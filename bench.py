@@ -152,6 +152,30 @@ def cfg_of(args):
 
 
 REF_SAMPLE_BATCH = 8   # BASELINE.md section 3: the reference's own CPU-runnable case is batch 8
+DUMP_SAMPLE = 1 << 20  # --dump-outputs: larger arrays are reduced to this many elements (4 MB each in float32)
+
+
+def step_outputs(eng):
+    """What one train step hands its caller, copied to the host as float32: the per-sample losses with their mean
+    (loss[0]), the action head's output, the pooled readout rows, and the parameters and gradients after the AdamW update.
+    An array of more than DUMP_SAMPLE elements is flattened and reduced to a sample at fixed, seeded positions (the same
+    positions for every run of the same shape), which keeps the five arrays under 20 MB at any batch."""
+    import numpy as np
+    import torch
+
+    out, positions = {}, {}
+    for name, t in (("loss", eng.loss), ("head_out", eng.head_out), ("readout", eng.readout), ("params", eng.params),
+                    ("grads", eng.grads)):
+        if t is None:
+            continue
+        if t.numel() > DUMP_SAMPLE:
+            if t.numel() not in positions:
+                idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_SAMPLE, replace=False))
+                positions[t.numel()] = torch.from_numpy(idx).to(t.device)
+            t = t.reshape(-1).index_select(0, positions[t.numel()])
+            name += "_sample"
+        out[name] = t.float().cpu().numpy()
+    return out
 
 
 def workload_config(args, world, B, T0):
@@ -329,10 +353,11 @@ def microbench(args):
 
 
 # ------------------------------------------------------------------------------------------------ this repo's arm
-def measure_workload(args, cfgname, rank, world, local, steps, warmup, with_extras=True):
+def measure_workload(args, cfgname, rank, world, local, steps, warmup, with_extras=True, dump_dir=None):
     """One workload measured three ways on this rank's GPU (max over ranks): device-timed steps with resident inputs
     (`value`), end to end through the public trainer API with pinned-host inputs (`e2e`), and a per-op CUDA-event pass
-    (`kernels`, `roofline`).  Returns the dict rank 0 prints (None on other ranks)."""
+    (`kernels`, `roofline`).  Returns the dict rank 0 prints (None on other ranks).  dump_dir: rank 0 writes what the last
+    timed step computed there (step_outputs), before the later passes train on further inputs."""
     import torch
     import torch.distributed as dist
 
@@ -397,6 +422,11 @@ def measure_workload(args, cfgname, rank, world, local, steps, warmup, with_extr
     launches = int(lib.tome_launch_count(1))
     loss_dev = float(eng.loss[0].item())
     value = world * B * steps / (ms * 1e-3)
+    if dump_dir is not None and rank == 0:
+        import numpy as np
+        os.makedirs(dump_dir, exist_ok=True)
+        for name, a in step_outputs(eng).items():
+            np.save(os.path.join(dump_dir, name + ".npy"), a)
 
     # every rank started from the same weights and applied the same summed gradients: the parameter vectors must be
     # bit-identical (a checksum of the fp32 bit patterns, min == max over the ranks)
@@ -629,7 +659,15 @@ def main():
     ap.add_argument("--microbench", action="store_true",
                     help="BASELINE.json configs[4]: standalone ToMe block kernels at 1k-8k tokens, d = 768 / 1024, merge-ratio "
                          "sweep, each against its roofline (one JSON object; N = 1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed train step computed to DIR/<name>.npy (float32): loss, head_out, readout, "
+                         "and seeded samples of the updated params and of the grads; inputs are seeded, so two builds run "
+                         "with the same arguments can be compared array by array")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "tome_b200" or args.microbench):
+        ap.error("--dump-outputs applies to the train-step workload of --impl tome_b200")
     args.warmup = max(args.warmup, 3) if args.impl == "tome_b200" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -655,7 +693,7 @@ def main():
         if world > 1:
             os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
             dist.init_process_group("nccl", device_id=torch.device("cuda", local), pg_options=nccl_options(args.comm_sms))
-        out = measure_workload(args, args.config, rank, world, local, args.steps, args.warmup)
+        out = measure_workload(args, args.config, rank, world, local, args.steps, args.warmup, dump_dir=args.dump_outputs)
         want_base = args.octo_base == "on" or (args.octo_base == "auto" and world == 8)
         if want_base and args.config == "octo_small":
             # BASELINE.json configs[2] (octo-base, batch 2048 over 8 GPUs) rides on the same line, so that the driver's scaling
