@@ -9,7 +9,7 @@ import ctypes as C
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.path.join(HERE, f"libtome_b200{os.environ.get('TOME_LIB_SUFFIX', '')}.so")   # suffix: experimental A/B builds (build.py)
+LIB_PATH = os.path.join(HERE, "libtome_b200.so")
 
 TOME_OK, TOME_ERR_INVALID, TOME_ERR_CUDA, TOME_ERR_UNSUPPORTED = 0, 1, 2, 3
 TOME_BF16, TOME_F32, TOME_U8 = 0, 1, 2
@@ -148,18 +148,15 @@ def lib() -> C.CDLL:
         for name in ("tome_gemm_workspace_bytes", "tome_stack_workspace_bytes", "tome_attention_workspace_bytes", "tome_sim_argmax_workspace_bytes",
                      "tome_attention_bwd_workspace_bytes", "tome_action_head_workspace_bytes", "tome_diffusion_head_workspace_bytes",
                      "tome_image_tokenizer_workspace_bytes"):
-            if hasattr(L, name):
-                getattr(L, name).restype = C.c_size_t
+            getattr(L, name).restype = C.c_size_t
         for name in ("tome_stack_param_count", "tome_stack_layer_offset", "tome_stack_head_offset", "tome_launch_count",
                      "tome_diffusion_head_param_count", "tome_diffusion_head_param_offset",
                      "tome_image_tokenizer_param_count", "tome_image_tokenizer_param_offset"):
-            if hasattr(L, name):
-                getattr(L, name).restype = ll
+            getattr(L, name).restype = ll
         for name in ("tome_stack_final_x", "tome_stack_final_size", "tome_stack_layer_edge_idx", "tome_stack_layer_dst_idx",
                      "tome_stack_layer_node_max", "tome_stack_layer_node_idx", "tome_stack_layer_relu_bits",
                      "tome_stack_layer_x_in", "tome_stack_layer_size_in", "tome_stack_layer_importance", "tome_stack_layer_prune_ids"):
-            if hasattr(L, name):
-                getattr(L, name).restype = vp
+            getattr(L, name).restype = vp
         P = C.POINTER
         sig = {
             "tome_clamp_r": [i32, i32, i32, i32],
@@ -177,16 +174,19 @@ def lib() -> C.CDLL:
             "tome_gemm_workspace_bytes": [P(GemmArgs)],
             "tome_gemm_bf16": [P(GemmArgs), vp, C.c_size_t, vp],
             "tome_gemm_set_sm_limit": [i32],
+            "tome_gemm_force_tile": [i32, i32],          # test hook, not in the header
             "tome_colsum_workspace_rows": [i32],
             "tome_reduce_rows_f32": [i32, i32, vp, vp, i32, vp],
             "tome_colsum_bf16": [i32, i32, vp, ll, vp, i32, vp, vp],
             "tome_dropout_colsum_bf16": [i32, i32, vp, vp, f32, C.c_uint64, C.c_uint32, vp, i32, vp, vp],
             "tome_layernorm_fwd": [i32, i32, i32, i32, f32, vp, vp, vp, vp, vp, vp, vp],
             "tome_layernorm_bwd": [i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp],
+            "tome_ln_force_cluster": [i32],              # test hook, not in the header
             "tome_attention_workspace_bytes": [P(AttnDesc)],
             "tome_attention_bwd_workspace_bytes": [P(AttnDesc)],
             "tome_attention_fwd": [P(AttnDesc), vp, vp, vp, vp, vp, vp, C.c_size_t, vp],
             "tome_attention_bwd": [P(AttnDesc), P(AttnGradStrides), vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_size_t, vp],
+            "tome_attention_set_dq_from_ds": [i32],      # test hook, not in the header
             "tome_add_pos_embedding": [i32, i32, i32, vp, i32, vp, vp, vp],
             "tome_pos_embedding_bwd": [i32, i32, i32, vp, vp, vp],
             "tome_chain_row_maps": [i32, i32, P(vp), P(i32), vp, i32, vp, vp],
@@ -230,8 +230,9 @@ def lib() -> C.CDLL:
             "tome_num_sms": [],
         }
         for name, args in sig.items():
-            if hasattr(L, name):
-                getattr(L, name).argtypes = args
+            getattr(L, name).argtypes = args
+        for name in ("tome_gemm_force_tile", "tome_ln_force_cluster", "tome_attention_set_dq_from_ds"):
+            getattr(L, name).restype = None
         _lib = L
     return _lib
 

@@ -12,14 +12,11 @@ from concurrent.futures import ThreadPoolExecutor
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
-# TOME_LIB_SUFFIX: an experimental build (with TOME_NVCC_EXTRA defines) beside the product library; _lib.py loads it when the
-# same variable is set.  Development aid for A/B measurements only.
-SUFFIX = os.environ.get("TOME_LIB_SUFFIX", "")
-BUILD = os.path.join(CSRC, "_build" + SUFFIX)
-LIB = os.path.join(HERE, f"libtome_b200{SUFFIX}.so")
+BUILD = os.path.join(CSRC, "_build")
+LIB = os.path.join(HERE, "libtome_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC",
-         "--expt-relaxed-constexpr", "-Xptxas", "-v"] + os.environ.get("TOME_NVCC_EXTRA", "").split()   # e.g. -DTOME_GEMM_EPI_WARPS=16 (A/B builds)
+         "--expt-relaxed-constexpr", "-Xptxas", "-v"]
 
 
 def _sources():

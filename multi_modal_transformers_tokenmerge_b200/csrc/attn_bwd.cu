@@ -5,7 +5,8 @@
 //   prep      delta[b,h,q] = sum_d dO*O and lse2 = lse*log2(e), both padded to 64-token tiles ([B,H,Tp]) so a tile is
 //             one aligned 256-byte bulk copy; attn_meta_kernel (attn_meta.cuh) builds the per-tile mask words
 //   dkdv      CTA = (128-key tile, head, batch), thread = key row, loop over 64-query tiles:
-//               S^T = K Q^T, dP^T = V dO^T (TMEM) -> P^T, dS^T (bf16, shared) -> dV += P^T dO, dK += dS^T Q (TMEM)
+//               S^T = K Q^T, dP^T = V dO^T (TMEM) -> P^T, dS^T (bf16, written over dP^T in TMEM) -> dV += P^T dO,
+//               dK += dS^T Q (TMEM)
 //   dq        CTA = (128-query tile, head, batch), thread = query row, loop over 64-key tiles:
 //               S = Q K^T, dP = dO V^T (TMEM) -> dS (bf16, shared, double-buffered) -> dQ += dS K (TMEM)
 // P is recomputed from the saved log-sum-exp: P = exp2(s2 - lse2), s2 = q.k*scale*log2e + log2(size_k);
@@ -14,8 +15,6 @@
 // bulk copies issued by the producer warp: the softmax threads run no global loads, ballots or CTA barriers per tile
 // (the first version did, and that dependent-load chain paced the kernels).
 #include <float.h>
-
-#include <stdlib.h>
 
 #include "attn_meta.cuh"
 #include "common.cuh"
@@ -56,13 +55,7 @@ struct AttnBwdParams {
   float* cs;
   long long cs_ld;
   int cs_q, cs_k, cs_v, n_t128;
-  int ablate;   // TOME_ATTN_ABLATE builds only (timing probes, wrong results): 1 = no softmax arithmetic, 2 = no MMAs
 };
-#ifdef TOME_ATTN_ABLATE
-#define AB_ABL(bit) ((p.ablate & (bit)) != 0)
-#else
-#define AB_ABL(bit) false
-#endif
 
 // one mbarrier arrival for the whole warp, after every lane has got here (the lanes' tensor-memory accesses are warp-collective
 // and already waited for; their shared-memory stores are ordered by the __syncwarp)
@@ -71,7 +64,7 @@ __device__ __forceinline__ void warp_arrive(uint64_t* bar, int lane) {
   if (lane == 0) mbar_arrive(bar);
 }
 
-// Epilogue shared by the four kernels below.  The 128 threads of warps 0-3 each own one row of a [128 x 64] fp32 accumulator in
+// Epilogue shared by the three kernels below.  The 128 threads of warps 0-3 each own one row of a [128 x 64] fp32 accumulator in
 // tensor memory.  The rows are rounded to bf16 and staged in shared memory (16 KB, 128-byte swizzled rows), then written out
 // by whole 128-byte lines (8 lanes per row, 4 rows per store instruction; a thread storing its own row scatters 32 partial
 // sectors per instruction) and, when asked, summed per column over the valid rows -- the Dense bias gradient of the q/k/v
@@ -120,7 +113,6 @@ __device__ __forceinline__ void ab_store_tile(uint8_t* stage, float* part, uint3
 __global__ void attn_bwd_prep_kernel(int B, int T, int Tp, int H, const __nv_bfloat16* __restrict__ o, long long o_bs,
                                      long long o_ts, const __nv_bfloat16* __restrict__ dout, long long do_bs, long long do_ts,
                                      const float* __restrict__ lse, float* __restrict__ delta, float* __restrict__ lse2) {
-  pdl_prologue();
   const long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x;  // (b, t, h, chunk of 8)
   const long long total = (long long)B * Tp * H * 8;
   if (idx < total) {  // total is a multiple of 8: the 8 lanes of a (b,t,h) group leave together
@@ -156,271 +148,13 @@ constexpr int DKV_KV_BYTES = DKV_BK * AB_D * 2;  // 16 KB
 constexpr int DKV_Q_BYTES = DKV_BQ * AB_D * 2;   // 8 KB
 constexpr int DKV_PT_BYTES = DKV_BK * DKV_BQ * 2;  // 16 KB
 constexpr int DKV_META_SLOT = 1280 + ATTN_DROP_TILE_BYTES;  // lse2[64] | delta[64] | pos[64] | qvis[32][2] | qvisc[32][2] | dropout keep words [128 keys][2]
-constexpr int DKV_SMEM = 2 * DKV_KV_BYTES + 2 * 2 * DKV_Q_BYTES + 2 * DKV_PT_BYTES + AB_MSLOTS * DKV_META_SLOT + 256 + 1024;
 
-template <bool DROP>  // attention-weight dropout compiled in or not
-__global__ void __launch_bounds__(AB_THREADS, 2)
-attn_bwd_dkdv_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
-                     const __grid_constant__ CUtensorMap tm_v, const __grid_constant__ CUtensorMap tm_do,
-                     const __grid_constant__ CUtensorMap tm_ds, const AttnBwdParams p) {
-  pdl_prologue();
-  extern __shared__ uint8_t smem_raw[];
-  // 1 KB alignment by pointer arithmetic on the __shared__ array itself, so every access below stays LDS/STS
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  uint8_t* s_k = smem;
-  uint8_t* s_v = s_k + DKV_KV_BYTES;
-  uint8_t* s_qdo = s_v + DKV_KV_BYTES;            // stage s: Q at s*16K, dO at s*16K + 8K
-  uint8_t* s_pt = s_qdo + 2 * 2 * DKV_Q_BYTES;    // P^T  [128 keys][64 queries] bf16, K-major swizzled
-  uint8_t* s_dst = s_pt + DKV_PT_BYTES;           // dS^T
-  uint8_t* s_meta = s_dst + DKV_PT_BYTES;         // slot i at i * DKV_META_SLOT
-  uint64_t* bars = reinterpret_cast<uint64_t*>(s_meta + AB_MSLOTS * DKV_META_SLOT);
-  uint64_t* kv_full = bars;        // 1
-  uint64_t* q_full = bars + 1;     // [2]
-  uint64_t* q_empty = bars + 3;    // [2]
-  uint64_t* st_full = bars + 5;    // S^T_i and dP^T_i in TMEM
-  uint64_t* ps_ready = bars + 6;   // P^T_i, dS^T_i in smem; TMEM S^T/dP^T consumed (128 arrivals)
-  uint64_t* pd_free = bars + 7;    // dV/dK MMAs of tile i done: smem P^T/dS^T reusable, accumulators final at the end
-  uint64_t* meta_full = bars + 8;  // [3]
-  uint64_t* meta_empty = bars + 11;  // [3]  128 arrivals
-  uint64_t* ds_stored = bars + 14;   // store_ds: the TMA store of dS^T_i has read the tile out of shared memory
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 15);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int kt = blockIdx.x, h = blockIdx.y, b = blockIdx.z;
-  const int T = p.tokens;
-  const int n_q = (T + DKV_BQ - 1) / DKV_BQ;
-  const bool has_mask = p.gid != nullptr;
-
-  if (threadIdx.x == 0) {
-    mbar_init(kv_full, 1);
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&q_full[i], 1);
-      mbar_init(&q_empty[i], 1);
-    }
-    mbar_init(st_full, 1);
-    mbar_init(ps_ready, DKV_BK);
-    mbar_init(pd_free, 1);
-    mbar_init(ds_stored, 1);
-    for (int i = 0; i < AB_MSLOTS; ++i) {
-      mbar_init(&meta_full[i], 1);
-      mbar_init(&meta_empty[i], DKV_BK);
-    }
-    fence_barrier_init();
-  }
-  if (warp == 4 && lane == 0) {
-    tma_prefetch_desc(&tm_q);
-    tma_prefetch_desc(&tm_k);
-    tma_prefetch_desc(&tm_v);
-    tma_prefetch_desc(&tm_do);
-  }
-  if (warp == 5) tmem_alloc(tmem_slot, AB_TMEM_COLS);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const uint32_t tm_st = tmem_base, tm_dpt = tmem_base + 64, tm_dk = tmem_base + 128, tm_dv = tmem_base + 192;
-
-  if (warp == 4) {
-    if (lane == 0) {
-      mbar_expect_tx(kv_full, 2 * DKV_KV_BYTES);
-      tma_load_3d(s_k, &tm_k, kv_full, h * AB_D, kt * DKV_BK, b);
-      tma_load_3d(s_v, &tm_v, kv_full, h * AB_D, kt * DKV_BK, b);
-      const float* lse_row = p.lse2 + ((size_t)b * p.heads + h) * p.tp;
-      const float* del_row = p.delta + ((size_t)b * p.heads + h) * p.tp;
-      const uint8_t* meta_b = p.meta + (size_t)b * n_q * ATTN_META_BYTES;
-      for (int i = 0; i < n_q; ++i) {
-        const int ms = i % AB_MSLOTS;
-        uint8_t* slot = s_meta + ms * DKV_META_SLOT;
-        mbar_wait(&meta_empty[ms], ((i / AB_MSLOTS) & 1) ^ 1);
-        mbar_expect_tx(&meta_full[ms], (has_mask ? 1280u : 512u) + (DROP ? ATTN_DROP_TILE_BYTES : 0));
-        if constexpr (DROP) bulk_g2s(slot + 1280, p.keep_k + ((size_t)kt * n_q + i) * ATTN_DROP_TILE_BYTES, ATTN_DROP_TILE_BYTES, &meta_full[ms]);
-        bulk_g2s(slot, lse_row + i * DKV_BQ, 256, &meta_full[ms]);
-        bulk_g2s(slot + 256, del_row + i * DKV_BQ, 256, &meta_full[ms]);
-        if (has_mask) bulk_g2s(slot + 512, meta_b + (size_t)i * ATTN_META_BYTES + ATTN_META_OFF_POS, 768, &meta_full[ms]);  // pos | qvis | qvisc
-        const int st = i & 1;
-        mbar_wait(&q_empty[st], ((i >> 1) & 1) ^ 1);
-        mbar_expect_tx(&q_full[st], 2 * DKV_Q_BYTES);
-        tma_load_3d(s_qdo + st * 2 * DKV_Q_BYTES, &tm_q, &q_full[st], h * AB_D, i * DKV_BQ, b);
-        tma_load_3d(s_qdo + st * 2 * DKV_Q_BYTES + DKV_Q_BYTES, &tm_do, &q_full[st], h * AB_D, i * DKV_BQ, b);
-      }
-    }
-  } else if (warp == 5) {
-    if (lane == 0) {
-      constexpr uint32_t idesc_s = make_idesc_bf16(DKV_BK, DKV_BQ, false, false);  // K/V K-major, Q/dO K-major
-      constexpr uint32_t idesc_g = make_idesc_bf16(DKV_BK, AB_D, false, true);     // P^T/dS^T K-major, dO/Q MN-major
-      const uint32_t ak = smem_u32(s_k), av = smem_u32(s_v), apt = smem_u32(s_pt), adst = smem_u32(s_dst);
-      mbar_wait(kv_full, 0);
-      for (int i = 0; i <= n_q; ++i) {
-        if (i >= 1) {
-          mbar_wait(ps_ready, (i - 1) & 1);
-          tc_fence_after();
-        }
-        if (i < n_q) {
-          const int st = i & 1;
-          mbar_wait(&q_full[st], (i >> 1) & 1);
-          tc_fence_after();
-          const uint32_t aq = smem_u32(s_qdo + st * 2 * DKV_Q_BYTES), ado = aq + DKV_Q_BYTES;
-#pragma unroll
-          for (int k = 0; k < AB_D / 16; ++k)
-            umma_bf16(tm_st, make_smem_desc(ak + k * 32, 16, 1024), make_smem_desc(aq + k * 32, 16, 1024), idesc_s, k > 0);
-#pragma unroll
-          for (int k = 0; k < AB_D / 16; ++k)
-            umma_bf16(tm_dpt, make_smem_desc(av + k * 32, 16, 1024), make_smem_desc(ado + k * 32, 16, 1024), idesc_s, k > 0);
-          umma_commit(st_full);
-        }
-        if (i >= 1) {
-          const int st = (i - 1) & 1;
-          const uint32_t aq = smem_u32(s_qdo + st * 2 * DKV_Q_BYTES), ado = aq + DKV_Q_BYTES;
-          if (p.store_ds) {  // dS^T tile (keys kt*128.., queries (i-1)*64..) -> global, in the layout it has in shared memory
-            asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-                         ::"l"(&tm_ds), "r"(adst), "r"((i - 1) * DKV_BQ), "r"(kt * DKV_BK), "r"(b * p.heads + h) : "memory");
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-          }
-#pragma unroll
-          for (int k = 0; k < DKV_BQ / 16; ++k)  // dV += P^T dO
-            umma_bf16(tm_dv, make_smem_desc(apt + k * 32, 16, 1024), make_smem_desc(ado + k * 2048, 8192, 1024), idesc_g,
-                      (i > 1 || k > 0) ? 1u : 0u);
-#pragma unroll
-          for (int k = 0; k < DKV_BQ / 16; ++k)  // dK += dS^T Q
-            umma_bf16(tm_dk, make_smem_desc(adst + k * 32, 16, 1024), make_smem_desc(aq + k * 2048, 8192, 1024), idesc_g,
-                      (i > 1 || k > 0) ? 1u : 0u);
-          umma_commit(pd_free);
-          umma_commit(&q_empty[st]);
-          if (p.store_ds) {  // after the commits, so neither the softmax warps nor the producer wait for the store's read
-            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-            mbar_arrive(ds_stored);
-          }
-        }
-      }
-      if (p.store_ds) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");  // stores complete before the CTA exits
-    }
-  } else {
-    const int row = threadIdx.x;  // key row == TMEM lane
-    const int kk = kt * DKV_BK + row;
-    const uint32_t lane_sel = ((uint32_t)(warp * 32)) << 16;
-    const bool k_valid = kk < T;
-    float bias2 = 0.f;
-    int gk = 0, pk = 0;
-    if (k_valid) {
-      if (p.size) bias2 = log2f(p.size[(long long)b * T + kk]);
-      if (has_mask) {
-        gk = p.gid[(long long)b * T + kk];
-        pk = p.pos[(long long)b * T + kk];
-      }
-    }
-    const float2 scale2 = make_float2(p.scale_log2, p.scale_log2), bias22 = make_float2(bias2, bias2);
-    const float2 sc2 = make_float2(p.scale, p.scale), ik2 = make_float2(p.inv_keep, p.inv_keep);
-    for (int i = 0; i < n_q; ++i) {
-      const int ms = i % AB_MSLOTS;
-      const uint8_t* slot = s_meta + ms * DKV_META_SLOT;
-      mbar_wait(&meta_full[ms], (i / AB_MSLOTS) & 1);
-      uint32_t vw[2] = {0xffffffffu, 0xffffffffu};
-      if (has_mask) {
-        const uint2 a = *reinterpret_cast<const uint2*>(slot + 768 + gk * 8);
-        const uint2 c = *reinterpret_cast<const uint2*>(slot + 1024 + gk * 8);
-        vw[0] = a.x; vw[1] = a.y;
-        if (c.x | c.y) {  // rare (Text sets): fold the causal rule into the visibility words
-          const int* posq = reinterpret_cast<const int*>(slot + 512);
-          for (int q = 0; q < 32; ++q) {
-            if (((c.x >> q) & 1u) && pk <= posq[q]) vw[0] |= 1u << q;
-            if (((c.y >> q) & 1u) && pk <= posq[32 + q]) vw[1] |= 1u << q;
-          }
-        }
-      }
-      if (!k_valid) vw[0] = vw[1] = 0u;  // rows past T contribute nothing
-      uint32_t kb[2] = {0xffffffffu, 0xffffffffu};  // dropout keep bits of this key against the tile's 64 queries
-      if constexpr (DROP) {
-        const uint2 t = *reinterpret_cast<const uint2*>(slot + 1280 + row * 8);
-        kb[0] = t.x; kb[1] = t.y;
-      }
-      const float4* lse4 = reinterpret_cast<const float4*>(slot);
-      const float4* del4 = reinterpret_cast<const float4*>(slot + 256);
-      mbar_wait(st_full, i & 1);
-      tc_fence_after();
-#pragma unroll
-      for (int cq = 0; cq < DKV_BQ / 32; ++cq) {
-        const int c0 = cq * 32;
-        float sv[32], dv[32];
-        tmem_ld_f32x32(tm_st + lane_sel + c0, sv);
-        tmem_ld_f32x32(tm_dpt + lane_sel + c0, dv);
-        tmem_ld_wait();
-        const uint32_t word = vw[cq];
-        uint32_t pw[16], dw[16];
-#pragma unroll
-        for (int c4 = 0; c4 < 8; ++c4) {
-          const float4 l4 = lse4[cq * 8 + c4], d4 = del4[cq * 8 + c4];
-#pragma unroll
-          for (int u = 0; u < 2; ++u) {
-            const int c = c4 * 4 + 2 * u;
-            const float2 lv = u ? make_float2(l4.z, l4.w) : make_float2(l4.x, l4.y);
-            const float2 dl = u ? make_float2(d4.z, d4.w) : make_float2(d4.x, d4.y);
-            float2 t = __ffma2_rn(make_float2(sv[c], sv[c + 1]), scale2, bias22);
-            t = __fadd2_rn(t, make_float2(-lv.x, -lv.y));
-            float2 pe = make_float2(fast_exp2(t.x), fast_exp2(t.y));
-            pe.x = ((word >> c) & 1u) ? pe.x : 0.f;
-            pe.y = ((word >> (c + 1)) & 1u) ? pe.y : 0.f;
-            // dropout (weights' = weights * keep / (1 - rate)): dP' = dP * keep / (1 - rate) enters dS, P' enters dV
-            float2 dp = make_float2(dv[c], dv[c + 1]), pd = pe;
-            if constexpr (DROP) {
-              const bool k0 = (kb[cq] >> c) & 1u, k1 = (kb[cq] >> (c + 1)) & 1u;
-              dp = __fmul2_rn(dp, ik2);
-              pd = __fmul2_rn(pd, ik2);
-              dp.x = k0 ? dp.x : 0.f; dp.y = k1 ? dp.y : 0.f;
-              pd.x = k0 ? pd.x : 0.f; pd.y = k1 ? pd.y : 0.f;
-            }
-            float2 g = __fadd2_rn(dp, make_float2(-dl.x, -dl.y));
-            g = __fmul2_rn(g, sc2);
-            g = __fmul2_rn(g, pe);
-            pw[c >> 1] = pack_bf16(pd.x, pd.y);
-            dw[c >> 1] = pack_bf16(g.x, g.y);
-          }
-        }
-        if (cq == 0 && i >= 1) {
-          mbar_wait(pd_free, (i - 1) & 1);  // previous P^T / dS^T fully consumed by the tensor core
-          if (p.store_ds) mbar_wait(ds_stored, (i - 1) & 1);  // ... and dS^T by its TMA store
-        }
-#pragma unroll
-        for (int ch = 0; ch < 4; ++ch) {
-          const int chunk = (c0 >> 3) + ch;
-          const int off = row * 128 + ((chunk ^ (row & 7)) << 4);
-          *reinterpret_cast<uint4*>(s_pt + off) = make_uint4(pw[4 * ch], pw[4 * ch + 1], pw[4 * ch + 2], pw[4 * ch + 3]);
-          *reinterpret_cast<uint4*>(s_dst + off) = make_uint4(dw[4 * ch], dw[4 * ch + 1], dw[4 * ch + 2], dw[4 * ch + 3]);
-        }
-      }
-      mbar_arrive(&meta_empty[ms]);
-      fence_proxy_async_smem();
-      tc_fence_before();
-      mbar_arrive(ps_ready);
-    }
-    mbar_wait(pd_free, (n_q - 1) & 1);  // accumulators final
-    tc_fence_after();
-    {
-      // every MMA has retired: the K and V tiles serve as staging for dK and dV, the Q/dO ring for the column-sum scratch
-      const int rows_valid = min(DKV_BK, T - kt * DKV_BK);
-      float* cs_row = p.cs ? p.cs + ((long long)b * p.n_t128 + kt) * p.cs_ld + h * AB_D : nullptr;
-      ab_store_tile(s_k, reinterpret_cast<float*>(s_qdo), tm_dk + lane_sel, rows_valid,
-                    p.dk + (long long)b * p.dk_bs + (long long)kt * DKV_BK * p.dk_ts + h * AB_D, p.dk_ts, cs_row ? cs_row + p.cs_k : nullptr, 1);
-      ab_store_tile(s_v, reinterpret_cast<float*>(s_qdo) + 256, tm_dv + lane_sel, rows_valid,
-                    p.dv + (long long)b * p.dv_bs + (long long)kt * DKV_BK * p.dv_ts + h * AB_D, p.dv_ts, cs_row ? cs_row + p.cs_v : nullptr, 1);
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 5) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, AB_TMEM_COLS);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------ dK / dV, P^T and dS^T in tensor memory
-// Same tiling and arithmetic as attn_bwd_dkdv_kernel, but the two products that consume what the softmax threads produce
-// take their A operand from TENSOR MEMORY (tcgen05.mma with [tmem] A): once a thread has read its row of dP^T_i, it
-// writes dS^T_i (two bf16 per column) over columns [64, 96) and P^T_i over [96, 128) of that very accumulator, and
-// dV += P^T dO / dK += dS^T Q read them from there.  Nothing the threads produce passes through shared memory any more:
-// per 128 x 64 tile the shared-memory traffic falls from 160 KB (four SS products 96 KB, P^T / dS^T staging 32 KB, TMA in
-// 16 KB, TMA store read 16 KB) to 80 KB, and with two CTAs per SM that traffic -- 2 x 1280 cycles of the SM's 128 B/clk
-// against ~5000 measured per tile pair -- was the largest single term of the kernel.  dS^T for the dQ GEMM is written to
-// global memory straight from the registers (a thread owns one 128-byte line per tile).
+// The two products that consume what the softmax threads produce take their A operand from TENSOR MEMORY (tcgen05.mma
+// with [tmem] A): once a thread has read its row of dP^T_i, it writes dS^T_i (two bf16 per column) over columns [64, 96)
+// and P^T_i over [96, 128) of that very accumulator, and dV += P^T dO / dK += dS^T Q read them from there.  Nothing the
+// threads produce passes through shared memory on its way to the tensor core: staging P^T / dS^T there doubled the
+// shared-memory traffic per 128 x 64 tile, the largest single term of the kernel at two CTAs per SM
+// (profiles/r02_attention_bwd.md).  dS^T for the dQ GEMM is staged in shared memory for one TMA store per tile.
 // S^T lives in columns [0, 64) and is free again as soon as every thread has read it (s_free), so S^T_{i+1} is computed
 // while the threads are still busy with dP^T_i; the order on the tensor pipe is S^T_{i+1}, dV_i, dK_i, dP^T_{i+1}.
 constexpr int DKT_SMEM = 2 * DKV_KV_BYTES + 2 * 2 * DKV_Q_BYTES + 2 * DKV_PT_BYTES + AB_MSLOTS * DKV_META_SLOT + 256 + 1024;
@@ -430,7 +164,6 @@ __global__ void __launch_bounds__(DKT_THREADS, 2)
 attn_bwd_dkdv_ts_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
                         const __grid_constant__ CUtensorMap tm_v, const __grid_constant__ CUtensorMap tm_do,
                         const __grid_constant__ CUtensorMap tm_ds, const AttnBwdParams p) {
-  pdl_prologue();
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   uint8_t* s_k = smem;
@@ -537,7 +270,7 @@ attn_bwd_dkdv_ts_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_c
           const uint32_t aq = smem_u32(s_qdo + st * 2 * DKV_Q_BYTES);
 #pragma unroll
           for (int k = 0; k < AB_D / 16; ++k)
-            if (!AB_ABL(2)) umma_bf16(tm_st, make_smem_desc(ak + k * 32, 16, 1024), make_smem_desc(aq + k * 32, 16, 1024), idesc_s, k > 0);
+            umma_bf16(tm_st, make_smem_desc(ak + k * 32, 16, 1024), make_smem_desc(aq + k * 32, 16, 1024), idesc_s, k > 0);
           umma_commit(s_full);
         }
         if (i >= 1) {
@@ -546,17 +279,16 @@ attn_bwd_dkdv_ts_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_c
           const int st = (i - 1) & 1;
           const uint32_t aq = smem_u32(s_qdo + st * 2 * DKV_Q_BYTES), ado = aq + DKV_Q_BYTES;
           if (p.store_ds) {  // dS^T tile (keys kt*128.., queries (i-1)*64..) -> global, in the layout it has in shared memory
-            if (!AB_ABL(4))
             asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
                          ::"l"(&tm_ds), "r"(smem_u32(s_dst + ((i - 1) & 1) * DKV_PT_BYTES)), "r"((i - 1) * DKV_BQ), "r"(kt * DKV_BK), "r"(b * p.heads + h) : "memory");
             asm volatile("cp.async.bulk.commit_group;" ::: "memory");
           }
 #pragma unroll
           for (int k = 0; k < DKV_BQ / 16; ++k)  // dV += P^T dO
-            if (!AB_ABL(2)) umma_bf16_ts(tm_dv, tm_pa(k), make_smem_desc(ado + k * 2048, 8192, 1024), idesc_g, (i > 1 || k > 0) ? 1u : 0u);
+            umma_bf16_ts(tm_dv, tm_pa(k), make_smem_desc(ado + k * 2048, 8192, 1024), idesc_g, (i > 1 || k > 0) ? 1u : 0u);
 #pragma unroll
           for (int k = 0; k < DKV_BQ / 16; ++k)  // dK += dS^T Q
-            if (!AB_ABL(2)) umma_bf16_ts(tm_dk, tm_dsa(k), make_smem_desc(aq + k * 2048, 8192, 1024), idesc_g, (i > 1 || k > 0) ? 1u : 0u);
+            umma_bf16_ts(tm_dk, tm_dsa(k), make_smem_desc(aq + k * 2048, 8192, 1024), idesc_g, (i > 1 || k > 0) ? 1u : 0u);
           umma_commit(pd_free);
           umma_commit(&q_empty[st]);
         }
@@ -565,11 +297,11 @@ attn_bwd_dkdv_ts_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_c
           const uint32_t ado = smem_u32(s_qdo + st * 2 * DKV_Q_BYTES) + DKV_Q_BYTES;
 #pragma unroll
           for (int k = 0; k < AB_D / 16; ++k)
-            if (!AB_ABL(2)) umma_bf16(tm_dpt, make_smem_desc(av + k * 32, 16, 1024), make_smem_desc(ado + k * 32, 16, 1024), idesc_s, k > 0);
+            umma_bf16(tm_dpt, make_smem_desc(av + k * 32, 16, 1024), make_smem_desc(ado + k * 32, 16, 1024), idesc_s, k > 0);
           umma_commit(dp_full);
         }
         if (i >= 2 && p.store_ds) {  // all but the newest store have left shared memory: buffer i & 1 (tile i - 2) is free again
-          if (!AB_ABL(16)) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+          asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
           mbar_arrive(&ds_stored[i & 1]);
         }
       }
@@ -607,7 +339,7 @@ attn_bwd_dkdv_ts_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_c
       const int ms = i % AB_MSLOTS;
       const uint8_t* slot = s_meta + ms * DKV_META_SLOT;
       mbar_wait(&meta_full[ms], (i / AB_MSLOTS) & 1);
-      if (!warp_active || AB_ABL(1)) {
+      if (!warp_active) {
         mbar_wait(s_full, i & 1);
         tc_fence_before();
         warp_arrive(s_free, lane);
@@ -617,7 +349,7 @@ attn_bwd_dkdv_ts_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_c
           if (i >= 2) mbar_wait(&ds_stored[i & 1], ((i - 2) >> 1) & 1);
 #pragma unroll
           for (int ch = 0; ch < 4; ++ch) *reinterpret_cast<uint4*>(dst_row + ((hq * 4 + ch) << 4)) = make_uint4(0u, 0u, 0u, 0u);
-          if (!AB_ABL(8)) fence_proxy_async_smem();
+          fence_proxy_async_smem();
         }
         warp_arrive(&meta_empty[ms], lane);
         tc_fence_before();
@@ -708,7 +440,7 @@ attn_bwd_dkdv_ts_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_c
 #pragma unroll
         for (int ch = 0; ch < 4; ++ch)
           *reinterpret_cast<uint4*>(dst_row + (((hq * 4 + ch) ^ (row & 7)) << 4)) = make_uint4(dw[4 * ch], dw[4 * ch + 1], dw[4 * ch + 2], dw[4 * ch + 3]);
-        if (!AB_ABL(8)) fence_proxy_async_smem();
+        fence_proxy_async_smem();
       }
       tmem_st_wait();
       warp_arrive(&meta_empty[ms], lane);
@@ -753,7 +485,6 @@ __global__ void __launch_bounds__(AB_THREADS, 2)
 attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
                    const __grid_constant__ CUtensorMap tm_v, const __grid_constant__ CUtensorMap tm_do,
                    const AttnBwdParams p) {
-  pdl_prologue();
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   uint8_t* s_q = smem;
@@ -987,22 +718,15 @@ static size_t bwd_pad_elems(const tome_attn_desc_t* d) {
 // 3 stages x 3 CTAs per SM: the kernel is a short stream of dS^T tiles (9 k-steps at T = 536), so more resident CTAs to
 // overlap one CTA's prologue / epilogue with another's loads beat a deeper ring (4 x 2: 892 us for the whole backward at the
 // bench shape, 2 x 4: 870, 3 x 3: 865)
-#ifndef TOME_DQG_STAGES
-#define TOME_DQG_STAGES 3
-#endif
-#ifndef TOME_DQG_CTAS
-#define TOME_DQG_CTAS 3
-#endif
-constexpr int DQG_BQ = 128, DQG_BK = 64, DQG_STAGES = TOME_DQG_STAGES;
+constexpr int DQG_BQ = 128, DQG_BK = 64, DQG_STAGES = 3, DQG_CTAS = 3;
 constexpr int DQG_A_BYTES = 2 * DQG_BK * 128;   // 16 KB: two [64 keys][64 queries] atoms
 constexpr int DQG_B_BYTES = DQG_BK * AB_D * 2;  // 8 KB
 constexpr int DQG_STAGE = DQG_A_BYTES + DQG_B_BYTES;
 constexpr int DQG_SMEM = DQG_STAGES * DQG_STAGE + 256 + 1024;
 
-__global__ void __launch_bounds__(AB_THREADS, TOME_DQG_CTAS)
+__global__ void __launch_bounds__(AB_THREADS, DQG_CTAS)
 attn_bwd_dq_gemm_kernel(const __grid_constant__ CUtensorMap tm_ds, const __grid_constant__ CUtensorMap tm_k,
                         const AttnBwdParams p) {
-  pdl_prologue();
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + DQG_STAGES * DQG_STAGE);
@@ -1094,10 +818,6 @@ static inline bool dq_from_ds(const tome_attn_desc_t* d) {
   return g_attn_dq_from_ds < 0 ? ds_buffer_bytes(d) <= ((size_t)8 << 30) : g_attn_dq_from_ds != 0;
 }
 
-// 1 (default): the dK/dV kernel keeps P^T / dS^T in tensor memory (attn_bwd_dkdv_ts_kernel); 0: the shared-memory version.
-static int g_attn_bwd_ts = 1;
-extern "C" void tome_attention_set_bwd_ts(int on) { g_attn_bwd_ts = on ? 1 : 0; }
-
 extern "C" void tome_attention_set_dq_from_ds(int mode) { g_attn_dq_from_ds = mode < 0 ? -1 : (mode ? 1 : 0); }
 
 extern "C" size_t tome_attention_bwd_workspace_bytes(const tome_attn_desc_t* d) {
@@ -1165,10 +885,6 @@ extern "C" int tome_attention_bwd(const tome_attn_desc_t* d, const tome_attn_gra
   p.cs = gs->bias_partial; p.cs_ld = gs->bias_partial_ld;
   p.cs_q = gs->bias_q_col; p.cs_k = gs->bias_k_col; p.cs_v = gs->bias_v_col;
   p.n_t128 = ceil_div(T, 128);
-  p.ablate = 0;
-#ifdef TOME_ATTN_ABLATE
-  if (const char* e = getenv("TOME_ATTN_ABLATE")) p.ablate = atoi(e);
-#endif
 
   // dS^T [B*H][ceil128(T) keys][ceil64(T) queries] bf16, after the (possibly absent) dropout bit tilings
   uint8_t* ds_buf = reinterpret_cast<uint8_t*>(lse2) + align256(bwd_pad_elems(d) * sizeof(float)) +
@@ -1186,14 +902,11 @@ extern "C" int tome_attention_bwd(const tome_attn_desc_t* d, const tome_attn_gra
   p.dk = reinterpret_cast<__nv_bfloat16*>(dk); p.dk_bs = gs->dk_batch_stride; p.dk_ts = gs->dk_token_stride;
   p.dv = reinterpret_cast<__nv_bfloat16*>(dv); p.dv_bs = gs->dv_batch_stride; p.dv_ts = gs->dv_token_stride;
   static DynSmemOnce once[5];
-  TOME_CUDA(ensure_dyn_smem(attn_bwd_dkdv_kernel<false>, DKV_SMEM, once[0]));
-  TOME_CUDA(ensure_dyn_smem(attn_bwd_dkdv_kernel<true>, DKV_SMEM, once[1]));
+  TOME_CUDA(ensure_dyn_smem(attn_bwd_dkdv_ts_kernel<false>, DKT_SMEM, once[0]));
+  TOME_CUDA(ensure_dyn_smem(attn_bwd_dkdv_ts_kernel<true>, DKT_SMEM, once[1]));
   TOME_CUDA(ensure_dyn_smem(attn_bwd_dq_kernel<false>, DQ_SMEM, once[2]));
   TOME_CUDA(ensure_dyn_smem(attn_bwd_dq_kernel<true>, DQ_SMEM, once[3]));
   TOME_CUDA(ensure_dyn_smem(attn_bwd_dq_gemm_kernel, DQG_SMEM, once[4]));
-  static DynSmemOnce once_ts[2];
-  TOME_CUDA(ensure_dyn_smem(attn_bwd_dkdv_ts_kernel<false>, DKT_SMEM, once_ts[0]));
-  TOME_CUDA(ensure_dyn_smem(attn_bwd_dkdv_ts_kernel<true>, DKT_SMEM, once_ts[1]));
   {
     CUtensorMap tq, tk, tv, tdo;
     if (int rc = make_tmap_3d_bf16(&tq, q, hd, T, B, d->q_token_stride, d->q_batch_stride, DKV_BQ)) return rc;
@@ -1201,11 +914,8 @@ extern "C" int tome_attention_bwd(const tome_attn_desc_t* d, const tome_attn_gra
     if (int rc = make_tmap_3d_bf16(&tv, v, hd, T, B, d->v_token_stride, d->v_batch_stride, DKV_BK)) return rc;
     if (int rc = make_tmap_3d_bf16(&tdo, dout, hd, T, B, gs->do_token_stride, gs->do_batch_stride, DKV_BQ)) return rc;
     dim3 grid(ceil_div(T, DKV_BK), H, B);
-    if (g_attn_bwd_ts) {
-      if (keep_k) launch_k(attn_bwd_dkdv_ts_kernel<true>, grid, DKT_THREADS, DKT_SMEM, stream, tq, tk, tv, tdo, tds_store, p);
-      else launch_k(attn_bwd_dkdv_ts_kernel<false>, grid, DKT_THREADS, DKT_SMEM, stream, tq, tk, tv, tdo, tds_store, p);
-    } else if (keep_k) launch_k(attn_bwd_dkdv_kernel<true>, grid, AB_THREADS, DKV_SMEM, stream, tq, tk, tv, tdo, tds_store, p);
-    else launch_k(attn_bwd_dkdv_kernel<false>, grid, AB_THREADS, DKV_SMEM, stream, tq, tk, tv, tdo, tds_store, p);
+    if (keep_k) launch_k(attn_bwd_dkdv_ts_kernel<true>, grid, DKT_THREADS, DKT_SMEM, stream, tq, tk, tv, tdo, tds_store, p);
+    else launch_k(attn_bwd_dkdv_ts_kernel<false>, grid, DKT_THREADS, DKT_SMEM, stream, tq, tk, tv, tdo, tds_store, p);
     TOME_CUDA(cudaGetLastError());
   }
   if (from_ds) {

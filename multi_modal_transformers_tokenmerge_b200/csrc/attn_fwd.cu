@@ -11,11 +11,13 @@
 //   warp 5      UMMA issuer:  S_j = Q K_j^T (128x64x64) into a DOUBLE-BUFFERED TMEM accumulator (S_{j+1} is computed
 //               while the softmax warps work on S_j); O += P_j V_j (128x64x64) accumulates IN TMEM across key tiles
 //   warps 0..3  softmax, thread = query row: S_j (TMEM) -> registers, scale + bias (packed f32x2 FMA), mask, row max,
-//               exp2, row sum, P_j -> bf16 K-major A operand in shared memory (double-buffered).
+//               exp2, row sum, P_j -> bf16 written over the first 32 columns of S_j in TMEM.
 //               The running maximum is LAZY: O and l are rescaled only when a row's maximum grows by more than 2^8,
 //               which after the first tile is rare, so the usual tile needs no TMEM correction pass at all; when a
 //               warp does need one it multiplies its 32 rows of O in TMEM by alpha (tcgen05.ld / st) before it
 //               publishes P_j -- the PV MMA that reads O next is only issued after that.
+// Both MMAs take their A operand from tensor memory: the softmax warps copy Q there once per CTA, and P_j overwrites S_j,
+// so P never passes through shared memory.
 // Logits are kept in the log2 domain: s2 = (q.k) * scale * log2(e) + log2(size_k); masked -> -FLT_MAX (finite, as
 // flax's finfo.min), keys past T -> -inf.
 #include <float.h>
@@ -32,20 +34,14 @@ constexpr int ATT_D = 64;
 constexpr int ATT_THREADS = 192;
 constexpr int ATT_Q_BYTES = ATT_BM * ATT_D * 2;         // 16 KB
 constexpr int ATT_KV_BYTES = ATT_BN * ATT_D * 2;        // 8 KB each for K and V
-constexpr int ATT_P_BYTES = ATT_BM * ATT_BN * 2;        // 16 KB, x2 buffers
 constexpr int ATT_SLOTS = 5;  // ring of 8 KB slots; items are loaded in the order K_0 K_1 V_0 K_2 V_1 ...
 constexpr int ATT_MSLOTS = 4; // metadata ring
 constexpr int ATT_QAUG_BYTES = ATT_BM * ATTN_AUG_K * 2;   // 4 KB: mask augmentation operand of the query tile (attn_meta.cuh)
 constexpr int ATT_KAUG_BYTES = ATT_BN * ATTN_AUG_K * 2;   // 2 KB per key tile, one per ring slot
 constexpr int ATT_META_SLOT = ATTN_META_KEY_BYTES + ATTN_DROP_TILE_BYTES;  // bias2 | vis[32][2] | visc[32][2] | pos | dropout keep words [128][2]
 static_assert(ATT_BN == ATTN_META_TILE, "key tiles and metadata tiles must coincide");
-// TS = both MMAs take their A operand from tensor memory: Q is copied there once per CTA and P_j overwrites the first 32
-// columns of S_j (two bf16 per column), so no P buffer exists in shared memory
-template <bool TS>
-constexpr int att_smem() {
-  return ATT_Q_BYTES + ATT_SLOTS * ATT_KV_BYTES + (TS ? 0 : 2 * ATT_P_BYTES) + ATT_QAUG_BYTES + ATT_SLOTS * ATT_KAUG_BYTES +
-         ATT_MSLOTS * ATT_META_SLOT + 512 + 1024;
-}
+constexpr int ATT_SMEM = ATT_Q_BYTES + ATT_SLOTS * ATT_KV_BYTES + ATT_QAUG_BYTES + ATT_SLOTS * ATT_KAUG_BYTES +
+                         ATT_MSLOTS * ATT_META_SLOT + 512 + 1024;
 constexpr uint32_t ATT_TMEM_COLS = 256;  // S0 [0,64) S1 [64,128) O [128,192) Q [192,224)
 constexpr float ATT_LAZY_LOG2 = 8.0f;    // rescale O only when the row maximum grows by more than 2^8
 
@@ -81,19 +77,17 @@ __device__ __forceinline__ void tmem_ld_f32x32(uint32_t taddr, float (&r)[N]) {
 }
 
 // DROP: attention-weight dropout compiled in (the keep words ride in the metadata ring); the rate-0 instantiation carries none of it
-template <bool DROP, bool TS>
+template <bool DROP>
 __global__ void __launch_bounds__(ATT_THREADS, 2)
 attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
                 const __grid_constant__ CUtensorMap tm_v, const __grid_constant__ CUtensorMap tm_qaug,
                 const __grid_constant__ CUtensorMap tm_kaug, const AttnFwdParams p) {
-  pdl_prologue();
   extern __shared__ uint8_t smem_raw[];
   // 1 KB alignment by pointer arithmetic on the __shared__ array itself, so every access below stays LDS/STS
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   uint8_t* s_q = smem;
   uint8_t* s_kv = s_q + ATT_Q_BYTES;                        // slot i at i * 8 KB
-  uint8_t* s_p = s_kv + ATT_SLOTS * ATT_KV_BYTES;           // buffer i at i * 16 KB (absent with TS)
-  uint8_t* s_qaug = s_p + (TS ? 0 : 2 * ATT_P_BYTES);       // [128 rows][16] bf16, 32-byte swizzle
+  uint8_t* s_qaug = s_kv + ATT_SLOTS * ATT_KV_BYTES;        // [128 rows][16] bf16, 32-byte swizzle
   uint8_t* s_kaug = s_qaug + ATT_QAUG_BYTES;                // slot i at i * 2 KB (only K slots use theirs)
   uint8_t* s_meta = s_kaug + ATT_SLOTS * ATT_KAUG_BYTES;    // metadata slot i at i * ATT_META_SLOT
   uint64_t* bars = reinterpret_cast<uint64_t*>(s_meta + ATT_MSLOTS * ATT_META_SLOT);
@@ -101,11 +95,11 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
   uint64_t* kv_full = bars + 1;            // [ATT_SLOTS] (room for 6)
   uint64_t* kv_empty = bars + 7;           // [ATT_SLOTS] (room for 6)
   uint64_t* s_full = bars + 13;            // [2]  S_j ready in TMEM buffer j&1
-  uint64_t* p_ready = bars + 15;           // [2]  P_j in smem buffer j&1, S_j consumed, O corrected (128 arrivals)
-  uint64_t* pv_done = bars + 17;           // [2]  O += P_j V_j retired: P buffer j&1 reusable, O readable
+  uint64_t* p_ready = bars + 15;           // [2]  P_j in TMEM buffer j&1, S_j consumed, O corrected (128 arrivals)
+  uint64_t* pv_done = bars + 17;           // [2]  O += P_j V_j retired: O readable
   uint64_t* meta_full = bars + 19;         // [ATT_MSLOTS]  bulk copy of the tile's metadata block landed
   uint64_t* meta_empty = bars + 23;        // [ATT_MSLOTS]  128 arrivals (softmax threads), after the P stores of the tile
-  uint64_t* q_ready = bars + 27;           // TS: the query tile has been copied into tensor memory (128 arrivals)
+  uint64_t* q_ready = bars + 27;           // the query tile has been copied into tensor memory (128 arrivals)
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 28);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -142,7 +136,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const uint32_t tmem_o = tmem_base + 128;   // 64 columns; S buffers at +0 and +64
-  const uint32_t tmem_q = tmem_base + 192;   // TS: 32 columns = 128 x 64 bf16
+  const uint32_t tmem_q = tmem_base + 192;   // 32 columns = 128 x 64 bf16
   const bool has_mask = p.gid != nullptr;
   // the mask rides in the QK^T contraction (attn_meta.cuh) when the table allows it; CTA-uniform
   const bool use_aug = has_mask && *p.aug_flag != 0u;
@@ -184,7 +178,6 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
     if (lane == 0) {
       constexpr uint32_t idesc_s = make_idesc_bf16(ATT_BM, ATT_BN, false, false);  // Q K-major, K K-major
       constexpr uint32_t idesc_o = make_idesc_bf16(ATT_BM, ATT_D, false, true);    // P K-major, V MN-major
-      const uint32_t aq = smem_u32(s_q), ap = smem_u32(s_p);
       const int n_items = 2 * n_kv;
       auto issue_s = [&](int t) {  // S_t = Q K_t^T into TMEM buffer t&1
         const int item = t == 0 ? 0 : 2 * t - 1, slot = item % ATT_SLOTS;
@@ -192,43 +185,29 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
         tc_fence_after();
         const uint32_t ak = smem_u32(s_kv + slot * ATT_KV_BYTES);
 #pragma unroll
-        for (int k = 0; k < ATT_D / 16; ++k) {
-          if constexpr (TS)
-            umma_bf16_ts(tmem_base + (t & 1) * ATT_BN, tmem_q + k * 8, make_smem_desc(ak + k * 32, 16, 1024), idesc_s, k > 0 ? 1u : 0u);
-          else
-            umma_bf16(tmem_base + (t & 1) * ATT_BN, make_smem_desc(aq + k * 32, 16, 1024), make_smem_desc(ak + k * 32, 16, 1024),
-                      idesc_s, k > 0 ? 1u : 0u);
-        }
+        for (int k = 0; k < ATT_D / 16; ++k)
+          umma_bf16_ts(tmem_base + (t & 1) * ATT_BN, tmem_q + k * 8, make_smem_desc(ak + k * 32, 16, 1024), idesc_s, k > 0 ? 1u : 0u);
         if (use_aug)  // S += Mq Ek^T: 0 where the query's group sees the key's group, -2^100 (absorbing) where it does not
           umma_bf16(tmem_base + (t & 1) * ATT_BN, make_smem_desc_sw32(smem_u32(s_qaug)),
                     make_smem_desc_sw32(smem_u32(s_kaug + slot * ATT_KAUG_BYTES)), idesc_s, 1u);
         umma_commit(&s_full[t & 1]);
         umma_commit(&kv_empty[slot]);
       };
-      if constexpr (TS) {
-        mbar_wait(q_ready, 0);
-        tc_fence_after();
-      } else {
-        mbar_wait(q_full, 0);
-      }
+      mbar_wait(q_ready, 0);
+      tc_fence_after();
       issue_s(0);
       if (n_kv > 1) issue_s(1);
       for (int j = 0; j < n_kv; ++j) {
-        mbar_wait(&p_ready[j & 1], (j >> 1) & 1);  // P_j in smem, S_j consumed, O corrected
+        mbar_wait(&p_ready[j & 1], (j >> 1) & 1);  // P_j in TMEM, S_j consumed, O corrected
         tc_fence_after();
         const int item = j == n_kv - 1 ? n_items - 1 : 2 * j + 2, slot = item % ATT_SLOTS;
         mbar_wait(&kv_full[slot], (item / ATT_SLOTS) & 1);
         tc_fence_after();
-        const uint32_t av = smem_u32(s_kv + slot * ATT_KV_BYTES), apj = ap + (j & 1) * ATT_P_BYTES;
+        const uint32_t av = smem_u32(s_kv + slot * ATT_KV_BYTES);
 #pragma unroll
-        for (int k = 0; k < ATT_BN / 16; ++k) {  // O += P_j V_j
-          if constexpr (TS)
-            umma_bf16_ts(tmem_o, tmem_base + (j & 1) * ATT_BN + k * 8, make_smem_desc(av + k * 2048, 8192, 1024), idesc_o,
-                         (j > 0 || k > 0) ? 1u : 0u);
-          else
-            umma_bf16(tmem_o, make_smem_desc(apj + k * 32, 16, 1024), make_smem_desc(av + k * 2048, 8192, 1024), idesc_o,
-                      (j > 0 || k > 0) ? 1u : 0u);
-        }
+        for (int k = 0; k < ATT_BN / 16; ++k)  // O += P_j V_j
+          umma_bf16_ts(tmem_o, tmem_base + (j & 1) * ATT_BN + k * 8, make_smem_desc(av + k * 2048, 8192, 1024), idesc_o,
+                       (j > 0 || k > 0) ? 1u : 0u);
         umma_commit(&pv_done[j & 1]);
         umma_commit(&kv_empty[slot]);
         if (j + 2 < n_kv) issue_s(j + 2);
@@ -247,7 +226,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
     }
     float m_run = -INFINITY, l_run = 0.f;
     const float2 scale2 = make_float2(p.scale_log2, p.scale_log2);
-    if constexpr (TS) {  // this thread's query row: shared memory (128B-swizzled, as TMA wrote it) -> 32 TMEM columns
+    {  // this thread's query row: shared memory (128B-swizzled, as TMA wrote it) -> 32 TMEM columns
       mbar_wait(q_full, 0);
       uint32_t qw[32];
 #pragma unroll
@@ -348,18 +327,13 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
         }
       }
 
-      // P = exp2(s2 - m_run) -> bf16: the A operand of the PV product.  TS: written over the first 32 columns of S_j in
-      // tensor memory (every logit of this row is already in registers; S_{j+2}, which reuses the buffer, is issued behind
-      // P_j V_j).  Otherwise: K-major 128B-swizzled rows of shared-memory buffer j&1.
-      if constexpr (!TS) {
-        if (j >= 2) mbar_wait(&pv_done[j & 1], ((j - 2) >> 1) & 1);  // P V_{j-2} has finished reading this buffer
-      }
+      // P = exp2(s2 - m_run) -> bf16: the A operand of the PV product, written over the first 32 columns of S_j in tensor
+      // memory (every logit of this row is already in registers; S_{j+2}, which reuses the buffer, is issued behind P_j V_j)
       const float2 nm2 = make_float2(-m_run, -m_run);
       float2 l2[4];  // four independent partial row sums (same reason as the maxima)
 #pragma unroll
       for (int u = 0; u < 4; ++u) l2[u] = make_float2(0.f, 0.f);
-      uint8_t* prow = s_p + (j & 1) * ATT_P_BYTES + row * 128;
-      uint32_t pw[TS ? 32 : 1];
+      uint32_t pw[32];
 #pragma unroll
       for (int ch = 0; ch < ATT_BN / 8; ++ch) {  // 8 chunks of 8 keys = 16 bytes
         uint32_t w[4];
@@ -376,16 +350,10 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
           }
           w[u] = pack_bf16(e.x, e.y);
         }
-        if constexpr (TS) {
-          pw[4 * ch] = w[0]; pw[4 * ch + 1] = w[1]; pw[4 * ch + 2] = w[2]; pw[4 * ch + 3] = w[3];
-        } else {
-          *reinterpret_cast<uint4*>(prow + ((ch ^ (row & 7)) << 4)) = make_uint4(w[0], w[1], w[2], w[3]);
-        }
+        pw[4 * ch] = w[0]; pw[4 * ch + 1] = w[1]; pw[4 * ch + 2] = w[2]; pw[4 * ch + 3] = w[3];
       }
-      if constexpr (TS) {
-        tmem_st_x32(ts, pw);
-        tmem_st_wait();
-      }
+      tmem_st_x32(ts, pw);
+      tmem_st_wait();
       const float2 lsum = __fadd2_rn(__fadd2_rn(l2[0], l2[1]), __fadd2_rn(l2[2], l2[3]));
       l_run += lsum.x + lsum.y;
       // Release the metadata slot only HERE, after the P stores above: they consume every value loaded from the slot (bias,
@@ -394,7 +362,6 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant_
       // MUFU / tcgen05.ld traffic: rows then saw the bias of the tile three ahead (-inf past T) -- wrong, and different
       // from run to run.  Found by the full-size reproducibility test; invisible at small batch.
       mbar_arrive(&meta_empty[ms]);
-      if constexpr (!TS) fence_proxy_async_smem();  // P visible to the tensor core (async proxy)
       tc_fence_before();         // our TMEM reads of S_j / writes of O (and P_j) are ordered before the MMAs that follow
       mbar_arrive(&p_ready[j & 1]);
     }
@@ -437,7 +404,6 @@ __global__ void __launch_bounds__(ATTN_META_TILE)
 attn_meta_kernel(int T, const uint8_t* __restrict__ gid, const int32_t* __restrict__ pos, const uint8_t* __restrict__ allow,
                  int G, const float* __restrict__ size, uint8_t* __restrict__ meta, uint32_t* __restrict__ aug_flag,
                  uint4* __restrict__ aug_q, uint4* __restrict__ aug_k) {
-  pdl_prologue();
   const int tile = blockIdx.x, b = blockIdx.y, t = threadIdx.x, warp = t >> 5, lane = t & 31;
   const int idx = tile * ATTN_META_TILE + t;
   const bool valid = idx < T;
@@ -514,7 +480,6 @@ int launch_attn_meta(int B, int T, const uint8_t* gid, const int32_t* pos, const
 // come from 32 ballots
 __global__ void __launch_bounds__(256)
 attn_dropbits_kernel(int n128, int n64, DropoutCfg d, uint32_t* __restrict__ keep_q, uint32_t* __restrict__ keep_k) {
-  pdl_prologue();
   const int Tq = n128 * 128;                       // padded query / key range: both arrays are written completely
   const long long t = blockIdx.x * 256ll + threadIdx.x;
   const int q = (int)(t % Tq), w = (int)(t / Tq);  // w < n128 * 4
@@ -579,11 +544,6 @@ int check_attn_desc(const tome_attn_desc_t* d, const char* who) {
 }
 }  // namespace tome
 
-// 1 (default): A operands (Q, P) in tensor memory; 0: both operands of both products in shared memory (round-1 kernel, kept
-// as the A/B cross-check).  Process-wide tuning aid, not part of the public header.
-static int g_attn_fwd_ts = 1;
-extern "C" void tome_attention_set_fwd_ts(int on) { g_attn_fwd_ts = on ? 1 : 0; }
-
 static size_t fwd_ws_bytes(const tome_attn_desc_t* d) {
   const size_t meta = (attn_meta_bytes(d->batch, d->tokens) + 255) & ~size_t(255);
   return meta + (d->dropout_rate > 0.f ? attn_dropbits_bytes(d->tokens) : 0);
@@ -642,19 +602,14 @@ extern "C" int tome_attention_fwd(const tome_attn_desc_t* d, const void* q, cons
   p.o_batch_stride = d->o_batch_stride; p.o_token_stride = d->o_token_stride;
   p.lse = lse;
   dim3 grid(ceil_div(d->tokens, ATT_BM), d->heads, d->batch);
-#define TOME_ATT_LAUNCH(DROP_, TS_)                                                                          \
-  do {                                                                                                       \
-    static DynSmemOnce once;                                                                                 \
-    TOME_CUDA(ensure_dyn_smem(attn_fwd_kernel<DROP_, TS_>, att_smem<TS_>(), once));                          \
-    launch_k(attn_fwd_kernel<DROP_, TS_>, grid, ATT_THREADS, att_smem<TS_>(), stream, tq, tk, tv, tqa, tka, p);    \
+#define TOME_ATT_LAUNCH(DROP_)                                                                     \
+  do {                                                                                             \
+    static DynSmemOnce once;                                                                       \
+    TOME_CUDA(ensure_dyn_smem(attn_fwd_kernel<DROP_>, ATT_SMEM, once));                            \
+    launch_k(attn_fwd_kernel<DROP_>, grid, ATT_THREADS, ATT_SMEM, stream, tq, tk, tv, tqa, tka, p); \
   } while (0)
-  if (g_attn_fwd_ts) {
-    if (p.keep_q) TOME_ATT_LAUNCH(true, true);
-    else TOME_ATT_LAUNCH(false, true);
-  } else {
-    if (p.keep_q) TOME_ATT_LAUNCH(true, false);
-    else TOME_ATT_LAUNCH(false, false);
-  }
+  if (p.keep_q) TOME_ATT_LAUNCH(true);
+  else TOME_ATT_LAUNCH(false);
 #undef TOME_ATT_LAUNCH
   TOME_CUDA(cudaGetLastError());
   return TOME_OK;

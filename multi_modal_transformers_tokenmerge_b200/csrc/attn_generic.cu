@@ -46,7 +46,6 @@ __device__ __forceinline__ bool ag_keep(const AttnGenericParams& p, DropStream& 
 // ------------------------------------------------------------------------------------------------ forward: warp = query row
 __global__ void __launch_bounds__(AG_WARPS * 32)
 attn_generic_fwd_kernel(const AttnGenericParams p) {
-  pdl_prologue();
   const int lane = threadIdx.x & 31;
   const int q = blockIdx.x * AG_WARPS + (threadIdx.x >> 5), h = blockIdx.y, b = blockIdx.z;
   if (q >= p.tokens) return;
@@ -100,7 +99,6 @@ attn_generic_fwd_kernel(const AttnGenericParams p) {
 // ------------------------------------------------------------------------------------------------ dQ: warp = query row
 __global__ void __launch_bounds__(AG_WARPS * 32)
 attn_generic_dq_kernel(const AttnGenericParams p) {
-  pdl_prologue();
   const int lane = threadIdx.x & 31;
   const int q = blockIdx.x * AG_WARPS + (threadIdx.x >> 5), h = blockIdx.y, b = blockIdx.z;
   if (q >= p.tokens) return;
@@ -160,7 +158,6 @@ attn_generic_dq_kernel(const AttnGenericParams p) {
 // ------------------------------------------------------------------------------------------------ dK / dV: warp = key row
 __global__ void __launch_bounds__(AG_WARPS * 32)
 attn_generic_dkdv_kernel(const AttnGenericParams p) {
-  pdl_prologue();
   const int lane = threadIdx.x & 31;
   const int kk = blockIdx.x * AG_WARPS + (threadIdx.x >> 5), h = blockIdx.y, b = blockIdx.z;
   if (kk >= p.tokens) return;

@@ -20,7 +20,6 @@ constexpr int AP_MAX_KEYS = 64;
 // q[j] = scale * (sum_c learnt[c] * wq[c, j] + bq[j]),  j < H * D: one thread per output (E x HD multiply-adds in total)
 __global__ void pool_query_kernel(int E, int HD, const float* __restrict__ learnt, const float* __restrict__ wq,
                                   const float* __restrict__ bq, float scale, float* __restrict__ q) {
-  pdl_prologue();
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= HD) return;
   float acc = 0.f;
@@ -32,7 +31,6 @@ __global__ void pool_query_kernel(int E, int HD, const float* __restrict__ learn
 __global__ void __launch_bounds__(128)
 attn_pool_kernel(int B, int n, int H, int D, const float* __restrict__ q, const __nv_bfloat16* __restrict__ kv, long long ld,
                  int v_off, __nv_bfloat16* __restrict__ out) {
-  pdl_prologue();
   const int lane = threadIdx.x & 31;
   const int w = blockIdx.x * 4 + (threadIdx.x >> 5);
   if (w >= B * H) return;

@@ -49,19 +49,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   }
 }
 
-// ------------------------------------------------------------------------------------------------ programmatic dependent launch
-// First statement of every kernel of this library.  Launched with the programmatic-stream-serialization attribute
-// (host_util.h launch_k) a grid may be scheduled onto SMs while its predecessor in the stream is still draining; `wait` then
-// blocks until that predecessor has completed and its memory is visible, so nothing below it ever runs early -- what could be
-// saved is the launch latency between dependent kernels (~500 launches per training step).  Without the attribute both
-// instructions do nothing.  The trigger follows the wait, so a kernel never runs more than one grid ahead.
-// Measured on the octo-small step (TOME_PDL=1 / 0 alternating on one box): 33.52 / 33.76 / 33.67 / 33.65 ms -- no gain, so
-// the attribute is off by default; the step's distance from the sum of its kernels is the power-capped clock, not gaps.
-__device__ __forceinline__ void pdl_prologue() {
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
-
 // ------------------------------------------------------------------------------------------------ TMA
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* tm) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(tm) : "memory");
@@ -84,12 +71,6 @@ __device__ __forceinline__ void tma_load_2d_mc(void* dst, const CUtensorMap* tm,
   asm volatile(
       "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
       ::"r"(smem_u32(dst)), "l"(tm), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(cta_mask)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_3d_mc(void* dst, const CUtensorMap* tm, uint64_t* bar, int c0, int c1, int c2, uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5}], [%2], %6;"
-      ::"r"(smem_u32(dst)), "l"(tm), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "h"(cta_mask)
       : "memory");
 }
 __device__ __forceinline__ uint32_t cluster_ctarank() {

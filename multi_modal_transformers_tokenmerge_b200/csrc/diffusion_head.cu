@@ -87,7 +87,6 @@ diff_prep_kernel(const tome_diffusion_desc_t d, const __nv_bfloat16* __restrict_
                  const float* __restrict__ fourier, const float* __restrict__ actions, const float* __restrict__ noise,
                  const int32_t* __restrict__ time, const float* __restrict__ alpha_hats, __nv_bfloat16* __restrict__ ff,
                  __nv_bfloat16* __restrict__ cat) {
-  pdl_prologue();
   const int b = blockIdx.x, C = d.channels, A = d.action_dim, F2 = d.fourier_dim / 2, n = d.n_readout;
   const long long Dc = (long long)A + d.time_out + C;
   const int t = min(max(time[b], 0), d.diffusion_steps - 1);
@@ -115,7 +114,6 @@ __global__ void __launch_bounds__(DH_THREADS)
 diff_out_kernel(const tome_diffusion_desc_t d, const __nv_bfloat16* __restrict__ h, const float* __restrict__ w2,
                 const float* __restrict__ b2, const float* __restrict__ noise, float* __restrict__ pred,
                 float* __restrict__ loss, float* __restrict__ dpred) {
-  pdl_prologue();
   __shared__ float lsum[DH_THREADS / 32];
   const int b = blockIdx.x, H = d.hidden, A = d.action_dim;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -143,7 +141,6 @@ diff_out_kernel(const tome_diffusion_desc_t d, const __nv_bfloat16* __restrict__
   }
 }
 __global__ void diff_loss_final_kernel(int B, float* loss) {
-  pdl_prologue();
   float t = 0.f;
   for (int b = 0; b < B; ++b) t += loss[1 + b];
   loss[0] = t / (float)B;
@@ -154,7 +151,6 @@ __global__ void __launch_bounds__(DH_THREADS)
 diff_out_bwd_kernel(const tome_diffusion_desc_t d, const __nv_bfloat16* __restrict__ h, const float* __restrict__ w2,
                     const float* __restrict__ dpred, float* __restrict__ dw2, float* __restrict__ db2,
                     __nv_bfloat16* __restrict__ dh) {
-  pdl_prologue();
   const int H = d.hidden, A = d.action_dim, B = d.batch;
   const long long i = blockIdx.x * (long long)DH_THREADS + threadIdx.x;
   if (i < (long long)H * A) {                       // weight gradient, fixed order over the batch
@@ -181,7 +177,6 @@ diff_out_bwd_kernel(const tome_diffusion_desc_t d, const __nv_bfloat16* __restri
 __global__ void __launch_bounds__(DH_THREADS)
 diff_scatter_kernel(const tome_diffusion_desc_t d, const int32_t* __restrict__ origin, const __nv_bfloat16* __restrict__ dcat,
                     __nv_bfloat16* __restrict__ dx) {
-  pdl_prologue();
   const int b = blockIdx.x, C = d.channels, n = d.n_readout;
   const long long Dc = (long long)d.action_dim + d.time_out + C;
   const float inv_n = 1.0f / (float)n;
@@ -196,7 +191,6 @@ diff_scatter_kernel(const tome_diffusion_desc_t d, const int32_t* __restrict__ o
 __global__ void __launch_bounds__(DH_THREADS)
 diff_fourier_bwd_kernel(const tome_diffusion_desc_t d, const int32_t* __restrict__ time, const float* __restrict__ fourier,
                         const float* __restrict__ dff, float* __restrict__ dfourier) {
-  pdl_prologue();
   const int j = blockIdx.x * DH_THREADS + threadIdx.x, F2 = d.fourier_dim / 2;
   if (j >= F2) return;
   const float w = fourier[j];
@@ -365,7 +359,6 @@ extern "C" int tome_diffusion_head_bwd(const tome_diffusion_desc_t* d, const flo
 namespace tome {
 __global__ void ddpm_step_kernel(long long n, const float* __restrict__ sample, const float* __restrict__ eps,
                                  const float* __restrict__ noise, float c1, float c2, float c3, float clip, float* __restrict__ out) {
-  pdl_prologue();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const float v = c1 * (sample[i] - c2 * eps[i]) + c3 * noise[i];

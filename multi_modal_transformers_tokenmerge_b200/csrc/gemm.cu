@@ -27,10 +27,7 @@ namespace tome {
 
 constexpr int GEMM_BM = 128;
 constexpr int GEMM_BK = 64;
-#ifndef TOME_GEMM_EPI_WARPS
-#define TOME_GEMM_EPI_WARPS 8
-#endif
-constexpr int GEMM_EPI_WARPS = TOME_GEMM_EPI_WARPS;   // 4 per TMEM lane quadrant x NSPLIT column groups
+constexpr int GEMM_EPI_WARPS = 8;   // 4 per TMEM lane quadrant x NSPLIT column groups
 constexpr int GEMM_NSPLIT = GEMM_EPI_WARPS / 4;
 static_assert(GEMM_EPI_WARPS % 4 == 0 && GEMM_NSPLIT >= 1 && GEMM_NSPLIT <= 4, "epilogue warps come in groups of four (one per lane quadrant)");
 constexpr int GEMM_THREADS = 64 + 32 * GEMM_EPI_WARPS;
@@ -60,17 +57,11 @@ struct GemmShape {
   int m, n, k;
   int m_tiles, n_tiles, k_splits, kb_per_split, kb_total;
   int m_items;  // m_tiles, or ceil(m_tiles / 2) when CTA pairs share the B operand
-  int ablate;   // TOME_GEMM_ABLATE builds only: 1 = no output stores, 2 = no operand loads, 4 = no MMAs (wrong results; timing probes)
   // Row-shifted A windows (tome_gemm_args_t.a_row_shift): K is a_groups groups of a_group_kb k-blocks; group g reads columns
   // [0, a_group_kb * 64) of A at rows m0 + a_shift[g] (TMA zero-fills rows outside the matrix).  a_groups == 0: plain GEMM.
   int a_groups, a_group_kb;
   int a_shift[TOME_GEMM_MAX_SHIFTS];
 };
-#ifdef TOME_GEMM_ABLATE
-#define TOME_ABL(bit) ((s.ablate & (bit)) != 0)
-#else
-#define TOME_ABL(bit) false
-#endif
 
 constexpr int GEMM_BRES_KB = 6;   // k-blocks (of 64) a resident B operand may have: K <= 384
 
@@ -84,10 +75,9 @@ struct GemmSmem {
   static constexpr int B_BYTES = B_ATOMS * 64 * GEMM_BK * 2;
   static constexpr int STAGE_BYTES = BRES ? A_BYTES : A_BYTES + B_BYTES;
   static constexpr int RES_BYTES = BRES ? GEMM_BRES_KB * B_BYTES : 0;
-  // 6 x 32 KB, 5 x 40 KB, 4 x 48 KB; with 16 epilogue warps the staging tiles take 32 KB and the widest tile keeps 3 stages
   static constexpr int STAGES = BRES ? 6                        // 6 x 16 KB of A (one whole K = 384 tile ahead) + 96 KB of B
                               : PAIR ? ((BN <= 128) ? 8 : 6)   // 8 x 24 KB, 6 x 32 KB (BN = 192 and 256)
-                                     : (BN <= 128) ? 6 : (BN <= 192) ? (GEMM_EPI_WARPS > 8 ? 4 : 5) : (GEMM_EPI_WARPS > 8 ? 3 : 4);
+                                     : (BN <= 128) ? 6 : (BN <= 192) ? 5 : 4;   // 6 x 32 KB, 5 x 40 KB, 4 x 48 KB
   static constexpr int STORE_BYTES = GEMM_EPI_WARPS * 2048;  // per epilogue warp: 32 rows x 64 B staging tile for TMA stores
   static constexpr int BAR_BYTES = 256 + 2 * BN * 4;  // barriers + double-buffered bias tile
   static constexpr int COL_BYTES = 2 * 4 * BN * 4;    // column sums: [accumulator stage][lane quadrant][BN] f32
@@ -107,7 +97,6 @@ template <int BN, bool A_MN, bool B_MN, int MC, int EPI>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
                  const __grid_constant__ CUtensorMap tma_c, const GemmShape s, const GemmEpilogue e) {
-  pdl_prologue();
   constexpr bool PAIR = MC >= 2;   // one 256-row cta_group::2 MMA per cluster pair (MC == 1: two 128-row MMAs sharing a multicast B)
   constexpr bool BRES = MC == 3;   // ... with the B operand resident in shared memory (K <= 384)
   using L = GemmSmem<BN, PAIR, BRES>;
@@ -221,16 +210,11 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
           if constexpr (PAIR) {
             // both CTAs' loads are counted on the LEADER's barrier: its MMA thread is the only consumer
             const uint32_t fb = map_to_cta(&full_bar[stage], 0);
-            if (TOME_ABL(2)) {
-              if (leader) mbar_arrive(&full_bar[stage]);
-              if (++stage == STAGES) { stage = 0; phase ^= 1; }
-              continue;
-            }
             // bytes both CTAs' boxes deliver (a K-major half of BN = 192 is one 96-row box: 12 KB of the 16 KB slot)
             constexpr uint32_t kPairTx = 2 * (L::A_BYTES + (B_MN ? L::B_BYTES : (BN / 2) * GEMM_BK * 2));
             if (leader) mbar_expect_tx(&full_bar[stage], kPairTx);
             if (!A_MN) {
-              tma_load_2d_pair(sa, &tma_a, fb, ka, TOME_ABL(32) ? (m0 & 1023) : ma);   // 32: operand stream from 1024 rows (L2-resident)
+              tma_load_2d_pair(sa, &tma_a, fb, ka, ma);
             } else {
 #pragma unroll
               for (int j = 0; j < GEMM_BM / 64; ++j) tma_load_2d_pair(sa + j * 8192, &tma_a, fb, m0 + 64 * j, k0);
@@ -242,11 +226,6 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
 #pragma unroll
               for (int j = 0; j < L::B_ATOMS; ++j) tma_load_2d_pair(sb + j * 8192, &tma_b, fb, nh + 64 * j, k0);   // BN = 192: the second atom is half used
             }
-            if (++stage == STAGES) { stage = 0; phase ^= 1; }
-            continue;
-          }
-          if (TOME_ABL(2) && !MC) {
-            mbar_arrive(&full_bar[stage]);
             if (++stage == STAGES) { stage = 0; phase ^= 1; }
             continue;
           }
@@ -304,7 +283,6 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
           const uint32_t sb = BRES ? smem_u32(s_bres + kb * L::B_BYTES) : sa + L::A_BYTES;
 #pragma unroll
           for (int k = 0; k < GEMM_BK / 16; ++k) {
-            if (TOME_ABL(4)) break;
             const uint64_t da = A_MN ? make_smem_desc(sa + k * 2048, 8192, 1024) : make_smem_desc(sa + k * 32, 16, 1024);
             const uint64_t db = B_MN ? make_smem_desc(sb + k * 2048, 8192, 1024) : make_smem_desc(sb + k * 32, 16, 1024);
             if constexpr (PAIR) umma2_bf16(d_tmem, da, db, idesc, (kb > kb0 || k > 0) ? 1u : 0u);
@@ -377,10 +355,10 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
         const uint32_t t_addr = tmem_base + acc * BN + ((uint32_t)(quad * 32) << 16);
         // the TMEM read of chunk c + 1 is in flight while chunk c is processed (two register sets, compile-time ping-pong)
         float va[32], vb[32];
-        if (!TOME_ABL(8)) tmem_ld_f32x32(t_addr + TOME_CHUNK(0) * 32, va);
+        tmem_ld_f32x32(t_addr + TOME_CHUNK(0) * 32, va);
 #pragma unroll
         for (int c = 0; c < NCH; ++c) {
-          if (!TOME_CHUNK_OK(c) || TOME_ABL(8)) break;   // warp-uniform: this warp owns one chunk fewer
+          if (!TOME_CHUNK_OK(c)) break;   // warp-uniform: this warp owns one chunk fewer
           float (&v)[32] = (c & 1) ? vb : va;
           tmem_ld_wait();
           if (c + 1 < NCH && TOME_CHUNK_OK(c + 1)) tmem_ld_f32x32(t_addr + TOME_CHUNK(c + 1) * 32, (c & 1) ? va : vb);
@@ -456,8 +434,8 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
           fence_proxy_async_smem();
           __syncwarp();
           if (lane == 0) {
-            const int row0 = (TOME_ABL(16) ? (m_blk & 7) : m_blk) * GEMM_BM + quad * 32;   // 16: all stores into 1024 rows (L2-resident)
-            if (col < s.n && row0 < s.m && !TOME_ABL(1)) {
+            const int row0 = m_blk * GEMM_BM + quad * 32;
+            if (col < s.n && row0 < s.m) {
               asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
                            ::"l"(&tma_c), "r"(smem_u32(stg)), "r"(col), "r"(row0) : "memory");
             }
@@ -676,7 +654,6 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
 // sum split-K partials: out[i] = sum_s part[s*stride + i]      (fp32, deterministic order)
 __global__ void splitk_reduce_kernel(const float* __restrict__ part, float* __restrict__ out, long long n4,
                                      long long stride4, int splits, int accumulate) {
-  pdl_prologue();
   const float4* p = reinterpret_cast<const float4*>(part);
   float4* o = reinterpret_cast<float4*>(out);
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
@@ -719,18 +696,17 @@ static int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const CUten
   cfg.blockDim = dim3(GEMM_THREADS);
   cfg.dynamicSmemBytes = SM::TOTAL;
   cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_attr(&attr[0]);
+  cudaLaunchAttribute attr[1];
   if (MC) {
     int clusters = items < gemm_sms() / 2 ? items : gemm_sms() / 2;
     if (MC == 3) clusters = bres_clusters(s.n_tiles, s.m_items);   // a multiple of the column tiles
     cfg.gridDim = dim3(2 * clusters);
-    cudaLaunchAttribute& ca = attr[cfg.numAttrs++];
-    ca.id = cudaLaunchAttributeClusterDimension;
-    ca.val.clusterDim.x = 2;
-    ca.val.clusterDim.y = 1;
-    ca.val.clusterDim.z = 1;
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 2;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
   } else {
     cfg.gridDim = dim3(items < gemm_sms() ? items : gemm_sms());
   }
@@ -752,14 +728,6 @@ static int pick_bn(int n) {  // least padded MMA work (tiles x width), then the 
 static int g_gemm_force_mode = -1, g_gemm_force_bn = 0;
 // tuning aid: force the CTA mode (0 single, 1 multicast pairs, 2 pair MMA; -1 = automatic) and the tile width (0 = automatic)
 extern "C" void tome_gemm_force_tile(int mode, int bn) { g_gemm_force_mode = mode; g_gemm_force_bn = bn; }
-// g_gemm_pair = 1 (default): CTA pairs may run one cta_group::2 MMA per k-step (256 x BN tile, each CTA holding half of B);
-// 0: never (two 128-row MMAs sharing a TMA-multicast B tile, round 1).  Process-wide tuning aid, not in the public header.
-static int g_gemm_pair = 1;
-extern "C" void tome_gemm_set_pair_mma(int on) { g_gemm_pair = on ? 1 : 0; }
-static int g_gemm_bres = 1;   // tuning aid: 0 = never keep B resident
-extern "C" void tome_gemm_set_b_resident(int on) { g_gemm_bres = on ? 1 : 0; }
-static int g_gemm_ablate = 0;
-extern "C" void tome_gemm_set_ablate(int bits) { g_gemm_ablate = bits; }   // has an effect in TOME_GEMM_ABLATE builds only
 
 struct TileChoice { int bn, mode; };   // mode 0: one CTA per tile; 1: CTA pairs, multicast B; 2: CTA pairs, one 256-row MMA
 static TileChoice pick_tile(const tome_gemm_args_t* a) {
@@ -774,7 +742,7 @@ static TileChoice pick_tile(const tome_gemm_args_t* a) {
   // profiles/r02_gemm_tile_sweep.md): with the tile width below it is the fastest or within 2 % of the fastest mode at every
   // shape that can form pairs (octo-base: 1.46 - 1.56 PF/s against 1.31 - 1.41 for multicast pairs, above cuBLAS).  A pair
   // MMA narrower than 192 columns is not: 256 x 128 x 16 occupies the tensor pipe as long as 256 x 256 x 16 does.
-  if (pairs_ok && g_gemm_pair) {
+  if (pairs_ok) {
     t.mode = 2;
     // activations x weights with a wide output: the 256-wide pair tile beats the exactly fitting 192 (qkv, N = 1152: 112 vs 121 us)
     if (t.bn == 192 && a->n >= 1024 && a->a_major == TOME_MAJOR_K) t.bn = 256;
@@ -783,7 +751,7 @@ static TileChoice pick_tile(const tome_gemm_args_t* a) {
   // K <= 384 with a specialised epilogue: keep B in shared memory (mode 3; the caller checks the epilogue)
   // (with two column tiles the epilogue, not the operand stream, paces the kernel and the fixed column assignment only costs
   // balance: out projection 137216 x 384 x 384, 78 vs 76 us)
-  if (t.mode == 2 && g_gemm_bres && a->k <= GEMM_BRES_KB * GEMM_BK && a->a_major == TOME_MAJOR_K && ceil_div(a->n, t.bn) >= 3 &&
+  if (t.mode == 2 && a->k <= GEMM_BRES_KB * GEMM_BK && a->a_major == TOME_MAJOR_K && ceil_div(a->n, t.bn) >= 3 &&
       ceil_div(a->n, t.bn) <= gemm_sms() / 2)
     t.mode = 3;
   if (g_gemm_force_bn == 128 || g_gemm_force_bn == 192 || g_gemm_force_bn == 256) t.bn = g_gemm_force_bn;
@@ -853,7 +821,6 @@ extern "C" int tome_gemm_bf16(const tome_gemm_args_t* a, void* workspace, size_t
   s.kb_per_split = ceil_div(s.kb_total, s.k_splits);
   s.k_splits = ceil_div(s.kb_total, s.kb_per_split);  // drop empty splits
   s.m_items = mc ? ceil_div(s.m_tiles, 2) : s.m_tiles;
-  s.ablate = g_gemm_ablate;
   s.a_groups = 0; s.a_group_kb = 1;
   if (a->a_row_shift) {
     TOME_CHECK(a->a_shift_groups >= 1 && a->a_shift_groups <= TOME_GEMM_MAX_SHIFTS && a->k % a->a_shift_groups == 0 &&

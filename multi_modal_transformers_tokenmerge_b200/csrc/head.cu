@@ -55,7 +55,6 @@ __global__ void __launch_bounds__(HEAD_THREADS)
 head_fwd_kernel(const tome_head_desc_t d, const void* __restrict__ x, const int32_t* __restrict__ origin,
                 const float* __restrict__ w, const float* __restrict__ bias, const float* __restrict__ actions,
                 float* __restrict__ out, float* __restrict__ loss, float* __restrict__ pooled_g, float* __restrict__ dz_g) {
-  pdl_prologue();
   extern __shared__ float head_sm[];
   const int b = blockIdx.x, C = d.channels, G = d.groups, F = d.features, m = d.n_readout / d.groups;
   float* pooled = head_sm;        // [G*C]
@@ -139,7 +138,6 @@ head_fwd_kernel(const tome_head_desc_t d, const void* __restrict__ x, const int3
 }
 
 __global__ void head_loss_final_kernel(int B, float inv_count, float* loss) {
-  pdl_prologue();
   float t = 0.f;
   for (int b = 0; b < B; ++b) t += loss[1 + b];
   loss[0] = t * inv_count;
@@ -151,7 +149,6 @@ __global__ void head_loss_final_kernel(int B, float inv_count, float* loss) {
 __global__ void __launch_bounds__(HEAD_THREADS)
 head_wgrad_kernel(const tome_head_desc_t d, const float* __restrict__ pooled, const float* __restrict__ dz,
                   float* __restrict__ dw, float* __restrict__ dbias) {
-  pdl_prologue();
   __shared__ float part[HEAD_THREADS / 32][32];
   const int C = d.channels, F = d.features, BG = d.batch * d.groups;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = HEAD_THREADS / 32;
@@ -180,7 +177,6 @@ template <bool BF16>
 __global__ void __launch_bounds__(HEAD_THREADS)
 head_dgrad_kernel(const tome_head_desc_t d, const int32_t* __restrict__ origin, const float* __restrict__ w,
                   const float* __restrict__ dz, void* __restrict__ dx) {
-  pdl_prologue();
   extern __shared__ float head_sm[];
   const int b = blockIdx.x, C = d.channels, G = d.groups, F = d.features, m = d.n_readout / d.groups;
   float* dzs = head_sm;  // [G*F]

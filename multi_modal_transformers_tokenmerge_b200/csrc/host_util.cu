@@ -1,6 +1,4 @@
 // Error string + TMA tensor-map encoding (driver entry point fetched at run time; the library links only cudart).
-#include <stdlib.h>
-
 #include "host_util.h"
 
 #include <string.h>
@@ -169,17 +167,5 @@ extern "C" int tome_profile_collect(int n_tags, float* ms, double* work, int* co
 }
 
 extern "C" const char* tome_last_error(void) { return tome::g_err; }
-namespace tome {
-static int g_pdl = -1;   // -1: read TOME_PDL from the environment on first use
-bool pdl_enabled() {
-  if (g_pdl < 0) {
-    const char* e = getenv("TOME_PDL");
-    g_pdl = (e && e[0] == '1') ? 1 : 0;   // off unless asked for: measured neutral (profiles/r02_graph_probe.txt)
-  }
-  return g_pdl != 0;
-}
-}  // namespace tome
-/* tuning aid (not in the public header): programmatic dependent launch on / off for every kernel of the library */
-extern "C" void tome_set_pdl(int on) { tome::g_pdl = on ? 1 : 0; }
 
 extern "C" int tome_abi_version(void) { return TOME_ABI_VERSION; }

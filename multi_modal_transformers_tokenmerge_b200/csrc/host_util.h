@@ -65,13 +65,7 @@ inline cudaError_t ensure_dyn_smem(Kernel kernel, int bytes, DynSmemOnce& once) 
   return e;
 }
 
-// ---- kernel launches with programmatic dependent launch (common.cuh pdl_prologue) ----
-bool pdl_enabled();   // TOME_PDL=1 in the environment, or tome_set_pdl(1), turns the attribute on (off by default: measured neutral)
-inline int pdl_attr(cudaLaunchAttribute* a) {   // fills *a; returns the number of attributes to pass (0 or 1)
-  a->id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  a->val.programmaticStreamSerializationAllowed = 1;
-  return pdl_enabled() ? 1 : 0;
-}
+// ---- kernel launches: the arguments are converted to the kernel's parameter types ----
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args&&... args) {
   cudaLaunchConfig_t cfg;
@@ -80,9 +74,6 @@ inline cudaError_t launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  cfg.numAttrs = pdl_attr(attr);
-  cfg.attrs = attr;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 

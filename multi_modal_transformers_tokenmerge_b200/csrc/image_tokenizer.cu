@@ -28,8 +28,6 @@
 // What is left HBM-bound is the input convolution (its im2col rows are k*k*C_in / (s*s*C_in) = 36x the pixels); the batch
 // is processed in chunks of whole batch rows so that buffer stays near 1 GiB whatever the batch.  Measurements and the
 // versions that led here: DESIGN.md 4.5, profiles/r02c_image_tokenizer.md.
-#include <stdlib.h>
-
 #include <algorithm>
 
 #include "common.cuh"
@@ -83,9 +81,7 @@ static int it_geometry(const tome_image_tokenizer_desc_t* d, ItGeom* g, const ch
   TOME_CHECK(g->o2 >= 1, TOME_ERR_INVALID, "%s: a %d-wide pool does not fit the %d x %d convolution output", who, d->pool_window, g->o1, g->o1);
   g->k0 = d->conv_kernel * d->conv_kernel * d->channels_in;
   g->kd = g->o2 * g->o2 * d->features;
-  // TOME_IT_NO_SHIFT (environment; A/B measurements and bisection only) forces the im2col path of the 3 x 3 convolutions
-  static const bool no_shift = getenv("TOME_IT_NO_SHIFT") != nullptr;
-  g->pad = (d->features % 64 == 0 && !no_shift) ? 1 : 0;
+  g->pad = d->features % 64 == 0 ? 1 : 0;
   TOME_CHECK(g->k0 % 16 == 0, TOME_ERR_UNSUPPORTED, "%s: conv_kernel^2 * channels_in (%d) must be a multiple of 16", who, g->k0);
   g->wp = g->o2 + 2 * g->pad;
   g->imgs = (long long)d->batch * d->n_images;
@@ -150,7 +146,6 @@ struct Im2col0Args {
 template <typename PixT>
 __global__ void __launch_bounds__(IT_THREADS)
 it_im2col0_kernel(const PixT* __restrict__ image, __nv_bfloat16* __restrict__ col, uint32_t n_vec, const Im2col0Args a) {
-  pdl_prologue();
   __shared__ uint16_t lut[256];
   if (sizeof(PixT) == 1) {
     float x = (float)threadIdx.x;
@@ -194,7 +189,6 @@ it_im2col0_kernel(const PixT* __restrict__ image, __nv_bfloat16* __restrict__ co
 template <typename PixT>
 __global__ void __launch_bounds__(IT_THREADS)
 it_pixels_bf16_kernel(const PixT* __restrict__ image, __nv_bfloat16* __restrict__ out, long long n, int normalize) {
-  pdl_prologue();
   const long long i = ((long long)blockIdx.x * IT_THREADS + threadIdx.x) * 8;
   if (i >= n) return;
   uint32_t w[4];
@@ -214,7 +208,6 @@ it_pixels_bf16_kernel(const PixT* __restrict__ image, __nv_bfloat16* __restrict_
 // is even (host-checked: k * C_in, W * C_in, stride * C_in and patch * C_in even), so a word never straddles a (dy) row.
 __global__ void __launch_bounds__(IT_THREADS)
 it_im2col0_words_kernel(const uint32_t* __restrict__ pix, __nv_bfloat16* __restrict__ col, uint32_t n_vec, const Im2col0Args a) {
-  pdl_prologue();
   const uint32_t v = (blockIdx.x * IT_THREADS + threadIdx.x) * 2;   // two consecutive 16-byte vectors of one row
   if (v >= n_vec) return;
   uint32_t m, kc, ox, oy, patch, img, py, px, dy, rem, t;
@@ -253,7 +246,6 @@ __device__ __forceinline__ uint32_t bf16x2_max(uint32_t a, uint32_t b) {
 __global__ void __launch_bounds__(IT_THREADS)
 it_pool_kernel(const __nv_bfloat16* __restrict__ y0, __nv_bfloat16* __restrict__ pooled, uint32_t n_vec, FastDiv nchunk, int o1,
                FastDiv o2, int window, int wp, int pad) {
-  pdl_prologue();
   const uint32_t v = blockIdx.x * IT_THREADS + threadIdx.x;
   if (v >= n_vec) return;
   uint32_t c, t, ox, oy, ip;
@@ -277,7 +269,6 @@ it_pool_kernel(const __nv_bfloat16* __restrict__ y0, __nv_bfloat16* __restrict__
 // of batch row b -> part [rows_b, gridDim.x, F, 2].  Thread = (8-channel chunk, row lane); lanes are added in lane order.
 __global__ void __launch_bounds__(IT_THREADS)
 it_gn_partial_kernel(const __nv_bfloat16* __restrict__ x, float* __restrict__ part, long long R, int nchunk, FastDiv wp, int pad) {
-  pdl_prologue();
   __shared__ float sm[2][IT_THREADS * 8];
   const int F = nchunk << 3;
   const int lanes = blockDim.x / nchunk;
@@ -319,7 +310,6 @@ it_gn_partial_kernel(const __nv_bfloat16* __restrict__ x, float* __restrict__ pa
 __global__ void __launch_bounds__(128)
 it_gn_final_kernel(const float* __restrict__ part, float* __restrict__ stats, int rows_b, int n_ctas, int F, int G, long long R,
                    float eps) {
-  pdl_prologue();
   const int i = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (i >= rows_b * G) return;
   const int b = i / G, g = i - b * G, cg = F / G;
@@ -350,7 +340,6 @@ __device__ __forceinline__ float gelu_tanh(float x) {   // flax.linen.gelu, appr
 // channel) affine (rstd * scale, bias - mean * rstd * scale) the preceding tiny kernel folded the statistics into.
 __global__ void it_gn_fold_kernel(const float* __restrict__ stats, const float* __restrict__ scale, const float* __restrict__ bias,
                                   float* __restrict__ ab, int rows_b, int F, int G) {
-  pdl_prologue();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= rows_b * F) return;
   const int b = i / F, ch = i - b * F;
@@ -363,7 +352,6 @@ __global__ void it_gn_fold_kernel(const float* __restrict__ stats, const float* 
 __global__ void __launch_bounds__(IT_THREADS)
 it_gn_gelu_kernel(const __nv_bfloat16* __restrict__ x, const float* __restrict__ ab, __nv_bfloat16* __restrict__ h, uint32_t n_vec,
                   FastDiv nchunk, FastDiv pix_per_row, FastDiv wp, int pad) {
-  pdl_prologue();
   const uint32_t v = blockIdx.x * IT_THREADS + threadIdx.x;
   if (v >= n_vec) return;
   uint32_t m, c;
@@ -396,7 +384,6 @@ it_gn_gelu_kernel(const __nv_bfloat16* __restrict__ x, const float* __restrict__
 // (pixel, tap, 8 channels): output vector index == thread index, so the stores are one contiguous stream.
 __global__ void __launch_bounds__(IT_THREADS)
 it_im2col3_kernel(const __nv_bfloat16* __restrict__ h, __nv_bfloat16* __restrict__ col, uint32_t n_vec, FastDiv nchunk, FastDiv o2) {
-  pdl_prologue();
   const uint32_t v = blockIdx.x * IT_THREADS + threadIdx.x;
   if (v >= n_vec) return;
   uint32_t c, t, tap, m, ox, oy, q;
@@ -420,7 +407,6 @@ it_im2col3_kernel(const __nv_bfloat16* __restrict__ h, __nv_bfloat16* __restrict
 __global__ void __launch_bounds__(IT_THREADS)
 it_compact_kernel(const __nv_bfloat16* __restrict__ xp, const __nv_bfloat16* __restrict__ res, __nv_bfloat16* __restrict__ out,
                   uint32_t n_vec, FastDiv nchunk, FastDiv o2, int wp, int pad) {
-  pdl_prologue();
   const uint32_t v = blockIdx.x * IT_THREADS + threadIdx.x;
   if (v >= n_vec) return;
   uint32_t c, t, ox, oy, ip;
@@ -442,7 +428,6 @@ __global__ void __launch_bounds__(IT_THREADS)
 it_posadd_kernel(const float* __restrict__ dense, const float* __restrict__ row_emb, const float* __restrict__ col_emb,
                  const int32_t* __restrict__ row_tok, const int32_t* __restrict__ col_tok, void* __restrict__ out, long long n_vec,
                  int E, int np, long long img0, int per_image_tokens, int P, int out_bf16) {
-  pdl_prologue();
   const long long v = (long long)blockIdx.x * IT_THREADS + threadIdx.x;
   if (v >= n_vec) return;
   const int e4 = E >> 2;

@@ -58,7 +58,6 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 template <int D, bool ROWS_ARE_KEYS, bool MASKED>
 __global__ void __launch_bounds__(IMP_WARPS * 32)
 attn_importance_kernel(const ImpParams p) {
-  pdl_prologue();
   constexpr int PITCH = D + 8;   // bf16 elements per staged row
   constexpr int IMP_COLS = D > 128 ? 32 : 64;   // rows of the swept operand staged per step (static shared memory <= 48 KB)
   __shared__ __align__(16) __nv_bfloat16 ys[2][IMP_COLS * PITCH];

@@ -29,7 +29,6 @@ __global__ void __launch_bounds__(LN_THREADS)
 ln_seq_fwd_kernel(int T, int C, float eps, const __nv_bfloat16* __restrict__ x, const float* __restrict__ gamma,
                   const float* __restrict__ beta, __nv_bfloat16* __restrict__ y, float* __restrict__ mean,
                   float* __restrict__ rstd) {
-  pdl_prologue();
   __shared__ float s_sum[LN_RG][LN_SLAB + 1];
   __shared__ float s_sq[LN_RG][LN_SLAB + 1];
   __shared__ float s_mean[LN_SLAB], s_rstd[LN_SLAB];
@@ -100,7 +99,6 @@ __global__ void __launch_bounds__(LN_THREADS)
 ln_seq_bwd_kernel(int B, int T, int C, const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
                   const float* __restrict__ gamma, const float* __restrict__ mean, const float* __restrict__ rstd,
                   const __nv_bfloat16* __restrict__ dres, __nv_bfloat16* __restrict__ dx, float* __restrict__ partial) {
-  pdl_prologue();
   __shared__ float s_a[LN_RG][LN_SLAB + 1];
   __shared__ float s_b[LN_RG][LN_SLAB + 1];
   __shared__ float s_A[LN_SLAB], s_B[LN_SLAB];
@@ -183,7 +181,6 @@ template <int G>
 __global__ void __launch_bounds__(32 * G)
 reduce_rows_kernel(int R, int N, const float* __restrict__ ws, long long plane_stride, float* __restrict__ out0,
                    float* __restrict__ out1, int accumulate) {
-  pdl_prologue();
   __shared__ float s[G][33];
   const int n = blockIdx.x * 32 + (threadIdx.x & 31), rgp = threadIdx.x >> 5;
   const float* w = ws + blockIdx.y * plane_stride;
@@ -231,7 +228,6 @@ __global__ void __launch_bounds__(LN_THREADS)
 ln_seq_fwd_smem_kernel(const __grid_constant__ CUtensorMap tm_x, int T, int C, int nb, float eps, const float* __restrict__ gamma,
                        const float* __restrict__ beta, __nv_bfloat16* __restrict__ y, float* __restrict__ mean,
                        float* __restrict__ rstd) {
-  pdl_prologue();
   extern __shared__ uint8_t ln_smem_raw[];
   uint8_t* slab = ln_smem_raw + ((1024u - (smem_u32(ln_smem_raw) & 1023u)) & 1023u);
   const int t0 = CL ? (int)blockIdx.z * nb * LN_BOX : 0;   // first token row of this CTA
@@ -350,7 +346,6 @@ __global__ void __launch_bounds__(LN_THREADS)
 ln_seq_bwd_smem_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_dy, int B, int T, int C, int nb,
                        const float* __restrict__ gamma, const float* __restrict__ mean, const float* __restrict__ rstd,
                        const __nv_bfloat16* __restrict__ dres, __nv_bfloat16* __restrict__ dx, float* __restrict__ partial) {
-  pdl_prologue();
   extern __shared__ uint8_t ln_smem_raw[];
   uint8_t* slab_x = ln_smem_raw + ((128u - (smem_u32(ln_smem_raw) & 127u)) & 127u);
   const int t0 = CL ? (int)blockIdx.z * nb * LN_BOX : 0;   // first token row of this CTA
@@ -493,7 +488,6 @@ ln_seq_bwd_smem_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_co
 __global__ void __launch_bounds__(LN_THREADS)
 colsum_partial_kernel(int M, int N, long long ldx, int rows_per_chunk, const __nv_bfloat16* __restrict__ x,
                       float* __restrict__ ws) {
-  pdl_prologue();
   __shared__ float s_sum[LN_RG][LN_SLAB + 1];
   const int chunk = blockIdx.y, c0 = blockIdx.x * LN_SLAB;
   const int ct = threadIdx.x & 7, rg = threadIdx.x >> 3;
@@ -526,7 +520,6 @@ colsum_partial_kernel(int M, int N, long long ldx, int rows_per_chunk, const __n
 __global__ void __launch_bounds__(LN_THREADS)
 dropout_colsum_kernel(int M, int N, int rows_per_chunk, const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __restrict__ y,
                       DropoutCfg d, float* __restrict__ ws) {
-  pdl_prologue();
   __shared__ float s_sum[LN_RG][LN_SLAB + 1];
   const int chunk = blockIdx.y, c0 = blockIdx.x * LN_SLAB;
   const int ct = threadIdx.x & 7, rg = threadIdx.x >> 3;
@@ -566,7 +559,6 @@ __global__ void __launch_bounds__(256)
 ln_feat_fwd_kernel(long long rows, int C, float eps, const __nv_bfloat16* __restrict__ x, const float* __restrict__ gamma,
                    const float* __restrict__ beta, __nv_bfloat16* __restrict__ y, float* __restrict__ mean,
                    float* __restrict__ rstd) {
-  pdl_prologue();
   const long long row = blockIdx.x * 8ll + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (row >= rows) return;
@@ -603,7 +595,6 @@ __global__ void __launch_bounds__(256)
 ln_feat_bwd_kernel(long long rows, int C, const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ dy,
                    const float* __restrict__ gamma, const float* __restrict__ mean, const float* __restrict__ rstd,
                    const __nv_bfloat16* __restrict__ dres, __nv_bfloat16* __restrict__ dx) {
-  pdl_prologue();
   const long long row = blockIdx.x * 8ll + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (row >= rows) return;
@@ -643,7 +634,6 @@ __global__ void __launch_bounds__(LN_THREADS)
 ln_feat_param_grad_kernel(long long rows, int C, int rows_per_chunk, int n_chunks, const __nv_bfloat16* __restrict__ x,
                           const __nv_bfloat16* __restrict__ dy, const float* __restrict__ mean,
                           const float* __restrict__ rstd, float* __restrict__ ws) {
-  pdl_prologue();
   __shared__ float s_a[LN_RG][LN_SLAB + 1];
   __shared__ float s_b[LN_RG][LN_SLAB + 1];
   const int chunk = blockIdx.y, c0 = blockIdx.x * LN_SLAB;
@@ -696,7 +686,6 @@ using namespace tome;
 
 extern "C" int tome_colsum_workspace_rows(int m) { return colsum_rows(m); }
 
-static int g_ln_smem_fwd = 1, g_ln_smem_bwd = 1;
 static int g_ln_force_cluster = 0;
 /* testing aid (not in the public header): 1 = take the cluster kernels even when one CTA per slab would do; n > 1 = split the
  * tokens over exactly n CTAs */
@@ -716,19 +705,16 @@ static int launch_cluster_z(K kern, dim3 grid, int smem, cudaStream_t stream, Ar
   cfg.blockDim = dim3(LN_THREADS);
   cfg.dynamicSmemBytes = (size_t)smem;
   cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 1;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = grid.z;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_attr(&attr[0]);
-  cudaLaunchAttribute& ca = attr[cfg.numAttrs++];
-  ca.id = cudaLaunchAttributeClusterDimension;
-  ca.val.clusterDim.x = 1;
-  ca.val.clusterDim.y = 1;
-  ca.val.clusterDim.z = grid.z;
+  cfg.numAttrs = 1;
   TOME_CUDA(cudaLaunchKernelEx(&cfg, kern, args...));
   return TOME_OK;
 }
-/* tuning aid (not part of the public header): bit 0 = forward, bit 1 = backward may take the shared-memory-slab kernels */
-extern "C" void tome_ln_set_smem_path(int mask) { g_ln_smem_fwd = mask & 1; g_ln_smem_bwd = (mask >> 1) & 1; }
 
 extern "C" int tome_reduce_rows_f32(int rows, int n, const float* partial, float* out, int accumulate, void* stream_) {
   clear_error();
@@ -798,7 +784,7 @@ extern "C" int tome_layernorm_fwd(int batch, int tokens, int channels, int axis,
     const int nb_all = ln_boxes(tokens);
     const int split = g_ln_force_cluster > 1 ? g_ln_force_cluster : ln_token_split(nb_all);   // CTAs (one cluster) per (batch, slab)
     const int nb = ceil_div(nb_all, split);
-    if (g_ln_smem_fwd && ((uintptr_t)x & 15) == 0 && nb * LN_BOX <= LN_SMEM_T_FWD) {
+    if (((uintptr_t)x & 15) == 0 && nb * LN_BOX <= LN_SMEM_T_FWD) {
       CUtensorMap tx;
       if (int rc = make_tmap_3d_bf16(&tx, x, channels, tokens, batch, channels, (uint64_t)tokens * channels, LN_BOX)) return rc;
       const int smem = nb * LN_BOX * 128 + nb * 8 + 1024;
@@ -844,7 +830,7 @@ extern "C" int tome_layernorm_bwd(int batch, int tokens, int channels, int axis,
     const int nb_all = ln_boxes(tokens);
     const int split = g_ln_force_cluster > 1 ? g_ln_force_cluster : ln_token_split(nb_all);
     const int nb = ceil_div(nb_all, split);
-    if (g_ln_smem_bwd && nb <= LNB_MAX_BOXES && (((uintptr_t)x | (uintptr_t)dy) & 15) == 0) {
+    if (nb <= LNB_MAX_BOXES && (((uintptr_t)x | (uintptr_t)dy) & 15) == 0) {
       CUtensorMap tx, tdy;
       if (int rc = make_tmap_3d_bf16_plain(&tx, x, channels, tokens, batch, channels, (uint64_t)tokens * channels, LNB_SLAB, LN_BOX)) return rc;
       if (int rc = make_tmap_3d_bf16_plain(&tdy, dy, channels, tokens, batch, channels, (uint64_t)tokens * channels, LNB_SLAB, LN_BOX)) return rc;

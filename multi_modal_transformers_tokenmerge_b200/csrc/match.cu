@@ -9,8 +9,6 @@
 // numpy), so indices are bit-exact given the same fp32 scores.  The similarity product is fp32 FMA on CUDA cores
 // on purpose: it is 0.1 % of the block's FLOPs (SURVEY.md 8d) and fp32 keeps the arg max aligned with the fp32
 // reference; the scores tile lives in registers and never reaches HBM unless scores_out is given.
-#include <string.h>
-
 #include "common.cuh"
 #include "host_util.h"
 
@@ -84,7 +82,6 @@ template <typename T>
 __global__ void __launch_bounds__(SIM_THREADS)
 sim_argmax_kernel(const tome_metric_desc_t d, const T* __restrict__ src, float* __restrict__ node_max,
                   int32_t* __restrict__ node_idx, float* __restrict__ scores_out) {
-  pdl_prologue();
   extern __shared__ float4 sm4[];
   float* sm = reinterpret_cast<float*>(sm4);
   const int dpad = (d.dim + 3) & ~3, pitch = dpad + 4;
@@ -179,7 +176,6 @@ template <typename T>
 __global__ void __launch_bounds__(256)
 metric_norm_kernel(const tome_metric_desc_t d, const T* __restrict__ src, float* __restrict__ plane_a,
                    float* __restrict__ plane_b) {
-  pdl_prologue();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long tok = (long long)blockIdx.x * 8 + warp;   // b * T + t
   if (tok >= (long long)d.batch * d.tokens) return;
@@ -216,7 +212,6 @@ metric_norm_kernel(const tome_metric_desc_t d, const T* __restrict__ src, float*
 __global__ void __launch_bounds__(256)
 metric_norm64_kernel(const tome_metric_desc_t d, const __nv_bfloat16* __restrict__ src, float* __restrict__ plane_a,
                      float* __restrict__ plane_b) {
-  pdl_prologue();
   const long long tok = ((long long)blockIdx.x * 256 + threadIdx.x) >> 3;   // b * T + t
   const int sub = threadIdx.x & 7;
   const bool valid = tok < (long long)d.batch * d.tokens;   // every lane stays for the shuffles
@@ -268,7 +263,6 @@ __device__ __forceinline__ void load_tile_async(float* dst, const float* plane, 
 __global__ void __launch_bounds__(SIM_THREADS)
 sim_argmax_planes_kernel(const tome_metric_desc_t d, const float* __restrict__ plane_a, const float* __restrict__ plane_b,
                          float* __restrict__ node_max, int32_t* __restrict__ node_idx, float* __restrict__ scores_out) {
-  pdl_prologue();
   extern __shared__ float4 sm4[];
   float* sm = reinterpret_cast<float*>(sm4);
   const int dpad = (d.dim + 3) & ~3, pitch = dpad + 4;
@@ -385,10 +379,6 @@ sim_argmax_planes_kernel(const tome_metric_desc_t d, const float* __restrict__ p
 // max / first arg max of tile j from tensor memory while tile j + 1 is being computed.  (A first version stored the six
 // operand chunks per row explicitly, 768 B per token: its 295 MB of L2 -> SM traffic per call, not the tensor pipe, set
 // its 93 us -- profiles/r02_sim_argmax_tc.md.)
-// Optional (tome_sim_argmax_set_tc(2), off by default): the a tiles of one batch element form a thread-block cluster (up to
-// 8 CTAs) and every b chunk is fetched from L2 by ONE of them and TMA-multicast into the ring slot of all.  Measured: no
-// gain (93 vs 89 us at B = 256, T = 536; 393 vs 390 us at T = 8192) -- after the three-chunk layout the kernel is bound by
-// the per-CTA latency chain (ncu: the epilogue warps wait for the first score tile, 25 % tensor pipe), not by L2 -> SM bytes.
 //   warp 4  TMA: the a tile's three chunks once (48 KB, resident), then the b tiles chunk by chunk through a 3-slot ring
 //   warp 5  MMA issuer: per b chunk h: a_h, a_m, a_l;  m: a_h, a_m;  l: a_h        warps 0..3  epilogue
 constexpr int SIMT_BM = 128, SIMT_BN = 128, SIMT_CHUNKS = 3, SIMT_SLOTS = 3, SIMT_ROW = 192;
@@ -400,7 +390,6 @@ constexpr int SIMT_THREADS = 192;
 __global__ void __launch_bounds__(256)
 metric_split64_kernel(const tome_metric_desc_t d, const __nv_bfloat16* __restrict__ src, __nv_bfloat16* __restrict__ plane_a,
                       __nv_bfloat16* __restrict__ plane_b) {
-  pdl_prologue();
   const long long tok = ((long long)blockIdx.x * 256 + threadIdx.x) >> 3;   // b * T + t
   const int sub = threadIdx.x & 7;
   const bool valid = tok < (long long)d.batch * d.tokens;   // every lane stays for the shuffles
@@ -451,7 +440,6 @@ template <typename T>
 __global__ void __launch_bounds__(256)
 metric_split_kernel(const tome_metric_desc_t d, const T* __restrict__ src, __nv_bfloat16* __restrict__ plane_a,
                     __nv_bfloat16* __restrict__ plane_b) {
-  pdl_prologue();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long tok = (long long)blockIdx.x * 8 + warp;   // b * T + t
   if (tok >= (long long)d.batch * d.tokens) return;
@@ -488,8 +476,7 @@ metric_split_kernel(const tome_metric_desc_t d, const T* __restrict__ src, __nv_
 
 __global__ void __launch_bounds__(SIMT_THREADS, 2)
 sim_argmax_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, const tome_metric_desc_t d,
-                     float* __restrict__ node_max, int32_t* __restrict__ node_idx, float* __restrict__ scores_out, const int csize) {
-  pdl_prologue();
+                     float* __restrict__ node_max, int32_t* __restrict__ node_idx, float* __restrict__ scores_out) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   uint8_t* s_a = smem;                                   // chunk c at c * 16 KB
@@ -510,7 +497,7 @@ sim_argmax_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_cons
     mbar_init(a_full, 1);
     for (int i = 0; i < SIMT_SLOTS; ++i) {
       mbar_init(&b_full[i], 1);
-      mbar_init(&b_empty[i], csize);   // one commit from the MMA issuer of every CTA of the cluster
+      mbar_init(&b_empty[i], 1);
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(&s_full[i], 1);
@@ -525,11 +512,8 @@ sim_argmax_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_cons
   if (warp == 5) tmem_alloc(tmem_slot, 256);
   tc_fence_before();
   __syncthreads();
-  if (csize > 1) cluster_sync_all();   // the peers' barriers exist before anything is multicast at them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  const uint32_t crank = csize > 1 ? cluster_ctarank() : 0u;
-  const uint16_t cmask = (uint16_t)((1u << csize) - 1u);
 
   if (warp == 4) {
     if (lane == 0) {
@@ -539,11 +523,9 @@ sim_argmax_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_cons
       for (int jt = 0; jt < n_bt; ++jt)
         for (int c = 0; c < SIMT_CHUNKS; ++c, ++item) {
           const int slot = item % SIMT_SLOTS;
-          mbar_wait(&b_empty[slot], ((item / SIMT_SLOTS) & 1) ^ 1);   // every CTA of the cluster has drained the slot
+          mbar_wait(&b_empty[slot], ((item / SIMT_SLOTS) & 1) ^ 1);
           mbar_expect_tx(&b_full[slot], SIMT_CHUNK_BYTES);
-          if (csize == 1) tma_load_3d(s_b + slot * SIMT_CHUNK_BYTES, &tm_b, &b_full[slot], c * 64, jt * SIMT_BN, b);
-          else if ((uint32_t)(item % csize) == crank)   // this chunk is ours to fetch, for everybody
-            tma_load_3d_mc(s_b + slot * SIMT_CHUNK_BYTES, &tm_b, &b_full[slot], c * 64, jt * SIMT_BN, b, cmask);
+          tma_load_3d(s_b + slot * SIMT_CHUNK_BYTES, &tm_b, &b_full[slot], c * 64, jt * SIMT_BN, b);
         }
     }
   } else if (warp == 5) {
@@ -569,8 +551,7 @@ sim_argmax_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_cons
               umma_bf16(td, make_smem_desc(aa + k * 32, 16, 1024), make_smem_desc(ab + k * 32, 16, 1024), idesc,
                         (c > 0 || ca > 0 || k > 0) ? 1u : 0u);
           }
-          if (csize == 1) umma_commit(&b_empty[slot]);
-          else umma_commit_mc(&b_empty[slot], cmask);   // tell every producer of the cluster
+          umma_commit(&b_empty[slot]);
         }
         umma_commit(&s_full[jt & 1]);
       }
@@ -620,7 +601,6 @@ sim_argmax_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_cons
   }
   tc_fence_before();
   __syncthreads();
-  if (csize > 1) cluster_sync_all();   // peers may still multicast into this CTA's ring / arrive on its barriers
   if (warp == 5) {
     tc_fence_after();
     tmem_dealloc(tmem_base, 256);
@@ -667,7 +647,6 @@ __host__ __device__ inline int sel_pow2(int n) { int p = 1; while (p < n) p <<= 
 __global__ void __launch_bounds__(SEL_THREADS)
 select_topr_kernel(const tome_plan_shape_t s, const float* __restrict__ node_max, const int32_t* __restrict__ node_idx,
                    const tome_plan_t p) {
-  pdl_prologue();
   extern __shared__ __align__(8) unsigned char sel_raw[];
   const int T = s.tokens, r = s.r;
   const int ta = (T + 1) / 2, tb = T / 2;
@@ -779,11 +758,7 @@ extern "C" int tome_clamp_r(int tokens, int r, int class_token, int distill_toke
   return r > 0 ? r : 0;
 }
 
-// 1 (default): the tensor-core path (split-bf16 K = 384 contraction) whenever the input allows it; 0: fp32 CUDA-core planes.
-// Process-wide tuning aid (A/B measurements, cross-check), not part of the public header.
-static int g_sim_tc = 1, g_sim_mc = 0;
-extern "C" void tome_sim_argmax_set_tc(int on) { g_sim_tc = on ? 1 : 0; g_sim_mc = on == 2 ? 1 : 0; }   // 2: tensor cores + cluster multicast of the b rows
-
+// the tensor-core path (split-bf16 K = 384 contraction) whenever the input allows it, else fp32 CUDA-core planes
 static bool sim_tc_eligible(const tome_metric_desc_t* d) { return d->dim == 64; }
 static bool sim_fast64(const tome_metric_desc_t* d, const void* src) {   // 128-bit loads, 8 lanes per row
   return d->dtype == TOME_BF16 && d->dim == 64 && d->token_stride % 8 == 0 && d->batch_stride % 8 == 0 &&
@@ -819,7 +794,7 @@ extern "C" int tome_sim_argmax(const tome_metric_desc_t* d, const void* src, flo
                "sim_argmax: workspace must be 16-byte aligned and hold %zu bytes (got %zu)", tome_sim_argmax_workspace_bytes(d),
                workspace_bytes);
     ProfScope prof(PROF_SIM, 2.0 * d->batch * ta * (double)tb * d->dim, 2, stream);
-    if (g_sim_tc && sim_tc_eligible(d)) {
+    if (sim_tc_eligible(d)) {
       __nv_bfloat16* pa = reinterpret_cast<__nv_bfloat16*>(workspace);
       __nv_bfloat16* pb = pa + (size_t)d->batch * ta * SIMT_ROW;
       const long long toks = (long long)d->batch * d->tokens;
@@ -835,26 +810,8 @@ extern "C" int tome_sim_argmax(const tome_metric_desc_t* d, const void* src, flo
       if (int rc = make_tmap_3d_bf16(&tma_b, pb, SIMT_ROW, tb, d->batch, SIMT_ROW, (uint64_t)tb * SIMT_ROW, SIMT_BN)) return rc;
       static DynSmemOnce once;
       TOME_CUDA(ensure_dyn_smem(sim_argmax_tc_kernel, SIMT_SMEM, once));
-      const int n_at = ceil_div(ta, SIMT_BM);
-      int csize = 1;   // the largest cluster size <= 8 that divides the number of a tiles
-      for (int c = 8; c > 1; --c)
-        if (n_at % c == 0) { csize = c; break; }
-      if (!g_sim_mc) csize = 1;
-      cudaLaunchConfig_t cfg;
-      memset(&cfg, 0, sizeof(cfg));
-      cfg.gridDim = dim3(n_at, d->batch);
-      cfg.blockDim = dim3(SIMT_THREADS);
-      cfg.dynamicSmemBytes = SIMT_SMEM;
-      cfg.stream = stream;
-      cudaLaunchAttribute attr[2];
-      cfg.attrs = attr;
-      cfg.numAttrs = pdl_attr(&attr[0]);
-      cudaLaunchAttribute& ca = attr[cfg.numAttrs++];
-      ca.id = cudaLaunchAttributeClusterDimension;
-      ca.val.clusterDim.x = csize;
-      ca.val.clusterDim.y = 1;
-      ca.val.clusterDim.z = 1;
-      TOME_CUDA(cudaLaunchKernelEx(&cfg, sim_argmax_tc_kernel, tma_a, tma_b, *d, node_max, node_idx, scores_out, csize));
+      TOME_CUDA(launch_k(sim_argmax_tc_kernel, dim3(ceil_div(ta, SIMT_BM), d->batch), SIMT_THREADS, SIMT_SMEM, stream, tma_a, tma_b, *d,
+                         node_max, node_idx, scores_out));
       return TOME_OK;
     }
     float* plane_a = reinterpret_cast<float*>(workspace);

@@ -46,7 +46,6 @@ merge_fwd_kernel(const tome_merge_shape_t s, const tome_plan_t p, const T* __res
                  const float* __restrict__ size, T* __restrict__ x_out, float* __restrict__ size_out,
                  const uint8_t* __restrict__ gid, const int32_t* __restrict__ pos, uint8_t* __restrict__ gid_out,
                  int32_t* __restrict__ pos_out) {
-  pdl_prologue();
   constexpr int N = Vec<T>::N;
   const int Tn = s.tokens, r = s.r, C = s.channels;
   const int ta = (Tn + 1) / 2, tb = Tn / 2, n_unm = ta - r, To = Tn - r;
@@ -135,7 +134,6 @@ merge_fwd_bulk_kernel(const tome_merge_shape_t s, const tome_plan_t p, const T* 
                       const float* __restrict__ size, T* __restrict__ x_out, float* __restrict__ size_out,
                       const uint8_t* __restrict__ gid, const int32_t* __restrict__ pos, uint8_t* __restrict__ gid_out,
                       int32_t* __restrict__ pos_out, int rows_per_cta) {
-  pdl_prologue();
   constexpr int N = Vec<T>::N;
   extern __shared__ __align__(128) uint8_t smem_merge[];
   const int Tn = s.tokens, r = s.r, C = s.channels;
@@ -251,13 +249,10 @@ merge_fwd_bulk_kernel(const tome_merge_shape_t s, const tome_plan_t p, const T* 
   }
 }
 
-static int g_merge_rows_override = 0;  // tuning aid for scripts/bench_kernels.py (0 = choose automatically)
-
 template <typename T, bool WAVG>
 __global__ void __launch_bounds__(MERGE_THREADS)
 merge_bwd_kernel(const tome_merge_shape_t s, const int32_t* __restrict__ row_map, const float* __restrict__ size,
                  const float* __restrict__ size_out, const T* __restrict__ dy, T* __restrict__ dx) {
-  pdl_prologue();
   constexpr int N = Vec<T>::N;
   const int Tn = s.tokens, C = s.channels, To = Tn - s.r;
   const int vpr = C / N;
@@ -323,7 +318,7 @@ extern "C" int tome_merge_fwd(const tome_merge_shape_t* s, const tome_plan_t* pl
   const int row_bytes = s->channels * (int)esz;
   if (row_bytes <= 32768 && s->batch <= 65535) {
     // bulk-copy path: rows * row_bytes ~ 24 KB per CTA, so 8 CTAs (~190 KB in flight) fit one SM
-    int rows = g_merge_rows_override > 0 ? g_merge_rows_override : 24576 / row_bytes;
+    int rows = 24576 / row_bytes;
     if (rows < 1) rows = 1;
     if (rows > 128) rows = 128;
     if (rows > s->tokens - s->r) rows = s->tokens - s->r;
@@ -354,9 +349,6 @@ extern "C" int tome_merge_fwd(const tome_merge_shape_t* s, const tome_plan_t* pl
   TOME_CUDA(cudaGetLastError());
   return TOME_OK;
 }
-
-/* tuning aid (not part of the public header): force the bulk kernel's rows per CTA; 0 restores the default */
-extern "C" void tome_merge_set_rows_per_cta(int rows) { g_merge_rows_override = rows; }
 
 extern "C" int tome_merge_bwd(const tome_merge_shape_t* s, const tome_plan_t* plan, const float* size,
                               const float* size_out, const void* dy, void* dx, void* stream_) {

@@ -16,7 +16,6 @@ __device__ __forceinline__ uint4 pack8m(const float (&f)[8]) {
 template <bool X_F32>
 __global__ void add_pos_kernel(long long n8, long long tc8, const void* __restrict__ x, const float* __restrict__ pe,
                                __nv_bfloat16* __restrict__ y) {
-  pdl_prologue();
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n8; i += (long long)gridDim.x * blockDim.x) {
     float f[8];
     if (X_F32) {
@@ -33,7 +32,6 @@ __global__ void add_pos_kernel(long long n8, long long tc8, const void* __restri
 }
 
 __global__ void pos_bwd_kernel(int B, long long tc8, const __nv_bfloat16* __restrict__ dy, float* __restrict__ dpe) {
-  pdl_prologue();
   const long long j = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (j >= tc8) return;
   float a[8];
@@ -58,7 +56,6 @@ struct ChainArgs {
 };
 __global__ void chain_kernel(int B, int layers, const ChainArgs a, const int32_t* __restrict__ readout_idx, int n,
                              int32_t* __restrict__ origin) {
-  pdl_prologue();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * n) return;
   const int b = i / n;
@@ -73,7 +70,6 @@ __global__ void __launch_bounds__(256)
 readout_mse_kernel(int B, int T, int C, int n, const __nv_bfloat16* __restrict__ x, const int32_t* __restrict__ origin,
                    const float* __restrict__ target, float* __restrict__ loss, __nv_bfloat16* __restrict__ dx,
                    float* __restrict__ out) {
-  pdl_prologue();
   __shared__ float red[8];
   const int b = blockIdx.x;
   const float gscale = 2.0f / ((float)B * (float)n * (float)C);
@@ -99,7 +95,6 @@ readout_mse_kernel(int B, int T, int C, int n, const __nv_bfloat16* __restrict__
   }
 }
 __global__ void loss_final_kernel(int B, float inv_count, float* loss) {
-  pdl_prologue();
   float t = 0.f;
   for (int b = 0; b < B; ++b) t += loss[1 + b];
   loss[0] = t * inv_count;
@@ -108,7 +103,6 @@ __global__ void loss_final_kernel(int B, float inv_count, float* loss) {
 __global__ void adamw_kernel(long long n, float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                              float* __restrict__ v, __nv_bfloat16* __restrict__ w16, float lr, float b1, float b2, float eps,
                              float wd, float gs, float bc1, float bc2) {
-  pdl_prologue();
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     const float gi = g[i] * gs;
     const float mi = b1 * m[i] + (1.f - b1) * gi;
@@ -123,7 +117,6 @@ __global__ void adamw_kernel(long long n, float* __restrict__ p, const float* __
 }
 
 __global__ void cast_kernel(long long n, const float* __restrict__ s, __nv_bfloat16* __restrict__ d) {
-  pdl_prologue();
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
     d[i] = __float2bfloat16(s[i]);
 }

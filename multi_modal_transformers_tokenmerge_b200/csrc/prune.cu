@@ -27,7 +27,6 @@ __device__ __forceinline__ bool topk_before(float vj, int j, float vi, int i) {
 __global__ void __launch_bounds__(PRUNE_THREADS)
 topk_prune_kernel(const tome_prune_desc_t d, const uint8_t* __restrict__ emb, const float* __restrict__ score,
                   uint8_t* __restrict__ out, int32_t* __restrict__ ids) {
-  pdl_prologue();
   extern __shared__ float prune_sm[];
   const int s = blockIdx.x, b = blockIdx.y;
   const int start = d.set_start[s], n = d.set_n[s], k = d.set_k[s];
@@ -82,7 +81,6 @@ __device__ __forceinline__ unsigned long long prune_key(float v, int i) {
 
 __global__ void __launch_bounds__(PRUNE_SORT_THREADS)
 topk_sort_kernel(const tome_prune_desc_t d, const float* __restrict__ score, int32_t* __restrict__ ids) {
-  pdl_prologue();
   extern __shared__ __align__(8) unsigned char prune_sort_raw[];
   unsigned long long* keys = reinterpret_cast<unsigned long long*>(prune_sort_raw);
   const int s = blockIdx.x, b = blockIdx.y, tid = threadIdx.x, nt = blockDim.x;
@@ -122,7 +120,6 @@ topk_sort_kernel(const tome_prune_desc_t d, const float* __restrict__ score, int
 __global__ void __launch_bounds__(256)
 prune_gather_kernel(long long n_vec, int T, int K, int vpr, const int32_t* __restrict__ ids, const uint4* __restrict__ emb,
                     uint4* __restrict__ out) {
-  pdl_prologue();
   for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n_vec; i += (long long)gridDim.x * 256) {
     const long long rowg = i / vpr;           // b * K + j
     const int v = (int)(i - rowg * vpr);
@@ -136,7 +133,6 @@ prune_gather_kernel(long long n_vec, int T, int K, int vpr, const int32_t* __res
 __global__ void prune_row_map_kernel(int B, int T, int K, const int32_t* __restrict__ ids, const uint8_t* __restrict__ gid,
                                      const int32_t* __restrict__ pos, int32_t* __restrict__ row_map, uint8_t* __restrict__ gid_out,
                                      int32_t* __restrict__ pos_out) {
-  pdl_prologue();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (long long)B * K) return;
   const int b = (int)(i / K), j = (int)(i - (long long)b * K);
@@ -150,7 +146,6 @@ __global__ void prune_row_map_kernel(int B, int T, int K, const int32_t* __restr
 __global__ void __launch_bounds__(256)
 prune_bwd_kernel(long long n_vec, int T, int K, int vpr, const int32_t* __restrict__ row_map, const uint4* __restrict__ dy,
                  uint4* __restrict__ dx) {
-  pdl_prologue();
   for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n_vec; i += (long long)gridDim.x * 256) {
     const long long rowg = i / vpr;
     const int v = (int)(i - rowg * vpr);

@@ -301,7 +301,6 @@ static StackLayout make_layout(const tome_stack_cfg_t* c, void* workspace) {
 
 __global__ void broadcast_groups_kernel(int B, int T, const uint8_t* __restrict__ gid, const int32_t* __restrict__ pos,
                                         uint8_t* __restrict__ gid_out, int32_t* __restrict__ pos_out) {
-  pdl_prologue();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < B * T) {
     gid_out[i] = gid[i % T];

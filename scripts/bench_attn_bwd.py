@@ -3,8 +3,7 @@ import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from multi_modal_transformers_tokenmerge_b200 import ops
-from bench_attn_variants import inputs
-from bench_kernels import timeit
+from bench_kernels import attn_inputs as inputs, timeit
 drop = dict(dropout_rate=0.1, dropout_seed=3, dropout_site=5)
 for (B, T, H) in [(256, 536, 6), (256, 440, 6), (256, 392, 6), (256, 536, 12)]:
     q, k, v, kw = inputs(B, T, H)

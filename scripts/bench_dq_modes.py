@@ -1,5 +1,4 @@
 """Backward attention with dQ from stored dS^T tiles (mode 1) against the recomputing dQ kernel (mode 0) at several lengths."""
-import ctypes
 import os
 import sys
 
@@ -9,8 +8,6 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from multi_modal_transformers_tokenmerge_b200 import _lib, ops  # noqa: E402
 
 setter = _lib.lib().tome_attention_set_dq_from_ds
-setter.argtypes = [ctypes.c_int]
-setter.restype = None
 for B, T, H in ((256, 536, 6), (32, 2080, 12), (20, 3072, 12), (16, 4096, 12), (8, 6144, 12)):
     qkv = torch.randn(B, T, 3, H, 64, device="cuda").bfloat16()
     q, k, v = qkv[:, :, 0], qkv[:, :, 1], qkv[:, :, 2]

@@ -10,6 +10,7 @@ import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from multi_modal_transformers_tokenmerge_b200 import ops  # noqa: E402
+from multi_modal_transformers_tokenmerge_b200.tokenizers.token_sequencer import sequence_groups  # noqa: E402
 
 PEAKS = json.load(open(os.path.join(os.path.dirname(__file__), "..", "MEASURED_PEAKS.json"))) if os.path.exists(
     os.path.join(os.path.dirname(__file__), "..", "MEASURED_PEAKS.json")) else {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0}
@@ -36,6 +37,17 @@ def timeit(fn, iters=10, warmup=3, flush=True):
     return tot / iters * 1e-3
 
 
+def attn_inputs(B, T, H):
+    """q, k, v of B x T x H heads of 64 and the stack's block-causal group mask in a scrambled token order (as after a merge)."""
+    qkv = torch.randn(B, T, 3, H, 64, device="cuda").bfloat16()
+    n_img = (T - 16) // 2 - 4
+    g1, p1, allow, _ = sequence_groups(f"[TaskDescriptionPrefix{{16}}] [Image{{{n_img}}};Readout{{4}}]*2")
+    rng = np.random.default_rng(0)
+    kw = dict(size=torch.ones(B, T, device="cuda"), gid=torch.tensor(np.stack([rng.permutation(g1) for _ in range(B)])).cuda(),
+              pos=torch.tensor(np.broadcast_to(p1, (B, len(g1))).copy()).cuda(), allow=torch.tensor(allow).cuda())
+    return qkv[:, :, 0], qkv[:, :, 1], qkv[:, :, 2], kw
+
+
 def bench_merge():
     for (B, T, C, r) in [(256, 536, 384, 16), (256, 536, 768, 32), (32, 4096, 1024, 1024), (16, 8192, 768, 2048), (128, 1024, 768, 128)]:
         x = torch.randn(B, T, C, device="cuda").bfloat16()
@@ -45,12 +57,8 @@ def bench_merge():
         size = torch.ones(B, T, device="cuda")
         ta = (T + 1) // 2
         by = B * (T * C * 2 + 4 * T + 4 * (ta + r) + (T - r) * C * 2 + 4 * (T - r))
-        from multi_modal_transformers_tokenmerge_b200 import _lib
-        for rows in ([0] if "sweep" not in sys.argv else [0, 8, 16, 32, 48, 64]):
-            _lib.lib().tome_merge_set_rows_per_cta(rows)
-            t = timeit(lambda: ops.merge_fwd(plan, x, size, 1))
-            print(f"merge_fwd  B{B} T{T} C{C} r{r} rows/cta {rows}: {t*1e6:8.1f} us  {by/t/1e9:7.1f} GB/s  frac {by/t/1e9/PEAKS['hbm_gbs']:.3f}")
-        _lib.lib().tome_merge_set_rows_per_cta(0)
+        t = timeit(lambda: ops.merge_fwd(plan, x, size, 1))
+        print(f"merge_fwd  B{B} T{T} C{C} r{r}: {t*1e6:8.1f} us  {by/t/1e9:7.1f} GB/s  frac {by/t/1e9/PEAKS['hbm_gbs']:.3f}")
         size2 = torch.randint(1, 4, (B, T), device="cuda").float()   # sizes != 1: every row takes the arithmetic path
         t = timeit(lambda: ops.merge_fwd(plan, x, size2, 1))
         print(f"merge_fwd  (all rows patched) : {t*1e6:8.1f} us  {by/t/1e9:7.1f} GB/s  frac {by/t/1e9/PEAKS['hbm_gbs']:.3f}")
@@ -65,29 +73,11 @@ def bench_merge():
         H = C // 64   # the stack's call: keys read in place from the packed bf16 qkv buffer, mean over heads
         qkv = torch.randn(B, T, 3, H, 64, device="cuda").bfloat16()
         kwm = dict(heads=H, dim=64, batch=B, tokens=T, batch_stride=T * 3 * H * 64, token_stride=3 * H * 64, head_stride=64, offset_elems=H * 64)
-        ref = None
-        for tc in (0, 2, 1):
-            _lib.lib().tome_sim_argmax_set_tc(tc)
-            t = timeit(lambda: ops.sim_argmax(qkv, **kwm))
-            nm2, ni2, _ = ops.sim_argmax(qkv, **kwm)
-            if ref is None:
-                ref = (nm2.clone(), ni2.clone())
-            same = (ni2 == ref[1]).float().mean().item()
-            print(f"   sim_argmax from packed bf16 keys, {H} heads, {('fp32 CUDA cores', 'tensor cores', 'tensor cores + cluster multicast')[tc]}: {t*1e6:8.1f} us"
-                  f"  (arg max equal to fp32 path: {same:.5f}, max |node_max diff| {(nm2 - ref[0]).abs().max().item():.2e})")
-        _lib.lib().tome_sim_argmax_set_tc(1)
+        t = timeit(lambda: ops.sim_argmax(qkv, **kwm))
+        print(f"   sim_argmax from packed bf16 keys, {H} heads: {t*1e6:8.1f} us")
 
 
 def bench_gemm():
-    from multi_modal_transformers_tokenmerge_b200 import _lib
-    for pair in (1, 0):
-        _lib.lib().tome_gemm_set_pair_mma(pair)
-        print("cta_group::2 pair MMA:", "on" if pair else "off (two 128-row MMAs, multicast B)")
-        _bench_gemm()
-    _lib.lib().tome_gemm_set_pair_mma(1)
-
-
-def _bench_gemm():
     for (m, n, k, bmn) in [(137216, 1152, 384, 1), (137216, 384, 384, 1), (133120, 1536, 384, 1), (133120, 384, 1536, 1),
                            (137216, 2304, 768, 1), (129024, 3072, 768, 1), (129024, 768, 3072, 1), (8192, 8192, 8192, 0)]:
         a = torch.randn(m, k, device="cuda").bfloat16()
@@ -147,15 +137,6 @@ def bench_attn():
 
 
 def bench_ln():
-    from multi_modal_transformers_tokenmerge_b200 import _lib
-    for mask in (0, 3):
-        _lib.lib().tome_ln_set_smem_path(mask)
-        print("shared-memory slab path:", "on" if mask else "off")
-        _bench_ln()
-    _lib.lib().tome_ln_set_smem_path(3)
-
-
-def _bench_ln():
     for (B, T, C) in [(256, 536, 384), (256, 536, 768)]:
         x = torch.randn(B, T, C, device="cuda").bfloat16()
         g = torch.ones(C, device="cuda")
@@ -172,6 +153,6 @@ def _bench_ln():
 
 
 if __name__ == "__main__":
-    which = [a for a in sys.argv[1:] if a != "sweep"] or ["merge", "gemm", "attn", "ln"]
+    which = sys.argv[1:] or ["merge", "gemm", "attn", "ln"]
     for w in which:
         globals()["bench_" + w]()

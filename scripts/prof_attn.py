@@ -7,7 +7,7 @@ import torch
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from multi_modal_transformers_tokenmerge_b200 import ops  # noqa: E402
-from bench_attn_variants import inputs  # noqa: E402
+from bench_kernels import attn_inputs as inputs  # noqa: E402
 
 T = int(sys.argv[1]) if len(sys.argv) > 1 else 536
 H = int(sys.argv[2]) if len(sys.argv) > 2 else 6

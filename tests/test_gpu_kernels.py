@@ -817,11 +817,8 @@ def test_attention_bwd_dq_paths_agree(ops, T, rate):
     """dQ as a batched GEMM over the dS^T tiles stored by the dK/dV kernel (the default up to 3 072 tokens) against the
     recomputing dQ kernel: same bf16 dS (both form it from the bf16-rounded P, in the same operation order), same accumulation
     order, so dq must agree bit for bit; dk / dv come from the same kernel in both modes."""
-    import ctypes
     from multi_modal_transformers_tokenmerge_b200 import _lib as L
     setter = L.lib().tome_attention_set_dq_from_ds
-    setter.argtypes = [ctypes.c_int]
-    setter.restype = None
     rng = np.random.default_rng(T)
     B, H, D = 4, 3, 64
     qkv = dev(rng.standard_normal((B, T, 3, H, D)).astype(np.float32), torch.bfloat16)
@@ -852,7 +849,6 @@ def test_gemm_epilogue_column_sums(ops, m, n, k):
     pass over the tensor): reduced over the tiles they must equal the column sums of the output it wrote -- rows past M
     excluded even when the epilogue adds a bias to them -- for the gated data gradient, the plain one and a forward layer, in
     every CTA mode; asking for them must not change the output; and the result is reproducible bit for bit."""
-    import ctypes
     from multi_modal_transformers_tokenmerge_b200 import _lib as L
     rng = np.random.default_rng(m + n + k)
     A = dev(rng.standard_normal((m, k)).astype(np.float32) * 0.5, torch.bfloat16)
@@ -892,11 +888,8 @@ def test_attention_bwd_bias_partials(ops, T, H, rate, from_ds):
     """The attention-backward epilogues can leave the column sums of every 128-token tile of dq / dk / dv (the packed q/k/v
     projection's bias gradient): reduced over the tiles they equal the column sums of the gradients written, on both dQ paths,
     and asking for them changes no gradient bit."""
-    import ctypes
     from multi_modal_transformers_tokenmerge_b200 import _lib as L
     setter = L.lib().tome_attention_set_dq_from_ds
-    setter.argtypes = [ctypes.c_int]
-    setter.restype = None
     rng = np.random.default_rng(T + H)
     B, D = 3, 64
     qkv = dev(rng.standard_normal((B, T, 3, H, D)).astype(np.float32), torch.bfloat16)
