@@ -704,8 +704,6 @@ attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
 
 using namespace tome;
 
-static size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
-
 static size_t bwd_pad_elems(const tome_attn_desc_t* d) {
   return (size_t)d->batch * d->heads * (size_t)(((d->tokens + 63) / 64) * 64);
 }
@@ -811,7 +809,7 @@ static inline size_t ds_buffer_bytes(const tome_attn_desc_t* d) {
   // [B*H][T keys][T queries, rows pitched to 16 bytes]: the TMA stores clip the tiles' rows / columns past T and the loads
   // zero-fill them, so no padding is written or read (T = 536: 575 KB per head instead of the 737 KB of whole 128 x 64 tiles)
   const size_t tq = ((size_t)d->tokens + 7) / 8 * 8, tk = (size_t)d->tokens;
-  return align256((size_t)d->batch * d->heads * tq * tk * 2);
+  return (size_t)d->batch * d->heads * tq * tk * 2;
 }
 static inline bool dq_from_ds(const tome_attn_desc_t* d) {
   if (d->head_dim != AB_D) return false;
@@ -820,11 +818,28 @@ static inline bool dq_from_ds(const tome_attn_desc_t* d) {
 
 extern "C" void tome_attention_set_dq_from_ds(int mode) { g_attn_dq_from_ds = mode < 0 ? -1 : (mode ? 1 : 0); }
 
+struct BwdWs {
+  uint8_t* meta;        // per-tile metadata (launch_attn_meta)
+  float *delta, *lse2;  // [B, H, ceil64(T)] each (attn_bwd_prep_kernel)
+  uint8_t* bits;        // dropout keep bits, both tilings (launch_attn_dropbits), only with dropout
+  uint8_t* ds;          // dS^T (ds_buffer_bytes), only when dQ is the GEMM over it
+  size_t total;
+};
+static BwdWs bwd_ws(const tome_attn_desc_t* d, void* base) {
+  Bump b{reinterpret_cast<uint8_t*>(base)};
+  BwdWs w;
+  w.meta = b.take<uint8_t>(attn_meta_bytes(d->batch, d->tokens));
+  w.delta = b.take<float>(bwd_pad_elems(d));
+  w.lse2 = b.take<float>(bwd_pad_elems(d));
+  w.bits = b.take<uint8_t>(d->dropout_rate > 0.f ? attn_dropbits_bytes(d->tokens) : 0);
+  w.ds = b.take<uint8_t>(dq_from_ds(d) ? ds_buffer_bytes(d) : 0);
+  w.total = b.total();
+  return w;
+}
+
 extern "C" size_t tome_attention_bwd_workspace_bytes(const tome_attn_desc_t* d) {
   if (!d || d->batch <= 0 || d->tokens <= 0 || d->heads <= 0) return 0;
-  return align256(attn_meta_bytes(d->batch, d->tokens)) + 2 * align256(bwd_pad_elems(d) * sizeof(float)) +
-         align256(d->dropout_rate > 0.f ? attn_dropbits_bytes(d->tokens) : 0) +
-         (dq_from_ds(d) ? ds_buffer_bytes(d) : 0);
+  return bwd_ws(d, nullptr).total;
 }
 
 extern "C" int tome_attention_bwd(const tome_attn_desc_t* d, const tome_attn_grad_strides_t* gs, const void* q, const void* k,
@@ -843,42 +858,37 @@ extern "C" int tome_attention_bwd(const tome_attn_desc_t* d, const tome_attn_gra
   }
   TOME_CHECK(workspace != nullptr, TOME_ERR_INVALID, "attention_bwd: null workspace");
   TOME_CHECK(((uintptr_t)workspace & 255) == 0, TOME_ERR_INVALID, "attention_bwd: workspace must be 256-byte aligned");
-  TOME_CHECK(workspace_bytes >= tome_attention_bwd_workspace_bytes(d), TOME_ERR_INVALID,
-             "attention_bwd: workspace too small (%zu < %zu, see tome_attention_bwd_workspace_bytes)", workspace_bytes,
-             tome_attention_bwd_workspace_bytes(d));
+  const BwdWs ws = bwd_ws(d, workspace);
+  TOME_CHECK(workspace_bytes >= ws.total, TOME_ERR_INVALID,
+             "attention_bwd: workspace too small (%zu < %zu, see tome_attention_bwd_workspace_bytes)", workspace_bytes, ws.total);
   const long long st[8] = {gs->dq_batch_stride, gs->dq_token_stride, gs->dk_batch_stride, gs->dk_token_stride,
                            gs->dv_batch_stride, gs->dv_token_stride, gs->do_batch_stride, gs->do_token_stride};
   for (int i = 0; i < 8; ++i) TOME_CHECK(st[i] % 8 == 0, TOME_ERR_INVALID, "attention_bwd: strides must be multiples of 8");
   const int B = d->batch, T = d->tokens, H = d->heads;
   ProfScope prof(PROF_ATTN_BWD, 10.0 * d->batch * d->heads * (double)d->tokens * d->tokens * d->head_dim, 4, stream);
   const int Tp = ((T + 63) / 64) * 64;
-  uint8_t* meta = reinterpret_cast<uint8_t*>(workspace);
-  float* delta = reinterpret_cast<float*>(meta + align256(attn_meta_bytes(B, T)));
-  float* lse2 = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(delta) + align256(bwd_pad_elems(d) * sizeof(float)));
-  if (int rc = launch_attn_meta(B, T, d->gid, d->pos, d->allow, d->num_groups, d->size, meta, stream)) return rc;
+  if (int rc = launch_attn_meta(B, T, d->gid, d->pos, d->allow, d->num_groups, d->size, ws.meta, stream)) return rc;
   TOME_CHECK(d->dropout_rate >= 0.f && d->dropout_rate < 1.f, TOME_ERR_INVALID, "attention_bwd: dropout_rate must be in [0, 1)");
   const uint8_t *keep_q = nullptr, *keep_k = nullptr;
   float inv_keep = 1.0f;
   if (d->dropout_rate > 0.f) {  // the same (seed, site) as the forward call regenerates the same mask
-    uint8_t* bits = reinterpret_cast<uint8_t*>(lse2) + align256(bwd_pad_elems(d) * sizeof(float));
-    if (int rc = launch_attn_dropbits(T, d->dropout_rate, d->dropout_seed, d->dropout_site, bits, stream)) return rc;
-    keep_q = bits;
-    keep_k = bits + attn_dropbits_bytes(T) / 2;
-    const uint32_t th = (uint32_t)(d->dropout_rate * 65536.0f + 0.5f);
-    inv_keep = 1.0f / (1.0f - (float)th / 65536.0f);
+    if (int rc = launch_attn_dropbits(T, d->dropout_rate, d->dropout_seed, d->dropout_site, ws.bits, stream)) return rc;
+    keep_q = ws.bits;
+    keep_k = ws.bits + attn_dropbits_bytes(T) / 2;
+    inv_keep = make_dropout(d->dropout_rate, d->dropout_seed, d->dropout_site).inv_keep;
   }
   {
     const long long total = (long long)B * Tp * H * 8;
     launch_k(attn_bwd_prep_kernel, (unsigned)((total + 255) / 256), 256, 0, stream, 
         B, T, Tp, H, reinterpret_cast<const __nv_bfloat16*>(out), d->o_batch_stride, d->o_token_stride,
-        reinterpret_cast<const __nv_bfloat16*>(dout), gs->do_batch_stride, gs->do_token_stride, lse, delta, lse2);
+        reinterpret_cast<const __nv_bfloat16*>(dout), gs->do_batch_stride, gs->do_token_stride, lse, ws.delta, ws.lse2);
     TOME_CUDA(cudaGetLastError());
   }
   const uint64_t hd = (uint64_t)H * d->head_dim;
   AttnBwdParams p;
   p.batch = B; p.tokens = T; p.heads = H; p.tp = Tp;
   p.scale = d->scale; p.scale_log2 = d->scale * 1.4426950408889634f;
-  p.gid = d->gid; p.pos = d->pos; p.meta = meta; p.size = d->size; p.lse2 = lse2; p.delta = delta;
+  p.gid = d->gid; p.pos = d->pos; p.meta = ws.meta; p.size = d->size; p.lse2 = ws.lse2; p.delta = ws.delta;
   p.keep_q = keep_q; p.keep_k = keep_k; p.inv_keep = inv_keep;
   const bool from_ds = dq_from_ds(d);
   p.store_ds = from_ds ? 1 : 0;
@@ -886,15 +896,11 @@ extern "C" int tome_attention_bwd(const tome_attn_desc_t* d, const tome_attn_gra
   p.cs_q = gs->bias_q_col; p.cs_k = gs->bias_k_col; p.cs_v = gs->bias_v_col;
   p.n_t128 = ceil_div(T, 128);
 
-  // dS^T [B*H][ceil128(T) keys][ceil64(T) queries] bf16, after the (possibly absent) dropout bit tilings
-  uint8_t* ds_buf = reinterpret_cast<uint8_t*>(lse2) + align256(bwd_pad_elems(d) * sizeof(float)) +
-                    align256(d->dropout_rate > 0.f ? attn_dropbits_bytes(T) : 0);
   const uint64_t ds_tq = ((uint64_t)T + 7) / 8 * 8, ds_tk = (uint64_t)T;   // row pitch, rows (see ds_buffer_bytes)
   CUtensorMap tds_store, tds_load;
   if (from_ds) {
-
-    if (int rc = make_tmap_3d_bf16(&tds_store, ds_buf, (uint64_t)T, ds_tk, (uint64_t)B * H, ds_tq, ds_tq * ds_tk, DKV_BK)) return rc;
-    if (int rc = make_tmap_3d_bf16(&tds_load, ds_buf, (uint64_t)T, ds_tk, (uint64_t)B * H, ds_tq, ds_tq * ds_tk, DQG_BK)) return rc;
+    if (int rc = make_tmap_3d_bf16(&tds_store, ws.ds, (uint64_t)T, ds_tk, (uint64_t)B * H, ds_tq, ds_tq * ds_tk, DKV_BK)) return rc;
+    if (int rc = make_tmap_3d_bf16(&tds_load, ws.ds, (uint64_t)T, ds_tk, (uint64_t)B * H, ds_tq, ds_tq * ds_tk, DQG_BK)) return rc;
   } else {
     memset(&tds_store, 0, sizeof(tds_store));
   }

@@ -507,11 +507,7 @@ int launch_attn_dropbits(int T, float rate, uint64_t seed, uint32_t site, uint8_
   TOME_CHECK(bits != nullptr && ((uintptr_t)bits & 15) == 0, TOME_ERR_INVALID, "attention: dropout workspace must be 16-byte aligned");
   TOME_CHECK(rate > 0.f && rate < 1.f, TOME_ERR_INVALID, "attention: dropout_rate must be in [0, 1)");
   const int n128 = (T + 127) / 128, n64 = (T + 63) / 64;
-  DropoutCfg d;
-  d.thresh16 = (uint32_t)(rate * 65536.0f + 0.5f);
-  d.inv_keep = 1.0f / (1.0f - (float)d.thresh16 / 65536.0f);
-  d.seed_lo = (uint32_t)seed; d.seed_hi = (uint32_t)(seed >> 32);
-  d.site = site;
+  const DropoutCfg d = make_dropout(rate, seed, site);
   uint32_t* kq = reinterpret_cast<uint32_t*>(bits);
   uint32_t* kk = kq + (size_t)n128 * n64 * (ATTN_DROP_TILE_BYTES / 4);
   const long long threads = (long long)n128 * 128 * n128 * 4;
@@ -544,14 +540,23 @@ int check_attn_desc(const tome_attn_desc_t* d, const char* who) {
 }
 }  // namespace tome
 
-static size_t fwd_ws_bytes(const tome_attn_desc_t* d) {
-  const size_t meta = (attn_meta_bytes(d->batch, d->tokens) + 255) & ~size_t(255);
-  return meta + (d->dropout_rate > 0.f ? attn_dropbits_bytes(d->tokens) : 0);
+struct FwdWs {
+  uint8_t* meta;  // per-tile metadata (launch_attn_meta)
+  uint8_t* bits;  // dropout keep bits (launch_attn_dropbits), only with dropout
+  size_t total;
+};
+static FwdWs fwd_ws(const tome_attn_desc_t* d, void* base) {
+  Bump b{reinterpret_cast<uint8_t*>(base)};
+  FwdWs w;
+  w.meta = b.take<uint8_t>(attn_meta_bytes(d->batch, d->tokens));
+  w.bits = b.take<uint8_t>(d->dropout_rate > 0.f ? attn_dropbits_bytes(d->tokens) : 0);
+  w.total = b.total();
+  return w;
 }
 
 extern "C" size_t tome_attention_workspace_bytes(const tome_attn_desc_t* d) {
   if (!d || d->batch <= 0 || d->tokens <= 0) return 0;
-  return fwd_ws_bytes(d);
+  return fwd_ws(d, nullptr).total;
 }
 
 extern "C" int tome_attention_fwd(const tome_attn_desc_t* d, const void* q, const void* k, const void* v, void* out,
@@ -566,22 +571,22 @@ extern "C" int tome_attention_fwd(const tome_attn_desc_t* d, const void* q, cons
     ProfScope prof(PROF_ATTN_FWD, 4.0 * d->batch * d->heads * (double)d->tokens * d->tokens * d->head_dim, 1, stream);
     return attn_generic_fwd(d, q, k, v, out, lse, stream);
   }
-  TOME_CHECK(workspace && workspace_bytes >= fwd_ws_bytes(d), TOME_ERR_INVALID,
-             "attention_fwd: workspace too small (%zu < %zu, see tome_attention_workspace_bytes)", workspace_bytes, fwd_ws_bytes(d));
+  const FwdWs ws = fwd_ws(d, workspace);
+  TOME_CHECK(workspace && workspace_bytes >= ws.total, TOME_ERR_INVALID,
+             "attention_fwd: workspace too small (%zu < %zu, see tome_attention_workspace_bytes)", workspace_bytes, ws.total);
   TOME_CHECK(((uintptr_t)workspace & 255) == 0, TOME_ERR_INVALID, "attention_fwd: workspace must be 256-byte aligned");
   TOME_CHECK(d->dropout_rate >= 0.f && d->dropout_rate < 1.f, TOME_ERR_INVALID, "attention_fwd: dropout_rate must be in [0, 1)");
   CUtensorMap tq, tk, tv;
   const uint64_t hd = (uint64_t)d->heads * d->head_dim;
   ProfScope prof(PROF_ATTN_FWD, 4.0 * d->batch * d->heads * (double)d->tokens * d->tokens * d->head_dim, 2, stream);
-  if (int rc = launch_attn_meta(d->batch, d->tokens, d->gid, d->pos, d->allow, d->num_groups, d->size,
-                                reinterpret_cast<uint8_t*>(workspace), stream)) return rc;
+  if (int rc = launch_attn_meta(d->batch, d->tokens, d->gid, d->pos, d->allow, d->num_groups, d->size, ws.meta, stream)) return rc;
   if (int rc = make_tmap_3d_bf16(&tq, q, hd, d->tokens, d->batch, d->q_token_stride, d->q_batch_stride, ATT_BM)) return rc;
   if (int rc = make_tmap_3d_bf16(&tk, k, hd, d->tokens, d->batch, d->k_token_stride, d->k_batch_stride, ATT_BN)) return rc;
   if (int rc = make_tmap_3d_bf16(&tv, v, hd, d->tokens, d->batch, d->v_token_stride, d->v_batch_stride, ATT_BN)) return rc;
   AttnFwdParams p;
   p.batch = d->batch; p.tokens = d->tokens; p.heads = d->heads;
   p.scale_log2 = d->scale * 1.4426950408889634f;
-  p.gid = d->gid; p.pos = d->pos; p.meta = reinterpret_cast<const uint8_t*>(workspace);
+  p.gid = d->gid; p.pos = d->pos; p.meta = ws.meta;
   p.aug_flag = attn_aug_flag(p.meta, d->batch, d->tokens);
   CUtensorMap tqa, tka;
   {
@@ -592,11 +597,9 @@ extern "C" int tome_attention_fwd(const tome_attn_desc_t* d, const void* q, cons
   p.keep_q = nullptr;
   p.inv_keep = 1.0f;
   if (d->dropout_rate > 0.f) {
-    uint8_t* bits = reinterpret_cast<uint8_t*>(workspace) + ((attn_meta_bytes(d->batch, d->tokens) + 255) & ~size_t(255));
-    if (int rc = launch_attn_dropbits(d->tokens, d->dropout_rate, d->dropout_seed, d->dropout_site, bits, stream)) return rc;
-    p.keep_q = bits;
-    const uint32_t th = (uint32_t)(d->dropout_rate * 65536.0f + 0.5f);
-    p.inv_keep = 1.0f / (1.0f - (float)th / 65536.0f);
+    if (int rc = launch_attn_dropbits(d->tokens, d->dropout_rate, d->dropout_seed, d->dropout_site, ws.bits, stream)) return rc;
+    p.keep_q = ws.bits;
+    p.inv_keep = make_dropout(d->dropout_rate, d->dropout_seed, d->dropout_site).inv_keep;
   }
   p.out = reinterpret_cast<__nv_bfloat16*>(out);
   p.o_batch_stride = d->o_batch_stride; p.o_token_stride = d->o_token_stride;

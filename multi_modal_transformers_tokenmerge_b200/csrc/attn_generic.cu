@@ -231,10 +231,7 @@ static void fill_params(AttnGenericParams& p, const tome_attn_desc_t* d, const v
   p.batch = d->batch; p.tokens = d->tokens; p.heads = d->heads; p.dim = d->head_dim;
   p.scale = d->scale; p.scale_log2 = d->scale * 1.4426950408889634f;
   p.gid = d->gid; p.pos = d->pos; p.allow = d->allow; p.num_groups = d->num_groups; p.size = d->size;
-  p.drop.thresh16 = (uint32_t)(d->dropout_rate * 65536.0f + 0.5f);
-  p.drop.inv_keep = 1.0f / (1.0f - (float)p.drop.thresh16 / 65536.0f);
-  p.drop.seed_lo = (uint32_t)d->dropout_seed; p.drop.seed_hi = (uint32_t)(d->dropout_seed >> 32);
-  p.drop.site = d->dropout_site;
+  p.drop = make_dropout(d->dropout_rate, d->dropout_seed, d->dropout_site);
   p.q = reinterpret_cast<const __nv_bfloat16*>(q); p.k = reinterpret_cast<const __nv_bfloat16*>(k);
   p.v = reinterpret_cast<const __nv_bfloat16*>(v);
   p.q_bs = d->q_batch_stride; p.q_ts = d->q_token_stride; p.k_bs = d->k_batch_stride; p.k_ts = d->k_token_stride;

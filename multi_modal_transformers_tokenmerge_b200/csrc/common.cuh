@@ -299,6 +299,16 @@ struct DropoutCfg {
   uint32_t seed_lo, seed_hi;
   uint32_t site;  // distinguishes call sites / layers
 };
+// The one rate -> threshold conversion: forward and backward regenerate the same mask only if every call site rounds
+// `rate` the same way (and a dgrad's gate_scale must equal the forward epilogue's inv_keep).
+inline DropoutCfg make_dropout(float rate, uint64_t seed, uint32_t site) {
+  DropoutCfg d;
+  d.thresh16 = (uint32_t)(rate * 65536.0f + 0.5f);
+  d.inv_keep = 1.0f / (1.0f - (float)d.thresh16 / 65536.0f);
+  d.seed_lo = (uint32_t)seed; d.seed_hi = (uint32_t)(seed >> 32);
+  d.site = site;
+  return d;
+}
 constexpr uint32_t DROP_A = 0x915F77F5u;  // LCG multiplier (A % 8 == 5: full period for any odd increment)
 __host__ __device__ constexpr uint32_t drop_pow(int n) { uint32_t r = 1; for (int i = 0; i < n; ++i) r *= DROP_A; return r; }
 __host__ __device__ constexpr uint32_t drop_geo(int n) { uint32_t r = 0, a = 1; for (int i = 0; i < n; ++i) { r += a; a *= DROP_A; } return r; }  // 1 + A + ... + A^(n-1)

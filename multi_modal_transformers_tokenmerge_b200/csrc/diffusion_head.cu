@@ -54,30 +54,23 @@ struct DiffWs {
   float *dpred, *colsum, *dff;
   size_t total;
 };
-static DiffWs diff_ws(const tome_diffusion_desc_t* d, void* base_) {
+static DiffWs diff_ws(const tome_diffusion_desc_t* d, void* base) {
   const DiffDims s = diff_dims(d);
-  uint8_t* base = reinterpret_cast<uint8_t*>(base_);
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    off = (off + 255) & ~size_t(255);
-    uint8_t* p = base ? base + off : nullptr;
-    off += bytes;
-    return p;
-  };
+  Bump b{reinterpret_cast<uint8_t*>(base)};
   DiffWs w;
-  w.ff = reinterpret_cast<__nv_bfloat16*>(take(s.B * s.F * 2));
-  w.th = reinterpret_cast<__nv_bfloat16*>(take(s.B * s.Ht * 2));
-  w.cat = reinterpret_cast<__nv_bfloat16*>(take(s.B * s.Dc * 2));
-  w.h = reinterpret_cast<__nv_bfloat16*>(take(s.B * s.H * 2));
-  w.dpred = reinterpret_cast<float*>(take(s.B * s.A * 4));
-  w.dh = reinterpret_cast<__nv_bfloat16*>(take(s.B * s.H * 2));
-  w.dcat = reinterpret_cast<__nv_bfloat16*>(take(s.B * s.Dc * 2));
-  w.dth = reinterpret_cast<__nv_bfloat16*>(take(s.B * s.Ht * 2));
-  w.dff = reinterpret_cast<float*>(take(s.B * s.F * 4));   // fp32: it feeds the Fourier-kernel gradient, a sum with cancellation
+  w.ff = b.take<__nv_bfloat16>(s.B * s.F);
+  w.th = b.take<__nv_bfloat16>(s.B * s.Ht);
+  w.cat = b.take<__nv_bfloat16>(s.B * s.Dc);
+  w.h = b.take<__nv_bfloat16>(s.B * s.H);
+  w.dpred = b.take<float>(s.B * s.A);
+  w.dh = b.take<__nv_bfloat16>(s.B * s.H);
+  w.dcat = b.take<__nv_bfloat16>(s.B * s.Dc);
+  w.dth = b.take<__nv_bfloat16>(s.B * s.Ht);
+  w.dff = b.take<float>(s.B * s.F);   // fp32: it feeds the Fourier-kernel gradient, a sum with cancellation
   long long widest = s.H > s.Ht ? s.H : s.Ht;
   if (s.To > widest) widest = s.To;
-  w.colsum = reinterpret_cast<float*>(take((size_t)tome_colsum_workspace_rows((int)s.B) * widest * 4));
-  w.total = (off + 255) & ~size_t(255);
+  w.colsum = b.take<float>((size_t)tome_colsum_workspace_rows((int)s.B) * widest);
+  w.total = b.total();
   return w;
 }
 

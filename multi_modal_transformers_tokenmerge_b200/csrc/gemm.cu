@@ -839,10 +839,7 @@ extern "C" int tome_gemm_bf16(const tome_gemm_args_t* a, void* workspace, size_t
   e.colsum_part = a->colsum_partial;
   e.ldc = a->ldc; e.ldr = a->ldr; e.ldg = a->ldg;
   e.gate_scale = a->gate_scale; e.relu = a->relu; e.c_is_f32 = (a->c_dtype == TOME_F32);
-  e.drop.thresh16 = (uint32_t)(a->dropout_rate * 65536.0f + 0.5f);
-  e.drop.inv_keep = 1.0f / (1.0f - (float)e.drop.thresh16 / 65536.0f);
-  e.drop.seed_lo = (uint32_t)a->dropout_seed; e.drop.seed_hi = (uint32_t)(a->dropout_seed >> 32);
-  e.drop.site = a->dropout_site;
+  e.drop = make_dropout(a->dropout_rate, a->dropout_seed, a->dropout_site);
   e.split_stride = 0;
   e.accumulate = a->accumulate;
   TOME_CHECK(!a->accumulate || e.c_is_f32, TOME_ERR_INVALID, "gemm: accumulate requires an fp32 output");

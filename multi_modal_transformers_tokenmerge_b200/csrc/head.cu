@@ -21,14 +21,14 @@ constexpr int HEAD_THREADS = 256;
 struct HeadWs {
   float* pooled;  // [B, G, C]
   float* dz;      // [B, G, F]   dL/dz of the mean loss
+  size_t total;
 };
-static inline size_t head_pooled_bytes(const tome_head_desc_t* d) {
-  return (((size_t)d->batch * d->groups * d->channels * sizeof(float)) + 255) & ~size_t(255);
-}
-static inline HeadWs head_ws(const tome_head_desc_t* d, void* ws) {
+static HeadWs head_ws(const tome_head_desc_t* d, void* base) {
+  Bump b{reinterpret_cast<uint8_t*>(base)};
   HeadWs w;
-  w.pooled = reinterpret_cast<float*>(ws);
-  w.dz = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(ws) + head_pooled_bytes(d));
+  w.pooled = b.take<float>((size_t)d->batch * d->groups * d->channels);
+  w.dz = b.take<float>((size_t)d->batch * d->groups * d->features);
+  w.total = b.total();
   return w;
 }
 
@@ -228,7 +228,7 @@ using namespace tome;
 extern "C" size_t tome_action_head_workspace_bytes(const tome_head_desc_t* d) {
   clear_error();
   if (check_head(d) != TOME_OK) return 0;
-  return head_pooled_bytes(d) + (((size_t)d->batch * d->groups * d->features * sizeof(float) + 255) & ~size_t(255));
+  return head_ws(d, nullptr).total;
 }
 
 extern "C" int tome_action_head_fwd(const tome_head_desc_t* d, const void* x, const int32_t* origin, const float* w,
@@ -239,10 +239,9 @@ extern "C" int tome_action_head_fwd(const tome_head_desc_t* d, const void* x, co
   if (int rc = check_head(d)) return rc;
   TOME_CHECK(x && origin && w && out, TOME_ERR_INVALID, "action_head_fwd: null argument");
   TOME_CHECK(!loss || actions, TOME_ERR_INVALID, "action_head_fwd: a loss needs the target actions");
-  TOME_CHECK(!workspace || (workspace_bytes >= tome_action_head_workspace_bytes(d) && ((uintptr_t)workspace & 255) == 0),
-             TOME_ERR_INVALID, "action_head_fwd: workspace too small or not 256-byte aligned");
-  HeadWs ws{nullptr, nullptr};
-  if (workspace) ws = head_ws(d, workspace);
+  const HeadWs ws = head_ws(d, workspace);  // no workspace: nothing kept for the backward
+  TOME_CHECK(!workspace || (workspace_bytes >= ws.total && ((uintptr_t)workspace & 255) == 0), TOME_ERR_INVALID,
+             "action_head_fwd: workspace too small or not 256-byte aligned");
   const size_t smem = ((size_t)d->groups * d->channels + (size_t)d->groups * d->features) * sizeof(float);
   ProfScope prof(PROF_OTHER, 0.0, loss ? 2 : 1, stream);
   if (d->x_dtype == TOME_BF16) {

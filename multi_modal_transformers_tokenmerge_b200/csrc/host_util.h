@@ -48,6 +48,26 @@ int make_tmap_3d_bf16_sw32(CUtensorMap* out, const void* base, uint64_t d1, uint
 
 inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 
+// Carves a workspace into 256-byte aligned buffers, in call order.  A module's `*_workspace_bytes` and its launch run
+// the same carving function, the query with base == nullptr (every pointer comes back null), so the size it reports is
+// the size the launch uses.
+struct Bump {
+  uint8_t* base;
+  size_t off = 0;
+  size_t reserve(size_t bytes) {  // returns the new buffer's offset from base
+    off = (off + 255) & ~size_t(255);
+    const size_t at = off;
+    off += bytes;
+    return at;
+  }
+  template <typename T>
+  T* take(size_t count) {
+    const size_t at = reserve(count * sizeof(T));
+    return base ? reinterpret_cast<T*>(base + at) : nullptr;
+  }
+  size_t total() const { return (off + 255) & ~size_t(255); }
+};
+
 // cudaFuncAttributeMaxDynamicSharedMemorySize is a PER-DEVICE attribute: a process that drives several GPUs (JAX's
 // default) must set it on each one.  One DynSmemOnce per call site remembers, per device, the largest size already set.
 struct DynSmemOnce {

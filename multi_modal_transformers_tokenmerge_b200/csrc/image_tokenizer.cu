@@ -53,8 +53,6 @@ struct ItGeom {
   size_t off_col, off_y0, off_pool, off_xa, off_xb, off_h, off_pix, off_dense, off_part, off_stats, off_ab, total;
 };
 
-static size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
-
 static int it_geometry(const tome_image_tokenizer_desc_t* d, ItGeom* g, const char* who) {
   TOME_CHECK(d != nullptr, TOME_ERR_INVALID, "%s: null descriptor", who);
   TOME_CHECK(d->batch > 0 && d->n_images > 0 && d->image_size > 0 && d->channels_in > 0, TOME_ERR_INVALID, "%s: bad image shape", who);
@@ -99,19 +97,19 @@ static int it_geometry(const tome_image_tokenizer_desc_t* d, ItGeom* g, const ch
   g->chunk_rows = (int)cr;
   long long want = m2_row * (d->features / 8) / (IT_THREADS * 4);
   g->gn_ctas = (int)std::min<long long>(IT_GN_MAX_CTAS, std::max<long long>(1, want));
-  size_t o = 0;
-  g->off_col = o;   o += align256(col_row * cr);
-  g->off_y0 = o;    o += align256((size_t)2 * m0_row * cr * d->features);
-  g->off_pool = o;  o += align256((size_t)2 * m2p_row * cr * d->features);
-  g->off_xa = o;    o += align256((size_t)2 * m2p_row * cr * d->features);
-  g->off_xb = o;    o += align256((size_t)2 * m2p_row * cr * d->features);
-  g->off_h = o;     o += align256((size_t)2 * m2p_row * cr * d->features);
-  g->off_pix = o;   o += align256((size_t)2 * cr * d->n_images * d->image_size * d->image_size * d->channels_in + 16);
-  g->off_dense = o; o += align256((size_t)4 * cr * d->n_images * g->np * d->embed_dim);
-  g->off_part = o;  o += align256((size_t)4 * cr * g->gn_ctas * d->features * 2);
-  g->off_stats = o; o += align256((size_t)4 * cr * d->num_groups * 2);
-  g->off_ab = o;    o += align256((size_t)4 * cr * d->features * 2);
-  g->total = o;
+  Bump b{nullptr};
+  g->off_col = b.reserve(col_row * cr);
+  g->off_y0 = b.reserve((size_t)2 * m0_row * cr * d->features);
+  g->off_pool = b.reserve((size_t)2 * m2p_row * cr * d->features);
+  g->off_xa = b.reserve((size_t)2 * m2p_row * cr * d->features);
+  g->off_xb = b.reserve((size_t)2 * m2p_row * cr * d->features);
+  g->off_h = b.reserve((size_t)2 * m2p_row * cr * d->features);
+  g->off_pix = b.reserve((size_t)2 * cr * d->n_images * d->image_size * d->image_size * d->channels_in + 16);
+  g->off_dense = b.reserve((size_t)4 * cr * d->n_images * g->np * d->embed_dim);
+  g->off_part = b.reserve((size_t)4 * cr * g->gn_ctas * d->features * 2);
+  g->off_stats = b.reserve((size_t)4 * cr * d->num_groups * 2);
+  g->off_ab = b.reserve((size_t)4 * cr * d->features * 2);
+  g->total = b.total();
   return TOME_OK;
 }
 

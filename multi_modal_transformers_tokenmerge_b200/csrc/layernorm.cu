@@ -750,11 +750,7 @@ extern "C" int tome_dropout_colsum_bf16(int m, int n, const void* x, void* y, fl
   TOME_CHECK(m > 0 && n > 0 && x && y && out && workspace, TOME_ERR_INVALID, "dropout_colsum: bad argument");
   TOME_CHECK(n % 8 == 0, TOME_ERR_INVALID, "dropout_colsum: n must be a multiple of 8");
   TOME_CHECK(rate >= 0.f && rate < 1.f, TOME_ERR_INVALID, "dropout_colsum: rate must be in [0, 1)");
-  DropoutCfg d;
-  d.thresh16 = (uint32_t)(rate * 65536.0f + 0.5f);
-  d.inv_keep = 1.0f / (1.0f - (float)d.thresh16 / 65536.0f);
-  d.seed_lo = (uint32_t)seed; d.seed_hi = (uint32_t)(seed >> 32);
-  d.site = site;
+  const DropoutCfg d = make_dropout(rate, seed, site);
   const int chunks = colsum_rows(m);
   ProfScope prof(PROF_COLSUM, (double)m * n * 4.0, 2, stream);
   const int rpc = ceil_div(m, chunks);

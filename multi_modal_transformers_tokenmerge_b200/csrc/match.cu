@@ -765,11 +765,19 @@ static bool sim_fast64(const tome_metric_desc_t* d, const void* src) {   // 128-
          d->head_stride % 8 == 0 && ((uintptr_t)src & 15) == 0;
 }
 
+// The normalised metric in the workspace: plane A (the ta even tokens of every batch row), then plane B (the tb odd ones),
+// packed.  A token's row is three bf16 chunks of 64 (SIMT_ROW) on the tensor-core path, else dim floats padded to a multiple of 4.
+struct SimPlanes { uint8_t *a, *b; size_t total; };
+static SimPlanes sim_planes(const tome_metric_desc_t* d, void* base) {
+  const size_t row = sim_tc_eligible(d) ? SIMT_ROW * sizeof(__nv_bfloat16) : ((d->dim + 3) & ~3) * sizeof(float);
+  uint8_t* a = reinterpret_cast<uint8_t*>(base);
+  const size_t ta = (d->tokens + 1) / 2;
+  return {a, a ? a + d->batch * ta * row : nullptr, (size_t)d->batch * d->tokens * row};
+}
+
 extern "C" size_t tome_sim_argmax_workspace_bytes(const tome_metric_desc_t* d) {
   if (!d || d->batch <= 0 || d->tokens <= 0 || d->dim <= 0) return 0;
-  const size_t f32_planes = (size_t)d->batch * d->tokens * ((d->dim + 3) & ~3) * sizeof(float);
-  const size_t split_planes = (size_t)d->batch * d->tokens * SIMT_ROW * 2;   // three bf16 chunks of 64 per token (dim 64 only)
-  return d->dim == 64 && split_planes > f32_planes ? split_planes : f32_planes;
+  return sim_planes(d, nullptr).total;
 }
 
 extern "C" int tome_sim_argmax(const tome_metric_desc_t* d, const void* src, float* node_max, int32_t* node_idx,
@@ -790,13 +798,13 @@ extern "C" int tome_sim_argmax(const tome_metric_desc_t* d, const void* src, flo
   dim3 grid(ceil_div(ta, SIM_TILE), d->batch);
   if (workspace != nullptr) {
     // ---- normalise once, then stream tiles (see the comment above metric_norm_kernel)
-    TOME_CHECK(workspace_bytes >= tome_sim_argmax_workspace_bytes(d) && ((uintptr_t)workspace & 15) == 0, TOME_ERR_INVALID,
-               "sim_argmax: workspace must be 16-byte aligned and hold %zu bytes (got %zu)", tome_sim_argmax_workspace_bytes(d),
-               workspace_bytes);
+    const SimPlanes planes = sim_planes(d, workspace);
+    TOME_CHECK(workspace_bytes >= planes.total && ((uintptr_t)workspace & 15) == 0, TOME_ERR_INVALID,
+               "sim_argmax: workspace must be 16-byte aligned and hold %zu bytes (got %zu)", planes.total, workspace_bytes);
     ProfScope prof(PROF_SIM, 2.0 * d->batch * ta * (double)tb * d->dim, 2, stream);
     if (sim_tc_eligible(d)) {
-      __nv_bfloat16* pa = reinterpret_cast<__nv_bfloat16*>(workspace);
-      __nv_bfloat16* pb = pa + (size_t)d->batch * ta * SIMT_ROW;
+      __nv_bfloat16* pa = reinterpret_cast<__nv_bfloat16*>(planes.a);
+      __nv_bfloat16* pb = reinterpret_cast<__nv_bfloat16*>(planes.b);
       const long long toks = (long long)d->batch * d->tokens;
       if (sim_fast64(d, src))
         launch_k(metric_split64_kernel, (unsigned)((toks * 8 + 255) / 256), 256, 0, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), pa, pb);
@@ -814,8 +822,8 @@ extern "C" int tome_sim_argmax(const tome_metric_desc_t* d, const void* src, flo
                          node_max, node_idx, scores_out));
       return TOME_OK;
     }
-    float* plane_a = reinterpret_cast<float*>(workspace);
-    float* plane_b = plane_a + (size_t)d->batch * ta * dpad;
+    float* plane_a = reinterpret_cast<float*>(planes.a);
+    float* plane_b = reinterpret_cast<float*>(planes.b);
     const long long toks = (long long)d->batch * d->tokens;
     const unsigned nblk = (unsigned)((toks + 7) / 8);
     if (sim_fast64(d, src))

@@ -169,18 +169,6 @@ static std::vector<LayerShape> layer_shapes(const tome_stack_cfg_t* c) {
   return s;
 }
 
-struct Bump {
-  uint8_t* base;
-  size_t off = 0;
-  template <typename T>
-  T* take(size_t count) {
-    off = (off + 255) & ~size_t(255);
-    T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
-    off += count * sizeof(T);
-    return p;
-  }
-};
-
 // One function computes the layout for both the size query (base == nullptr) and the real pointers.
 static StackLayout make_layout(const tome_stack_cfg_t* c, void* workspace) {
   StackLayout S;
@@ -295,7 +283,7 @@ static StackLayout make_layout(const tome_stack_cfg_t* c, void* workspace) {
     S.ws_head_bytes = tome_action_head_workspace_bytes(&h);
     S.ws_head = b.take<uint8_t>(S.ws_head_bytes);
   }
-  S.total = (b.off + 255) & ~size_t(255);
+  S.total = b.total();
   return S;
 }
 
@@ -308,14 +296,21 @@ __global__ void broadcast_groups_kernel(int B, int T, const uint8_t* __restrict_
   }
 }
 
-static DropoutCfg make_drop(const tome_stack_cfg_t* c, uint32_t site) {
-  DropoutCfg d;
-  d.thresh16 = (uint32_t)(c->dropout_rate * 65536.0f + 0.5f);
-  d.inv_keep = 1.0f / (1.0f - (float)d.thresh16 / 65536.0f);
-  d.seed_lo = (uint32_t)c->dropout_seed;
-  d.seed_hi = (uint32_t)(c->dropout_seed >> 32);
-  d.site = site;
-  return d;
+// Layer l's attention over its packed qkv: forward and backward must describe it identically (the attention-dropout
+// mask is regenerated from the seed and site given here).
+static tome_attn_desc_t attn_desc(const tome_stack_cfg_t* c, const tome_stack_io_t* io, const LayerBufs& Lb, int T, int l) {
+  const int HD = c->heads * c->head_dim;
+  tome_attn_desc_t ad;
+  memset(&ad, 0, sizeof(ad));
+  ad.batch = c->batch; ad.tokens = T; ad.heads = c->heads; ad.head_dim = c->head_dim;
+  ad.q_batch_stride = ad.k_batch_stride = ad.v_batch_stride = (long long)T * 3 * HD;
+  ad.q_token_stride = ad.k_token_stride = ad.v_token_stride = 3 * HD;
+  ad.o_batch_stride = (long long)T * HD; ad.o_token_stride = HD;
+  ad.scale = 1.0f / sqrtf((float)c->head_dim);
+  if (c->num_groups) { ad.gid = Lb.gid_in; ad.pos = Lb.pos_in; ad.allow = io->allow; ad.num_groups = c->num_groups; }
+  ad.size = c->prop_attn ? Lb.size_in : nullptr;
+  ad.dropout_rate = c->attn_dropout_rate; ad.dropout_seed = c->dropout_seed; ad.dropout_site = kAttnDropSite + (uint32_t)l;
+  return ad;
 }
 
 #define RC(expr)                 \
@@ -427,16 +422,7 @@ extern "C" int tome_stack_forward(const tome_stack_cfg_t* c, const tome_stack_io
                           Lb.ln1_rstd, st));
     RC(gemm(c, S, st, M, 3 * HD, C, Lb.h, C, TOME_MAJOR_K, pw + o.wqkv, 3 * HD, TOME_MAJOR_MN, Lb.qkv, 3 * HD, TOME_BF16,
             pf + o.bqkv, 0, nullptr, nullptr, 1.f, -1, 0));
-    tome_attn_desc_t ad;
-    memset(&ad, 0, sizeof(ad));
-    ad.batch = B; ad.tokens = T; ad.heads = H; ad.head_dim = D;
-    ad.q_batch_stride = ad.k_batch_stride = ad.v_batch_stride = (long long)T * 3 * HD;
-    ad.q_token_stride = ad.k_token_stride = ad.v_token_stride = 3 * HD;
-    ad.o_batch_stride = (long long)T * HD; ad.o_token_stride = HD;
-    ad.scale = 1.0f / sqrtf((float)D);
-    if (c->num_groups) { ad.gid = Lb.gid_in; ad.pos = Lb.pos_in; ad.allow = io->allow; ad.num_groups = c->num_groups; }
-    ad.size = c->prop_attn ? Lb.size_in : nullptr;
-    ad.dropout_rate = c->attn_dropout_rate; ad.dropout_seed = c->dropout_seed; ad.dropout_site = kAttnDropSite + (uint32_t)l;
+    const tome_attn_desc_t ad = attn_desc(c, io, Lb, T, l);
     RC(tome_attention_fwd(&ad, Lb.qkv, Lb.qkv + HD, Lb.qkv + 2 * HD, Lb.attn_o, Lb.lse, S.ws_attn, S.ws_attn_bytes, st));
     __nv_bfloat16* x1 = r > 0 ? S.x1_scratch : Lb.x1m;
     RC(gemm(c, S, st, M, C, HD, Lb.attn_o, HD, TOME_MAJOR_K, pw + o.wo, C, TOME_MAJOR_MN, x1, C, TOME_BF16, pf + o.bo, 0,
@@ -531,7 +517,7 @@ extern "C" int tome_stack_backward(const tome_stack_cfg_t* c, const tome_stack_i
   const __nv_bfloat16* pw = reinterpret_cast<const __nv_bfloat16*>(io->params_bf16);
   float* gr = io->grads_f32;
   const bool drop = c->dropout_rate > 0.f;
-  const float inv_keep = drop ? make_drop(c, 0).inv_keep : 1.0f;
+  const float inv_keep = drop ? make_dropout(c->dropout_rate, c->dropout_seed, 0).inv_keep : 1.0f;
   const int TL = S.shapes.back().t_out;
 
   __nv_bfloat16 *g0 = S.g0, *g1 = S.g1, *g2 = S.g2, *g3 = S.g3;
@@ -607,16 +593,7 @@ extern "C" int tome_stack_backward(const tome_stack_cfg_t* c, const tome_stack_i
     RC(gemm(c, S, st, M, HD, C, dyo, C, TOME_MAJOR_K, pw + o.wo, C, TOME_MAJOR_K, g3, HD, TOME_BF16, nullptr, 0, nullptr, nullptr,
             1.f, -1, 0));  // d attn_o
     // ---- attention backward -> dqkv in big
-    tome_attn_desc_t ad;
-    memset(&ad, 0, sizeof(ad));
-    ad.batch = B; ad.tokens = T; ad.heads = H; ad.head_dim = D;
-    ad.q_batch_stride = ad.k_batch_stride = ad.v_batch_stride = (long long)T * 3 * HD;
-    ad.q_token_stride = ad.k_token_stride = ad.v_token_stride = 3 * HD;
-    ad.o_batch_stride = (long long)T * HD; ad.o_token_stride = HD;
-    ad.scale = 1.0f / sqrtf((float)D);
-    if (c->num_groups) { ad.gid = Lb.gid_in; ad.pos = Lb.pos_in; ad.allow = io->allow; ad.num_groups = c->num_groups; }
-    ad.size = c->prop_attn ? Lb.size_in : nullptr;
-    ad.dropout_rate = c->attn_dropout_rate; ad.dropout_seed = c->dropout_seed; ad.dropout_site = kAttnDropSite + (uint32_t)l;
+    const tome_attn_desc_t ad = attn_desc(c, io, Lb, T, l);
     tome_attn_grad_strides_t gs;
     memset(&gs, 0, sizeof(gs));
     gs.dq_batch_stride = gs.dk_batch_stride = gs.dv_batch_stride = (long long)T * 3 * HD;

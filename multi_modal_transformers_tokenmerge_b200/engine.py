@@ -16,6 +16,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
+from .ops import _scratch
 
 PARAM_ORDER = ["ln1_scale", "ln1_bias", "wqkv", "bqkv", "wo", "bo", "ln2_scale", "ln2_bias", "w1", "b1", "w2", "b2"]
 
@@ -101,8 +102,7 @@ class ToMeStackEngine:
         self.adam_m = self.adam_v = None
         self.step_count = 0
         ws = self.lib.tome_stack_workspace_bytes(C.byref(self.ccfg))
-        self.workspace = torch.empty(ws + 256, dtype=torch.uint8, device=self.dev)
-        self._ws_off = (-self.workspace.data_ptr()) % 256
+        self.workspace = _scratch(ws, self.dev)
         self._ws_bytes = ws
         self.gid = None if gid is None else torch.as_tensor(np.asarray(gid, np.uint8)).to(self.dev)
         self.pos = None if pos is None else torch.as_tensor(np.asarray(pos, np.int32)).to(self.dev)
@@ -213,7 +213,7 @@ class ToMeStackEngine:
                          None if self.allow is None else self.allow.data_ptr(),
                          None if self.readout_idx is None else self.readout_idx.data_ptr(),
                          None if target is None else target.data_ptr(),
-                         self.workspace.data_ptr() + self._ws_off, self._ws_bytes, None,
+                         self.workspace.data_ptr(), self._ws_bytes, None,
                          None if self.readout is None else self.readout.data_ptr(), self.loss.data_ptr(),
                          None if self.grads is None else self.grads.data_ptr(),
                          None if ev is None else C.cast(ev, C.POINTER(C.c_void_p)),

@@ -74,11 +74,13 @@ class MatchPlan:
                       self.dst_off.data_ptr(), self.dst_src.data_ptr())
 
 
-def _scratch(nbytes: int, device) -> torch.Tensor:
-    """uint8 device scratch of `nbytes` whose data pointer is 256-byte aligned (torch's allocator aligns to 512)."""
-    t = torch.empty(max(int(nbytes), 256), dtype=torch.uint8, device=device)
-    assert t.data_ptr() % 256 == 0
-    return t
+def _scratch(nbytes: int, device, buf: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """uint8 device view of at least `nbytes` bytes whose data pointer is 256-byte aligned (the library's workspaces): a
+    slice of `buf` (uint8, nbytes + 256 bytes or more) or of a new allocation of that size, so it keeps the storage alive."""
+    if buf is None:
+        buf = torch.empty(int(nbytes) + 256, dtype=torch.uint8, device=device)
+    assert buf.numel() >= nbytes + 256, (buf.numel(), nbytes)
+    return buf[(-buf.data_ptr()) % 256:]
 
 
 def sim_argmax(src: torch.Tensor, *, heads: int = 1, dim: Optional[int] = None, batch_stride=None, token_stride=None,
@@ -333,7 +335,6 @@ class HeadState:
     origin: torch.Tensor
     w: torch.Tensor
     workspace: torch.Tensor
-    off: int
 
 
 def action_head_fwd(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], *, kind: int, max_action: float,
@@ -358,16 +359,15 @@ def action_head_fwd(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tenso
         want = (B, feats) if kind == L.HEAD_CONTINUOUS_L2 else (B, groups)
         assert tuple(actions.shape) == want, (actions.shape, want)
         loss = torch.zeros(1 + B, dtype=torch.float32, device=x.device)
-    ws, off, nbytes = None, 0, 0
+    ws, nbytes = None, 0
     if keep_for_backward:
         nbytes = int(L.lib().tome_action_head_workspace_bytes(C.byref(d)))
         if nbytes == 0:
             L.check(1)
-        ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=x.device)
-        off = (-ws.data_ptr()) % 256
+        ws = _scratch(nbytes, x.device)
     L.check(L.lib().tome_action_head_fwd(C.byref(d), _ptr(x), _ptr(origin), _ptr(w), _ptr(bias), _ptr(actions), _ptr(out),
-                                         _ptr(loss), None if ws is None else C.c_void_p(ws.data_ptr() + off), nbytes, _stream()))
-    return out, loss, (HeadState(d, origin, w, ws, off) if keep_for_backward else None)
+                                         _ptr(loss), _ptr(ws), nbytes, _stream()))
+    return out, loss, (HeadState(d, origin, w, ws) if keep_for_backward else None)
 
 
 def action_head_bwd(state: HeadState, dw: torch.Tensor, dbias: Optional[torch.Tensor], want_dx: bool = True):
@@ -377,9 +377,8 @@ def action_head_bwd(state: HeadState, dw: torch.Tensor, dbias: Optional[torch.Te
     if want_dx:
         dx = torch.empty(d.batch, d.tokens, d.channels, dtype=torch.bfloat16 if d.x_dtype == L.TOME_BF16 else torch.float32,
                          device=dw.device)
-    L.check(L.lib().tome_action_head_bwd(C.byref(d), _ptr(state.origin), _ptr(state.w),
-                                         C.c_void_p(state.workspace.data_ptr() + state.off), _ptr(dw), _ptr(dbias), _ptr(dx),
-                                         _stream()))
+    L.check(L.lib().tome_action_head_bwd(C.byref(d), _ptr(state.origin), _ptr(state.w), _ptr(state.workspace), _ptr(dw),
+                                         _ptr(dbias), _ptr(dx), _stream()))
     return dx
 
 
@@ -391,7 +390,6 @@ class DiffusionState:
     origin: torch.Tensor
     time: torch.Tensor
     workspace: torch.Tensor
-    off: int
 
 
 def diffusion_head_fwd(x: torch.Tensor, params: torch.Tensor, desc: "L.DiffusionDesc", actions: torch.Tensor, noise: torch.Tensor,
@@ -409,24 +407,21 @@ def diffusion_head_fwd(x: torch.Tensor, params: torch.Tensor, desc: "L.Diffusion
     assert params.numel() == n, (params.numel(), n)
     p16 = params.to(torch.bfloat16)
     nbytes = int(L.lib().tome_diffusion_head_workspace_bytes(C.byref(desc)))
-    ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=x.device)
-    off = (-ws.data_ptr()) % 256
+    ws = _scratch(nbytes, x.device)
     pred = torch.empty(B, desc.action_dim, dtype=torch.float32, device=x.device)
     loss = torch.zeros(1 + B, dtype=torch.float32, device=x.device)
     for t, dt in ((actions, torch.float32), (noise, torch.float32), (time, torch.int32), (alpha_hats, torch.float32)):
         assert t.dtype == dt and t.is_contiguous()
     L.check(L.lib().tome_diffusion_head_fwd(C.byref(desc), _ptr(params), _ptr(p16), _ptr(x), _ptr(origin), _ptr(actions), _ptr(noise),
-                                            _ptr(time), _ptr(alpha_hats), _ptr(pred), _ptr(loss), C.c_void_p(ws.data_ptr() + off),
-                                            nbytes, _stream()))
-    return pred, loss, DiffusionState(desc, params, p16, origin, time, ws, off)
+                                            _ptr(time), _ptr(alpha_hats), _ptr(pred), _ptr(loss), _ptr(ws), nbytes, _stream()))
+    return pred, loss, DiffusionState(desc, params, p16, origin, time, ws)
 
 
 def diffusion_head_bwd(state: DiffusionState, grads: torch.Tensor, want_dx: bool = True):
     d = state.desc
     dx = torch.empty(d.batch, d.tokens, d.channels, dtype=torch.bfloat16, device=grads.device) if want_dx else None
     L.check(L.lib().tome_diffusion_head_bwd(C.byref(d), _ptr(state.params), _ptr(state.params_bf16), _ptr(state.origin),
-                                            _ptr(state.time), C.c_void_p(state.workspace.data_ptr() + state.off), _ptr(grads),
-                                            _ptr(dx), _stream()))
+                                            _ptr(state.time), _ptr(state.workspace), _ptr(grads), _ptr(dx), _stream()))
     return dx
 
 
@@ -445,16 +440,14 @@ def image_tokenizer_fwd(image: torch.Tensor, params: torch.Tensor, desc: "L.Imag
     assert params.numel() == n, (params.numel(), n)
     p16 = params.to(torch.bfloat16) if params_bf16 is None else params_bf16
     nbytes = int(L.lib().tome_image_tokenizer_workspace_bytes(C.byref(desc)))
-    ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=image.device) if workspace is None else workspace
-    assert ws.numel() >= nbytes + 256
-    off = (-ws.data_ptr()) % 256
+    ws = _scratch(nbytes, image.device, workspace)
     n_patches = (desc.image_size // desc.patch_size) ** 2
     for t in (row_tokens, col_tokens):
         assert t.dtype == torch.int32 and t.is_contiguous() and t.numel() == desc.token_rows * n_patches
     out = torch.empty(desc.batch, desc.n_images, n_patches, desc.embed_dim, device=image.device,
                       dtype=torch.bfloat16 if desc.out_dtype == L.TOME_BF16 else torch.float32)
     L.check(L.lib().tome_image_tokenizer_fwd(C.byref(desc), _ptr(image), _ptr(params), _ptr(p16), _ptr(row_tokens), _ptr(col_tokens),
-                                             _ptr(out), C.c_void_p(ws.data_ptr() + off), nbytes, _stream()))
+                                             _ptr(out), _ptr(ws), nbytes, _stream()))
     return out
 
 
