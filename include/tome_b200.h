@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define TOME_ABI_VERSION 13
+#define TOME_ABI_VERSION 14
 
 enum tome_status { TOME_OK = 0, TOME_ERR_INVALID = 1, TOME_ERR_CUDA = 2, TOME_ERR_UNSUPPORTED = 3 };
 enum tome_dtype { TOME_BF16 = 0, TOME_F32 = 1, TOME_U8 = 2 /* raw pixels: image front end only */ };
@@ -58,9 +58,11 @@ typedef struct {
  * node_max f32 [B,Ta], node_idx i32 [B,Ta]  (Ta = ceil(T/2), Tb = floor(T/2)).
  * scores_out: optional f32 [B,Ta,Tb] dump of the exact fp32 scores the arg max was taken from (parity protocol:
  * "indices bit-exact from the same fp32 scores"); pass NULL on the fast path and the scores never touch HBM.
- * workspace: optional, tome_sim_argmax_workspace_bytes(desc) bytes, 16-byte aligned.  With it the rows are
- * normalised once into fp32 planes and the score kernel streams them; with NULL every
- * CTA normalises the rows it needs itself.  Both normalise first; the workspace path sums even and odd k separately (packed FMAs). */
+ * dim: even, 2 .. 296.  workspace: required, tome_sim_argmax_workspace_bytes(desc) bytes, 16-byte aligned; a NULL or
+ * smaller one is TOME_ERR_INVALID.  The rows are normalised once into the workspace, then scored:
+ *   dim == 64  each row as three bf16 planes (hi + mid + lo: the fp32 value), a b^T on the tensor cores (tcgen05);
+ *   otherwise  fp32 planes, a b^T as fp32 FMAs on CUDA cores (even and odd k summed separately).
+ * (ABI 14: the workspace became required.  Dims 297 .. 448 ran only without a workspace before and are now refused.) */
 size_t tome_sim_argmax_workspace_bytes(const tome_metric_desc_t* desc);
 int tome_sim_argmax(const tome_metric_desc_t* desc, const void* src, float* node_max, int32_t* node_idx,
                     float* scores_out, void* workspace, size_t workspace_bytes, void* stream);
@@ -134,7 +136,6 @@ typedef struct {
   float dropout_rate; uint64_t dropout_seed; uint32_t dropout_site;
   int k_splits;
   int accumulate;
-  int no_multicast; /* debugging aid: 1 disables the CTA-pair TMA multicast of the B operand */
   /* The ReLU gate as one bit per element instead of bf16 rows ([M, ld_bits] u32 words, bit j of word w = column 32 w + j):
    * a ReLU epilogue with relu_bits_out != NULL also writes bit = (output > 0) (after dropout, so the dropped elements are
    * gated too); a later GEMM with gate_bits != NULL multiplies by (bit ? gate_scale : 0) exactly as `gate` would, reading

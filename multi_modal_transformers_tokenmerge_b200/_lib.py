@@ -15,7 +15,7 @@ TOME_OK, TOME_ERR_INVALID, TOME_ERR_CUDA, TOME_ERR_UNSUPPORTED = 0, 1, 2, 3
 TOME_BF16, TOME_F32, TOME_U8 = 0, 1, 2
 TOME_MAJOR_K, TOME_MAJOR_MN = 0, 1
 TOME_MERGE_SUM, TOME_MERGE_WAVG = 0, 1
-ABI_VERSION = 13
+ABI_VERSION = 14
 
 vp, ll, i32, f32, u64, u32 = C.c_void_p, C.c_longlong, C.c_int, C.c_float, C.c_uint64, C.c_uint32
 
@@ -60,7 +60,7 @@ class GemmArgs(C.Structure):
                 ("gate", vp), ("ldg", ll),
                 ("gate_scale", f32), ("relu", i32),
                 ("dropout_rate", f32), ("dropout_seed", u64), ("dropout_site", u32),
-                ("k_splits", i32), ("accumulate", i32), ("no_multicast", i32),
+                ("k_splits", i32), ("accumulate", i32),
                 ("gate_bits", vp), ("relu_bits_out", vp), ("ld_bits", ll), ("colsum_partial", vp),
                 ("a_row_shift", vp), ("a_shift_groups", i32)]
 

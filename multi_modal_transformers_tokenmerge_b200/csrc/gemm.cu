@@ -733,7 +733,7 @@ struct TileChoice { int bn, mode; };   // mode 0: one CTA per tile; 1: CTA pairs
 static TileChoice pick_tile(const tome_gemm_args_t* a) {
   const int m_tiles = ceil_div(a->m, GEMM_BM);
   // CTA pairs: worth it unless an odd, small tile count would leave a large share of dummy tiles
-  const bool pairs_ok = a->no_multicast == 0 && m_tiles >= 2 && (m_tiles % 2 == 0 || m_tiles >= 16);
+  const bool pairs_ok = m_tiles >= 2 && (m_tiles % 2 == 0 || m_tiles >= 16);
   TileChoice t;
   t.bn = pick_bn(a->n);
   t.mode = pairs_ok ? 1 : 0;

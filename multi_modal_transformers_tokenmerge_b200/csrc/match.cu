@@ -39,139 +39,11 @@ __device__ __forceinline__ float2 load2<__nv_bfloat16>(const __nv_bfloat16* p) {
   return __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(p));
 }
 
-// Load `SIM_TILE` metric rows (token = 2*row + parity) into smem as normalised fp32 rows, zero-padded to a multiple of 4
-// columns, pitch = padded dim + 4 floats (16-byte aligned rows; consecutive rows start 4 banks apart).
-template <typename T>
-__device__ __forceinline__ void load_rows_normalised(float* dst, const T* src, const tome_metric_desc_t& d, int b,
-                                                     int row0, int nrows_total, int parity) {
-  // 4 threads per row, all 64 rows of the tile in flight at once (one memory-latency chain per tile)
-  const int rr = threadIdx.x >> 2, part = threadIdx.x & 3;
-  const int dpad = (d.dim + 3) & ~3, pitch = dpad + 4;
-  const float inv_h = 1.0f / (float)d.heads;
-  const int row = row0 + rr;
-  float* drow = dst + rr * pitch;
-  const bool valid = row < nrows_total;  // rows past the end become zero rows; every lane still takes the shuffles
-  const T* base = src + (long long)b * d.batch_stride + (long long)(2 * (valid ? row : 0) + parity) * d.token_stride;
-  float ss = 0.f;
-  for (int c = 2 * part; c < d.dim; c += 8) {
-    float2 acc = make_float2(0.f, 0.f);
-    for (int h = 0; h < (valid ? d.heads : 0); ++h) {
-      const float2 v = load2<T>(base + (long long)h * d.head_stride + c);
-      acc.x += v.x;
-      acc.y += v.y;
-    }
-    if (d.heads > 1) {  // jnp.mean over heads = sum / H
-      acc.x *= inv_h;
-      acc.y *= inv_h;
-    }
-    drow[c] = acc.x;
-    drow[c + 1] = acc.y;
-    ss += acc.x * acc.x + acc.y * acc.y;
-  }
-  ss += __shfl_xor_sync(0xffffffffu, ss, 1);
-  ss += __shfl_xor_sync(0xffffffffu, ss, 2);
-  const float nrm = valid ? sqrtf(ss) : 1.0f;  // no epsilon (token_compression.py:72): a zero row becomes NaN
-  for (int c = 2 * part; c < d.dim; c += 8) {
-    drow[c] = drow[c] / nrm;
-    drow[c + 1] = drow[c + 1] / nrm;
-  }
-  if (part < dpad - d.dim) drow[d.dim + part] = 0.f;
-}
-
-template <typename T>
-__global__ void __launch_bounds__(SIM_THREADS)
-sim_argmax_kernel(const tome_metric_desc_t d, const T* __restrict__ src, float* __restrict__ node_max,
-                  int32_t* __restrict__ node_idx, float* __restrict__ scores_out) {
-  extern __shared__ float4 sm4[];
-  float* sm = reinterpret_cast<float*>(sm4);
-  const int dpad = (d.dim + 3) & ~3, pitch = dpad + 4;
-  float* sa = sm;
-  float* sb = sm + SIM_TILE * pitch;
-  const int b = blockIdx.y;
-  const int ta = (d.tokens + 1) / 2, tb = d.tokens / 2;
-  const int a0 = blockIdx.x * SIM_TILE;
-  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-
-  load_rows_normalised<T>(sa, src, d, b, a0, ta, 0);
-
-  float best_v[4];
-  int best_j[4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    best_v[i] = -INFINITY;
-    best_j[i] = 0x7fffffff;
-  }
-
-  for (int b0 = 0; b0 < tb; b0 += SIM_TILE) {
-    __syncthreads();  // previous tile fully consumed (and sa visible on the first pass)
-    load_rows_normalised<T>(sb, src, d, b, b0, tb, 1);
-    __syncthreads();
-    float acc[4][4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-      for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-    for (int c = 0; c < dpad; c += 4) {  // one 128-bit shared-memory read feeds 4 k-steps: 8 LDS.128 per 64 FMAs
-      float4 av[4], bv[4];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) av[i] = *reinterpret_cast<const float4*>(sa + (ty + 16 * i) * pitch + c);
-#pragma unroll
-      for (int j = 0; j < 4; ++j) bv[j] = *reinterpret_cast<const float4*>(sb + (tx + 16 * j) * pitch + c);
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {  // ascending k, one accumulator: the order of a plain dot product
-          acc[i][j] = fmaf(av[i].x, bv[j].x, acc[i][j]);
-          acc[i][j] = fmaf(av[i].y, bv[j].y, acc[i][j]);
-          acc[i][j] = fmaf(av[i].z, bv[j].z, acc[i][j]);
-          acc[i][j] = fmaf(av[i].w, bv[j].w, acc[i][j]);
-        }
-    }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int ai = a0 + ty + 16 * i;
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const int bj = b0 + tx + 16 * j;
-        if (ai < ta && bj < tb) {
-          float s = acc[i][j];
-          if ((d.class_token && ai == 0) || (d.distill_token && bj == 0)) s = -INFINITY;  // :77-80
-          if (scores_out) scores_out[((long long)b * ta + ai) * tb + bj] = s;
-          if (argmax_better(s, bj, best_v[i], best_j[i])) {
-            best_v[i] = s;
-            best_j[i] = bj;
-          }
-        }
-      }
-    }
-  }
-  // reduce over the 16 tx lanes that share an a-row (contiguous half-warp)
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-#pragma unroll
-    for (int o = 8; o > 0; o >>= 1) {
-      const float ov = __shfl_xor_sync(0xffffffffu, best_v[i], o);
-      const int oj = __shfl_xor_sync(0xffffffffu, best_j[i], o);
-      if (argmax_better(ov, oj, best_v[i], best_j[i])) {
-        best_v[i] = ov;
-        best_j[i] = oj;
-      }
-    }
-    const int ai = a0 + ty + 16 * i;
-    if (tx == 0 && ai < ta) {
-      node_max[(long long)b * ta + ai] = best_v[i];
-      node_idx[(long long)b * ta + ai] = best_j[i] == 0x7fffffff ? 0 : best_j[i];
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------------------ K1, workspace path
-// The kernel above re-reads and re-normalises every b row once per 64-row a tile (5x at T = 536) with the head mean, the
-// square root and the divisions on its critical path: 229 us per layer for 2.4 GFLOP (profiles/r01b_launches_summary.csv).
-// With a workspace the normalisation happens ONCE (metric_norm_kernel: head mean, L2 norm, fp32, a rows and b rows in
-// separate contiguous planes) and the score kernel only streams 16 KB tiles through a cp.async double buffer into the
-// 4x4-per-thread fp32 loop, now on packed f32x2 FMAs (even-k and odd-k partial sums, added at the end).
-// generic version: one warp per token row, 2 columns per lane per step (any even dim <= 512, any even strides)
+// ------------------------------------------------------------------------------------------------ K1, fp32 planes (dim != 64)
+// The rows are normalised ONCE into the workspace (metric_norm_kernel: head mean, L2 norm, fp32, a rows and b rows in
+// separate contiguous planes), so the score kernel only streams 16 KB tiles through a cp.async double buffer into the
+// 4x4-per-thread fp32 loop on packed f32x2 FMAs (even-k and odd-k partial sums, added at the end).
+// generic version: one warp per token row, 2 columns per lane per step (any even dim, any even strides)
 template <typename T>
 __global__ void __launch_bounds__(256)
 metric_norm_kernel(const tome_metric_desc_t d, const T* __restrict__ src, float* __restrict__ plane_a,
@@ -259,6 +131,17 @@ __device__ __forceinline__ void load_tile_async(float* dst, const float* plane, 
     cp_async_16(dst + rr * pitch + 4 * v, plane + (long long)(ok ? r0 + rr : 0) * dpad + 4 * v, ok);
   }
 }
+
+// Dynamic shared memory of sim_argmax_planes_kernel: the a tile and two b tiles of SIM_TILE rows, pitch pad4(dim) + 4 floats.
+// It bounds the metric width the library accepts: the widest even dim whose tiles fit the 227 KB a block may opt into.
+constexpr size_t sim_planes_smem(int dim) { return (size_t)3 * SIM_TILE * (((dim + 3) & ~3) + 4) * sizeof(float); }
+constexpr int sim_max_dim() {
+  int dim = 2;
+  while (sim_planes_smem(dim + 2) <= 232448) dim += 2;
+  return dim;
+}
+constexpr int SIM_MAX_DIM = sim_max_dim();
+static_assert(SIM_MAX_DIM == 296, "include/tome_b200.h states the accepted dims of tome_sim_argmax");
 
 __global__ void __launch_bounds__(SIM_THREADS)
 sim_argmax_planes_kernel(const tome_metric_desc_t d, const float* __restrict__ plane_a, const float* __restrict__ plane_b,
@@ -787,70 +670,52 @@ extern "C" int tome_sim_argmax(const tome_metric_desc_t* d, const void* src, flo
   TOME_CHECK(d && src && node_max && node_idx, TOME_ERR_INVALID, "sim_argmax: null argument");
   TOME_CHECK(d->batch > 0 && d->tokens >= 2 && d->heads >= 1, TOME_ERR_INVALID,
              "sim_argmax: need batch > 0, tokens >= 2, heads >= 1 (got %d, %d, %d)", d->batch, d->tokens, d->heads);
-  TOME_CHECK(d->dim >= 2 && d->dim % 2 == 0 && d->dim <= 512, TOME_ERR_INVALID,
-             "sim_argmax: metric dim must be even and in [2, 512] (got %d)", d->dim);
+  TOME_CHECK(d->dim >= 2 && d->dim % 2 == 0 && d->dim <= SIM_MAX_DIM, TOME_ERR_INVALID,
+             "sim_argmax: metric dim must be even and in [2, %d] (got %d)", SIM_MAX_DIM, d->dim);
   TOME_CHECK(d->dtype == TOME_BF16 || d->dtype == TOME_F32, TOME_ERR_INVALID, "sim_argmax: dtype must be bf16 or f32");
   TOME_CHECK(d->token_stride % 2 == 0 && d->batch_stride % 2 == 0 && d->head_stride % 2 == 0, TOME_ERR_INVALID,
              "sim_argmax: strides must be even (vector loads)");
   TOME_CHECK(d->batch <= 65535, TOME_ERR_INVALID, "sim_argmax: batch too large for one launch");
+  const SimPlanes planes = sim_planes(d, workspace);
+  TOME_CHECK(workspace != nullptr && workspace_bytes >= planes.total && ((uintptr_t)workspace & 15) == 0, TOME_ERR_INVALID,
+             "sim_argmax: workspace must be 16-byte aligned and hold tome_sim_argmax_workspace_bytes = %zu bytes (got %p, %zu bytes)",
+             planes.total, workspace, workspace_bytes);
   const int ta = (d->tokens + 1) / 2, tb = d->tokens / 2;
-  const int dpad = (d->dim + 3) & ~3;
-  dim3 grid(ceil_div(ta, SIM_TILE), d->batch);
-  if (workspace != nullptr) {
-    // ---- normalise once, then stream tiles (see the comment above metric_norm_kernel)
-    const SimPlanes planes = sim_planes(d, workspace);
-    TOME_CHECK(workspace_bytes >= planes.total && ((uintptr_t)workspace & 15) == 0, TOME_ERR_INVALID,
-               "sim_argmax: workspace must be 16-byte aligned and hold %zu bytes (got %zu)", planes.total, workspace_bytes);
-    ProfScope prof(PROF_SIM, 2.0 * d->batch * ta * (double)tb * d->dim, 2, stream);
-    if (sim_tc_eligible(d)) {
-      __nv_bfloat16* pa = reinterpret_cast<__nv_bfloat16*>(planes.a);
-      __nv_bfloat16* pb = reinterpret_cast<__nv_bfloat16*>(planes.b);
-      const long long toks = (long long)d->batch * d->tokens;
-      if (sim_fast64(d, src))
-        launch_k(metric_split64_kernel, (unsigned)((toks * 8 + 255) / 256), 256, 0, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), pa, pb);
-      else if (d->dtype == TOME_BF16)
-        launch_k(metric_split_kernel<__nv_bfloat16>, (unsigned)((toks + 7) / 8), 256, 0, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), pa, pb);
-      else
-        launch_k(metric_split_kernel<float>, (unsigned)((toks + 7) / 8), 256, 0, stream, *d, reinterpret_cast<const float*>(src), pa, pb);
-      TOME_CUDA(cudaGetLastError());
-      CUtensorMap tma_a, tma_b;
-      if (int rc = make_tmap_3d_bf16(&tma_a, pa, SIMT_ROW, ta, d->batch, SIMT_ROW, (uint64_t)ta * SIMT_ROW, SIMT_BM)) return rc;
-      if (int rc = make_tmap_3d_bf16(&tma_b, pb, SIMT_ROW, tb, d->batch, SIMT_ROW, (uint64_t)tb * SIMT_ROW, SIMT_BN)) return rc;
-      static DynSmemOnce once;
-      TOME_CUDA(ensure_dyn_smem(sim_argmax_tc_kernel, SIMT_SMEM, once));
-      TOME_CUDA(launch_k(sim_argmax_tc_kernel, dim3(ceil_div(ta, SIMT_BM), d->batch), SIMT_THREADS, SIMT_SMEM, stream, tma_a, tma_b, *d,
-                         node_max, node_idx, scores_out));
-      return TOME_OK;
-    }
-    float* plane_a = reinterpret_cast<float*>(planes.a);
-    float* plane_b = reinterpret_cast<float*>(planes.b);
-    const long long toks = (long long)d->batch * d->tokens;
-    const unsigned nblk = (unsigned)((toks + 7) / 8);
+  const long long toks = (long long)d->batch * d->tokens;
+  ProfScope prof(PROF_SIM, 2.0 * d->batch * ta * (double)tb * d->dim, 2, stream);
+  if (sim_tc_eligible(d)) {
+    __nv_bfloat16* pa = reinterpret_cast<__nv_bfloat16*>(planes.a);
+    __nv_bfloat16* pb = reinterpret_cast<__nv_bfloat16*>(planes.b);
     if (sim_fast64(d, src))
-      launch_k(metric_norm64_kernel, (unsigned)((toks * 8 + 255) / 256), 256, 0, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), plane_a, plane_b);
+      launch_k(metric_split64_kernel, (unsigned)((toks * 8 + 255) / 256), 256, 0, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), pa, pb);
     else if (d->dtype == TOME_BF16)
-      launch_k(metric_norm_kernel<__nv_bfloat16>, nblk, 256, 0, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), plane_a, plane_b);
+      launch_k(metric_split_kernel<__nv_bfloat16>, (unsigned)((toks + 7) / 8), 256, 0, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), pa, pb);
     else
-      launch_k(metric_norm_kernel<float>, nblk, 256, 0, stream, *d, reinterpret_cast<const float*>(src), plane_a, plane_b);
+      launch_k(metric_split_kernel<float>, (unsigned)((toks + 7) / 8), 256, 0, stream, *d, reinterpret_cast<const float*>(src), pa, pb);
     TOME_CUDA(cudaGetLastError());
-    const size_t smem = (size_t)3 * SIM_TILE * (dpad + 4) * sizeof(float);
-    TOME_CUDA(cudaFuncSetAttribute(sim_argmax_planes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    launch_k(sim_argmax_planes_kernel, grid, SIM_THREADS, smem, stream, *d, plane_a, plane_b, node_max, node_idx, scores_out);
-    TOME_CUDA(cudaGetLastError());
+    CUtensorMap tma_a, tma_b;
+    if (int rc = make_tmap_3d_bf16(&tma_a, pa, SIMT_ROW, ta, d->batch, SIMT_ROW, (uint64_t)ta * SIMT_ROW, SIMT_BM)) return rc;
+    if (int rc = make_tmap_3d_bf16(&tma_b, pb, SIMT_ROW, tb, d->batch, SIMT_ROW, (uint64_t)tb * SIMT_ROW, SIMT_BN)) return rc;
+    static DynSmemOnce once;
+    TOME_CUDA(ensure_dyn_smem(sim_argmax_tc_kernel, SIMT_SMEM, once));
+    TOME_CUDA(launch_k(sim_argmax_tc_kernel, dim3(ceil_div(ta, SIMT_BM), d->batch), SIMT_THREADS, SIMT_SMEM, stream, tma_a, tma_b, *d,
+                       node_max, node_idx, scores_out));
     return TOME_OK;
   }
-  const size_t smem = (size_t)2 * SIM_TILE * (dpad + 4) * sizeof(float);
-  ProfScope prof(PROF_SIM, 2.0 * d->batch * ta * (double)tb * d->dim, 1, stream);
-  if (d->dtype == TOME_BF16) {
-    auto kern = sim_argmax_kernel<__nv_bfloat16>;
-    TOME_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    launch_k(kern, grid, SIM_THREADS, smem, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), node_max, node_idx,
-                                              scores_out);
-  } else {
-    auto kern = sim_argmax_kernel<float>;
-    TOME_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    launch_k(kern, grid, SIM_THREADS, smem, stream, *d, reinterpret_cast<const float*>(src), node_max, node_idx, scores_out);
-  }
+  float* plane_a = reinterpret_cast<float*>(planes.a);
+  float* plane_b = reinterpret_cast<float*>(planes.b);
+  const unsigned nblk = (unsigned)((toks + 7) / 8);
+  if (sim_fast64(d, src))
+    launch_k(metric_norm64_kernel, (unsigned)((toks * 8 + 255) / 256), 256, 0, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), plane_a, plane_b);
+  else if (d->dtype == TOME_BF16)
+    launch_k(metric_norm_kernel<__nv_bfloat16>, nblk, 256, 0, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), plane_a, plane_b);
+  else
+    launch_k(metric_norm_kernel<float>, nblk, 256, 0, stream, *d, reinterpret_cast<const float*>(src), plane_a, plane_b);
+  TOME_CUDA(cudaGetLastError());
+  const size_t smem = sim_planes_smem(d->dim);
+  TOME_CUDA(cudaFuncSetAttribute(sim_argmax_planes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  launch_k(sim_argmax_planes_kernel, dim3(ceil_div(ta, SIM_TILE), d->batch), SIM_THREADS, smem, stream, *d, plane_a, plane_b,
+           node_max, node_idx, scores_out);
   TOME_CUDA(cudaGetLastError());
   return TOME_OK;
 }

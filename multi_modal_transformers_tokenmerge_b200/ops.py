@@ -85,9 +85,8 @@ def _scratch(nbytes: int, device, buf: Optional[torch.Tensor] = None) -> torch.T
 
 def sim_argmax(src: torch.Tensor, *, heads: int = 1, dim: Optional[int] = None, batch_stride=None, token_stride=None,
                head_stride=None, tokens=None, batch=None, class_token=False, distill_token=False, dump_scores=False,
-               offset_elems: int = 0, use_workspace: bool = True):
-    """K1.  `src` is either a [B,T,Dm] metric (heads=1) or a packed buffer addressed by the given strides.
-    `use_workspace=False` takes the library's no-scratch path (every CTA normalises its own rows)."""
+               offset_elems: int = 0):
+    """K1.  `src` is either a [B,T,Dm] metric (heads=1) or a packed buffer addressed by the given strides."""
     _need_cuda(src)
     if heads == 1 and dim is None:
         assert src.dim() == 3 and src.is_contiguous()
@@ -100,9 +99,9 @@ def sim_argmax(src: torch.Tensor, *, heads: int = 1, dim: Optional[int] = None, 
     d = L.MetricDesc(batch, tokens, dim, heads, _dt(src), batch_stride, token_stride, head_stride,
                      int(bool(class_token)), int(bool(distill_token)))
     base = C.c_void_p(src.data_ptr() + offset_elems * src.element_size())
-    ws = _scratch(L.lib().tome_sim_argmax_workspace_bytes(C.byref(d)), src.device) if use_workspace else None
-    L.check(L.lib().tome_sim_argmax(C.byref(d), base, _ptr(node_max), _ptr(node_idx), _ptr(scores), _ptr(ws),
-                                    0 if ws is None else ws.numel(), _stream()))
+    ws = _scratch(L.lib().tome_sim_argmax_workspace_bytes(C.byref(d)), src.device)
+    L.check(L.lib().tome_sim_argmax(C.byref(d), base, _ptr(node_max), _ptr(node_idx), _ptr(scores), _ptr(ws), ws.numel(),
+                                    _stream()))
     return node_max, node_idx, scores
 
 
@@ -177,7 +176,7 @@ def topk_prune(emb: torch.Tensor, importance: torch.Tensor, set_start, set_n, se
 def gemm(a: torch.Tensor, b: torch.Tensor, *, m: int, n: int, k: int, a_major=L.TOME_MAJOR_K, b_major=L.TOME_MAJOR_K,
          lda=None, ldb=None, out: Optional[torch.Tensor] = None, out_dtype=torch.bfloat16, bias=None, residual=None,
          gate=None, gate_scale=1.0, relu=False, dropout_rate=0.0, dropout_seed=0, dropout_site=0, k_splits=0,
-         accumulate=False, no_multicast=False, gate_bits: Optional[torch.Tensor] = None,
+         accumulate=False, gate_bits: Optional[torch.Tensor] = None,
          relu_bits_out: Optional[torch.Tensor] = None, colsum_partial: Optional[torch.Tensor] = None,
          a_row_shift=None) -> torch.Tensor:
     """C[M,N] = epilogue(A * B^T) on tcgen05.  a/b are 2-D bf16 tensors whose rows are M/N (K-major) or K (MN-major).
@@ -195,7 +194,7 @@ def gemm(a: torch.Tensor, b: torch.Tensor, *, m: int, n: int, k: int, a_major=L.
                       None if residual is None else residual.data_ptr(), 0 if residual is None else residual.stride(0),
                       None if gate is None else gate.data_ptr(), 0 if gate is None else gate.stride(0),
                       float(gate_scale), int(relu), float(dropout_rate), int(dropout_seed), int(dropout_site),
-                      int(k_splits), int(accumulate), int(no_multicast),
+                      int(k_splits), int(accumulate),
                       None if gate_bits is None else gate_bits.data_ptr(),
                       None if relu_bits_out is None else relu_bits_out.data_ptr(),
                       0 if (gate_bits is None and relu_bits_out is None) else (gate_bits if gate_bits is not None else relu_bits_out).stride(0),

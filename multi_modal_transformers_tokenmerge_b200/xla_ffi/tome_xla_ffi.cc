@@ -12,6 +12,7 @@
 // and register from Python with tome_jax.py (same directory).  INTEGRATION.md shows the Flax-side wiring.
 #include <cstdint>
 #include <cstring>
+#include <optional>
 
 #include <cuda_runtime_api.h>
 
@@ -27,16 +28,20 @@ static ffi::Error Status(int rc) {
 static int DType(ffi::DataType t) { return t == ffi::DataType::BF16 ? TOME_BF16 : TOME_F32; }
 
 // ---- tome_sim_argmax: metric [B,T,Dm] -> node_max f32 [B,Ta], node_idx s32 [B,Ta]        token_compression.py:72-83
-static ffi::Error SimArgmax(cudaStream_t s, ffi::AnyBuffer metric, ffi::Result<ffi::Buffer<ffi::F32>> node_max,
-                            ffi::Result<ffi::Buffer<ffi::S32>> node_idx, int32_t class_token, int32_t distill_token) {
+// workspace: tome_sim_argmax_workspace_bytes(desc) bytes from XLA's scratch allocator
+static ffi::Error SimArgmax(cudaStream_t s, ffi::ScratchAllocator scratch, ffi::AnyBuffer metric,
+                            ffi::Result<ffi::Buffer<ffi::F32>> node_max, ffi::Result<ffi::Buffer<ffi::S32>> node_idx,
+                            int32_t class_token, int32_t distill_token) {
   auto d = metric.dimensions();
   tome_metric_desc_t m{(int)d[0], (int)d[1], (int)d[2], 1, DType(metric.element_type()), (long long)(d[1] * d[2]), (long long)d[2], 0,
                        class_token, distill_token};
-  return Status(tome_sim_argmax(&m, metric.untyped_data(), node_max->typed_data(), node_idx->typed_data(), nullptr,
-                                /*workspace=*/nullptr, 0, s));  // no-scratch path; add a u8 Ret buffer to take the faster one
+  const size_t ws_bytes = tome_sim_argmax_workspace_bytes(&m);
+  std::optional<void*> ws = scratch.Allocate(ws_bytes, 256);
+  if (!ws.has_value()) return ffi::Error(ffi::ErrorCode::kResourceExhausted, "tome_sim_argmax: scratch allocation failed");
+  return Status(tome_sim_argmax(&m, metric.untyped_data(), node_max->typed_data(), node_idx->typed_data(), nullptr, *ws, ws_bytes, s));
 }
 XLA_FFI_DEFINE_HANDLER_SYMBOL(TomeSimArgmax, SimArgmax,
-                              ffi::Ffi::Bind().Ctx<ffi::PlatformStream<cudaStream_t>>().Arg<ffi::AnyBuffer>()
+                              ffi::Ffi::Bind().Ctx<ffi::PlatformStream<cudaStream_t>>().Ctx<ffi::ScratchAllocator>().Arg<ffi::AnyBuffer>()
                                   .Ret<ffi::Buffer<ffi::F32>>().Ret<ffi::Buffer<ffi::S32>>()
                                   .Attr<int32_t>("class_token").Attr<int32_t>("distill_token"));
 

@@ -35,7 +35,7 @@ def test_every_declared_symbol_is_exported(lib):
 def test_abi_version_and_struct_sizes(lib):
     from multi_modal_transformers_tokenmerge_b200 import _lib as L
     assert lib.tome_abi_version() == L.ABI_VERSION
-    # layout agreement between the ctypes mirrors and the C structs is checked through behaviour below; sizes are sane
+    # field-by-field layout agreement with the C structs: test_ctypes_mirrors_match_header_layout; sizes are sane
     assert C.sizeof(L.GemmArgs) % 8 == 0 and C.sizeof(L.AttnDesc) % 8 == 0 and C.sizeof(L.StackCfg) % 8 == 0
 
 
@@ -117,6 +117,16 @@ def test_validation_errors_are_reported_not_thrown(lib):
     assert b"mode" in lib.tome_last_error()
     d = L.AttnDesc(1, 8, 1, 260, 0, 0, 0, 0, 0, 0, 0, 0, 1.0, None, None, None, 0, None)  # head_dim 260: not a multiple of 8
     assert lib.tome_attention_fwd(C.byref(d), None, None, None, None, None, None, 0, None) == L.TOME_ERR_UNSUPPORTED
+    # tome_sim_argmax refuses these before any CUDA call, so the (16-byte aligned) fake device pointers are never touched
+    fake = C.c_void_p(1 << 20)
+    for dim, ws, ws_delta, msg in ((64, None, 0, b"tome_sim_argmax_workspace_bytes"),   # the workspace is required
+                                   (64, fake, -1, b"tome_sim_argmax_workspace_bytes"),   # one byte short
+                                   (48, fake, -1, b"tome_sim_argmax_workspace_bytes"),
+                                   (298, fake, 0, b"metric dim")):                       # planes tiles exceed 227 KB of smem
+        d = L.MetricDesc(2, 64, dim, 1, L.TOME_BF16, 64 * dim, dim, 0, 0, 0)
+        ws_bytes = lib.tome_sim_argmax_workspace_bytes(C.byref(d)) + ws_delta
+        assert lib.tome_sim_argmax(C.byref(d), fake, fake, fake, None, ws, ws_bytes, None) == L.TOME_ERR_INVALID, (dim, ws_delta)
+        assert msg in lib.tome_last_error(), (dim, ws_delta, lib.tome_last_error())
 
 
 def test_product_path_has_no_cpu_fallback():
@@ -200,3 +210,34 @@ def test_header_is_plain_c(tmp_path):
                    '(void)g; (void)c; (void)d; return TOME_ABI_VERSION > 0 ? 0 : 1; }\n')
     r = subprocess.run(["gcc", "-std=c99", "-Wall", "-Werror", "-fsyntax-only", f"-I{root}", str(src)], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
+
+
+def test_ctypes_mirrors_match_header_layout(tmp_path):
+    """Every struct _lib.py mirrors has the header's size, and every mirrored field the header's offset and size, as gcc
+    lays them out (a field that moves into or out of padding changes no size, so behaviour alone would not show it)."""
+    import shutil
+    import subprocess
+    from multi_modal_transformers_tokenmerge_b200 import _lib as L
+    if shutil.which("gcc") is None:
+        pytest.skip("no gcc")
+    mirrors = {"tome_metric_desc_t": L.MetricDesc, "tome_plan_t": L.Plan, "tome_plan_shape_t": L.PlanShape,
+               "tome_prune_desc_t": L.PruneDesc, "tome_merge_shape_t": L.MergeShape, "tome_gemm_args_t": L.GemmArgs,
+               "tome_attn_desc_t": L.AttnDesc, "tome_attn_grad_strides_t": L.AttnGradStrides, "tome_stack_cfg_t": L.StackCfg,
+               "tome_diffusion_desc_t": L.DiffusionDesc, "tome_image_tokenizer_desc_t": L.ImageTokenizerDesc,
+               "tome_head_desc_t": L.HeadDesc, "tome_stack_io_t": L.StackIO}
+    lines, want = [], []
+    for cname, cls in mirrors.items():
+        lines.append(f'printf("{cname} %zu\\n", sizeof({cname}));')
+        want.append(f"{cname} {C.sizeof(cls)}")
+        for fname, _ in cls._fields_:
+            lines.append(f'printf("{cname}.{fname} %zu %zu\\n", offsetof({cname}, {fname}), sizeof((({cname}*)0)->{fname}));')
+            f = getattr(cls, fname)
+            want.append(f"{cname}.{fname} {f.offset} {f.size}")
+    src = tmp_path / "layout.c"
+    src.write_text('#include <stddef.h>\n#include <stdio.h>\n#include "include/tome_b200.h"\nint main(void) {\n' + "\n".join(lines) +
+                   "\nreturn 0;\n}\n")
+    exe = tmp_path / "layout"
+    r = subprocess.run(["gcc", "-std=c99", "-Wall", "-Werror", f"-I{ROOT}", str(src), "-o", str(exe)], capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr
+    got = subprocess.run([str(exe)], capture_output=True, text=True, check=True).stdout.splitlines()
+    assert got == want

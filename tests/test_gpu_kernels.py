@@ -365,22 +365,19 @@ def test_attention_fwd_lazy_rescale(ops, T, growth):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("B,T,H,D", [(3, 536, 6, 64), (2, 75, 1, 30), (2, 300, 3, 128)])
-def test_sim_argmax_workspace_and_scratchless_paths_agree(ops, B, T, H, D):
-    """tome_sim_argmax has two code paths (normalise once into a workspace, or normalise inside every CTA); both follow the
-    reference order (normalise, then an ascending-k fp32 dot product), so their scores agree to fp32 rounding of the
-    norm and each path's arg max is the exact first maximum of ITS OWN dumped scores."""
+@pytest.mark.parametrize("B,T,H,D", [(3, 536, 6, 64), (2, 75, 1, 30), (2, 300, 3, 128), (2, 64, 1, 296)])
+def test_sim_argmax_scores_match_reference(ops, B, T, H, D):
+    """tome_sim_argmax on both of its paths (tcgen05 for dim 64, fp32 planes otherwise, up to the widest accepted dim 296):
+    the dumped scores match the reference's fp32 similarity of the head-mean metric, and the arg max is the exact first
+    maximum of the kernel's own dumped scores."""
     rng = np.random.default_rng(B * T + D)
     src = torch.tensor(rng.standard_normal((B, T, H, D)).astype(np.float32)).cuda().bfloat16()
-    kw = dict(heads=H, dim=D, batch=B, tokens=T, batch_stride=T * H * D, token_stride=H * D, head_stride=D, dump_scores=True)
-    nm1, ni1, sc1 = ops.sim_argmax(src, use_workspace=True, **kw)
-    nm0, ni0, sc0 = ops.sim_argmax(src, use_workspace=False, **kw)
-    torch.cuda.synchronize()
-    assert (sc1 - sc0).abs().max().item() <= 2e-6
-    for nm, ni, sc in ((nm1, ni1, sc1), (nm0, ni0, sc0)):
-        s = sc.cpu().numpy()
-        np.testing.assert_array_equal(ni.cpu().numpy(), s.argmax(-1).astype(np.int32))
-        np.testing.assert_array_equal(nm.cpu().numpy(), s.max(-1))
+    nm, ni, sc = ops.sim_argmax(src, heads=H, dim=D, batch=B, tokens=T, batch_stride=T * H * D, token_stride=H * D, head_stride=D,
+                                dump_scores=True)
+    s = sc.cpu().numpy()
+    np.testing.assert_allclose(s, O.similarity_scores(src.float().mean(dim=2).cpu().numpy()), atol=2e-5, rtol=0)
+    np.testing.assert_array_equal(ni.cpu().numpy(), s.argmax(-1).astype(np.int32))
+    np.testing.assert_array_equal(nm.cpu().numpy(), s.max(-1))
 
 
 # ------------------------------------------------------------------------------------------------ top-k pruning
