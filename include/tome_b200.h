@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define TOME_ABI_VERSION 14
+#define TOME_ABI_VERSION 15
 
 enum tome_status { TOME_OK = 0, TOME_ERR_INVALID = 1, TOME_ERR_CUDA = 2, TOME_ERR_UNSUPPORTED = 3 };
 enum tome_dtype { TOME_BF16 = 0, TOME_F32 = 1, TOME_U8 = 2 /* raw pixels: image front end only */ };
@@ -43,6 +43,22 @@ int tome_abi_version(void);
 /* r = min(r, (tokens - protected) / 2), clamped at 0            token_compression.py:60-67 */
 int tome_clamp_r(int tokens, int r, int class_token, int distill_token);
 
+/* Token sets for matching INSIDE each set (ABI 15): the sequence is n_sets consecutive sets in order, set s holding tokens
+ * [set_start[s], set_start[s] + set_n[s]), set_start[0] = 0, the sets covering `tokens` without gap or overlap.  Set s loses
+ * set_r[s] tokens, 0 <= set_r[s] <= set_n[s] / 2: its part of the output is bipartite_soft_matching + merge of the set's
+ * slice on its own (even / odd split relative to set_start[s], the same tie rules and fp32 rank-order adds), the parts
+ * concatenated in set order; a set with set_r[s] == 0 is copied unchanged.  So a token never merges with a token of another
+ * set: with one set per frame and modality the block-causal group mask keeps holding after a merge.  Not combinable with
+ * class_token / distill_token (TOME_ERR_INVALID).  A NULL `sets` pointer below means one set spanning the sequence: the
+ * behaviour and results of ABI 14. */
+#define TOME_MAX_TOKEN_SETS 16
+typedef struct {
+  int n_sets;
+  int set_start[TOME_MAX_TOKEN_SETS];
+  int set_n[TOME_MAX_TOKEN_SETS];
+  int set_r[TOME_MAX_TOKEN_SETS];
+} tome_token_sets_t;
+
 /* Where the matching metric comes from.  metric[b,t,d] = (1/heads) * sum_h src[b,t,h,d]; with heads == 1 this is a
  * plain [B,T,Dm] tensor (the `metric` argument of bipartite_soft_matching); with heads > 1 it is "keys averaged
  * over heads" read in place from a packed qkv buffer (intended call site tome_attention.py:249-256). */
@@ -51,11 +67,15 @@ typedef struct {
   int dtype; /* tome_dtype of src */
   long long batch_stride, token_stride, head_stride;
   int class_token, distill_token;
+  const tome_token_sets_t* sets; /* NULL: one set (set_r is ignored here apart from its range check) */
 } tome_metric_desc_t;
 
 /* L2-normalise rows (no epsilon), split even/odd, scores = a b^T in fp32, protect row/column 0, then
  * node_max[b,i] = max_j scores, node_idx[b,i] = first arg max.                       token_compression.py:72-83
  * node_max f32 [B,Ta], node_idx i32 [B,Ta]  (Ta = ceil(T/2), Tb = floor(T/2)).
+ * With sets: every set is scored against its own odd tokens only; node_max / node_idx are [B, sum_s ceil(n_s/2)], set after
+ * set, node_idx local to the set; scores_out is [B, sum_s ceil(n_s/2) * floor(n_s/2)], each set's [ceil, floor] block in
+ * turn.  A one-token set has no partner: node_max = -inf, node_idx = 0.
  * scores_out: optional f32 [B,Ta,Tb] dump of the exact fp32 scores the arg max was taken from (parity protocol:
  * "indices bit-exact from the same fp32 scores"); pass NULL on the fast path and the scores never touch HBM.
  * dim: even, 2 .. 296.  workspace: required, tome_sim_argmax_workspace_bytes(desc) bytes, 16-byte aligned; a NULL or
@@ -77,10 +97,14 @@ typedef struct {
   int32_t* dst_off;  /* [B,Tb+1] CSR offsets: sources merged into odd token j are dst_src[dst_off[j]..)     */
   int32_t* dst_src;  /* [B,r]    even-set indices grouped by destination, in rank order inside a group      */
 } tome_plan_t;
+/* With sets the arrays are concatenated set by set inside each batch row, indices local to the set: edge_idx [B, sum
+ * ceil(n_s/2)] (the identity order for a set with r = 0), dst_idx / dst_src [B, sum r_s], dst_off [B, sum (floor(n_s/2) + 1)];
+ * row_map [B,T] holds GLOBAL output rows, so tome_merge_bwd and tome_chain_row_maps read it as they read a one-set plan. */
 
 typedef struct {
-  int batch, tokens, r; /* r already clamped (tome_clamp_r), r >= 1 */
+  int batch, tokens, r; /* r already clamped (tome_clamp_r), r >= 1; with sets: sum_s set_r[s] */
   int distill_token;
+  const tome_token_sets_t* sets; /* NULL: one set */
 } tome_plan_shape_t;
 
 /* Edge ranking and index split.                                                       token_compression.py:84-88 */
@@ -95,6 +119,7 @@ typedef struct {
   int distill_token;
   int dtype; /* of x / x_out / dy / dx */
   int mode;  /* TOME_MERGE_SUM: merge(x, "sum") :90-109;  TOME_MERGE_WAVG: merge_wavg :114-129 */
+  const tome_token_sets_t* sets; /* NULL: one set; else r = sum_s set_r[s] and the plan has the per-set layout above */
 } tome_merge_shape_t;
 
 /* x [B,T,C] -> x_out [B,T-r,C].  WAVG: x_out = merge(x*size)/merge(size), size_out = merge(size), fp32 arithmetic in
@@ -260,7 +285,6 @@ int tome_attention_bwd(const tome_attn_desc_t* desc, const tome_attn_grad_stride
  * 5b. Per-modality top-k pruning       tokenizers/token_compression.py:15-46 (compute_top_k_tokens): the sibling
  *                                      compression path of SURVEY.md 8(f) rank 2
  * ------------------------------------------------------------------------------------------------------------ */
-#define TOME_MAX_TOKEN_SETS 16
 typedef struct {
   int batch, tokens, channels;
   int dtype;        /* tome_dtype of the embeddings */
@@ -445,6 +469,11 @@ typedef struct {
   int prune_set_n[TOME_MAX_TOKEN_SETS];
   int prune_set_c[TOME_MAX_TOKEN_SETS];
   int prune_importance;
+  /* set_merge != 0 (with prune_sets > 0): every layer MERGES prune_set_c[i] tokens inside set i instead of pruning them --
+   * bipartite soft matching on the keys averaged over heads, merge_wavg after the attention residual, sizes carried (prop_attn
+   * allowed), group id / position carried as by the global merge (tome_token_sets_t).  r must be 0, no class / distill token,
+   * prune_set_c[i] <= floor(n_i(l) / 2) at every layer l, and layer_gid / layer_pos are not taken. */
+  int set_merge;
 } tome_stack_cfg_t;
 
 /* Per-layer parameter offsets (elements) into one flat fp32 vector (master weights / gradients / Adam moments)

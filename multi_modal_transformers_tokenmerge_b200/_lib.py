@@ -15,7 +15,7 @@ TOME_OK, TOME_ERR_INVALID, TOME_ERR_CUDA, TOME_ERR_UNSUPPORTED = 0, 1, 2, 3
 TOME_BF16, TOME_F32, TOME_U8 = 0, 1, 2
 TOME_MAJOR_K, TOME_MAJOR_MN = 0, 1
 TOME_MERGE_SUM, TOME_MERGE_WAVG = 0, 1
-ABI_VERSION = 14
+ABI_VERSION = 15
 
 vp, ll, i32, f32, u64, u32 = C.c_void_p, C.c_longlong, C.c_int, C.c_float, C.c_uint64, C.c_uint32
 
@@ -26,10 +26,19 @@ class TomeError(RuntimeError):
         self.code = code
 
 
+MAX_TOKEN_SETS = 16
+
+
+class TokenSets(C.Structure):
+    """tome_token_sets_t: consecutive token sets covering the sequence; set s loses set_r[s] tokens to merging inside it."""
+    _fields_ = [("n_sets", i32), ("set_start", i32 * MAX_TOKEN_SETS), ("set_n", i32 * MAX_TOKEN_SETS),
+                ("set_r", i32 * MAX_TOKEN_SETS)]
+
+
 class MetricDesc(C.Structure):
     _fields_ = [("batch", i32), ("tokens", i32), ("dim", i32), ("heads", i32), ("dtype", i32),
                 ("batch_stride", ll), ("token_stride", ll), ("head_stride", ll),
-                ("class_token", i32), ("distill_token", i32)]
+                ("class_token", i32), ("distill_token", i32), ("sets", vp)]
 
 
 class Plan(C.Structure):
@@ -37,7 +46,7 @@ class Plan(C.Structure):
 
 
 class PlanShape(C.Structure):
-    _fields_ = [("batch", i32), ("tokens", i32), ("r", i32), ("distill_token", i32)]
+    _fields_ = [("batch", i32), ("tokens", i32), ("r", i32), ("distill_token", i32), ("sets", vp)]
 
 
 class PruneDesc(C.Structure):
@@ -47,7 +56,7 @@ class PruneDesc(C.Structure):
 
 class MergeShape(C.Structure):
     _fields_ = [("batch", i32), ("tokens", i32), ("channels", i32), ("r", i32), ("distill_token", i32),
-                ("dtype", i32), ("mode", i32)]
+                ("dtype", i32), ("mode", i32), ("sets", vp)]
 
 
 class GemmArgs(C.Structure):
@@ -88,7 +97,8 @@ class StackCfg(C.Structure):
                 ("head", i32), ("head_groups", i32), ("head_features", i32), ("max_action", f32),
                 ("head_fourier_dim", i32), ("head_time_hidden", i32), ("head_time_out", i32), ("head_hidden", i32),
                 ("diffusion_steps", i32),
-                ("prune_sets", i32), ("prune_set_n", i32 * 16), ("prune_set_c", i32 * 16), ("prune_importance", i32)]
+                ("prune_sets", i32), ("prune_set_n", i32 * 16), ("prune_set_c", i32 * 16), ("prune_importance", i32),
+                ("set_merge", i32)]
 
 
 IMPORTANCE_ROW_MEAN, IMPORTANCE_RECEIVED = 0, 1

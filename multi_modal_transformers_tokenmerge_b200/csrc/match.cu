@@ -11,6 +11,7 @@
 // reference; the scores tile lives in registers and never reaches HBM unless scores_out is given.
 #include "common.cuh"
 #include "host_util.h"
+#include "token_sets.cuh"
 
 namespace tome {
 
@@ -46,16 +47,18 @@ __device__ __forceinline__ float2 load2<__nv_bfloat16>(const __nv_bfloat16* p) {
 // generic version: one warp per token row, 2 columns per lane per step (any even dim, any even strides)
 template <typename T>
 __global__ void __launch_bounds__(256)
-metric_norm_kernel(const tome_metric_desc_t d, const T* __restrict__ src, float* __restrict__ plane_a,
-                   float* __restrict__ plane_b) {
+metric_norm_kernel(const tome_metric_desc_t d, const __grid_constant__ SetTable tab, const T* __restrict__ src,
+                   float* __restrict__ plane_a, float* __restrict__ plane_b) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long tok = (long long)blockIdx.x * 8 + warp;   // b * T + t
   if (tok >= (long long)d.batch * d.tokens) return;
   const int b = (int)(tok / d.tokens), t = (int)(tok % d.tokens);
   const int dpad = (d.dim + 3) & ~3;
-  const int ta = (d.tokens + 1) / 2, tb = d.tokens / 2;
+  const int ta = tab.a_off[tab.n], tb = tab.b_off[tab.n];
   const T* base = src + (long long)b * d.batch_stride + (long long)t * d.token_stride;
-  float* out = (t & 1) ? plane_b + ((long long)b * tb + (t >> 1)) * dpad : plane_a + ((long long)b * ta + (t >> 1)) * dpad;
+  bool odd;
+  const int pr = set_plane_row(tab, t, odd);
+  float* out = odd ? plane_b + ((long long)b * tb + pr) * dpad : plane_a + ((long long)b * ta + pr) * dpad;
   const float inv_h = 1.0f / (float)d.heads;
   float ss = 0.f;
   for (int c = 2 * lane; c < d.dim; c += 64) {  // pass 1: head mean -> out (un-normalised), sum of squares
@@ -82,14 +85,14 @@ metric_norm_kernel(const tome_metric_desc_t d, const T* __restrict__ src, float*
 
 // bf16, dim == 64, 16-byte aligned rows (the stack's case): 8 lanes per token row, one 128-bit load per head per lane
 __global__ void __launch_bounds__(256)
-metric_norm64_kernel(const tome_metric_desc_t d, const __nv_bfloat16* __restrict__ src, float* __restrict__ plane_a,
-                     float* __restrict__ plane_b) {
+metric_norm64_kernel(const tome_metric_desc_t d, const __grid_constant__ SetTable tab, const __nv_bfloat16* __restrict__ src,
+                     float* __restrict__ plane_a, float* __restrict__ plane_b) {
   const long long tok = ((long long)blockIdx.x * 256 + threadIdx.x) >> 3;   // b * T + t
   const int sub = threadIdx.x & 7;
   const bool valid = tok < (long long)d.batch * d.tokens;   // every lane stays for the shuffles
   const long long tk = valid ? tok : 0;
   const int b = (int)(tk / d.tokens), t = (int)(tk % d.tokens);
-  const int ta = (d.tokens + 1) / 2, tb = d.tokens / 2;
+  const int ta = tab.a_off[tab.n], tb = tab.b_off[tab.n];
   const __nv_bfloat16* base = src + (long long)b * d.batch_stride + (long long)t * d.token_stride + sub * 8;
   float acc[8];
 #pragma unroll
@@ -111,7 +114,9 @@ metric_norm64_kernel(const tome_metric_desc_t d, const __nv_bfloat16* __restrict
   ss += __shfl_xor_sync(0xffffffffu, ss, 4);
   const float nrm = sqrtf(ss);
   if (valid) {
-    float* out = ((t & 1) ? plane_b + ((long long)b * tb + (t >> 1)) * 64 : plane_a + ((long long)b * ta + (t >> 1)) * 64) + sub * 8;
+    bool odd;
+    const int pr = set_plane_row(tab, t, odd);
+    float* out = (odd ? plane_b + ((long long)b * tb + pr) * 64 : plane_a + ((long long)b * ta + pr) * 64) + sub * 8;
     reinterpret_cast<float4*>(out)[0] = make_float4(acc[0] / nrm, acc[1] / nrm, acc[2] / nrm, acc[3] / nrm);
     reinterpret_cast<float4*>(out)[1] = make_float4(acc[4] / nrm, acc[5] / nrm, acc[6] / nrm, acc[7] / nrm);
   }
@@ -144,19 +149,24 @@ constexpr int SIM_MAX_DIM = sim_max_dim();
 static_assert(SIM_MAX_DIM == 296, "include/tome_b200.h states the accepted dims of tome_sim_argmax");
 
 __global__ void __launch_bounds__(SIM_THREADS)
-sim_argmax_planes_kernel(const tome_metric_desc_t d, const float* __restrict__ plane_a, const float* __restrict__ plane_b,
-                         float* __restrict__ node_max, int32_t* __restrict__ node_idx, float* __restrict__ scores_out) {
+sim_argmax_planes_kernel(const tome_metric_desc_t d, const __grid_constant__ SetTable tab, const float* __restrict__ plane_a,
+                         const float* __restrict__ plane_b, float* __restrict__ node_max, int32_t* __restrict__ node_idx,
+                         float* __restrict__ scores_out) {
   extern __shared__ float4 sm4[];
   float* sm = reinterpret_cast<float*>(sm4);
   const int dpad = (d.dim + 3) & ~3, pitch = dpad + 4;
   float* sa = sm;
   float* sb0 = sm + SIM_TILE * pitch;
   const int b = blockIdx.y;
-  const int ta = (d.tokens + 1) / 2, tb = d.tokens / 2;
-  const int a0 = blockIdx.x * SIM_TILE;
+  // CTA = (a-row tile of a token set, batch row): rows and columns are the set's own even and odd tokens
+  const int set = set_of(tab.tile_off, tab.n, blockIdx.x);
+  const int ta = (tab.len[set] + 1) / 2, tb = tab.len[set] / 2;
+  const int a0 = (blockIdx.x - tab.tile_off[set]) * SIM_TILE;
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-  const float* pa = plane_a + (long long)b * ta * dpad;
-  const float* pb = plane_b + (long long)b * tb * dpad;
+  const long long arow = (long long)b * tab.a_off[tab.n] + tab.a_off[set];   // node_max / plane A row of the set's token 0
+  const float* pa = plane_a + arow * dpad;
+  const float* pb = plane_b + ((long long)b * tab.b_off[tab.n] + tab.b_off[set]) * dpad;
+  float* dump = scores_out ? scores_out + (long long)b * tab.sc_off[tab.n] + tab.sc_off[set] : nullptr;
   const int n_bt = (tb + SIM_TILE - 1) / SIM_TILE;
 
   load_tile_async(sa, pa, a0, ta, dpad);
@@ -221,7 +231,7 @@ sim_argmax_planes_kernel(const tome_metric_desc_t d, const float* __restrict__ p
         if (ai < ta && bj < tb) {
           float s = acc[i][j];
           if ((d.class_token && ai == 0) || (d.distill_token && bj == 0)) s = -INFINITY;  // :77-80
-          if (scores_out) scores_out[((long long)b * ta + ai) * tb + bj] = s;
+          if (dump) dump[(long long)ai * tb + bj] = s;
           if (argmax_better(s, bj, best_v[i], best_j[i])) {
             best_v[i] = s;
             best_j[i] = bj;
@@ -231,6 +241,7 @@ sim_argmax_planes_kernel(const tome_metric_desc_t d, const float* __restrict__ p
     }
     __syncthreads();  // tile bt fully consumed before tile bt+2 overwrites its buffer
   }
+  if (n_bt == 0) asm volatile("cp.async.wait_all;" ::: "memory");   // a one-token set: no b tile, the a tile still in flight
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
 #pragma unroll
@@ -244,8 +255,8 @@ sim_argmax_planes_kernel(const tome_metric_desc_t d, const float* __restrict__ p
     }
     const int ai = a0 + ty + 16 * i;
     if (tx == 0 && ai < ta) {
-      node_max[(long long)b * ta + ai] = best_v[i];
-      node_idx[(long long)b * ta + ai] = best_j[i] == 0x7fffffff ? 0 : best_j[i];
+      node_max[arow + ai] = best_v[i];
+      node_idx[arow + ai] = best_j[i] == 0x7fffffff ? 0 : best_j[i];
     }
   }
 }
@@ -271,14 +282,14 @@ constexpr int SIMT_THREADS = 192;
 
 // bf16, dim == 64, 16-byte aligned rows: 8 lanes per token row; head mean, L2 norm (no epsilon), three-way bf16 split
 __global__ void __launch_bounds__(256)
-metric_split64_kernel(const tome_metric_desc_t d, const __nv_bfloat16* __restrict__ src, __nv_bfloat16* __restrict__ plane_a,
-                      __nv_bfloat16* __restrict__ plane_b) {
+metric_split64_kernel(const tome_metric_desc_t d, const __grid_constant__ SetTable tab, const __nv_bfloat16* __restrict__ src,
+                      __nv_bfloat16* __restrict__ plane_a, __nv_bfloat16* __restrict__ plane_b) {
   const long long tok = ((long long)blockIdx.x * 256 + threadIdx.x) >> 3;   // b * T + t
   const int sub = threadIdx.x & 7;
   const bool valid = tok < (long long)d.batch * d.tokens;   // every lane stays for the shuffles
   const long long tk = valid ? tok : 0;
   const int b = (int)(tk / d.tokens), t = (int)(tk % d.tokens);
-  const int ta = (d.tokens + 1) / 2, tb = d.tokens / 2;
+  const int ta = tab.a_off[tab.n], tb = tab.b_off[tab.n];
   const __nv_bfloat16* base = src + (long long)b * d.batch_stride + (long long)t * d.token_stride + sub * 8;
   float acc[8];
 #pragma unroll
@@ -310,8 +321,9 @@ metric_split64_kernel(const tome_metric_desc_t d, const __nv_bfloat16* __restric
     lo[i] = __bfloat162float(__float2bfloat16_rn(r1 - mi[i]));
   }
   const uint4 wh = pack8(hi), wm = pack8(mi), wl = pack8(lo);
-  const bool odd = t & 1;
-  uint4* out = reinterpret_cast<uint4*>((odd ? plane_b + ((long long)b * tb + (t >> 1)) * SIMT_ROW : plane_a + ((long long)b * ta + (t >> 1)) * SIMT_ROW)) + sub;
+  bool odd;
+  const int pr = set_plane_row(tab, t, odd);
+  uint4* out = reinterpret_cast<uint4*>((odd ? plane_b + ((long long)b * tb + pr) * SIMT_ROW : plane_a + ((long long)b * ta + pr) * SIMT_ROW)) + sub;
   out[0] = wh;    // chunk c starts 64 elements = 8 uint4 further
   out[8] = wm;
   out[16] = wl;
@@ -321,13 +333,13 @@ metric_split64_kernel(const tome_metric_desc_t d, const __nv_bfloat16* __restric
 // bipartite_soft_matching takes this one)
 template <typename T>
 __global__ void __launch_bounds__(256)
-metric_split_kernel(const tome_metric_desc_t d, const T* __restrict__ src, __nv_bfloat16* __restrict__ plane_a,
-                    __nv_bfloat16* __restrict__ plane_b) {
+metric_split_kernel(const tome_metric_desc_t d, const __grid_constant__ SetTable tab, const T* __restrict__ src,
+                    __nv_bfloat16* __restrict__ plane_a, __nv_bfloat16* __restrict__ plane_b) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long tok = (long long)blockIdx.x * 8 + warp;   // b * T + t
   if (tok >= (long long)d.batch * d.tokens) return;
   const int b = (int)(tok / d.tokens), t = (int)(tok % d.tokens);
-  const int ta = (d.tokens + 1) / 2, tb = d.tokens / 2;
+  const int ta = tab.a_off[tab.n], tb = tab.b_off[tab.n];
   const T* base = src + (long long)b * d.batch_stride + (long long)t * d.token_stride + 2 * lane;
   float2 acc = make_float2(0.f, 0.f);
   for (int h = 0; h < d.heads; ++h) {
@@ -350,8 +362,9 @@ metric_split_kernel(const tome_metric_desc_t d, const T* __restrict__ src, __nv_
     lo[i] = __bfloat162float(__float2bfloat16_rn(r1 - mi[i]));
   }
   const uint32_t wh = pack_bf16(hi[0], hi[1]), wm = pack_bf16(mi[0], mi[1]), wl = pack_bf16(lo[0], lo[1]);
-  const bool odd = t & 1;
-  uint32_t* out = reinterpret_cast<uint32_t*>(odd ? plane_b + ((long long)b * tb + (t >> 1)) * SIMT_ROW : plane_a + ((long long)b * ta + (t >> 1)) * SIMT_ROW) + lane;
+  bool odd;
+  const int pr = set_plane_row(tab, t, odd);
+  uint32_t* out = reinterpret_cast<uint32_t*>(odd ? plane_b + ((long long)b * tb + pr) * SIMT_ROW : plane_a + ((long long)b * ta + pr) * SIMT_ROW) + lane;
   out[0] = wh;            // chunk c starts 64 elements = 32 words further
   out[32] = wm;
   out[64] = wl;
@@ -359,7 +372,8 @@ metric_split_kernel(const tome_metric_desc_t d, const T* __restrict__ src, __nv_
 
 __global__ void __launch_bounds__(SIMT_THREADS, 2)
 sim_argmax_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, const tome_metric_desc_t d,
-                     float* __restrict__ node_max, int32_t* __restrict__ node_idx, float* __restrict__ scores_out) {
+                     const __grid_constant__ SetTable tab, float* __restrict__ node_max, int32_t* __restrict__ node_idx,
+                     float* __restrict__ scores_out) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   uint8_t* s_a = smem;                                   // chunk c at c * 16 KB
@@ -372,8 +386,12 @@ sim_argmax_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_cons
   uint64_t* s_free = bars + 11;       // [2] 128 arrivals: the epilogue has read it
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 13);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int at = blockIdx.x, b = blockIdx.y;
-  const int ta = (d.tokens + 1) / 2, tb = d.tokens / 2;
+  // CTA = (a-row tile of a token set, batch row).  The tiles are read at the set's rows of the planes: a rows past the set's
+  // end (the next set's, or TMA zero fill) are never stored, b columns past it are skipped in the epilogue (j < tb).
+  const int b = blockIdx.y;
+  const int set = set_of(tab.tile_off, tab.n, blockIdx.x);
+  const int at = blockIdx.x - tab.tile_off[set];
+  const int ta = (tab.len[set] + 1) / 2, tb = tab.len[set] / 2;
   const int n_bt = (tb + SIMT_BN - 1) / SIMT_BN;
 
   if (threadIdx.x == 0) {
@@ -401,14 +419,15 @@ sim_argmax_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_cons
   if (warp == 4) {
     if (lane == 0) {
       mbar_expect_tx(a_full, SIMT_CHUNKS * SIMT_CHUNK_BYTES);
-      for (int c = 0; c < SIMT_CHUNKS; ++c) tma_load_3d(s_a + c * SIMT_CHUNK_BYTES, &tm_a, a_full, c * 64, at * SIMT_BM, b);
+      for (int c = 0; c < SIMT_CHUNKS; ++c)
+        tma_load_3d(s_a + c * SIMT_CHUNK_BYTES, &tm_a, a_full, c * 64, tab.a_off[set] + at * SIMT_BM, b);
       int item = 0;
       for (int jt = 0; jt < n_bt; ++jt)
         for (int c = 0; c < SIMT_CHUNKS; ++c, ++item) {
           const int slot = item % SIMT_SLOTS;
           mbar_wait(&b_empty[slot], ((item / SIMT_SLOTS) & 1) ^ 1);
           mbar_expect_tx(&b_full[slot], SIMT_CHUNK_BYTES);
-          tma_load_3d(s_b + slot * SIMT_CHUNK_BYTES, &tm_b, &b_full[slot], c * 64, jt * SIMT_BN, b);
+          tma_load_3d(s_b + slot * SIMT_CHUNK_BYTES, &tm_b, &b_full[slot], c * 64, tab.b_off[set] + jt * SIMT_BN, b);
         }
     }
   } else if (warp == 5) {
@@ -447,7 +466,8 @@ sim_argmax_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_cons
     const bool row_protected = d.class_token && ai == 0;   // :77-78
     float bv = -INFINITY;
     int bj = 0x7fffffff;
-    float* dump = (scores_out && row_ok) ? scores_out + ((long long)b * ta + ai) * tb : nullptr;
+    const long long arow = (long long)b * tab.a_off[tab.n] + tab.a_off[set] + ai;
+    float* dump = (scores_out && row_ok) ? scores_out + (long long)b * tab.sc_off[tab.n] + tab.sc_off[set] + (long long)ai * tb : nullptr;
     for (int jt = 0; jt < n_bt; ++jt) {
       mbar_wait(&s_full[jt & 1], (jt >> 1) & 1);
       tc_fence_after();
@@ -478,8 +498,8 @@ sim_argmax_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_cons
       mbar_arrive(&s_free[jt & 1]);
     }
     if (row_ok) {
-      node_max[(long long)b * ta + ai] = bv;
-      node_idx[(long long)b * ta + ai] = bj == 0x7fffffff ? 0 : bj;
+      node_max[arow] = bv;
+      node_idx[arow] = bj == 0x7fffffff ? 0 : bj;
     }
   }
   tc_fence_before();
@@ -528,23 +548,35 @@ constexpr int SEL_THREADS = 1024;
 __host__ __device__ inline int sel_pow2(int n) { int p = 1; while (p < n) p <<= 1; return p; }
 
 __global__ void __launch_bounds__(SEL_THREADS)
-select_topr_kernel(const tome_plan_shape_t s, const float* __restrict__ node_max, const int32_t* __restrict__ node_idx,
-                   const tome_plan_t p) {
+select_topr_kernel(const tome_plan_shape_t s, const __grid_constant__ SetTable tab, const float* __restrict__ node_max,
+                   const int32_t* __restrict__ node_idx, const tome_plan_t p) {
   extern __shared__ __align__(8) unsigned char sel_raw[];
-  const int T = s.tokens, r = s.r;
+  // CTA = (token set, batch row); every index below is local to the set, the arrays are concatenated set by set
+  const int set = blockIdx.x, b = blockIdx.y, tid = threadIdx.x, nt = blockDim.x;
+  const int T = tab.len[set], r = tab.r[set];
   const int ta = (T + 1) / 2, tb = T / 2;
+  const long long arow = (long long)b * tab.a_off[tab.n] + tab.a_off[set];    // node_max / node_idx / edge_idx
+  const long long rrow = (long long)b * tab.r_off[tab.n] + tab.r_off[set];    // dst_idx / dst_src
+  const long long orow = (long long)b * tab.off_off[tab.n] + tab.off_off[set];  // dst_off
+  int32_t* row_map = p.row_map + (long long)b * s.tokens + tab.start[set];
+  const int out0 = tab.out_off[set];   // global output row of the set's first row
+  if (r == 0) {   // the set is copied unchanged: identity ranking and row map, no sources
+    for (int i = tid; i < ta; i += nt) p.edge_idx[arow + i] = i;
+    for (int j = tid; j <= tb; j += nt) p.dst_off[orow + j] = 0;
+    for (int t = tid; t < T; t += nt) row_map[t] = out0 + t;
+    return;
+  }
   const int n2 = sel_pow2(ta);
   unsigned long long* keys = reinterpret_cast<unsigned long long*>(sel_raw);  // [n2]
   int* nidx = reinterpret_cast<int*>(keys + n2);   // [ta]
   int* rnk = nidx + ta;                            // [ta]   rank of even token i
   int* cnt = rnk + ta;                             // [tb+1] counts then exclusive offsets
   int* part = cnt + tb + 1;                        // [SEL_THREADS] scan partials
-  const int b = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
 
   for (int i = tid; i < n2; i += nt) {
     if (i < ta) {
-      keys[i] = rank_key(node_max[(long long)b * ta + i], i);
-      nidx[i] = node_idx[(long long)b * ta + i];
+      keys[i] = rank_key(node_max[arow + i], i);
+      nidx[i] = node_idx[arow + i];
     } else {
       keys[i] = 0ull;   // below every real key (the smallest real high word is that of -inf, 0x007FFFFF)
     }
@@ -555,12 +587,12 @@ select_topr_kernel(const tome_plan_shape_t s, const float* __restrict__ node_max
   for (int rk = tid; rk < ta; rk += nt) {
     const int i = (int)(uint32_t)keys[rk];
     rnk[i] = rk;
-    p.edge_idx[(long long)b * ta + rk] = i;
+    p.edge_idx[arow + rk] = i;
   }
   __syncthreads();
   for (int i = tid; i < r; i += nt) {
     const int d = nidx[(int)(uint32_t)keys[i]];
-    p.dst_idx[(long long)b * r + i] = d;
+    p.dst_idx[rrow + i] = d;
     atomicAdd(&cnt[d], 1);
   }
   __syncthreads();
@@ -587,7 +619,7 @@ select_topr_kernel(const tome_plan_shape_t s, const float* __restrict__ node_max
     if (tid == 0) cnt[tb] = r;
     __syncthreads();
   }
-  for (int j = tid; j <= tb; j += nt) p.dst_off[(long long)b * (tb + 1) + j] = cnt[j];
+  for (int j = tid; j <= tb; j += nt) p.dst_off[orow + j] = cnt[j];
   // placement: the merged sources sorted by (destination, rank) are the CSR lists in order -- sources of one destination
   // keep their rank order (the reference adds them in that order, :100-101).  Descending sort of the complemented key.
   {
@@ -607,7 +639,7 @@ select_topr_kernel(const tome_plan_shape_t s, const float* __restrict__ node_max
     }
     __syncthreads();
     bitonic_sort_desc(keys, r2, tid, nt);
-    for (int q = tid; q < r; q += nt) p.dst_src[(long long)b * r + q] = (int)(keys[q] & 0xFFFFFFull);
+    for (int q = tid; q < r; q += nt) p.dst_src[rrow + q] = (int)(keys[q] & 0xFFFFFFull);
   }
   // row map: where every input token lands in the concatenation [unm | dst] (:103-108)
   const int n_unm = ta - r;
@@ -626,7 +658,7 @@ select_topr_kernel(const tome_plan_shape_t s, const float* __restrict__ node_max
         row = s.distill_token ? (j == 0 ? 1 : n_unm + j) : n_unm + j;
       }
     }
-    p.row_map[(long long)b * T + t] = row;
+    row_map[t] = out0 + row;
   }
 }
 
@@ -648,19 +680,19 @@ static bool sim_fast64(const tome_metric_desc_t* d, const void* src) {   // 128-
          d->head_stride % 8 == 0 && ((uintptr_t)src & 15) == 0;
 }
 
-// The normalised metric in the workspace: plane A (the ta even tokens of every batch row), then plane B (the tb odd ones),
-// packed.  A token's row is three bf16 chunks of 64 (SIMT_ROW) on the tensor-core path, else dim floats padded to a multiple of 4.
+// The normalised metric in the workspace: plane A (the ta even tokens of every batch row, set after set), then plane B (the tb
+// odd ones), packed.  A token's row is three bf16 chunks of 64 (SIMT_ROW) on the tensor-core path, else dim floats padded to a
+// multiple of 4.  ta + tb = tokens whatever the sets, so the size does not depend on them.
 struct SimPlanes { uint8_t *a, *b; size_t total; };
-static SimPlanes sim_planes(const tome_metric_desc_t* d, void* base) {
+static SimPlanes sim_planes(const tome_metric_desc_t* d, size_t ta, void* base) {
   const size_t row = sim_tc_eligible(d) ? SIMT_ROW * sizeof(__nv_bfloat16) : ((d->dim + 3) & ~3) * sizeof(float);
   uint8_t* a = reinterpret_cast<uint8_t*>(base);
-  const size_t ta = (d->tokens + 1) / 2;
   return {a, a ? a + d->batch * ta * row : nullptr, (size_t)d->batch * d->tokens * row};
 }
 
 extern "C" size_t tome_sim_argmax_workspace_bytes(const tome_metric_desc_t* d) {
   if (!d || d->batch <= 0 || d->tokens <= 0 || d->dim <= 0) return 0;
-  return sim_planes(d, nullptr).total;
+  return sim_planes(d, (d->tokens + 1) / 2, nullptr).total;
 }
 
 extern "C" int tome_sim_argmax(const tome_metric_desc_t* d, const void* src, float* node_max, int32_t* node_idx,
@@ -676,29 +708,34 @@ extern "C" int tome_sim_argmax(const tome_metric_desc_t* d, const void* src, flo
   TOME_CHECK(d->token_stride % 2 == 0 && d->batch_stride % 2 == 0 && d->head_stride % 2 == 0, TOME_ERR_INVALID,
              "sim_argmax: strides must be even (vector loads)");
   TOME_CHECK(d->batch <= 65535, TOME_ERR_INVALID, "sim_argmax: batch too large for one launch");
-  const SimPlanes planes = sim_planes(d, workspace);
+  SetTable tab;
+  if (int rc = make_set_table(d->sets, d->tokens, -1, d->class_token, d->distill_token, &tab, "sim_argmax")) return rc;
+  const int ta = tab.a_off[tab.n], tb = tab.b_off[tab.n];   // even / odd tokens of a batch row, over all sets
+  const SimPlanes planes = sim_planes(d, ta, workspace);
   TOME_CHECK(workspace != nullptr && workspace_bytes >= planes.total && ((uintptr_t)workspace & 15) == 0, TOME_ERR_INVALID,
              "sim_argmax: workspace must be 16-byte aligned and hold tome_sim_argmax_workspace_bytes = %zu bytes (got %p, %zu bytes)",
              planes.total, workspace, workspace_bytes);
-  const int ta = (d->tokens + 1) / 2, tb = d->tokens / 2;
   const long long toks = (long long)d->batch * d->tokens;
-  ProfScope prof(PROF_SIM, 2.0 * d->batch * ta * (double)tb * d->dim, 2, stream);
+  ProfScope prof(PROF_SIM, 2.0 * d->batch * (double)tab.sc_off[tab.n] * d->dim, 2, stream);
   if (sim_tc_eligible(d)) {
     __nv_bfloat16* pa = reinterpret_cast<__nv_bfloat16*>(planes.a);
     __nv_bfloat16* pb = reinterpret_cast<__nv_bfloat16*>(planes.b);
     if (sim_fast64(d, src))
-      launch_k(metric_split64_kernel, (unsigned)((toks * 8 + 255) / 256), 256, 0, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), pa, pb);
+      launch_k(metric_split64_kernel, (unsigned)((toks * 8 + 255) / 256), 256, 0, stream, *d, tab, reinterpret_cast<const __nv_bfloat16*>(src), pa, pb);
     else if (d->dtype == TOME_BF16)
-      launch_k(metric_split_kernel<__nv_bfloat16>, (unsigned)((toks + 7) / 8), 256, 0, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), pa, pb);
+      launch_k(metric_split_kernel<__nv_bfloat16>, (unsigned)((toks + 7) / 8), 256, 0, stream, *d, tab, reinterpret_cast<const __nv_bfloat16*>(src), pa, pb);
     else
-      launch_k(metric_split_kernel<float>, (unsigned)((toks + 7) / 8), 256, 0, stream, *d, reinterpret_cast<const float*>(src), pa, pb);
+      launch_k(metric_split_kernel<float>, (unsigned)((toks + 7) / 8), 256, 0, stream, *d, tab, reinterpret_cast<const float*>(src), pa, pb);
     TOME_CUDA(cudaGetLastError());
     CUtensorMap tma_a, tma_b;
     if (int rc = make_tmap_3d_bf16(&tma_a, pa, SIMT_ROW, ta, d->batch, SIMT_ROW, (uint64_t)ta * SIMT_ROW, SIMT_BM)) return rc;
-    if (int rc = make_tmap_3d_bf16(&tma_b, pb, SIMT_ROW, tb, d->batch, SIMT_ROW, (uint64_t)tb * SIMT_ROW, SIMT_BN)) return rc;
+    // tb == 0 (every set a single token): no b tile is ever loaded, the map only has to be well-formed
+    const int tbm = tb > 0 ? tb : 1;
+    if (int rc = make_tmap_3d_bf16(&tma_b, pb, SIMT_ROW, tbm, d->batch, SIMT_ROW, (uint64_t)tbm * SIMT_ROW, SIMT_BN)) return rc;
     static DynSmemOnce once;
     TOME_CUDA(ensure_dyn_smem(sim_argmax_tc_kernel, SIMT_SMEM, once));
-    TOME_CUDA(launch_k(sim_argmax_tc_kernel, dim3(ceil_div(ta, SIMT_BM), d->batch), SIMT_THREADS, SIMT_SMEM, stream, tma_a, tma_b, *d,
+    const int tiles = set_tiles(&tab, SIMT_BM);
+    TOME_CUDA(launch_k(sim_argmax_tc_kernel, dim3(tiles, d->batch), SIMT_THREADS, SIMT_SMEM, stream, tma_a, tma_b, *d, tab,
                        node_max, node_idx, scores_out));
     return TOME_OK;
   }
@@ -706,15 +743,16 @@ extern "C" int tome_sim_argmax(const tome_metric_desc_t* d, const void* src, flo
   float* plane_b = reinterpret_cast<float*>(planes.b);
   const unsigned nblk = (unsigned)((toks + 7) / 8);
   if (sim_fast64(d, src))
-    launch_k(metric_norm64_kernel, (unsigned)((toks * 8 + 255) / 256), 256, 0, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), plane_a, plane_b);
+    launch_k(metric_norm64_kernel, (unsigned)((toks * 8 + 255) / 256), 256, 0, stream, *d, tab, reinterpret_cast<const __nv_bfloat16*>(src), plane_a, plane_b);
   else if (d->dtype == TOME_BF16)
-    launch_k(metric_norm_kernel<__nv_bfloat16>, nblk, 256, 0, stream, *d, reinterpret_cast<const __nv_bfloat16*>(src), plane_a, plane_b);
+    launch_k(metric_norm_kernel<__nv_bfloat16>, nblk, 256, 0, stream, *d, tab, reinterpret_cast<const __nv_bfloat16*>(src), plane_a, plane_b);
   else
-    launch_k(metric_norm_kernel<float>, nblk, 256, 0, stream, *d, reinterpret_cast<const float*>(src), plane_a, plane_b);
+    launch_k(metric_norm_kernel<float>, nblk, 256, 0, stream, *d, tab, reinterpret_cast<const float*>(src), plane_a, plane_b);
   TOME_CUDA(cudaGetLastError());
   const size_t smem = sim_planes_smem(d->dim);
   TOME_CUDA(cudaFuncSetAttribute(sim_argmax_planes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  launch_k(sim_argmax_planes_kernel, dim3(ceil_div(ta, SIM_TILE), d->batch), SIM_THREADS, smem, stream, *d, plane_a, plane_b,
+  const int tiles = set_tiles(&tab, SIM_TILE);
+  launch_k(sim_argmax_planes_kernel, dim3(tiles, d->batch), SIM_THREADS, smem, stream, *d, tab, plane_a, plane_b,
            node_max, node_idx, scores_out);
   TOME_CUDA(cudaGetLastError());
   return TOME_OK;
@@ -727,17 +765,20 @@ extern "C" int tome_select_topr(const tome_plan_shape_t* s, const float* node_ma
   TOME_CHECK(s && node_max && node_idx && plan, TOME_ERR_INVALID, "select_topr: null argument");
   TOME_CHECK(plan->edge_idx && plan->dst_idx && plan->row_map && plan->dst_off && plan->dst_src, TOME_ERR_INVALID,
              "select_topr: every plan buffer must be provided");
-  TOME_CHECK(s->batch > 0 && s->tokens >= 2, TOME_ERR_INVALID, "select_topr: need batch > 0 and tokens >= 2");
-  const int ta = (s->tokens + 1) / 2, tb = s->tokens / 2;
-  TOME_CHECK(s->r >= 1 && s->r <= tb && s->r <= ta, TOME_ERR_INVALID,
+  TOME_CHECK(s->batch > 0 && s->batch <= 65535 && s->tokens >= 2, TOME_ERR_INVALID,
+             "select_topr: need 0 < batch <= 65535 and tokens >= 2");
+  TOME_CHECK(s->r >= 1 && s->r <= s->tokens / 2, TOME_ERR_INVALID,
              "select_topr: r (%d) must be clamped to [1, %d] first (tome_clamp_r; r == 0 is the identity, no plan needed)",
-             s->r, tb);
+             s->r, s->tokens / 2);
+  SetTable tab;
+  if (int rc = make_set_table(s->sets, s->tokens, s->r, 0, s->distill_token, &tab, "select_topr")) return rc;
+  const int ta = tab.max_ta, tb = tab.max_tb;   // shared memory for the largest set
   const size_t smem = sizeof(unsigned long long) * (size_t)sel_pow2(ta) + sizeof(int) * ((size_t)2 * ta + tb + 1 + SEL_THREADS);
   TOME_CHECK(smem <= 220 * 1024 && s->tokens < (1 << 20), TOME_ERR_UNSUPPORTED,
              "select_topr: tokens (%d) too large for the shared-memory ranking", s->tokens);
   TOME_CUDA(cudaFuncSetAttribute(select_topr_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   ProfScope prof(PROF_SELECT, 0.0, 1, stream);
-  launch_k(select_topr_kernel, s->batch, SEL_THREADS, smem, stream, *s, node_max, node_idx, *plan);
+  launch_k(select_topr_kernel, dim3(tab.n, s->batch), SEL_THREADS, smem, stream, *s, tab, node_max, node_idx, *plan);
   TOME_CUDA(cudaGetLastError());
   return TOME_OK;
 }

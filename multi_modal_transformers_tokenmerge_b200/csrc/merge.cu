@@ -9,6 +9,7 @@
 // algorithmic bytes / sample (merge fwd, SURVEY.md 8d):  T*C*e + 4T + 4(Ta + r) + (T-r)*C*e + 4(T-r)
 #include "common.cuh"
 #include "host_util.h"
+#include "token_sets.cuh"
 
 namespace tome {
 
@@ -40,15 +41,56 @@ struct Vec<__nv_bfloat16> {
 
 constexpr int MERGE_THREADS = 256;
 
+// Output row prow of batch row b, inverted through the concatenation order (:103-108) of its token set: the input token it
+// keeps (an unmerged even token or a destination), its CSR source range, and where the set's sources are listed: source e is
+// input token tok0 + 2 * dst_src[src_base + e].  Rows of a set with r == 0 are plain copies (copy = true).
+struct RowPlan {
+  int keep_tok, e0, e1, tok0;
+  long long src_base;
+  bool copy;
+};
+__device__ __forceinline__ RowPlan resolve_row(const SetTable& tab, bool distill, const tome_plan_t& p, int b, int prow) {
+  const int set = set_of(tab.out_off, tab.n, prow);
+  const int lrow = prow - tab.out_off[set], r = tab.r[set];
+  RowPlan m;
+  m.e0 = m.e1 = 0;
+  m.tok0 = tab.start[set];
+  m.src_base = (long long)b * tab.r_off[tab.n] + tab.r_off[set];
+  m.copy = r == 0;
+  if (m.copy) {
+    m.keep_tok = m.tok0 + lrow;
+    return m;
+  }
+  const int n_unm = (tab.len[set] + 1) / 2 - r;
+  int u = -1, j = -1;
+  if (!distill) {
+    if (lrow < n_unm) u = lrow; else j = lrow - n_unm;
+  } else {
+    if (lrow == 0) u = 0;
+    else if (lrow == 1) j = 0;
+    else if (lrow <= n_unm) u = lrow - 1;
+    else j = lrow - n_unm;
+  }
+  if (u >= 0) {
+    m.keep_tok = m.tok0 + 2 * p.edge_idx[(long long)b * tab.a_off[tab.n] + tab.a_off[set] + r + u];
+  } else {
+    m.keep_tok = m.tok0 + 2 * j + 1;
+    const long long o = (long long)b * tab.off_off[tab.n] + tab.off_off[set] + j;
+    m.e0 = p.dst_off[o];
+    m.e1 = p.dst_off[o + 1];
+  }
+  return m;
+}
+
 template <typename T, bool WAVG>
 __global__ void __launch_bounds__(MERGE_THREADS)
-merge_fwd_kernel(const tome_merge_shape_t s, const tome_plan_t p, const T* __restrict__ x,
+merge_fwd_kernel(const tome_merge_shape_t s, const __grid_constant__ SetTable tab, const tome_plan_t p, const T* __restrict__ x,
                  const float* __restrict__ size, T* __restrict__ x_out, float* __restrict__ size_out,
                  const uint8_t* __restrict__ gid, const int32_t* __restrict__ pos, uint8_t* __restrict__ gid_out,
                  int32_t* __restrict__ pos_out) {
   constexpr int N = Vec<T>::N;
   const int Tn = s.tokens, r = s.r, C = s.channels;
-  const int ta = (Tn + 1) / 2, tb = Tn / 2, n_unm = ta - r, To = Tn - r;
+  const int To = Tn - r;
   const int vpr = C / N;  // vectors per row
   const long long total = (long long)s.batch * To * vpr;
   for (long long item = blockIdx.x * (long long)MERGE_THREADS + threadIdx.x; item < total;
@@ -57,40 +99,21 @@ merge_fwd_kernel(const tome_merge_shape_t s, const tome_plan_t p, const T* __res
     const long long rowg = item / vpr;
     const int prow = (int)(rowg % To);
     const int b = (int)(rowg / To);
-    // invert the concatenation order (:103-108): which unmerged (u) or destination (j) token is output row prow?
-    int u = -1, j = -1;
-    if (!s.distill_token) {
-      if (prow < n_unm) u = prow; else j = prow - n_unm;
-    } else {
-      if (prow == 0) u = 0;
-      else if (prow == 1) j = 0;
-      else if (prow <= n_unm) u = prow - 1;
-      else j = prow - n_unm;
-    }
+    const RowPlan m = resolve_row(tab, s.distill_token, p, b, prow);
     const T* xb = x + (long long)b * Tn * C;
     const float* sb = size ? size + (long long)b * Tn : nullptr;
     float acc[N];
-    float sacc;
-    int keep_tok;
-    if (u >= 0) {
-      keep_tok = 2 * p.edge_idx[(long long)b * ta + r + u];
-      Vec<T>::load(xb + (long long)keep_tok * C + v * N, acc);
-      sacc = sb ? sb[keep_tok] : 1.0f;
-      if (WAVG) {
-#pragma unroll
-        for (int i = 0; i < N; ++i) acc[i] = __fdiv_rn(__fmul_rn(acc[i], sacc), sacc);  // merge(x*size)/merge(size), literally
-      }
-    } else {
-      keep_tok = 2 * j + 1;
-      Vec<T>::load(xb + (long long)keep_tok * C + v * N, acc);
-      sacc = sb ? sb[keep_tok] : 1.0f;
+    const int keep_tok = m.keep_tok;
+    Vec<T>::load(xb + (long long)keep_tok * C + v * N, acc);
+    float sacc = sb ? sb[keep_tok] : 1.0f;
+    // merge(x*size)/merge(size), literally: an unmerged token or a destination without sources also becomes (x*s)/s
+    if (!m.copy) {
       if (WAVG) {
 #pragma unroll
         for (int i = 0; i < N; ++i) acc[i] = __fmul_rn(acc[i], sacc);
       }
-      const int e0 = p.dst_off[(long long)b * (tb + 1) + j], e1 = p.dst_off[(long long)b * (tb + 1) + j + 1];
-      for (int e = e0; e < e1; ++e) {
-        const int tok = 2 * p.dst_src[(long long)b * r + e];
+      for (int e = m.e0; e < m.e1; ++e) {
+        const int tok = m.tok0 + 2 * p.dst_src[m.src_base + e];
         float f[N];
         Vec<T>::load(xb + (long long)tok * C + v * N, f);
         const float sz = sb ? sb[tok] : 1.0f;
@@ -124,20 +147,21 @@ merge_fwd_kernel(const tome_merge_shape_t s, const tome_plan_t p, const T* __res
 struct MergeRowMeta {
   int keep_tok;
   int e0, e1;
+  int tok0, src0;   // the row's token set: first token, first dst_src entry in the batch row (RowPlan)
   float size_keep;  // size of the kept token
   float size_sum;   // size_out of the row
 };
 
 template <typename T, bool WAVG>
 __global__ void __launch_bounds__(MERGE_THREADS)
-merge_fwd_bulk_kernel(const tome_merge_shape_t s, const tome_plan_t p, const T* __restrict__ x,
+merge_fwd_bulk_kernel(const tome_merge_shape_t s, const __grid_constant__ SetTable tab, const tome_plan_t p, const T* __restrict__ x,
                       const float* __restrict__ size, T* __restrict__ x_out, float* __restrict__ size_out,
                       const uint8_t* __restrict__ gid, const int32_t* __restrict__ pos, uint8_t* __restrict__ gid_out,
                       int32_t* __restrict__ pos_out, int rows_per_cta) {
   constexpr int N = Vec<T>::N;
   extern __shared__ __align__(128) uint8_t smem_merge[];
   const int Tn = s.tokens, r = s.r, C = s.channels;
-  const int ta = (Tn + 1) / 2, tb = Tn / 2, n_unm = ta - r, To = Tn - r;
+  const int To = Tn - r;
   const int row_bytes = C * (int)sizeof(T);
   const int b = blockIdx.y;
   const int row0 = blockIdx.x * rows_per_cta;
@@ -160,24 +184,13 @@ merge_fwd_bulk_kernel(const tome_merge_shape_t s, const tome_plan_t p, const T* 
   if (tid == 0) mbar_expect_tx(bar, (uint32_t)(nrows * row_bytes));
   if (tid < nrows) {
     const int prow = row0 + tid;
-    int u = -1, j = -1;
-    if (!s.distill_token) {
-      if (prow < n_unm) u = prow; else j = prow - n_unm;
-    } else {
-      if (prow == 0) u = 0;
-      else if (prow == 1) j = 0;
-      else if (prow <= n_unm) u = prow - 1;
-      else j = prow - n_unm;
-    }
+    const RowPlan rp = resolve_row(tab, s.distill_token, p, b, prow);
     MergeRowMeta m;
-    m.e0 = m.e1 = 0;
-    if (u >= 0) {
-      m.keep_tok = 2 * p.edge_idx[(long long)b * ta + r + u];
-    } else {
-      m.keep_tok = 2 * j + 1;
-      m.e0 = p.dst_off[(long long)b * (tb + 1) + j];
-      m.e1 = p.dst_off[(long long)b * (tb + 1) + j + 1];
-    }
+    m.keep_tok = rp.keep_tok;
+    m.e0 = rp.e0;
+    m.e1 = rp.e1;
+    m.tok0 = rp.tok0;
+    m.src0 = (int)(rp.src_base - (long long)b * tab.r_off[tab.n]);
     // the copy first: everything below overlaps it
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                  ::"r"(smem_u32(s_rows + (size_t)tid * row_bytes)), "l"(xb + (long long)m.keep_tok * C), "r"(row_bytes),
@@ -185,10 +198,11 @@ merge_fwd_bulk_kernel(const tome_merge_shape_t s, const tome_plan_t p, const T* 
                  : "memory");
     m.size_keep = sb ? sb[m.keep_tok] : 1.0f;
     float sacc = m.size_keep;
-    for (int e = m.e0; e < m.e1; ++e) sacc = __fadd_rn(sacc, sb ? sb[2 * p.dst_src[(long long)b * r + e]] : 1.0f);
+    for (int e = m.e0; e < m.e1; ++e) sacc = __fadd_rn(sacc, sb ? sb[m.tok0 + 2 * p.dst_src[rp.src_base + e]] : 1.0f);
     m.size_sum = sacc;
     s_meta[tid] = m;
-    if ((WAVG && m.size_keep != 1.0f) || m.e1 > m.e0) s_fix[atomicAdd(s_nfix, 1)] = tid;
+    // rows of an r == 0 set stay the bit copies the bulk load made
+    if (!rp.copy && ((WAVG && m.size_keep != 1.0f) || m.e1 > m.e0)) s_fix[atomicAdd(s_nfix, 1)] = tid;
     if (size_out) size_out[(long long)b * To + prow] = sacc;
     if (gid_out) gid_out[(long long)b * To + prow] = gid[(long long)b * Tn + m.keep_tok];
     if (pos_out) pos_out[(long long)b * To + prow] = pos[(long long)b * Tn + m.keep_tok];
@@ -218,7 +232,7 @@ merge_fwd_bulk_kernel(const tome_merge_shape_t s, const tome_plan_t p, const T* 
         for (int i = 0; i < N; ++i) acc[i] = __fmul_rn(acc[i], m.size_keep);
       }
       for (int e = m.e0; e < m.e1; ++e) {
-        const int tok = 2 * p.dst_src[(long long)b * r + e];
+        const int tok = m.tok0 + 2 * p.dst_src[(long long)b * tab.r_off[tab.n] + m.src0 + e];
         float f[N];
         Vec<T>::load(xb + (long long)tok * C + v * N, f);
         const float sz = sb ? sb[tok] : 1.0f;
@@ -281,7 +295,7 @@ static inline int merge_grid(long long items) {
   return (int)(blocks > 0 ? blocks : 1);
 }
 
-static int check_merge_shape(const tome_merge_shape_t* s, const tome_plan_t* plan, const char* who) {
+static int check_merge_shape(const tome_merge_shape_t* s, const tome_plan_t* plan, SetTable* tab, const char* who) {
   TOME_CHECK(s && plan, TOME_ERR_INVALID, "%s: null shape/plan", who);
   TOME_CHECK(s->batch > 0 && s->tokens >= 2 && s->channels > 0, TOME_ERR_INVALID, "%s: bad shape", who);
   TOME_CHECK(s->dtype == TOME_BF16 || s->dtype == TOME_F32, TOME_ERR_INVALID, "%s: dtype must be bf16 or f32", who);
@@ -292,7 +306,7 @@ static int check_merge_shape(const tome_merge_shape_t* s, const tome_plan_t* pla
              s->tokens / 2);
   TOME_CHECK(s->mode == TOME_MERGE_SUM || s->mode == TOME_MERGE_WAVG, TOME_ERR_INVALID,
              "%s: unknown merge mode %d (the reference only implements \"sum\", token_compression.py:99)", who, s->mode);
-  return TOME_OK;
+  return make_set_table(s->sets, s->tokens, s->r, 0, s->distill_token, tab, who);
 }
 
 }  // namespace tome
@@ -304,7 +318,8 @@ extern "C" int tome_merge_fwd(const tome_merge_shape_t* s, const tome_plan_t* pl
                               int32_t* pos_out, void* stream_) {
   clear_error();
   cudaStream_t stream = (cudaStream_t)stream_;
-  if (int rc = check_merge_shape(s, plan, "merge_fwd")) return rc;
+  SetTable tab;
+  if (int rc = check_merge_shape(s, plan, &tab, "merge_fwd")) return rc;
   TOME_CHECK(x && x_out, TOME_ERR_INVALID, "merge_fwd: null x / x_out");
   TOME_CHECK(plan->edge_idx && plan->dst_off && plan->dst_src, TOME_ERR_INVALID, "merge_fwd: incomplete plan");
   TOME_CHECK((!gid_out || gid) && (!pos_out || pos), TOME_ERR_INVALID, "merge_fwd: gid_out/pos_out need gid/pos");
@@ -328,7 +343,7 @@ extern "C" int tome_merge_fwd(const tome_merge_shape_t* s, const tome_plan_t* pl
   do {                                                                                                                  \
     static DynSmemOnce once;                                                                                            \
     if (smem > 48 * 1024) TOME_CUDA(ensure_dyn_smem(merge_fwd_bulk_kernel<TT, W>, (int)smem, once));                   \
-    launch_k(merge_fwd_bulk_kernel<TT, W>, grid2, MERGE_THREADS, smem, stream, *s, *plan, reinterpret_cast<const TT*>(x), size, \
+    launch_k(merge_fwd_bulk_kernel<TT, W>, grid2, MERGE_THREADS, smem, stream, *s, tab, *plan, reinterpret_cast<const TT*>(x), size, \
                                                                          reinterpret_cast<TT*>(x_out), size_out, gid, pos, \
                                                                          gid_out, pos_out, rows);                       \
   } while (0)
@@ -340,7 +355,7 @@ extern "C" int tome_merge_fwd(const tome_merge_shape_t* s, const tome_plan_t* pl
   }
   const int grid = merge_grid(items);  // rows wider than 32 KB: thread-per-vector kernel
 #define LAUNCH(TT, W)                                                                                              \
-  launch_k(merge_fwd_kernel<TT, W>, grid, MERGE_THREADS, 0, stream, *s, *plan, reinterpret_cast<const TT*>(x), size,     \
+  launch_k(merge_fwd_kernel<TT, W>, grid, MERGE_THREADS, 0, stream, *s, tab, *plan, reinterpret_cast<const TT*>(x), size, \
                                                               reinterpret_cast<TT*>(x_out), size_out, gid, pos,   \
                                                               gid_out, pos_out)
   if (s->dtype == TOME_BF16) { if (wavg) LAUNCH(__nv_bfloat16, true); else LAUNCH(__nv_bfloat16, false); }
@@ -354,7 +369,8 @@ extern "C" int tome_merge_bwd(const tome_merge_shape_t* s, const tome_plan_t* pl
                               const float* size_out, const void* dy, void* dx, void* stream_) {
   clear_error();
   cudaStream_t stream = (cudaStream_t)stream_;
-  if (int rc = check_merge_shape(s, plan, "merge_bwd")) return rc;
+  SetTable tab;   // merge_bwd reads the global row map only; the table is validated so that both directions accept the same shapes
+  if (int rc = check_merge_shape(s, plan, &tab, "merge_bwd")) return rc;
   TOME_CHECK(dy && dx && plan->row_map, TOME_ERR_INVALID, "merge_bwd: null dy / dx / row_map");
   const bool wavg = s->mode == TOME_MERGE_WAVG;
   TOME_CHECK(!wavg || size_out, TOME_ERR_INVALID, "merge_bwd: WAVG needs size_out");

@@ -120,7 +120,22 @@ static int check_cfg(const tome_stack_cfg_t* c) {
   TOME_CHECK(c->n_readout >= 0, TOME_ERR_INVALID, "stack: n_readout must be >= 0");
   TOME_CHECK(c->prune_sets >= 0 && c->prune_sets <= TOME_MAX_TOKEN_SETS, TOME_ERR_INVALID, "stack: prune_sets must be in [0, %d]",
              TOME_MAX_TOKEN_SETS);
-  if (c->prune_sets > 0) {
+  TOME_CHECK(!c->set_merge || c->prune_sets > 0, TOME_ERR_INVALID, "stack: set_merge needs the token sets (prune_sets > 0)");
+  if (c->prune_sets > 0 && c->set_merge) {
+    TOME_CHECK(c->r == 0 && !c->class_token && !c->distill_token, TOME_ERR_INVALID,
+               "stack: a set-merging stack (set_merge) takes r = 0 and no class / distill token");
+    long long total = 0;
+    for (int i = 0; i < c->prune_sets; ++i) {
+      TOME_CHECK(c->prune_set_n[i] >= 1 && c->prune_set_c[i] >= 0, TOME_ERR_INVALID, "stack: token set %d: n >= 1, c >= 0", i);
+      // every layer merges c tokens of the set's n(l) = n - l c: bipartite matching needs c <= floor(n(l) / 2)
+      const long long n_last = (long long)c->prune_set_n[i] - (long long)(c->layers - 1) * c->prune_set_c[i];
+      TOME_CHECK(n_last >= 1 && c->prune_set_c[i] <= n_last / 2, TOME_ERR_INVALID,
+                 "stack: token set %d (%d tokens) cannot merge %d tokens in each of %d layers (c <= floor(n / 2) at every layer)", i,
+                 c->prune_set_n[i], c->prune_set_c[i], c->layers);
+      total += c->prune_set_n[i];
+    }
+    TOME_CHECK(total == c->tokens, TOME_ERR_INVALID, "stack: the token sets hold %lld tokens, the sequence %d", total, c->tokens);
+  } else if (c->prune_sets > 0) {
     TOME_CHECK(c->r == 0 && c->prop_attn == 0 && !c->class_token && !c->distill_token, TOME_ERR_INVALID,
                "stack: a pruning stack (prune_sets > 0) takes r = 0, prop_attn = 0 and no class / distill token");
     TOME_CHECK(c->prune_importance == TOME_IMPORTANCE_ROW_MEAN || c->prune_importance == TOME_IMPORTANCE_RECEIVED, TOME_ERR_INVALID,
@@ -153,6 +168,22 @@ static int check_cfg(const tome_stack_cfg_t* c) {
   return TOME_OK;
 }
 
+// The token sets entering `layer` of a pruning or set-merging stack (token_sequencer.py:236: n - layer * c), each losing c.
+static tome_token_sets_t layer_sets(const tome_stack_cfg_t* c, int layer) {
+  tome_token_sets_t ts;
+  memset(&ts, 0, sizeof(ts));
+  ts.n_sets = c->prune_sets;
+  for (int i = 0, start = 0; i < c->prune_sets; ++i) {
+    ts.set_start[i] = start;
+    ts.set_n[i] = c->prune_set_n[i] - layer * c->prune_set_c[i];
+    ts.set_r[i] = c->prune_set_c[i];
+    start += ts.set_n[i];
+  }
+  return ts;
+}
+
+static bool merges_in_sets(const tome_stack_cfg_t* c) { return c->prune_sets > 0 && c->set_merge; }
+
 static std::vector<LayerShape> layer_shapes(const tome_stack_cfg_t* c) {
   std::vector<LayerShape> s(c->layers);
   int t = c->tokens;
@@ -184,7 +215,16 @@ static StackLayout make_layout(const tome_stack_cfg_t* c, void* workspace) {
   for (int l = 0; l < c->layers; ++l) {
     LayerBufs& Lb = S.L[l];
     const size_t T = S.shapes[l].t_in, To = S.shapes[l].t_out, r = S.shapes[l].r;
-    const size_t ta = (T + 1) / 2, tb = T / 2;
+    // plan arrays: even tokens (node_max, node_idx, edge_idx) and dst_off entries, summed over the token sets when merging in sets
+    size_t ta = (T + 1) / 2, n_off = T / 2 + 1;
+    if (merges_in_sets(c)) {
+      const tome_token_sets_t ts = layer_sets(c, l);
+      ta = n_off = 0;
+      for (int i = 0; i < ts.n_sets; ++i) {
+        ta += (ts.set_n[i] + 1) / 2;
+        n_off += ts.set_n[i] / 2 + 1;
+      }
+    }
     const size_t st_in = c->ln_axis == 1 ? B * C : B * T, st_out = c->ln_axis == 1 ? B * C : B * To;
     Lb.x_in = x_prev;
     Lb.size_in = size_prev;
@@ -202,7 +242,7 @@ static StackLayout make_layout(const tome_stack_cfg_t* c, void* workspace) {
     Lb.node_idx = nullptr;
     Lb.importance = nullptr;
     Lb.prune_ids = nullptr;
-    if (r > 0 && c->prune_sets > 0) {
+    if (r > 0 && c->prune_sets > 0 && !c->set_merge) {
       Lb.importance = b.take<float>(B * T);
       Lb.prune_ids = b.take<int32_t>(B * To);
       Lb.plan.row_map = b.take<int32_t>(B * T);
@@ -215,7 +255,7 @@ static StackLayout make_layout(const tome_stack_cfg_t* c, void* workspace) {
       Lb.plan.edge_idx = b.take<int32_t>(B * ta);
       Lb.plan.dst_idx = b.take<int32_t>(B * r);
       Lb.plan.row_map = b.take<int32_t>(B * T);
-      Lb.plan.dst_off = b.take<int32_t>(B * (tb + 1));
+      Lb.plan.dst_off = b.take<int32_t>(B * n_off);
       Lb.plan.dst_src = b.take<int32_t>(B * r);
       Lb.size_out = b.take<float>(B * To);
       Lb.gid_out = c->num_groups ? b.take<uint8_t>(B * To) : nullptr;
@@ -388,6 +428,8 @@ static int check_io(const tome_stack_cfg_t* c, const tome_stack_io_t* io, const 
              "stack: a group mask needs gid, pos (or layer_gid, layer_pos) and allow");
   TOME_CHECK(!(io->layer_gid || io->layer_pos) || (c->prune_sets > 0 && c->num_groups > 0 && io->layer_gid && io->layer_pos), TOME_ERR_INVALID,
              "stack: layer_gid / layer_pos are the per-layer masks of a pruning stack with a group mask (both or neither)");
+  TOME_CHECK(!(c->set_merge && (io->layer_gid || io->layer_pos)), TOME_ERR_INVALID,
+             "stack: a set-merging stack carries gid / pos through its merges and takes no layer_gid / layer_pos");
   TOME_CHECK(c->n_readout == 0 || io->readout_idx, TOME_ERR_INVALID, "stack: readout_idx missing");
   if (backward) TOME_CHECK(io->grads_f32 && io->target && io->loss && c->n_readout > 0, TOME_ERR_INVALID,
                            "stack_backward: needs grads_f32, target, loss and n_readout > 0");
@@ -428,17 +470,17 @@ extern "C" int tome_stack_forward(const tome_stack_cfg_t* c, const tome_stack_io
     RC(gemm(c, S, st, M, C, HD, Lb.attn_o, HD, TOME_MAJOR_K, pw + o.wo, C, TOME_MAJOR_MN, x1, C, TOME_BF16, pf + o.bo, 0,
             Lb.x_in, nullptr, 1.f, 3 * l + 0, 0));
     grammar_off += T;
-    if (r > 0 && c->prune_sets > 0) {
+    if (r > 0 && c->prune_sets > 0 && !c->set_merge) {
       // importance from this layer's attention weights, per-set top-k, gather (compressed_attention.py:303-308)
       RC(tome_attention_importance(&ad, Lb.qkv, Lb.qkv + HD, Lb.lse, c->prune_importance, Lb.importance, st));
       tome_prune_desc_t pd;
       memset(&pd, 0, sizeof(pd));
       pd.batch = B; pd.tokens = T; pd.channels = C; pd.dtype = TOME_BF16; pd.n_sets = c->prune_sets; pd.score_planes = 1;
-      for (int i = 0, start = 0; i < c->prune_sets; ++i) {
-        pd.set_start[i] = start;
-        pd.set_n[i] = c->prune_set_n[i] - l * c->prune_set_c[i];
-        pd.set_k[i] = pd.set_n[i] - c->prune_set_c[i];
-        start += pd.set_n[i];
+      const tome_token_sets_t ts = layer_sets(c, l);
+      for (int i = 0; i < c->prune_sets; ++i) {
+        pd.set_start[i] = ts.set_start[i];
+        pd.set_n[i] = ts.set_n[i];
+        pd.set_k[i] = ts.set_n[i] - ts.set_r[i];
       }
       RC(tome_topk_prune(&pd, x1, Lb.importance, Lb.x1m, Lb.prune_ids, st));
       const bool grammar = io->layer_gid != nullptr && c->num_groups > 0;
@@ -451,14 +493,18 @@ extern "C" int tome_stack_forward(const tome_stack_cfg_t* c, const tome_stack_io
         TOME_CUDA(cudaGetLastError());
       }
     } else if (r > 0) {
+      // merging: over the whole sequence, or inside each token set (the sets of a set-merging stack)
+      const tome_token_sets_t ts = merges_in_sets(c) ? layer_sets(c, l) : tome_token_sets_t{};
+      const tome_token_sets_t* sets = merges_in_sets(c) ? &ts : nullptr;
       tome_metric_desc_t md;
+      memset(&md, 0, sizeof(md));
       md.batch = B; md.tokens = T; md.dim = D; md.heads = H; md.dtype = TOME_BF16;
       md.batch_stride = (long long)T * 3 * HD; md.token_stride = 3 * HD; md.head_stride = D;
-      md.class_token = c->class_token; md.distill_token = c->distill_token;
+      md.class_token = c->class_token; md.distill_token = c->distill_token; md.sets = sets;
       RC(tome_sim_argmax(&md, Lb.qkv + HD, Lb.node_max, Lb.node_idx, nullptr, S.ws_sim, S.ws_sim_bytes, st));
-      tome_plan_shape_t ps{B, T, r, c->distill_token};
+      tome_plan_shape_t ps{B, T, r, c->distill_token, sets};
       RC(tome_select_topr(&ps, Lb.node_max, Lb.node_idx, &Lb.plan, st));
-      tome_merge_shape_t ms{B, T, C, r, c->distill_token, TOME_BF16, TOME_MERGE_WAVG};
+      tome_merge_shape_t ms{B, T, C, r, c->distill_token, TOME_BF16, TOME_MERGE_WAVG, sets};
       RC(tome_merge_fwd(&ms, &Lb.plan, x1, Lb.size_in, Lb.x1m, Lb.size_out, Lb.gid_in, Lb.pos_in, Lb.gid_out, Lb.pos_out, st));
     }
     RC(tome_layernorm_fwd(B, To, C, c->ln_axis, c->ln_eps, Lb.x1m, pf + o.ln2_scale, pf + o.ln2_bias, Lb.h2, Lb.ln2_mean,
@@ -574,11 +620,13 @@ extern "C" int tome_stack_backward(const tome_stack_cfg_t* c, const tome_stack_i
                           gr + o.ln2_scale, gr + o.ln2_bias, S.ws_ln, st));
     // ---- merge backward -> dx1 in g0
     const __nv_bfloat16* dx1;
-    if (r > 0 && c->prune_sets > 0) {
+    if (r > 0 && c->prune_sets > 0 && !c->set_merge) {
       RC(tome_prune_bwd(B, T, To, C, TOME_BF16, Lb.plan.row_map, g2, g0, st));
       dx1 = g0;
     } else if (r > 0) {
-      tome_merge_shape_t ms{B, T, C, r, c->distill_token, TOME_BF16, TOME_MERGE_WAVG};
+      // the global row map: the same backward with or without token sets
+      const tome_token_sets_t ts = merges_in_sets(c) ? layer_sets(c, l) : tome_token_sets_t{};
+      tome_merge_shape_t ms{B, T, C, r, c->distill_token, TOME_BF16, TOME_MERGE_WAVG, merges_in_sets(c) ? &ts : nullptr};
       RC(tome_merge_bwd(&ms, &Lb.plan, Lb.size_in, Lb.size_out, g2, g0, st));
       dx1 = g0;
     } else {

@@ -57,6 +57,9 @@ class StackConfig:
     # as written) or "received"
     prune_sets: tuple = ()
     prune_importance: str = "received"
+    # with prune_sets: every layer MERGES its c tokens inside each set instead of pruning them (bipartite soft matching per
+    # token set, merge_wavg; include/tome_b200.h tome_stack_cfg_t.set_merge), so no token merges across a set boundary
+    set_merge: bool = False
 
     def c(self) -> L.StackCfg:
         return L.StackCfg(self.batch, self.tokens, self.channels, self.heads, self.head_dim, self.mlp_dim, self.layers,
@@ -66,7 +69,19 @@ class StackConfig:
                           self.head_groups, self.head_features, self.max_action, self.head_fourier_dim, self.head_time_hidden,
                           self.head_time_out, self.head_hidden, self.diffusion_steps, len(self.prune_sets),
                           (C.c_int * 16)(*[int(n) for n, _ in self.prune_sets]), (C.c_int * 16)(*[int(c) for _, c in self.prune_sets]),
-                          {"row_mean": L.IMPORTANCE_ROW_MEAN, "received": L.IMPORTANCE_RECEIVED}[self.prune_importance])
+                          {"row_mean": L.IMPORTANCE_ROW_MEAN, "received": L.IMPORTANCE_RECEIVED}[self.prune_importance],
+                          int(self.set_merge))
+
+    def layer_sets(self, layer: int):
+        """((start, n, r), ...) of the token sets entering `layer` of a set-merging stack, None for any other stack."""
+        if not (self.set_merge and self.prune_sets):
+            return None
+        out, start = [], 0
+        for n0, c in self.prune_sets:
+            n = int(n0) - layer * int(c)
+            out.append((start, n, int(c)))
+            start += n
+        return tuple(out)
 
     def diffusion_desc(self, tokens: int = 1) -> L.DiffusionDesc:
         return L.DiffusionDesc(self.batch, tokens, self.channels, self.n_readout, self.head_features, self.head_fourier_dim,
@@ -306,13 +321,16 @@ class ToMeStackEngine:
         return self._view(p, (self.cfg.batch, self.tokens_at(self.cfg.layers)), torch.float32)
 
     def layer_plan(self, layer: int):
-        """(node_max, node_idx, edge_idx, dst_idx) of one layer's matching, or None if that layer merged nothing."""
+        """(node_max, node_idx, edge_idx, dst_idx) of one layer's matching, or None if that layer merged nothing.  In a
+        set-merging stack the arrays are concatenated set by set (cfg.layer_sets(layer)), indices local to the set."""
         io = self._io(self._x, self._target)
         t = self.tokens_at(layer)
         r = t - self.tokens_at(layer + 1)
         if r == 0:
             return None
-        ta, b = (t + 1) // 2, self.cfg.batch
+        sets = self.cfg.layer_sets(layer)
+        ta = (t + 1) // 2 if sets is None else sum((n + 1) // 2 for _, n, _ in sets)
+        b = self.cfg.batch
         f = self.lib
         nm = self._view(f.tome_stack_layer_node_max(C.byref(self.ccfg), C.byref(io), layer), (b, ta), torch.float32)
         ni = self._view(f.tome_stack_layer_node_idx(C.byref(self.ccfg), C.byref(io), layer), (b, ta), torch.int32)

@@ -44,9 +44,26 @@ def clamp_r(tokens: int, r: int, class_token: bool = False, distill_token: bool 
 
 
 # ------------------------------------------------------------------------------------------------ matching
+def token_sets(sets) -> Optional[L.TokenSets]:
+    """tome_token_sets_t of `sets`, a sequence of (start, n, r) per token set (matching and merging stay inside each set; set s
+    loses r tokens), or None: one set spanning the sequence."""
+    if sets is None:
+        return None
+    sets = [tuple(int(v) for v in s_) for s_ in sets]
+    if not 1 <= len(sets) <= L.MAX_TOKEN_SETS:
+        raise ValueError(f"between 1 and {L.MAX_TOKEN_SETS} token sets are supported, got {len(sets)}")
+    pad = lambda xs: (C.c_int32 * L.MAX_TOKEN_SETS)(*xs)  # noqa: E731
+    return L.TokenSets(len(sets), pad([s_[0] for s_ in sets]), pad([s_[1] for s_ in sets]), pad([s_[2] for s_ in sets]))
+
+
+def _sets_ptr(ts: Optional[L.TokenSets]):
+    return None if ts is None else C.cast(C.pointer(ts), C.c_void_p)
+
+
 @dataclass
 class MatchPlan:
-    """Device-resident index set of one bipartite matching (token_compression.py:84-88)."""
+    """Device-resident index set of one bipartite matching (token_compression.py:84-88).  With token sets every array is
+    concatenated set by set and its indices are local to the set (include/tome_b200.h); row_map holds global output rows."""
 
     batch: int
     tokens: int
@@ -60,6 +77,7 @@ class MatchPlan:
     dst_off: torch.Tensor   # [B,Tb+1] i32
     dst_src: torch.Tensor   # [B,r] i32
     scores: Optional[torch.Tensor] = None
+    sets: Optional[tuple] = None   # ((start, n, r), ...) or None: one set
 
     @property
     def src_idx(self):
@@ -85,19 +103,27 @@ def _scratch(nbytes: int, device, buf: Optional[torch.Tensor] = None) -> torch.T
 
 def sim_argmax(src: torch.Tensor, *, heads: int = 1, dim: Optional[int] = None, batch_stride=None, token_stride=None,
                head_stride=None, tokens=None, batch=None, class_token=False, distill_token=False, dump_scores=False,
-               offset_elems: int = 0):
-    """K1.  `src` is either a [B,T,Dm] metric (heads=1) or a packed buffer addressed by the given strides."""
+               offset_elems: int = 0, sets=None):
+    """K1.  `src` is either a [B,T,Dm] metric (heads=1) or a packed buffer addressed by the given strides.
+    sets: ((start, n, r), ...) to match inside each token set; node_max / node_idx are then [B, sum ceil(n/2)] (indices local
+    to the set) and the scores dump [B, sum ceil(n/2) * floor(n/2)], each set's block row-major in turn."""
     _need_cuda(src)
     if heads == 1 and dim is None:
         assert src.dim() == 3 and src.is_contiguous()
         batch, tokens, dim = src.shape
         batch_stride, token_stride, head_stride = tokens * dim, dim, 0
-    ta, tb = (tokens + 1) // 2, tokens // 2
+    ts = token_sets(sets)
+    if ts is None:
+        ta, tb = (tokens + 1) // 2, tokens // 2
+        score_shape = (batch, ta, tb)
+    else:
+        ta = sum((int(n) + 1) // 2 for _, n, _ in sets)
+        score_shape = (batch, sum(((int(n) + 1) // 2) * (int(n) // 2) for _, n, _ in sets))
     node_max = torch.empty(batch, ta, dtype=torch.float32, device=src.device)
     node_idx = torch.empty(batch, ta, dtype=torch.int32, device=src.device)
-    scores = torch.empty(batch, ta, tb, dtype=torch.float32, device=src.device) if dump_scores else None
+    scores = torch.empty(score_shape, dtype=torch.float32, device=src.device) if dump_scores else None
     d = L.MetricDesc(batch, tokens, dim, heads, _dt(src), batch_stride, token_stride, head_stride,
-                     int(bool(class_token)), int(bool(distill_token)))
+                     int(bool(class_token)), int(bool(distill_token)), _sets_ptr(ts))
     base = C.c_void_p(src.data_ptr() + offset_elems * src.element_size())
     ws = _scratch(L.lib().tome_sim_argmax_workspace_bytes(C.byref(d)), src.device)
     L.check(L.lib().tome_sim_argmax(C.byref(d), base, _ptr(node_max), _ptr(node_idx), _ptr(scores), _ptr(ws), ws.numel(),
@@ -105,25 +131,34 @@ def sim_argmax(src: torch.Tensor, *, heads: int = 1, dim: Optional[int] = None, 
     return node_max, node_idx, scores
 
 
-def select_topr(node_max: torch.Tensor, node_idx: torch.Tensor, tokens: int, r: int, distill_token=False) -> MatchPlan:
-    """K2.  `r` must already be clamped and >= 1."""
+def select_topr(node_max: torch.Tensor, node_idx: torch.Tensor, tokens: int, r: Optional[int] = None, distill_token=False,
+                sets=None) -> MatchPlan:
+    """K2.  `r` must already be clamped and >= 1.  sets: ((start, n, r), ...) as for sim_argmax, whose node_max / node_idx
+    this takes; r defaults to (and must equal) the sum of the sets' r."""
     _need_cuda(node_max, node_idx)
     b = node_max.shape[0]
-    ta, tb = (tokens + 1) // 2, tokens // 2
+    ts = token_sets(sets)
+    if ts is None:
+        ta, n_off = (tokens + 1) // 2, tokens // 2 + 1
+    else:
+        sets = tuple(tuple(int(v) for v in s_) for s_ in sets)
+        r = sum(s_[2] for s_ in sets) if r is None else r
+        ta, n_off = sum((n + 1) // 2 for _, n, _ in sets), sum(n // 2 + 1 for _, n, _ in sets)
     dev = node_max.device
     i32 = torch.int32
     plan = MatchPlan(b, tokens, r, bool(distill_token), node_max, node_idx,
                      torch.empty(b, ta, dtype=i32, device=dev), torch.empty(b, r, dtype=i32, device=dev),
-                     torch.empty(b, tokens, dtype=i32, device=dev), torch.empty(b, tb + 1, dtype=i32, device=dev),
-                     torch.empty(b, r, dtype=i32, device=dev))
-    shp = L.PlanShape(b, tokens, r, int(bool(distill_token)))
+                     torch.empty(b, tokens, dtype=i32, device=dev), torch.empty(b, n_off, dtype=i32, device=dev),
+                     torch.empty(b, r, dtype=i32, device=dev), sets=sets)
+    shp = L.PlanShape(b, tokens, r, int(bool(distill_token)), _sets_ptr(ts))
     cp = plan.c_plan()
     L.check(L.lib().tome_select_topr(C.byref(shp), _ptr(node_max), _ptr(node_idx), C.byref(cp), _stream()))
     return plan
 
 
 def merge_fwd(plan: MatchPlan, x: torch.Tensor, size: Optional[torch.Tensor], mode: int, gid=None, pos=None):
-    """K3.  x [B,T,C] (bf16/fp32, contiguous); size f32 [B,T] or None.  Returns (x_out, size_out, gid_out, pos_out)."""
+    """K3.  x [B,T,C] (bf16/fp32, contiguous); size f32 [B,T] or None.  Returns (x_out, size_out, gid_out, pos_out).
+    A plan of select_topr(sets=...) merges inside each token set (its sets travel with the plan)."""
     _need_cuda(x, size)
     assert x.is_contiguous() and x.dim() == 3
     b, t, c = x.shape
@@ -133,7 +168,8 @@ def merge_fwd(plan: MatchPlan, x: torch.Tensor, size: Optional[torch.Tensor], mo
     size_out = torch.empty(b, to, dtype=torch.float32, device=x.device) if mode == L.TOME_MERGE_WAVG else None
     gid_out = torch.empty(b, to, dtype=torch.uint8, device=x.device) if gid is not None else None
     pos_out = torch.empty(b, to, dtype=torch.int32, device=x.device) if pos is not None else None
-    shp = L.MergeShape(b, t, c, plan.r, int(plan.distill_token), _dt(x), mode)
+    ts = token_sets(plan.sets)
+    shp = L.MergeShape(b, t, c, plan.r, int(plan.distill_token), _dt(x), mode, _sets_ptr(ts))
     cp = plan.c_plan()
     L.check(L.lib().tome_merge_fwd(C.byref(shp), C.byref(cp), _ptr(x), _ptr(size), _ptr(x_out), _ptr(size_out),
                                    _ptr(gid), _ptr(pos), _ptr(gid_out), _ptr(pos_out), _stream()))
@@ -147,7 +183,8 @@ def merge_bwd(plan: MatchPlan, dy: torch.Tensor, size: Optional[torch.Tensor], s
     b, to, c = dy.shape
     t = plan.tokens
     dx = torch.empty(b, t, c, dtype=dy.dtype, device=dy.device)
-    shp = L.MergeShape(b, t, c, plan.r, int(plan.distill_token), _dt(dy), mode)
+    ts = token_sets(plan.sets)
+    shp = L.MergeShape(b, t, c, plan.r, int(plan.distill_token), _dt(dy), mode, _sets_ptr(ts))
     cp = plan.c_plan()
     L.check(L.lib().tome_merge_bwd(C.byref(shp), C.byref(cp), _ptr(size), _ptr(size_out), _ptr(dy), _ptr(dx), _stream()))
     return dx

@@ -7,6 +7,10 @@ Mirror of multi_modal_transformers/tokenizers/token_compression.py (same names, 
     y = merge(x, mode="sum")                                                               # :90-109
     x, size = merge_wavg(merge, x, size=None)                                              # :114-129
 
+and, additive (the merging counterpart of compute_top_k_tokens' per-modality sets):
+
+    merge = tokenset_soft_matching(metric, tokenset_idx, tokenset_r)                       # matching inside each set
+
 Arrays are CUDA torch tensors (device memory is all torch is used for); every step launches a hand-written
 kernel through the C ABI (include/tome_b200.h: tome_sim_argmax, tome_select_topr, tome_merge_fwd / _bwd).  There is
 no CPU path: a CPU tensor raises.
@@ -131,6 +135,39 @@ def bipartite_soft_matching(metric: torch.Tensor, r: int, class_token: bool = Fa
     return _Merge(plan, t)
 
 
+def tokenset_soft_matching(metric: torch.Tensor, tokenset_idx, tokenset_r) -> Callable:
+    """Bipartite soft matching inside each token set: `merge` for merge_wavg / merge(x, "sum") that never merges a token
+    with one of another set.  tokenset_idx: (start_idx, num_tokens) per set as compute_top_k_tokens takes them, consecutive
+    and covering the sequence; tokenset_r: tokens each set loses (0 <= r <= num_tokens // 2; r = 0 leaves the set as it is).
+
+    The result for set s is bipartite_soft_matching(metric[:, s], r_s) + merge applied to the set's slice alone (the even /
+    odd split counted from the set's first token, the same tie rules and fp32 adds); the sets' outputs are concatenated in
+    order, so every set stays contiguous.  With one set per frame and modality of a block-causal sequence, a merged row keeps
+    the group of every token in it.  One launch each of K1, K2 (and K3 per merge) over all sets."""
+    if metric.dim() != 3:
+        raise ValueError(f"metric must be [batch, tokens, dim], got {tuple(metric.shape)}")
+    if len(tokenset_idx) != len(tokenset_r):
+        raise ValueError("tokenset_idx and tokenset_r must have one entry per token set")
+    if not 1 <= len(tokenset_r) <= L.MAX_TOKEN_SETS:
+        raise ValueError(f"between 1 and {L.MAX_TOKEN_SETS} token sets are supported, got {len(tokenset_r)}")
+    t = metric.shape[1]
+    sets, start = [], 0
+    for (s_, n), r in zip(tokenset_idx, tokenset_r):
+        s_, n, r = int(s_), int(n), int(r)
+        if s_ != start or n < 1:
+            raise ValueError(f"token sets must be consecutive and non-empty: expected a set starting at {start}, got ({s_}, {n})")
+        if not 0 <= r <= n // 2:
+            raise ValueError(f"token set ({s_}, {n}): r = {r} out of range [0, {n // 2}]")
+        sets.append((s_, n, r))
+        start += n
+    if start != t:
+        raise ValueError(f"the token sets cover {start} tokens, metric has {t}")
+    if sum(r for _, _, r in sets) == 0:
+        return _Merge(None, t)
+    node_max, node_idx, _ = ops.sim_argmax(metric.contiguous(), sets=sets)
+    return _Merge(ops.select_topr(node_max, node_idx, t, sets=sets), t)
+
+
 def merge_wavg(merge: Callable, x: torch.Tensor, size: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """token_compression.py:114-129.  Returns (x [n, t-r, c], size [n, t-r, 1] fp32)."""
     if isinstance(merge, _Merge):
@@ -139,4 +176,4 @@ def merge_wavg(merge: Callable, x: torch.Tensor, size: Optional[torch.Tensor] = 
         if size is None:
             size = torch.ones(x.shape[0], x.shape[1], 1, dtype=torch.float32, device=x.device)
         return x, size
-    raise TypeError("merge_wavg: `merge` must come from bipartite_soft_matching")
+    raise TypeError("merge_wavg: `merge` must come from bipartite_soft_matching or tokenset_soft_matching")

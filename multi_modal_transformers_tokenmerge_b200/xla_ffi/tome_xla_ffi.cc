@@ -34,7 +34,7 @@ static ffi::Error SimArgmax(cudaStream_t s, ffi::ScratchAllocator scratch, ffi::
                             int32_t class_token, int32_t distill_token) {
   auto d = metric.dimensions();
   tome_metric_desc_t m{(int)d[0], (int)d[1], (int)d[2], 1, DType(metric.element_type()), (long long)(d[1] * d[2]), (long long)d[2], 0,
-                       class_token, distill_token};
+                       class_token, distill_token, /*sets: one set (the FFI handlers take no token-set table)*/ nullptr};
   const size_t ws_bytes = tome_sim_argmax_workspace_bytes(&m);
   std::optional<void*> ws = scratch.Allocate(ws_bytes, 256);
   if (!ws.has_value()) return ffi::Error(ffi::ErrorCode::kResourceExhausted, "tome_sim_argmax: scratch allocation failed");
@@ -50,7 +50,7 @@ static ffi::Error SelectTopR(cudaStream_t s, ffi::Buffer<ffi::F32> node_max, ffi
                              ffi::Result<ffi::Buffer<ffi::S32>> edge, ffi::Result<ffi::Buffer<ffi::S32>> dst,
                              ffi::Result<ffi::Buffer<ffi::S32>> row_map, ffi::Result<ffi::Buffer<ffi::S32>> dst_off,
                              ffi::Result<ffi::Buffer<ffi::S32>> dst_src, int32_t tokens, int32_t r, int32_t distill_token) {
-  tome_plan_shape_t ps{(int)node_max.dimensions()[0], tokens, r, distill_token};
+  tome_plan_shape_t ps{(int)node_max.dimensions()[0], tokens, r, distill_token, /*sets=*/nullptr};
   tome_plan_t p{edge->typed_data(), dst->typed_data(), row_map->typed_data(), dst_off->typed_data(), dst_src->typed_data()};
   return Status(tome_select_topr(&ps, node_max.typed_data(), node_idx.typed_data(), &p, s));
 }
@@ -65,7 +65,7 @@ static ffi::Error MergeFwd(cudaStream_t s, ffi::AnyBuffer x, ffi::Buffer<ffi::F3
                            ffi::Buffer<ffi::S32> dst_off, ffi::Buffer<ffi::S32> dst_src, ffi::Result<ffi::AnyBuffer> x_out,
                            ffi::Result<ffi::Buffer<ffi::F32>> size_out, int32_t r, int32_t mode, int32_t distill_token) {
   auto d = x.dimensions();
-  tome_merge_shape_t ms{(int)d[0], (int)d[1], (int)d[2], r, distill_token, DType(x.element_type()), mode};
+  tome_merge_shape_t ms{(int)d[0], (int)d[1], (int)d[2], r, distill_token, DType(x.element_type()), mode, /*sets=*/nullptr};
   tome_plan_t p{};
   p.edge_idx = edge.typed_data(); p.dst_off = dst_off.typed_data(); p.dst_src = dst_src.typed_data();
   return Status(tome_merge_fwd(&ms, &p, x.untyped_data(), size.typed_data(), x_out->untyped_data(), size_out->typed_data(),
@@ -81,7 +81,7 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(TomeMergeFwd, MergeFwd,
 static ffi::Error MergeBwd(cudaStream_t s, ffi::AnyBuffer dy, ffi::Buffer<ffi::F32> size, ffi::Buffer<ffi::F32> size_out,
                            ffi::Buffer<ffi::S32> row_map, ffi::Result<ffi::AnyBuffer> dx, int32_t r, int32_t mode) {
   auto d = dx->dimensions();
-  tome_merge_shape_t ms{(int)d[0], (int)d[1], (int)d[2], r, 0, DType(dy.element_type()), mode};
+  tome_merge_shape_t ms{(int)d[0], (int)d[1], (int)d[2], r, 0, DType(dy.element_type()), mode, /*sets=*/nullptr};
   tome_plan_t p{};
   p.row_map = row_map.typed_data();
   return Status(tome_merge_bwd(&ms, &p, size.typed_data(), size_out.typed_data(), dy.untyped_data(), dx->untyped_data(), s));
