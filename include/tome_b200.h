@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define TOME_ABI_VERSION 15
+#define TOME_ABI_VERSION 16
 
 enum tome_status { TOME_OK = 0, TOME_ERR_INVALID = 1, TOME_ERR_CUDA = 2, TOME_ERR_UNSUPPORTED = 3 };
 enum tome_dtype { TOME_BF16 = 0, TOME_F32 = 1, TOME_U8 = 2 /* raw pixels: image front end only */ };
@@ -421,11 +421,27 @@ int tome_diffusion_head_bwd(const tome_diffusion_desc_t* desc, const float* para
                             const int32_t* origin, const int32_t* time, void* workspace, float* grads_f32, void* dx,
                             void* stream);
 
-/* One update of the diffusion head's sampling loop (action_heads/diffusion.py:182-190, inference): out = clip(c1 * (sample - c2 *
- * denoise_term) + c3 * noise, -clip, clip) over n floats; the denoise term of each step is tome_diffusion_head_fwd with an
- * alpha_hat table of ones (noisy = the current sample) -- the Python mirror's predict_action strings the steps together. */
-int tome_ddpm_step(long long n, const float* sample, const float* denoise_term, const float* noise, float c1, float c2, float c3,
-                   float clip, float* out, void* stream);
+/* Diffusion action head, inference: DiffusionActionHead.predict_action (action_heads/diffusion.py:146-213), the whole reverse
+ * process in one call.  Starting from init, for t = steps - 1 .. 0 (step i = steps - 1 - t):
+ *   eps = the denoiser of tome_diffusion_head_fwd on [sample | te(t) | emb];  sample = clip(c1 (sample - c2 eps) + c3 noise_i)
+ * with coef[t] = {c1 = 1/sqrt(alpha_t), c2 = (1 - alpha_t)/sqrt(1 - alpha_hat_t), c3 = sqrt(beta_t)} computed by the caller,
+ * noise_i = noise ([B, A], reused by every step as the reference does at :179) or noise + i B A ([steps, B, A]), clip to
+ * [-clip, clip] (:189).  x / origin as tome_diffusion_head_fwd; actions f32 [B, A] out.  The denoiser input's first A columns
+ * run in fp32 (W1[:A], W2 and b2 from params_f32); the readout mean and the time embedding through bf16 GEMMs as in training.
+ * One kernel runs every step, so the call makes six launches whatever `steps` is.  It needs action_dim <= 64, hidden <= 2048
+ * and W1[:A] and W2 in fp32 (8 A H bytes) within 227 KB of shared memory, else TOME_ERR_UNSUPPORTED.
+ * Deterministic: the same inputs give the same bits, whatever the batch size. */
+typedef struct {
+  const float* init;    /* f32 [B, A]: the Gaussian start (diffusion.py:203) */
+  const float* noise;   /* f32 [B, A] (noise_per_step = 0) or [steps, B, A] (noise_per_step = 1) */
+  int noise_per_step;
+  const float* coef;    /* f32 [steps, 3]: c1, c2, c3 of time step t in row t */
+  float clip;           /* > 0; the reference clips to 5.0 */
+} tome_ddpm_sample_t;
+size_t tome_diffusion_head_sample_workspace_bytes(const tome_diffusion_desc_t* desc);
+int tome_diffusion_head_sample(const tome_diffusion_desc_t* desc, const float* params_f32, const void* params_bf16, const void* x,
+                               const int32_t* origin, const tome_ddpm_sample_t* sample, float* actions, void* workspace,
+                               size_t workspace_bytes, void* stream);
 
 /* AdamW on an fp32 master vector with a bf16 working copy refreshed in the same pass (bf16_copy may be NULL).
  * grad_scale multiplies the gradient first (1/world_size after a sum all-reduce). */
@@ -544,6 +560,23 @@ const uint32_t* tome_stack_layer_relu_bits(const tome_stack_cfg_t* cfg, const to
 /* pruning stacks: f32 [B, T_in(layer)] importance scores the layer ranked, i32 [B, T_out(layer)] the token indices it kept */
 const float* tome_stack_layer_importance(const tome_stack_cfg_t* cfg, const tome_stack_io_t* io, int layer);
 const int32_t* tome_stack_layer_prune_ids(const tome_stack_cfg_t* cfg, const tome_stack_io_t* io, int layer);
+
+/* Forward-only executor: the forward of tome_stack_forward over a workspace that keeps nothing for backward.  The residual
+ * stream, sizes and group ids ping-pong between two buffers and every layer reuses one set of scratch; only each merging or
+ * pruning layer's row map (4 B T_in(l) bytes) stays, for the readout origins, so the workspace does not otherwise grow with
+ * `layers`.  Every stack kind tome_stack_forward accepts runs here.
+ *   - Dropout is off: cfg->dropout_rate and attn_dropout_rate are not applied, so one cfg serves a training executor and its
+ *     predictor.  The reference's Octo.generate_readouts passes train=True even when predicting (octo.py:120); stochastic
+ *     prediction as it does is tome_stack_forward with the dropout rates set.
+ *   - At dropout 0 x_final, readout and head_out (heads 1 and 2) equal tome_stack_forward's bit for bit.
+ *   - Outputs, each optional except head_out when cfg->head > 0: io->x_final (bf16 [B, T_L, C]), io->readout (f32
+ *     [B, n_readout, C]), io->head_out: tanh actions [B, A] (head 1), logits [B, groups, bins] (head 2), or actions [B, A]
+ *     sampled by tome_diffusion_head_sample with `sample` (head 3; sample must be NULL for any other head).
+ *   - io->target, loss, grads_f32, grad_trace, head_time, head_alpha_hats and layer_done_events are not read.
+ *   - io->workspace holds tome_stack_predict_workspace_bytes(cfg) bytes.  The tome_stack_layer_* / tome_stack_final_*
+ *     accessors describe the training workspace and are invalid on a predict workspace. */
+size_t tome_stack_predict_workspace_bytes(const tome_stack_cfg_t* cfg);
+int tome_stack_predict(const tome_stack_cfg_t* cfg, const tome_stack_io_t* io, const tome_ddpm_sample_t* sample, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * 7b. Image patch-embed front end (forward)   tokenizers/images/image_tokenizer.py:35-71 (image_to_patches), :74-140

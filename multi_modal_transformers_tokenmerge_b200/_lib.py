@@ -15,7 +15,7 @@ TOME_OK, TOME_ERR_INVALID, TOME_ERR_CUDA, TOME_ERR_UNSUPPORTED = 0, 1, 2, 3
 TOME_BF16, TOME_F32, TOME_U8 = 0, 1, 2
 TOME_MAJOR_K, TOME_MAJOR_MN = 0, 1
 TOME_MERGE_SUM, TOME_MERGE_WAVG = 0, 1
-ABI_VERSION = 15
+ABI_VERSION = 16
 
 vp, ll, i32, f32, u64, u32 = C.c_void_p, C.c_longlong, C.c_int, C.c_float, C.c_uint64, C.c_uint32
 
@@ -109,6 +109,11 @@ class DiffusionDesc(C.Structure):
                 ("fourier_dim", i32), ("time_hidden", i32), ("time_out", i32), ("hidden", i32), ("diffusion_steps", i32)]
 
 
+class DdpmSample(C.Structure):
+    """tome_ddpm_sample_t: the sampler's draws and schedule (tome_diffusion_head_sample, tome_stack_predict)."""
+    _fields_ = [("init", vp), ("noise", vp), ("noise_per_step", i32), ("coef", vp), ("clip", f32)]
+
+
 DIFFUSION_PARAMS = ["fourier_kernel", "tw1", "tb1", "tw2", "tb2", "w1", "b1", "w2", "b2"]
 
 
@@ -157,6 +162,7 @@ def lib() -> C.CDLL:
             raise ImportError(f"libtome_b200.so has ABI {L.tome_abi_version()}, python binding expects {ABI_VERSION}: rebuild")
         for name in ("tome_gemm_workspace_bytes", "tome_stack_workspace_bytes", "tome_attention_workspace_bytes", "tome_sim_argmax_workspace_bytes",
                      "tome_attention_bwd_workspace_bytes", "tome_action_head_workspace_bytes", "tome_diffusion_head_workspace_bytes",
+                     "tome_diffusion_head_sample_workspace_bytes", "tome_stack_predict_workspace_bytes",
                      "tome_image_tokenizer_workspace_bytes"):
             getattr(L, name).restype = C.c_size_t
         for name in ("tome_stack_param_count", "tome_stack_layer_offset", "tome_stack_head_offset", "tome_launch_count",
@@ -215,7 +221,8 @@ def lib() -> C.CDLL:
             "tome_image_tokenizer_param_offset": [P(ImageTokenizerDesc), i32],
             "tome_image_tokenizer_workspace_bytes": [P(ImageTokenizerDesc)],
             "tome_image_tokenizer_fwd": [P(ImageTokenizerDesc), vp, vp, vp, vp, vp, vp, vp, C.c_size_t, vp],
-            "tome_ddpm_step": [ll, vp, vp, vp, f32, f32, f32, f32, vp, vp],
+            "tome_diffusion_head_sample_workspace_bytes": [P(DiffusionDesc)],
+            "tome_diffusion_head_sample": [P(DiffusionDesc), vp, vp, vp, vp, P(DdpmSample), vp, vp, C.c_size_t, vp],
             "tome_adamw_step": [ll, vp, vp, vp, vp, vp, f32, f32, f32, f32, f32, f32, i32, vp],
             "tome_cast_f32_to_bf16": [ll, vp, vp, vp],
             "tome_launch_count": [i32],
@@ -227,6 +234,8 @@ def lib() -> C.CDLL:
             "tome_stack_workspace_bytes": [P(StackCfg)],
             "tome_stack_forward": [P(StackCfg), P(StackIO), vp],
             "tome_stack_backward": [P(StackCfg), P(StackIO), vp],
+            "tome_stack_predict_workspace_bytes": [P(StackCfg)],
+            "tome_stack_predict": [P(StackCfg), P(StackIO), P(DdpmSample), vp],
             "tome_stack_tokens_at": [P(StackCfg), i32],
             "tome_stack_final_x": [P(StackCfg), P(StackIO)],
             "tome_stack_final_size": [P(StackCfg), P(StackIO)],

@@ -9,8 +9,8 @@
 FourierFeatures + MLPBlock, mlp_block = the denoiser MLPBlock, num_blocks = 1).  Parameter tree, Flax names:
     denoiser/FourierFeatures_0/{fourier_kernel [F/2, 1], MLPBlock_0/Dense_{0,1}/{kernel, bias}}
     denoiser/MLPBlock_0/Dense_{0,1}/{kernel, bias}
-The sampling loop (`predict_action`, :145-213) is inference and outside the training path.  Random draws: jax's threefry
-cannot be reproduced, so `denoise_loss` draws time / noise from a numpy Generator seeded by `rng` (or takes them
+The sampling loop (`predict_action`, :145-213) runs as one call, tome_diffusion_head_sample.  Random draws: jax's threefry
+cannot be reproduced, so `denoise_loss` and `predict_action` draw from a numpy Generator seeded by `rng` (or take them
 explicitly) -- statistics, not bits, match the reference.
 """
 from __future__ import annotations
@@ -32,6 +32,16 @@ def cosine_beta_schedule(timesteps: int, s: float = 0.008) -> np.ndarray:
     ac = np.cos((t + f(s)) / f(1 + s) * f(np.pi) * f(0.5)) ** 2
     ac = ac / ac[0]
     return np.clip(f(1) - ac[1:] / ac[:-1], 0, 0.999).astype(np.float32)
+
+
+def ddpm_coefficients(betas: np.ndarray) -> np.ndarray:
+    """f32 [steps, 3]: row t = (c1, c2, c3) = (1 / sqrt(alpha_t), (1 - alpha_t) / sqrt(1 - alpha_hat_t), sqrt(beta_t)) of the
+    sampler's update (diffusion.py:183-186), in the precision the reference's host arithmetic gives."""
+    betas = np.asarray(betas, np.float32)
+    alphas = np.float32(1) - betas
+    ah = np.array([np.prod(alphas[: i + 1]) for i in range(len(betas))], np.float32)
+    return np.array([[1.0 / float(np.sqrt(alphas[t])), float((np.float32(1) - alphas[t]) / np.sqrt(np.float32(1) - ah[t])),
+                      float(np.sqrt(betas[t]))] for t in range(len(betas))], np.float32)
 
 
 class DiffusionActionHead(Module):
@@ -112,8 +122,7 @@ class DiffusionActionHead(Module):
         denoise term and apply algorithm 2 of arXiv:2006.11239 with the schedule's coefficients, clipping to [-5, 5] (:190).
         The reference draws its step noise from the SAME per-sample keys at every step (:179, "TODO: check keys here"), i.e. one
         noise tensor [B, A] reused by all steps; `noise` may also be [steps, B, A].  `init` / `noise` default to draws from `rng`
-        (numpy's generator, not jax.random's stream).  Every floating-point operation runs in the kernels."""
-        import ctypes as C_
+        (numpy's generator, not jax.random's stream).  All steps run in one call (tome_diffusion_head_sample)."""
         g = as_rng(rng)
         x = readouts.to(torch.bfloat16).contiguous()
         dev = x.device
@@ -122,24 +131,10 @@ class DiffusionActionHead(Module):
             init = torch.as_tensor(g.standard_normal((B, A)).astype(np.float32))
         if noise is None:
             noise = torch.as_tensor(g.standard_normal((B, A)).astype(np.float32))
-        sample = init.to(dev).float().contiguous().clone()
+        init = init.to(dev).float().contiguous()
         noise = noise.to(dev).float().contiguous()
-        desc, flat = self._desc(readouts), self._flat(variables["params"], dev)
-        ones = torch.ones(self.diffusion_steps, dtype=torch.float32, device=dev)
-        zeros = torch.zeros(B, A, dtype=torch.float32, device=dev)
-        strm = lambda: C_.c_void_p(torch.cuda.current_stream().cuda_stream)  # noqa: E731
-        for t in range(self.diffusion_steps - 1, -1, -1):                                              # :207-211
-            time = torch.full((B,), t, dtype=torch.int32, device=dev)
-            eps, _, _ = ops.diffusion_head_fwd(x, flat, desc, sample, zeros, time, ones)             # predict_denoise_term (:167-173)
-            c1 = 1.0 / float(np.sqrt(self.alphas[t]))                                                   # :183-185
-            c2 = float((np.float32(1) - self.alphas[t]) / np.sqrt(np.float32(1) - self.alpha_hats[t]))
-            c3 = float(np.sqrt(self.betas[t]))
-            nz = noise[self.diffusion_steps - 1 - t] if noise.dim() == 3 else noise
-            out = torch.empty_like(sample)
-            L.check(L.lib().tome_ddpm_step(B * A, C_.c_void_p(sample.data_ptr()), C_.c_void_p(eps.data_ptr()),
-                                           C_.c_void_p(nz.data_ptr()), c1, c2, c3, float(clip), C_.c_void_p(out.data_ptr()), strm()))
-            sample = out
-        return sample
+        coef = torch.as_tensor(ddpm_coefficients(self.betas)).to(dev)
+        return ops.diffusion_head_sample(x, self._flat(variables["params"], dev), self._desc(readouts), init, noise, coef, clip)
 
     def _apply(self, params, readouts, time, noisy_actions, dropout_rng=None):
         return self.predict_denoise_term({"params": params}, readouts, time, noisy_actions)

@@ -346,27 +346,188 @@ extern "C" int tome_diffusion_head_bwd(const tome_diffusion_desc_t* d, const flo
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// One step of the sampler's update (DiffusionActionHead.predict_action, action_heads/diffusion.py:182-190; algorithm 2 of
-// arXiv:2006.11239):  out = clip(c1 * (sample - c2 * denoise_term) + c3 * noise, -clip, clip), the coefficients taken from
-// the schedule by the caller (c1 = 1 / sqrt(alpha_t), c2 = (1 - alpha_t) / sqrt(1 - alpha_hat_t), c3 = sqrt(beta_t)).
+// The sampling loop (DiffusionActionHead.predict_action, action_heads/diffusion.py:146-213; algorithm 2 of arXiv:2006.11239):
+// for t = steps - 1 .. 0:  eps = OctoDenoise([sample | te(t) | emb]);  sample = clip(c1 (sample - c2 eps) + c3 noise).
+// Only the first A columns of the denoiser input change from step to step, so W1 splits by rows into [0, A) | [A, A + To) |
+// [A + To, Dc) and everything but the first block leaves the loop:
+//   zr[b]    = emb[b] W1[A + To:] + b1                         [B, H] fp32, one GEMM
+//   tproj[t] = te(t) W1[A:A + To], te(t) = time MLP(fourier(t)) [steps, H] fp32, GEMMs of M = steps (batch independent)
+// and one kernel runs all the steps: h = relu(zr + tproj[t] + sample W1[:A]), eps = h W2 + b2, with W1[:A] and W2 in fp32
+// shared memory and each row's sample on chip from the first step to the last.
 namespace tome {
-__global__ void ddpm_step_kernel(long long n, const float* __restrict__ sample, const float* __restrict__ eps,
-                                 const float* __restrict__ noise, float c1, float c2, float c3, float clip, float* __restrict__ out) {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const float v = c1 * (sample[i] - c2 * eps[i]) + c3 * noise[i];
-  out[i] = fminf(fmaxf(v, -clip), clip);
+
+constexpr int SMP_THREADS = 256;
+constexpr int SMP_MAX_ROWS = 8;        // batch rows per CTA: ceil(B / SMs) up to this, so B = 256 spans most SMs
+constexpr int SMP_MAX_A = 64, SMP_MAX_H = 2048;
+constexpr size_t SMP_MAX_SMEM = 227 * 1024;
+
+// W1[:A] [A, H] | W2^T [A, H] | b2 [A] | per row: zr [H], h [H], sample [A]
+static size_t sample_smem_bytes(long long A, long long H, int rows) {
+  return (size_t)(2 * A * H + A + (long long)rows * (2 * H + A)) * sizeof(float);
 }
+
+struct SampleWs {
+  __nv_bfloat16 *emb, *ff, *th, *te;
+  float *tproj, *zr;
+  size_t total;
+};
+static SampleWs sample_ws(const tome_diffusion_desc_t* d, void* base) {
+  const DiffDims s = diff_dims(d);
+  const long long S = d->diffusion_steps;
+  Bump b{reinterpret_cast<uint8_t*>(base)};
+  SampleWs w;
+  w.emb = b.take<__nv_bfloat16>(s.B * s.C);
+  w.ff = b.take<__nv_bfloat16>(S * s.F);
+  w.th = b.take<__nv_bfloat16>(S * s.Ht);
+  w.te = b.take<__nv_bfloat16>(S * s.To);
+  w.tproj = b.take<float>(S * s.H);
+  w.zr = b.take<float>(s.B * s.H);
+  w.total = b.total();
+  return w;
+}
+
+// blocks [0, B): emb[b] = mean of the readout rows (as diff_prep_kernel writes it into cat); blocks [B, B + steps): the
+// Fourier features of time step blockIdx.x - B
+__global__ void __launch_bounds__(DH_THREADS)
+diff_sample_prep_kernel(const tome_diffusion_desc_t d, const __nv_bfloat16* __restrict__ x, const int32_t* __restrict__ origin,
+                        const float* __restrict__ fourier, __nv_bfloat16* __restrict__ emb, __nv_bfloat16* __restrict__ ff) {
+  const int C = d.channels, n = d.n_readout, F2 = d.fourier_dim / 2;
+  if ((int)blockIdx.x < d.batch) {
+    const int b = blockIdx.x;
+    const float inv_n = 1.0f / (float)n;
+    for (int c = threadIdx.x; c < C; c += DH_THREADS) {
+      float s = 0.f;
+      for (int j = 0; j < n; ++j) s += __bfloat162float(x[((long long)b * d.tokens + origin[b * n + j]) * C + c]);
+      emb[(long long)b * C + c] = __float2bfloat16(s * inv_n);
+    }
+    return;
+  }
+  const int t = blockIdx.x - d.batch;
+  for (int j = threadIdx.x; j < F2; j += DH_THREADS) {
+    const float ang = 6.283185307179586f * (float)t * fourier[j];
+    float sn, cs;
+    sincosf(ang, &sn, &cs);
+    ff[(long long)t * d.fourier_dim + j] = __float2bfloat16(cs);
+    ff[(long long)t * d.fourier_dim + F2 + j] = __float2bfloat16(sn);
+  }
+}
+
+// All `steps` iterations for `rows` batch rows per CTA.  Fixed summation orders: the result does not depend on the grid.
+__global__ void __launch_bounds__(SMP_THREADS)
+diff_sample_loop_kernel(int B, int A, int H, int steps, int rows, const float* __restrict__ w1a, const float* __restrict__ w2,
+                        const float* __restrict__ b2, const float* __restrict__ zr, const float* __restrict__ tproj,
+                        const float* __restrict__ init, const float* __restrict__ noise, int noise_per_step,
+                        const float* __restrict__ coef, float clip, float* __restrict__ out) {
+  extern __shared__ float sm[];
+  float* W1 = sm;                 // [A, H]
+  float* W2t = W1 + A * H;        // [A, H]
+  float* bias = W2t + A * H;      // [A]
+  float* z = bias + A;            // [rows, H]
+  float* h = z + rows * H;        // [rows, H]
+  float* smp = h + rows * H;      // [rows, A]
+  const int r0 = blockIdx.x * rows, nr = min(rows, B - r0);
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int i = threadIdx.x; i < A * H; i += SMP_THREADS) {
+    W1[i] = w1a[i];
+    const int k = i / A, a = i - k * A;           // w2 is [H, A]
+    W2t[a * H + k] = w2[i];
+  }
+  for (int i = threadIdx.x; i < A; i += SMP_THREADS) bias[i] = b2[i];
+  for (int i = threadIdx.x; i < nr * H; i += SMP_THREADS) z[i] = zr[(long long)r0 * H + i];
+  for (int i = threadIdx.x; i < nr * A; i += SMP_THREADS) smp[i] = init[(long long)r0 * A + i];
+  __syncthreads();
+  for (int step = 0; step < steps; ++step) {
+    const int t = steps - 1 - step;                                          // diffusion.py:207-211
+    const float* tp = tproj + (long long)t * H;
+    for (int i = threadIdx.x; i < nr * H; i += SMP_THREADS) {               // h = relu(zr + tproj[t] + sample W1[:A])
+      const int r = i / H, k = i - r * H;
+      float acc = 0.f;
+      for (int a = 0; a < A; ++a) acc = fmaf(smp[r * A + a], W1[a * H + k], acc);
+      h[i] = fmaxf(z[i] + tp[k] + acc, 0.f);
+    }
+    __syncthreads();
+    const float c1 = coef[3 * t], c2 = coef[3 * t + 1], c3 = coef[3 * t + 2];
+    const float* nz = noise + (noise_per_step ? (long long)step * B * A : 0);
+    for (int o = warp; o < nr * A; o += SMP_THREADS / 32) {                  // eps = h W2 + b2, then the update (:182-190)
+      const int r = o / A, a = o - r * A;
+      float e = 0.f;
+      for (int k = lane; k < H; k += 32) e = fmaf(h[r * H + k], W2t[a * H + k], e);
+      e = warp_sum(e) + bias[a];
+      if (lane == 0) {
+        const float v = c1 * (smp[o] - c2 * e) + c3 * nz[(long long)(r0 + r) * A + a];
+        smp[o] = fminf(fmaxf(v, -clip), clip);
+      }
+    }
+    __syncthreads();
+  }
+  for (int i = threadIdx.x; i < nr * A; i += SMP_THREADS) out[(long long)r0 * A + i] = smp[i];
+}
+
+static DynSmemOnce g_sample_smem;
+
+static int check_sample_shape(const tome_diffusion_desc_t* d) {
+  TOME_CHECK(d->action_dim <= SMP_MAX_A && d->hidden <= SMP_MAX_H && sample_smem_bytes(d->action_dim, d->hidden, 1) <= SMP_MAX_SMEM,
+             TOME_ERR_UNSUPPORTED,
+             "diffusion_head_sample: action_dim %d / hidden %d outside the sampling kernel's limits (A <= %d, H <= %d, "
+             "W1[:A] and W2 in fp32: 8 A H bytes within %zu KB of shared memory)", d->action_dim, d->hidden, SMP_MAX_A, SMP_MAX_H,
+             SMP_MAX_SMEM / 1024);
+  return TOME_OK;
+}
+
 }  // namespace tome
 
-extern "C" int tome_ddpm_step(long long n, const float* sample, const float* denoise_term, const float* noise, float c1, float c2,
-                              float c3, float clip, float* out, void* stream_) {
+extern "C" size_t tome_diffusion_head_sample_workspace_bytes(const tome_diffusion_desc_t* d) {
+  clear_error();
+  if (check_diff(d) != TOME_OK || check_sample_shape(d) != TOME_OK) return 0;
+  return sample_ws(d, nullptr).total;
+}
+
+extern "C" int tome_diffusion_head_sample(const tome_diffusion_desc_t* d, const float* params_f32, const void* params_bf16_,
+                                          const void* x, const int32_t* origin, const tome_ddpm_sample_t* smp, float* actions,
+                                          void* workspace, size_t workspace_bytes, void* stream_) {
   clear_error();
   cudaStream_t st = (cudaStream_t)stream_;
-  TOME_CHECK(n > 0 && sample && denoise_term && noise && out, TOME_ERR_INVALID, "ddpm_step: bad argument");
-  TOME_CHECK(clip > 0.f, TOME_ERR_INVALID, "ddpm_step: clip must be positive");
+  DH_RC(check_diff(d));
+  DH_RC(check_sample_shape(d));
+  TOME_CHECK(smp != nullptr, TOME_ERR_INVALID, "diffusion_head_sample: null sample draws");
+  TOME_CHECK(smp->noise_per_step == 0 || smp->noise_per_step == 1, TOME_ERR_INVALID,
+             "diffusion_head_sample: noise_per_step must be 0 ([B, A] reused by every step) or 1 ([steps, B, A])");
+  TOME_CHECK(smp->clip > 0.f, TOME_ERR_INVALID, "diffusion_head_sample: clip must be positive");
+  TOME_CHECK(params_f32 && params_bf16_ && x && origin && smp->init && smp->noise && smp->coef && actions && workspace,
+             TOME_ERR_INVALID, "diffusion_head_sample: null argument");
+  TOME_CHECK(((uintptr_t)workspace & 255) == 0 && workspace_bytes >= sample_ws(d, nullptr).total, TOME_ERR_INVALID,
+             "diffusion_head_sample: workspace too small or not 256-byte aligned");
+  TOME_CHECK(((uintptr_t)params_bf16_ & 15) == 0, TOME_ERR_INVALID, "diffusion_head_sample: params_bf16 must be 16-byte aligned");
+  const DiffDims s = diff_dims(d);
+  const DiffOffsets o = diff_offsets(d);
+  const SampleWs w = sample_ws(d, workspace);
+  const __nv_bfloat16* pw = reinterpret_cast<const __nv_bfloat16*>(params_bf16_);
+  const int B = (int)s.B, S = d->diffusion_steps;
+  {
+    ProfScope prof(PROF_OTHER, 0.0, 1, st);
+    launch_k(diff_sample_prep_kernel, B + S, DH_THREADS, 0, st, *d, reinterpret_cast<const __nv_bfloat16*>(x), origin,
+             params_f32 + o.fourier, w.emb, w.ff);
+    TOME_CUDA(cudaGetLastError());
+  }
+  // the time-embedding table: th = relu(ff tw1 + tb1), te = th tw2 + tb2, tproj = te W1[A:A+To]
+  DH_RC(diff_gemm(st, S, (int)s.Ht, (int)s.F, w.ff, s.F, TOME_MAJOR_K, pw + o.tw1, s.Ht, TOME_MAJOR_MN, w.th, s.Ht, TOME_BF16,
+                  params_f32 + o.tb1, 1, nullptr, 0, 0));
+  DH_RC(diff_gemm(st, S, (int)s.To, (int)s.Ht, w.th, s.Ht, TOME_MAJOR_K, pw + o.tw2, s.To, TOME_MAJOR_MN, w.te, s.To, TOME_BF16,
+                  params_f32 + o.tb2, 0, nullptr, 0, 0));
+  DH_RC(diff_gemm(st, S, (int)s.H, (int)s.To, w.te, s.To, TOME_MAJOR_K, pw + o.w1 + s.A * s.H, s.H, TOME_MAJOR_MN, w.tproj, s.H,
+                  TOME_F32, nullptr, 0, nullptr, 0, 0));
+  // zr = emb W1[A+To:] + b1
+  DH_RC(diff_gemm(st, B, (int)s.H, (int)s.C, w.emb, s.C, TOME_MAJOR_K, pw + o.w1 + (s.A + s.To) * s.H, s.H, TOME_MAJOR_MN, w.zr, s.H,
+                  TOME_F32, params_f32 + o.b1, 0, nullptr, 0, 0));
+  int rows = (B + kNumSMs - 1) / kNumSMs;
+  if (rows > SMP_MAX_ROWS) rows = SMP_MAX_ROWS;
+  while (rows > 1 && sample_smem_bytes(s.A, s.H, rows) > SMP_MAX_SMEM) --rows;
+  const size_t smem = sample_smem_bytes(s.A, s.H, rows);
+  TOME_CUDA(ensure_dyn_smem(diff_sample_loop_kernel, (int)smem, g_sample_smem));
   ProfScope prof(PROF_OTHER, 0.0, 1, st);
-  launch_k(tome::ddpm_step_kernel, (unsigned)((n + 255) / 256), 256, 0, st, n, sample, denoise_term, noise, c1, c2, c3, clip, out);
+  launch_k(diff_sample_loop_kernel, (B + rows - 1) / rows, SMP_THREADS, smem, st, B, (int)s.A, (int)s.H, S, rows,
+           params_f32 + o.w1, params_f32 + o.w2, params_f32 + o.b2, w.zr, w.tproj, smp->init, smp->noise, smp->noise_per_step,
+           smp->coef, smp->clip, actions);
   TOME_CUDA(cudaGetLastError());
   return TOME_OK;
 }

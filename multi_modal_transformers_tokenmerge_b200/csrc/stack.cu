@@ -200,8 +200,10 @@ static std::vector<LayerShape> layer_shapes(const tome_stack_cfg_t* c) {
   return s;
 }
 
-// One function computes the layout for both the size query (base == nullptr) and the real pointers.
-static StackLayout make_layout(const tome_stack_cfg_t* c, void* workspace) {
+// One function computes the layout for both the size query (base == nullptr) and the real pointers.  Training keeps every
+// layer's activations for backward; predict (the forward-only executor) ping-pongs the residual stream, sizes and group ids
+// between two buffers, gives every layer the same scratch and keeps only the row maps the readout origins are chained from.
+static StackLayout make_layout(const tome_stack_cfg_t* c, void* workspace, bool predict = false) {
   StackLayout S;
   S.shapes = layer_shapes(c);
   S.L.resize(c->layers);
@@ -212,19 +214,97 @@ static StackLayout make_layout(const tome_stack_cfg_t* c, void* workspace) {
   float* size_prev = nullptr;
   uint8_t* gid_prev = c->num_groups ? b.take<uint8_t>(B * T0) : nullptr;
   int32_t* pos_prev = c->num_groups ? b.take<int32_t>(B * T0) : nullptr;
+  // plan arrays: even tokens (node_max, node_idx, edge_idx) and dst_off entries, summed over the token sets when merging in sets
+  auto plan_sizes = [&](int l, size_t* ta, size_t* n_off) {
+    const size_t T = S.shapes[l].t_in;
+    *ta = (T + 1) / 2;
+    *n_off = T / 2 + 1;
+    if (merges_in_sets(c)) {
+      const tome_token_sets_t ts = layer_sets(c, l);
+      *ta = *n_off = 0;
+      for (int i = 0; i < ts.n_sets; ++i) {
+        *ta += (ts.set_n[i] + 1) / 2;
+        *n_off += ts.set_n[i] / 2 + 1;
+      }
+    }
+  };
+  LayerBufs P;   // predict: the scratch every layer shares, sized for the widest layer
+  memset(&P, 0, sizeof(P));
+  __nv_bfloat16* x_pp[2] = {x_prev, nullptr};
+  float* size_pp[2] = {nullptr, nullptr};
+  uint8_t* gid_pp[2] = {gid_prev, nullptr};
+  int32_t* pos_pp[2] = {pos_prev, nullptr};
+  if (predict) {
+    size_t ta = 0, n_off = 0, r = 0;
+    for (int l = 0; l < c->layers; ++l) {
+      size_t a, o;
+      plan_sizes(l, &a, &o);
+      if (a > ta) ta = a;
+      if (o > n_off) n_off = o;
+      if ((size_t)S.shapes[l].r > r) r = S.shapes[l].r;
+    }
+    const size_t st = c->ln_axis == 1 ? B * C : B * T0;
+    x_pp[1] = b.take<__nv_bfloat16>(B * T0 * C);
+    if (r > 0 && !(c->prune_sets > 0 && !c->set_merge)) {
+      size_pp[0] = b.take<float>(B * T0);
+      size_pp[1] = b.take<float>(B * T0);
+    }
+    if (r > 0 && c->num_groups) {
+      gid_pp[1] = b.take<uint8_t>(B * T0);
+      pos_pp[1] = b.take<int32_t>(B * T0);
+    }
+    P.ln1_mean = b.take<float>(st);
+    P.ln1_rstd = b.take<float>(st);
+    P.h = b.take<__nv_bfloat16>(B * T0 * C);
+    P.qkv = b.take<__nv_bfloat16>(B * T0 * 3 * HD);
+    P.attn_o = b.take<__nv_bfloat16>(B * T0 * HD);
+    P.lse = b.take<float>(B * c->heads * T0);
+    P.x1m = b.take<__nv_bfloat16>(B * T0 * C);
+    if (r > 0 && c->prune_sets > 0 && !c->set_merge) {
+      P.importance = b.take<float>(B * T0);
+      P.prune_ids = b.take<int32_t>(B * T0);
+    } else if (r > 0) {
+      P.node_max = b.take<float>(B * ta);
+      P.node_idx = b.take<int32_t>(B * ta);
+      P.plan.edge_idx = b.take<int32_t>(B * ta);
+      P.plan.dst_idx = b.take<int32_t>(B * r);
+      P.plan.dst_off = b.take<int32_t>(B * n_off);
+      P.plan.dst_src = b.take<int32_t>(B * r);
+    }
+    P.ln2_mean = b.take<float>(st);
+    P.ln2_rstd = b.take<float>(st);
+    P.h2 = b.take<__nv_bfloat16>(B * T0 * C);
+    P.m1 = b.take<__nv_bfloat16>(B * T0 * F);
+  }
   for (int l = 0; l < c->layers; ++l) {
     LayerBufs& Lb = S.L[l];
     const size_t T = S.shapes[l].t_in, To = S.shapes[l].t_out, r = S.shapes[l].r;
-    // plan arrays: even tokens (node_max, node_idx, edge_idx) and dst_off entries, summed over the token sets when merging in sets
-    size_t ta = (T + 1) / 2, n_off = T / 2 + 1;
-    if (merges_in_sets(c)) {
-      const tome_token_sets_t ts = layer_sets(c, l);
-      ta = n_off = 0;
-      for (int i = 0; i < ts.n_sets; ++i) {
-        ta += (ts.set_n[i] + 1) / 2;
-        n_off += ts.set_n[i] / 2 + 1;
+    if (predict) {
+      // the other buffer of each pair than the one this layer reads (a layer that merges nothing passes its input on)
+      Lb = P;
+      Lb.x_in = x_prev;
+      Lb.x_out = x_prev == x_pp[0] ? x_pp[1] : x_pp[0];
+      Lb.size_in = size_prev;
+      Lb.gid_in = gid_prev;
+      Lb.pos_in = pos_prev;
+      if (r > 0) {
+        Lb.plan.row_map = b.take<int32_t>(B * T);
+        Lb.size_out = size_pp[0] ? (size_prev == size_pp[0] ? size_pp[1] : size_pp[0]) : nullptr;
+        Lb.gid_out = c->num_groups ? (gid_prev == gid_pp[0] ? gid_pp[1] : gid_pp[0]) : nullptr;
+        Lb.pos_out = c->num_groups ? (pos_prev == pos_pp[0] ? pos_pp[1] : pos_pp[0]) : nullptr;
+      } else {
+        Lb.size_out = Lb.size_in;
+        Lb.gid_out = Lb.gid_in;
+        Lb.pos_out = Lb.pos_in;
       }
+      x_prev = Lb.x_out;
+      size_prev = Lb.size_out;
+      gid_prev = Lb.gid_out;
+      pos_prev = Lb.pos_out;
+      continue;
     }
+    size_t ta, n_off;
+    plan_sizes(l, &ta, &n_off);
     const size_t st_in = c->ln_axis == 1 ? B * C : B * T, st_out = c->ln_axis == 1 ? B * C : B * To;
     Lb.x_in = x_prev;
     Lb.size_in = size_prev;
@@ -277,17 +357,22 @@ static StackLayout make_layout(const tome_stack_cfg_t* c, void* workspace) {
     pos_prev = Lb.pos_out;
   }
   S.x1_scratch = b.take<__nv_bfloat16>(B * T0 * C);
-  S.g0 = b.take<__nv_bfloat16>(B * T0 * C);
-  S.g1 = b.take<__nv_bfloat16>(B * T0 * C);
-  S.g2 = b.take<__nv_bfloat16>(B * T0 * C);
-  S.g3 = b.take<__nv_bfloat16>(B * T0 * HD);
-  S.big = b.take<__nv_bfloat16>(B * T0 * wide);
+  S.g0 = S.g1 = S.g2 = S.g3 = S.big = nullptr;
+  S.ws_gemm = S.ws_colsum = S.ws_ln = S.ws_colpart = nullptr;
+  S.ws_gemm_bytes = 0;
+  if (!predict) {
+    S.g0 = b.take<__nv_bfloat16>(B * T0 * C);
+    S.g1 = b.take<__nv_bfloat16>(B * T0 * C);
+    S.g2 = b.take<__nv_bfloat16>(B * T0 * C);
+    S.g3 = b.take<__nv_bfloat16>(B * T0 * HD);
+    S.big = b.take<__nv_bfloat16>(B * T0 * wide);
+  }
   {  // attention scratch (forward: per-tile metadata; backward: delta + metadata), sized for the widest layer
     tome_attn_desc_t ad;
     memset(&ad, 0, sizeof(ad));
     ad.batch = c->batch; ad.tokens = c->tokens; ad.heads = c->heads; ad.head_dim = c->head_dim;
     ad.dropout_rate = c->attn_dropout_rate;
-    const size_t f = tome_attention_workspace_bytes(&ad), bw = tome_attention_bwd_workspace_bytes(&ad);
+    const size_t f = tome_attention_workspace_bytes(&ad), bw = predict ? 0 : tome_attention_bwd_workspace_bytes(&ad);
     S.ws_attn_bytes = f > bw ? f : bw;
     S.ws_attn = b.take<uint8_t>(S.ws_attn_bytes);
   }
@@ -298,25 +383,27 @@ static StackLayout make_layout(const tome_stack_cfg_t* c, void* workspace) {
     S.ws_sim_bytes = tome_sim_argmax_workspace_bytes(&md);
   }
   S.ws_sim = b.take<uint8_t>(S.ws_sim_bytes);
-  // split-K workspace: the largest weight gradient, at most 64 splits are ever chosen but 148 tiles bound the product
-  size_t wmax = C * 3 * HD;
-  if (C * F > wmax) wmax = C * F;
-  if (HD * C > wmax) wmax = HD * C;
-  S.ws_gemm_bytes = wmax * sizeof(float) * 64;
-  S.ws_gemm = b.take<float>(wmax * 64);
-  S.ws_colsum = b.take<float>(256 * wide);
-  {  // rows: 128-row tiles of the flattened [B T0, N] GEMM outputs, or (batch row, 128-token tile) pairs of attention backward
-    const size_t r1 = (B * T0 + 127) / 128, r2 = B * ((T0 + 127) / 128);
-    S.ws_colpart = b.take<float>((r1 > r2 ? r1 : r2) * wide);
+  if (!predict) {
+    // split-K workspace: the largest weight gradient, at most 64 splits are ever chosen but 148 tiles bound the product
+    size_t wmax = C * 3 * HD;
+    if (C * F > wmax) wmax = C * F;
+    if (HD * C > wmax) wmax = HD * C;
+    S.ws_gemm_bytes = wmax * sizeof(float) * 64;
+    S.ws_gemm = b.take<float>(wmax * 64);
+    S.ws_colsum = b.take<float>(256 * wide);
+    {  // rows: 128-row tiles of the flattened [B T0, N] GEMM outputs, or (batch row, 128-token tile) pairs of attention backward
+      const size_t r1 = (B * T0 + 127) / 128, r2 = B * ((T0 + 127) / 128);
+      S.ws_colpart = b.take<float>((r1 > r2 ? r1 : r2) * wide);
+    }
+    const size_t ln_rows = c->ln_axis == 1 ? B : 256;
+    S.ws_ln = b.take<float>(2 * ln_rows * C);
   }
-  const size_t ln_rows = c->ln_axis == 1 ? B : 256;
-  S.ws_ln = b.take<float>(2 * ln_rows * C);
   S.origin = b.take<int32_t>(B * (c->n_readout > 0 ? c->n_readout : 1));
   S.ws_head_bytes = 0;
   S.ws_head = nullptr;
   if (c->head == 3) {
     tome_diffusion_desc_t d = diffusion_desc(c, 1);
-    S.ws_head_bytes = tome_diffusion_head_workspace_bytes(&d);
+    S.ws_head_bytes = predict ? tome_diffusion_head_sample_workspace_bytes(&d) : tome_diffusion_head_workspace_bytes(&d);
     S.ws_head = b.take<uint8_t>(S.ws_head_bytes);
   } else if (c->head > 0) {
     tome_head_desc_t h = head_desc(c, 1);
@@ -436,12 +523,8 @@ static int check_io(const tome_stack_cfg_t* c, const tome_stack_io_t* io, const 
   return TOME_OK;
 }
 
-extern "C" int tome_stack_forward(const tome_stack_cfg_t* c, const tome_stack_io_t* io, void* stream_) {
-  clear_error();
-  cudaStream_t st = (cudaStream_t)stream_;
-  RC(check_cfg(c));
-  StackLayout S = make_layout(c, io ? io->workspace : nullptr);
-  RC(check_io(c, io, S, false));
+// The forward of every layer, from the input embeddings to the last layer's x_out, over either layout of make_layout.
+static int forward_layers(const tome_stack_cfg_t* c, const tome_stack_io_t* io, const StackLayout& S, cudaStream_t st) {
   const int B = c->batch, C = c->channels, H = c->heads, D = c->head_dim, HD = H * D, F = c->mlp_dim;
   const float* pf = io->params_f32;
   const __nv_bfloat16* pw = reinterpret_cast<const __nv_bfloat16*>(io->params_bf16);
@@ -514,17 +597,33 @@ extern "C" int tome_stack_forward(const tome_stack_cfg_t* c, const tome_stack_io
     RC(gemm(c, S, st, Mo, C, F, Lb.m1, F, TOME_MAJOR_K, pw + o.w2, C, TOME_MAJOR_MN, Lb.x_out, C, TOME_BF16, pf + o.b2, 0, Lb.x1m,
             nullptr, 1.f, 3 * l + 2, 0));
   }
+  return TOME_OK;
+}
+
+// origin[b, i]: the final row readout token i ended up in, through every merging or pruning layer's row map
+static int chain_origin(const tome_stack_cfg_t* c, const tome_stack_io_t* io, const StackLayout& S, cudaStream_t st) {
+  const int32_t* maps[64];
+  int toks[64];
+  for (int l = 0; l < c->layers; ++l) {
+    maps[l] = S.shapes[l].r > 0 ? S.L[l].plan.row_map : nullptr;   // merge and prune layers both leave token -> output row
+    toks[l] = S.shapes[l].t_in;
+  }
+  return tome_chain_row_maps(c->batch, c->layers, maps, toks, io->readout_idx, c->n_readout, S.origin, st);
+}
+
+extern "C" int tome_stack_forward(const tome_stack_cfg_t* c, const tome_stack_io_t* io, void* stream_) {
+  clear_error();
+  cudaStream_t st = (cudaStream_t)stream_;
+  RC(check_cfg(c));
+  StackLayout S = make_layout(c, io ? io->workspace : nullptr);
+  RC(check_io(c, io, S, false));
+  const int B = c->batch, C = c->channels;
+  RC(forward_layers(c, io, S, st));
   const int TL = S.shapes.back().t_out;
   if (io->x_final)
     TOME_CUDA(cudaMemcpyAsync(io->x_final, S.L.back().x_out, (size_t)B * TL * C * 2, cudaMemcpyDeviceToDevice, st));
   if (c->n_readout > 0) {
-    const int32_t* maps[64];
-    int toks[64];
-    for (int l = 0; l < c->layers; ++l) {
-      maps[l] = S.shapes[l].r > 0 ? S.L[l].plan.row_map : nullptr;   // merge and prune layers both leave token -> output row
-      toks[l] = S.shapes[l].t_in;
-    }
-    RC(tome_chain_row_maps(B, c->layers, maps, toks, io->readout_idx, c->n_readout, S.origin, st));
+    RC(chain_origin(c, io, S, st));
     if (c->head == 3) {
       // diffusion head: denoise_loss on the pooled readout rows (diffusion.py:94-143); target = [actions | noise]
       tome_diffusion_desc_t d = diffusion_desc(c, TL);
@@ -549,6 +648,62 @@ extern "C" int tome_stack_forward(const tome_stack_cfg_t* c, const tome_stack_io
       RC(tome_readout_mse(B, TL, C, c->n_readout, S.L.back().x_out, S.origin, (io->target && io->loss) ? io->target : nullptr,
                           (io->target && io->loss) ? io->loss : nullptr, nullptr, io->readout, st));
   }
+  return TOME_OK;
+}
+
+// The forward-only executor runs the training forward with dropout off, over the predict layout.
+static tome_stack_cfg_t predict_cfg(const tome_stack_cfg_t* c) {
+  tome_stack_cfg_t p = *c;
+  p.dropout_rate = 0.f;
+  p.attn_dropout_rate = 0.f;
+  return p;
+}
+
+extern "C" size_t tome_stack_predict_workspace_bytes(const tome_stack_cfg_t* c) {
+  clear_error();
+  if (check_cfg(c)) return 0;
+  const tome_stack_cfg_t p = predict_cfg(c);
+  const StackLayout S = make_layout(&p, nullptr, true);
+  if (p.head == 3 && S.ws_head_bytes == 0) return 0;   // the sampler's shape check set the message
+  return S.total;
+}
+
+extern "C" int tome_stack_predict(const tome_stack_cfg_t* cfg, const tome_stack_io_t* io, const tome_ddpm_sample_t* sample,
+                                  void* stream_) {
+  clear_error();
+  cudaStream_t st = (cudaStream_t)stream_;
+  RC(check_cfg(cfg));
+  const tome_stack_cfg_t p = predict_cfg(cfg);
+  const tome_stack_cfg_t* c = &p;
+  TOME_CHECK((c->head == 3) == (sample != nullptr), TOME_ERR_INVALID,
+             "stack_predict: the diffusion head (head 3) needs the sampler's draws, every other head takes sample = NULL");
+  if (sample) {
+    TOME_CHECK(sample->noise_per_step == 0 || sample->noise_per_step == 1, TOME_ERR_INVALID,
+               "stack_predict: sample->noise_per_step must be 0 or 1");
+    TOME_CHECK(sample->clip > 0.f, TOME_ERR_INVALID, "stack_predict: sample->clip must be positive");
+  }
+  StackLayout S = make_layout(c, io ? io->workspace : nullptr, true);
+  if (c->head == 3 && S.ws_head_bytes == 0) return TOME_ERR_UNSUPPORTED;   // the sampler's shape check set the message
+  RC(check_io(c, io, S, false));
+  TOME_CHECK(c->head == 0 || io->head_out, TOME_ERR_INVALID, "stack_predict: head_out missing");
+  const int B = c->batch, C = c->channels;
+  RC(forward_layers(c, io, S, st));
+  const int TL = S.shapes.back().t_out;
+  const __nv_bfloat16* xf = S.L.back().x_out;
+  if (io->x_final) TOME_CUDA(cudaMemcpyAsync(io->x_final, xf, (size_t)B * TL * C * 2, cudaMemcpyDeviceToDevice, st));
+  if (c->n_readout == 0) return TOME_OK;
+  RC(chain_origin(c, io, S, st));
+  const long long ho = layer_offsets(c, c->layers).ln1_scale;
+  if (c->head == 3) {
+    tome_diffusion_desc_t d = diffusion_desc(c, TL);
+    RC(tome_diffusion_head_sample(&d, io->params_f32 + ho, reinterpret_cast<const __nv_bfloat16*>(io->params_bf16) + ho, xf,
+                                  S.origin, sample, io->head_out, S.ws_head, S.ws_head_bytes, st));
+  } else if (c->head > 0) {
+    tome_head_desc_t h = head_desc(c, TL);
+    RC(tome_action_head_fwd(&h, xf, S.origin, io->params_f32 + ho, io->params_f32 + ho + (long long)C * c->head_features, nullptr,
+                            io->head_out, nullptr, S.ws_head, S.ws_head_bytes, st));
+  }
+  if (io->readout) RC(tome_readout_mse(B, TL, C, c->n_readout, xf, S.origin, nullptr, nullptr, nullptr, io->readout, st));
   return TOME_OK;
 }
 

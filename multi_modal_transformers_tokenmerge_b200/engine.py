@@ -9,6 +9,7 @@ of this class.  torch is used for device memory, streams and (in `parallel.py`) 
 from __future__ import annotations
 
 import ctypes as C
+import dataclasses
 from dataclasses import dataclass, field
 from typing import Dict, List, Optional, Sequence
 
@@ -99,24 +100,39 @@ class StackConfig:
 
 
 class ToMeStackEngine:
+    """predict_only=True: a forward-only engine (tome_stack_predict) -- the predict workspace, no gradients, no Adam moments;
+    `predict` runs it, and forward / backward / the optimiser and the per-layer accessors raise.  `predictor()` builds one
+    from a training engine that shares its parameters."""
+
     def __init__(self, cfg: StackConfig, device="cuda", gid=None, pos=None, allow=None, readout_idx=None,
-                 training: bool = True, layer_gid=None, layer_pos=None):
+                 training: bool = True, layer_gid=None, layer_pos=None, predict_only: bool = False, _params=None):
         if not torch.cuda.is_available():
             raise RuntimeError("ToMeStackEngine needs a CUDA device (sm_100a); there is no CPU fallback")
         self.lib = L.lib()
         self.cfg = cfg
         self.dev = torch.device(device)
         self.ccfg = cfg.c()
+        self.predict_only = bool(predict_only)
         n = self.lib.tome_stack_param_count(C.byref(self.ccfg))
         if n < 0:
             L.check(1)
         self.n_params = int(n)
-        self.params = torch.zeros(self.n_params, dtype=torch.float32, device=self.dev)
-        self.params_bf16 = torch.zeros(self.n_params, dtype=torch.bfloat16, device=self.dev)
-        self.grads = torch.zeros(self.n_params, dtype=torch.float32, device=self.dev) if training else None
+        if _params is not None:   # predictor(): the training engine's storage, not a copy
+            self.params, self.params_bf16 = _params
+            assert self.params.numel() == self.n_params and self.params_bf16.numel() == self.n_params
+        else:
+            self.params = torch.zeros(self.n_params, dtype=torch.float32, device=self.dev)
+            self.params_bf16 = torch.zeros(self.n_params, dtype=torch.bfloat16, device=self.dev)
+        self.grads = (torch.zeros(self.n_params, dtype=torch.float32, device=self.dev)
+                      if training and not self.predict_only else None)
         self.adam_m = self.adam_v = None
         self.step_count = 0
-        ws = self.lib.tome_stack_workspace_bytes(C.byref(self.ccfg))
+        if self.predict_only:
+            ws = self.lib.tome_stack_predict_workspace_bytes(C.byref(self.ccfg))
+            if ws == 0:
+                L.check(L.TOME_ERR_UNSUPPORTED)
+        else:
+            ws = self.lib.tome_stack_workspace_bytes(C.byref(self.ccfg))
         self.workspace = _scratch(ws, self.dev)
         self._ws_bytes = ws
         self.gid = None if gid is None else torch.as_tensor(np.asarray(gid, np.uint8)).to(self.dev)
@@ -263,7 +279,12 @@ class ToMeStackEngine:
         self._base_seed = int(seed) & 0xFFFFFFFFFFFFFFFF
         self.ccfg.dropout_seed = self._base_seed
 
+    def _training_workspace(self, what: str) -> None:
+        if self.predict_only:
+            raise RuntimeError(f"{what} needs the training workspace: this engine is predict-only (use predict())")
+
     def forward(self, x: torch.Tensor, target: Optional[torch.Tensor] = None):
+        self._training_workspace("forward")
         cfg = self.cfg
         assert x.is_cuda and x.is_contiguous() and tuple(x.shape) == (cfg.batch, cfg.tokens, cfg.channels), x.shape
         assert x.dtype in (torch.float32, torch.bfloat16)
@@ -280,6 +301,7 @@ class ToMeStackEngine:
 
     def backward(self, events: Optional[List[torch.cuda.Event]] = None):
         """Loss gradient + full backward into `self.grads` (accumulating: call zero_grad() first)."""
+        self._training_workspace("backward")
         assert self._x is not None and self._target is not None, "forward(x, target) first"
         self._events = events
         io = self._io(self._x, self._target)
@@ -291,6 +313,7 @@ class ToMeStackEngine:
         self.grads.zero_()
 
     def adamw_step(self, lr=1e-4, beta1=0.9, beta2=0.999, eps=1e-8, weight_decay=0.0, grad_scale=1.0):
+        self._training_workspace("adamw_step")
         if self.adam_m is None:
             self.adam_m = torch.zeros_like(self.params)
             self.adam_v = torch.zeros_like(self.params)
@@ -299,11 +322,61 @@ class ToMeStackEngine:
                                          self.adam_v.data_ptr(), self.params_bf16.data_ptr(), lr, beta1, beta2, eps,
                                          weight_decay, grad_scale, self.step_count, self._stream()))
 
+    # ------------------------------------------------------------------ prediction (forward only)
+    def predictor(self, batch: Optional[int] = None) -> "ToMeStackEngine":
+        """A predict-only engine over THIS engine's params / params_bf16 storage (no copy), optionally at another batch size:
+        it sees every optimiser step without a reload.  Masks and readout indices are shared too."""
+        cfg = self.cfg if batch is None else dataclasses.replace(self.cfg, batch=int(batch))
+        p = ToMeStackEngine(cfg, device=self.dev, predict_only=True, _params=(self.params, self.params_bf16))
+        p.gid, p.pos, p.allow, p.readout_idx = self.gid, self.pos, self.allow, self.readout_idx
+        p.layer_gid, p.layer_pos = self.layer_gid, self.layer_pos
+        return p
+
+    def predict(self, x: torch.Tensor, init=None, noise=None, rng=0, x_final: Optional[torch.Tensor] = None):
+        """Forward only, dropout off (tome_stack_predict).  Returns (head_out, readout): head_out is the action head's output
+        -- tanh actions [B, A] (continuous), logits [B, groups, bins] (categorical), sampled actions [B, A] (diffusion) -- or
+        None without a head; readout f32 [B, n_readout, C] or None without readout tokens.  Diffusion head: init [B, A] and
+        noise [B, A] (reused by every step) or [steps, B, A] default to draws from `rng` (numpy's generator), as
+        DiffusionActionHead.predict_action draws them.  x_final: optional bf16 [B, T_L, C] output.  The returned tensors are
+        copies: a later predict() does not overwrite them."""
+        if not self.predict_only:
+            raise RuntimeError("predict() needs a predict-only engine: ToMeStackEngine(..., predict_only=True) or predictor()")
+        cfg = self.cfg
+        assert x.is_cuda and x.is_contiguous() and tuple(x.shape) == (cfg.batch, cfg.tokens, cfg.channels), x.shape
+        assert x.dtype in (torch.float32, torch.bfloat16)
+        smp = None
+        if cfg.head == "diffusion":
+            from .action_heads.diffusion import cosine_beta_schedule, ddpm_coefficients
+            from .attention_blocks._module import as_rng
+            g = as_rng(rng)
+            B, A = cfg.batch, cfg.head_features
+            if init is None:
+                init = torch.as_tensor(g.standard_normal((B, A)).astype(np.float32))
+            if noise is None:
+                noise = torch.as_tensor(g.standard_normal((B, A)).astype(np.float32))
+            init = torch.as_tensor(init).to(self.dev).float().contiguous()
+            noise = torch.as_tensor(noise).to(self.dev).float().contiguous()
+            assert tuple(init.shape) == (B, A) and tuple(noise.shape) in ((B, A), (cfg.diffusion_steps, B, A)), (init.shape, noise.shape)
+            coef = torch.as_tensor(ddpm_coefficients(cosine_beta_schedule(cfg.diffusion_steps))).to(self.dev)
+            self._draws = (init, noise, coef)   # alive until the kernels that read them have run
+            smp = L.DdpmSample(init.data_ptr(), noise.data_ptr(), int(noise.dim() == 3), coef.data_ptr(), 5.0)
+        if x_final is not None:
+            assert x_final.is_cuda and x_final.dtype == torch.bfloat16 and x_final.is_contiguous()
+            assert x_final.numel() == cfg.batch * self.tokens_at(cfg.layers) * cfg.channels
+        io = self._io(x, None)
+        io.x_final = None if x_final is None else x_final.data_ptr()
+        L.check(self.lib.tome_stack_predict(C.byref(self.ccfg), C.byref(io), None if smp is None else C.byref(smp), self._stream()))
+        out = None
+        if self.head_out is not None:
+            out = (self.head_out if cfg.head == "categorical" else self.head_out.view(cfg.batch, cfg.head_features)).clone()
+        return out, None if self.readout is None else self.readout.clone()
+
     # ------------------------------------------------------------------ results (views into the workspace)
     def tokens_at(self, layer: int) -> int:
         return int(self.lib.tome_stack_tokens_at(C.byref(self.ccfg), layer))
 
     def _view(self, ptr: int, shape, dtype) -> torch.Tensor:
+        self._training_workspace("the workspace accessors")
         off = ptr - self.workspace.data_ptr()
         n = int(np.prod(shape)) * torch.empty((), dtype=dtype).element_size()
         return self.workspace[off: off + n].view(dtype).view(*shape)

@@ -453,6 +453,28 @@ def diffusion_head_fwd(x: torch.Tensor, params: torch.Tensor, desc: "L.Diffusion
     return pred, loss, DiffusionState(desc, params, p16, origin, time, ws)
 
 
+def diffusion_head_sample(x: torch.Tensor, params: torch.Tensor, desc: "L.DiffusionDesc", init: torch.Tensor, noise: torch.Tensor,
+                          coef: torch.Tensor, clip: float = 5.0, origin: Optional[torch.Tensor] = None,
+                          params_bf16: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """DiffusionActionHead.predict_action's whole reverse process (tome_diffusion_head_sample) on the final sequence x bf16
+    [B, tokens, C]: init f32 [B, A], noise f32 [B, A] (every step) or [steps, B, A], coef f32 [steps, 3].  Returns [B, A]."""
+    _need_cuda(x, params, init, noise, coef, origin)
+    assert x.dtype == torch.bfloat16 and x.is_contiguous() and params.dtype == torch.float32
+    B, T, _ = x.shape
+    if origin is None:
+        origin = torch.arange(T, dtype=torch.int32, device=x.device).repeat(B, 1)
+    p16 = params.to(torch.bfloat16) if params_bf16 is None else params_bf16
+    for t in (init, noise, coef):
+        assert t.dtype == torch.float32 and t.is_contiguous()
+    nbytes = int(L.lib().tome_diffusion_head_sample_workspace_bytes(C.byref(desc)))   # 0 for a refused shape: the call says why
+    ws = _scratch(nbytes, x.device)
+    out = torch.empty(B, desc.action_dim, dtype=torch.float32, device=x.device)
+    smp = L.DdpmSample(_ptr(init), _ptr(noise), int(noise.dim() == 3), _ptr(coef), float(clip))
+    L.check(L.lib().tome_diffusion_head_sample(C.byref(desc), _ptr(params), _ptr(p16), _ptr(x), _ptr(origin), C.byref(smp), _ptr(out),
+                                               _ptr(ws), nbytes, _stream()))
+    return out
+
+
 def diffusion_head_bwd(state: DiffusionState, grads: torch.Tensor, want_dx: bool = True):
     d = state.desc
     dx = torch.empty(d.batch, d.tokens, d.channels, dtype=torch.bfloat16, device=grads.device) if want_dx else None
