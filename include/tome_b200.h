@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define TOME_ABI_VERSION 16
+#define TOME_ABI_VERSION 17
 
 enum tome_status { TOME_OK = 0, TOME_ERR_INVALID = 1, TOME_ERR_CUDA = 2, TOME_ERR_UNSUPPORTED = 3 };
 enum tome_dtype { TOME_BF16 = 0, TOME_F32 = 1, TOME_U8 = 2 /* raw pixels: image front end only */ };
@@ -444,9 +444,38 @@ int tome_diffusion_head_sample(const tome_diffusion_desc_t* desc, const float* p
                                size_t workspace_bytes, void* stream);
 
 /* AdamW on an fp32 master vector with a bf16 working copy refreshed in the same pass (bf16_copy may be NULL).
- * grad_scale multiplies the gradient first (1/world_size after a sum all-reduce). */
+ * grad_scale multiplies the gradient first (1/world_size after a sum all-reduce).  Per element, with g = grad_scale * grad:
+ *   m = b1 m + (1 - b1) g;  v = b2 v + (1 - b2) g^2;  p -= lr * ((m / bc1) / (sqrt(v / bc2) + eps) + wd * p)
+ * with bc1 = 1 - b1^step, bc2 = 1 - b2^step computed in fp32 on the host.
+ *
+ * opts == NULL is exactly this plain step (ABI 16).  opts adds, without any host synchronisation (ABI 17):
+ *   - the global L2 norm of g over all n elements, written to grad_norm when given.  It is a fixed-order reduction (a
+ *     compile-time partition into chunks, fp32 inside a chunk, fp64 across chunks), so the same gradient bits give the same
+ *     norm bits whatever the GPU, its SM count or tome_gemm_set_sm_limit: data-parallel replicas that all-reduced the same
+ *     gradient stay identical.  Computed when max_grad_norm > 0, skip_nonfinite or grad_norm != NULL;
+ *   - clipping as optax.clip_by_global_norm: g unchanged when norm < max_grad_norm, else g * (max_grad_norm / norm);
+ *   - skipping as optax.apply_if_finite: a NaN / Inf in g leaves param, m, v, bf16_copy and steps[0] untouched and adds 1 to
+ *     steps[1];
+ *   - steps != NULL: bias correction uses t = steps[0] + 1 (applied steps only) instead of `step`, computed on the device in
+ *     fp64 and rounded to fp32, and the call adds 1 to steps[0] when it applies the step;
+ *   - decay_ranges: weight decay only inside these element ranges (e.g. the Dense kernels; not LayerNorm, biases or embeddings).
+ * Malformed options return TOME_ERR_INVALID before any CUDA call. */
+#define TOME_ADAMW_MAX_DECAY_RANGES 512
+typedef struct {
+  float max_grad_norm;            /* > 0: clip g to this global L2 norm; 0: no clipping; negative or non-finite: refused */
+  int skip_nonfinite;             /* 1: a g with a NaN / Inf leaves every buffer untouched (needs steps) */
+  const long long* decay_ranges;  /* HOST array [2 * n_decay_ranges]: sorted, disjoint, non-empty half-open ranges [lo, hi) in
+                                     [0, n) that get weight decay; NULL: every element */
+  int n_decay_ranges;             /* 0 .. TOME_ADAMW_MAX_DECAY_RANGES */
+  float* grad_norm;               /* device f32 [1], optional: the norm of g before clipping */
+  int* steps;                     /* device i32 [2] {applied, skipped}, optional; required when skip_nonfinite */
+  void* workspace;                /* 16-byte aligned, tome_adamw_workspace_bytes(n) bytes; needed when the norm or steps is used */
+  size_t workspace_bytes;
+} tome_adamw_opts_t;
+size_t tome_adamw_workspace_bytes(long long n);
 int tome_adamw_step(long long n, float* param, const float* grad, float* m, float* v, void* bf16_copy, float lr,
-                    float beta1, float beta2, float eps, float weight_decay, float grad_scale, int step, void* stream);
+                    float beta1, float beta2, float eps, float weight_decay, float grad_scale, int step,
+                    const tome_adamw_opts_t* opts, void* stream);
 
 /* dst_bf16[i] = (bf16) src_f32[i] */
 int tome_cast_f32_to_bf16(long long n, const float* src, void* dst, void* stream);

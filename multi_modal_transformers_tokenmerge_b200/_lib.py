@@ -15,7 +15,7 @@ TOME_OK, TOME_ERR_INVALID, TOME_ERR_CUDA, TOME_ERR_UNSUPPORTED = 0, 1, 2, 3
 TOME_BF16, TOME_F32, TOME_U8 = 0, 1, 2
 TOME_MAJOR_K, TOME_MAJOR_MN = 0, 1
 TOME_MERGE_SUM, TOME_MERGE_WAVG = 0, 1
-ABI_VERSION = 16
+ABI_VERSION = 17
 
 vp, ll, i32, f32, u64, u32 = C.c_void_p, C.c_longlong, C.c_int, C.c_float, C.c_uint64, C.c_uint32
 
@@ -114,6 +114,15 @@ class DdpmSample(C.Structure):
     _fields_ = [("init", vp), ("noise", vp), ("noise_per_step", i32), ("coef", vp), ("clip", f32)]
 
 
+ADAMW_MAX_DECAY_RANGES = 512
+
+
+class AdamwOpts(C.Structure):
+    """tome_adamw_opts_t: global-norm clipping, non-finite skipping and a weight-decay mask for tome_adamw_step."""
+    _fields_ = [("max_grad_norm", f32), ("skip_nonfinite", i32), ("decay_ranges", C.POINTER(ll)), ("n_decay_ranges", i32),
+                ("grad_norm", vp), ("steps", vp), ("workspace", vp), ("workspace_bytes", C.c_size_t)]
+
+
 DIFFUSION_PARAMS = ["fourier_kernel", "tw1", "tb1", "tw2", "tb2", "w1", "b1", "w2", "b2"]
 
 
@@ -163,7 +172,7 @@ def lib() -> C.CDLL:
         for name in ("tome_gemm_workspace_bytes", "tome_stack_workspace_bytes", "tome_attention_workspace_bytes", "tome_sim_argmax_workspace_bytes",
                      "tome_attention_bwd_workspace_bytes", "tome_action_head_workspace_bytes", "tome_diffusion_head_workspace_bytes",
                      "tome_diffusion_head_sample_workspace_bytes", "tome_stack_predict_workspace_bytes",
-                     "tome_image_tokenizer_workspace_bytes"):
+                     "tome_image_tokenizer_workspace_bytes", "tome_adamw_workspace_bytes"):
             getattr(L, name).restype = C.c_size_t
         for name in ("tome_stack_param_count", "tome_stack_layer_offset", "tome_stack_head_offset", "tome_launch_count",
                      "tome_diffusion_head_param_count", "tome_diffusion_head_param_offset",
@@ -223,7 +232,8 @@ def lib() -> C.CDLL:
             "tome_image_tokenizer_fwd": [P(ImageTokenizerDesc), vp, vp, vp, vp, vp, vp, vp, C.c_size_t, vp],
             "tome_diffusion_head_sample_workspace_bytes": [P(DiffusionDesc)],
             "tome_diffusion_head_sample": [P(DiffusionDesc), vp, vp, vp, vp, P(DdpmSample), vp, vp, C.c_size_t, vp],
-            "tome_adamw_step": [ll, vp, vp, vp, vp, vp, f32, f32, f32, f32, f32, f32, i32, vp],
+            "tome_adamw_workspace_bytes": [ll],
+            "tome_adamw_step": [ll, vp, vp, vp, vp, vp, f32, f32, f32, f32, f32, f32, i32, P(AdamwOpts), vp],
             "tome_cast_f32_to_bf16": [ll, vp, vp, vp],
             "tome_launch_count": [i32],
             "tome_profile_enable": [i32],

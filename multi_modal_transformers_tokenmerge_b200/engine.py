@@ -127,6 +127,9 @@ class ToMeStackEngine:
                       if training and not self.predict_only else None)
         self.adam_m = self.adam_v = None
         self.step_count = 0
+        # adamw_step options: the gradient norm (device f32 [1]), {applied, skipped} counters, the decay mask, the norm scratch
+        self.grad_norm = (torch.zeros(1, dtype=torch.float32, device=self.dev) if self.grads is not None else None)
+        self._opt_steps = self._decay_ranges = self._adam_ws = None
         if self.predict_only:
             ws = self.lib.tome_stack_predict_workspace_bytes(C.byref(self.ccfg))
             if ws == 0:
@@ -312,15 +315,59 @@ class ToMeStackEngine:
     def zero_grad(self):
         self.grads.zero_()
 
-    def adamw_step(self, lr=1e-4, beta1=0.9, beta2=0.999, eps=1e-8, weight_decay=0.0, grad_scale=1.0):
+    def decay_ranges(self, decay: str = "dense_kernels") -> List[tuple]:
+        """Sorted [lo, hi) element ranges of the weight matrices that get weight decay under `decay="dense_kernels"`: every
+        layer's wqkv, wo, w1, w2, the continuous / categorical head kernel and the diffusion head's tw1, tw2, w1, w2 (the
+        Dense / DenseGeneral kernels).  LayerNorm parameters, biases, pos_embedding and the Fourier kernel get none."""
+        assert decay == "dense_kernels", decay
+        v = self.param_views(self.params)
+        mats = [d[k] for d in v["layers"] for k in ("wqkv", "wo", "w1", "w2")]
+        head = v.get("head", {})
+        mats += [head[k] for k in (("tw1", "tw2", "w1", "w2") if self.cfg.head == "diffusion" else ("kernel",)) if k in head]
+        return sorted((t.storage_offset(), t.storage_offset() + t.numel()) for t in mats)
+
+    def adamw_step(self, lr=1e-4, beta1=0.9, beta2=0.999, eps=1e-8, weight_decay=0.0, grad_scale=1.0,
+                   max_grad_norm: Optional[float] = None, skip_nonfinite: bool = False, decay: str = "all"):
+        """One AdamW step on the flat vectors (tome_adamw_step).  max_grad_norm: clip grad_scale * grads to this global L2
+        norm first (optax.clip_by_global_norm).  skip_nonfinite: a gradient holding a NaN / Inf changes nothing and counts
+        as skipped (optax.apply_if_finite); from the first such call on, bias correction counts applied steps only.
+        decay: "all" or "dense_kernels" (weight decay on the Dense kernels only, `decay_ranges`).  Steps that clip or skip
+        leave the norm of grad_scale * grads in `grad_norm` (device f32 [1]).  With none of these the step is the plain one."""
         self._training_workspace("adamw_step")
+        assert decay in ("all", "dense_kernels"), decay
         if self.adam_m is None:
             self.adam_m = torch.zeros_like(self.params)
             self.adam_v = torch.zeros_like(self.params)
+        if skip_nonfinite and self._opt_steps is None:   # {applied, skipped}: every earlier step was applied
+            self._opt_steps = torch.tensor([self.step_count, 0], dtype=torch.int32, device=self.dev)
         self.step_count += 1
+        opts = None
+        if max_grad_norm is not None or skip_nonfinite or decay != "all" or self._opt_steps is not None:
+            ranges = None
+            if decay != "all":
+                if self._decay_ranges is None:
+                    flat = [x for r in self.decay_ranges(decay) for x in r]
+                    self._decay_ranges = ((C.c_longlong * len(flat))(*flat), len(flat) // 2)
+                ranges = self._decay_ranges
+            norm = max_grad_norm is not None or skip_nonfinite
+            if self._adam_ws is None:
+                self._adam_ws = _scratch(self.lib.tome_adamw_workspace_bytes(self.n_params), self.dev)
+            opts = L.AdamwOpts(0.0 if max_grad_norm is None else float(max_grad_norm), int(bool(skip_nonfinite)),
+                               None if ranges is None else ranges[0], 0 if ranges is None else ranges[1],
+                               self.grad_norm.data_ptr() if norm else None,
+                               None if self._opt_steps is None else self._opt_steps.data_ptr(),
+                               self._adam_ws.data_ptr(), self._adam_ws.numel())
         L.check(self.lib.tome_adamw_step(self.n_params, self.params.data_ptr(), self.grads.data_ptr(), self.adam_m.data_ptr(),
                                          self.adam_v.data_ptr(), self.params_bf16.data_ptr(), lr, beta1, beta2, eps,
-                                         weight_decay, grad_scale, self.step_count, self._stream()))
+                                         weight_decay, grad_scale, self.step_count, None if opts is None else C.byref(opts),
+                                         self._stream()))
+
+    def optimizer_steps(self) -> tuple:
+        """(applied, skipped) optimiser steps so far.  Reads the device counters (a sync) once skip_nonfinite has been used."""
+        if self._opt_steps is None:
+            return self.step_count, 0
+        a, s = self._opt_steps.tolist()
+        return a, s
 
     # ------------------------------------------------------------------ prediction (forward only)
     def predictor(self, batch: Optional[int] = None) -> "ToMeStackEngine":

@@ -91,6 +91,9 @@ class DataParallelTrainer:
             ev.record()
 
     def train_step(self, x: torch.Tensor, target: torch.Tensor, lr: float = 1e-4, **adam) -> None:
+        """`adam` goes to `engine.adamw_step` (max_grad_norm, skip_nonfinite, decay, ...).  The step runs after the
+        all-reduce with grad_scale = 1/world, so its norm is the norm of the mean gradient and every rank computes the
+        same bits from the same reduced vector."""
         e = self.engine
         e.zero_grad()
         e.set_dropout_step(e.step_count)   # fresh dropout masks every step (forward and backward of a step share them)
