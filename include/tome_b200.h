@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define TOME_ABI_VERSION 17
+#define TOME_ABI_VERSION 18
 
 enum tome_status { TOME_OK = 0, TOME_ERR_INVALID = 1, TOME_ERR_CUDA = 2, TOME_ERR_UNSUPPORTED = 3 };
 enum tome_dtype { TOME_BF16 = 0, TOME_F32 = 1, TOME_U8 = 2 /* raw pixels: image front end only */ };
@@ -651,6 +651,53 @@ size_t tome_image_tokenizer_workspace_bytes(const tome_image_tokenizer_desc_t* d
 int tome_image_tokenizer_fwd(const tome_image_tokenizer_desc_t* desc, const void* image, const float* params_f32,
                              const void* params_bf16, const int32_t* row_tokens, const int32_t* col_tokens, void* out,
                              void* workspace, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------
+ * 7c. Pixels to actions in one call (ABI 18): Octo.generate_readouts (models/octo/octo.py:91-126) under
+ *     predict_continuous_action / predict_diffusion_action -- image front end -> sequence assembly -> forward-only stack -> head
+ * ------------------------------------------------------------------------------------------------------------ */
+/* One non-image token set of the sequence (text or readouts): bf16 [B or 1, n, C] rows copied to sequence rows
+ * first_row .. first_row + n - 1.  batch_stride (elements, a multiple of 8) is 0 to give every batch row the same n rows
+ * (readout embeddings) or >= n * C.  rows is 16-byte aligned. */
+typedef struct {
+  const void* rows;
+  long long batch_stride;
+  int n;
+  int first_row;
+} tome_policy_rows_t;
+
+typedef struct {
+  tome_image_tokenizer_desc_t image;  /* batch == cfg->batch, embed_dim == cfg->channels, out_dtype == TOME_BF16 */
+  const float* image_params_f32;      /* the front end's flat parameters (section 7b) and their bf16 copy */
+  const void* image_params_bf16;
+  const void* pixels;                 /* [B, N, H, W, C_in], u8 or f32 as image.image_dtype */
+  const int32_t* row_tokens;          /* i32 [image.token_rows, n_patches] (device), as tome_image_tokenizer_fwd */
+  const int32_t* col_tokens;
+  const int32_t* image_rows;          /* HOST i32 [N * n_patches]: sequence row of image token n * n_patches + p (the grammar's
+                                         image positions in order, TokenSequence.get_modality_idx("images")); at most 32 runs
+                                         of consecutive rows */
+  int n_sets;                         /* 0 .. TOME_MAX_TOKEN_SETS */
+  tome_policy_rows_t sets[TOME_MAX_TOKEN_SETS];
+} tome_policy_inputs_t;
+
+/* tome_policy_predict runs, on `stream`: the image front end of section 7b writing each bf16 token (b, n, p) straight into row
+ * image_rows[n * n_patches + p] of an assembled [B, T0, C] sequence; one kernel copying every non-image set into its rows; then
+ * tome_stack_predict on that sequence (io->x and io->x_dtype are not read; every other io field and `sample` as there).  The
+ * sequence, and with it every output, equals TokenSequence.assemble_embeddings of the front end's bf16 tokens fed to
+ * tome_stack_predict, bit for bit.
+ * Workspace (io->workspace, 256-byte aligned, tome_policy_predict_workspace_bytes bytes): the sequence, then one region the
+ * front end's scratch and the predict layout share, so the size is the sequence plus the larger of
+ * tome_image_tokenizer_workspace_bytes and tome_stack_predict_workspace_bytes.
+ * Validation runs on the host before any CUDA call and returns TOME_ERR_INVALID naming the fault: batch differs between cfg and
+ * the descriptor, embed_dim != channels, out_dtype not bf16, an image row outside [0, T0), image and set rows not covering
+ * [0, T0) exactly once, a malformed set; shapes the front end, the stack or the sampler refuse keep their own errors.
+ * Graph capture: for fixed pointers and shapes the call allocates nothing, never synchronises, reads no device memory on the
+ * host and launches the same kernels with the same parameters every time, so a caller may capture it in a CUDA graph and
+ * replay it with new pixels, sets and draws written into the same buffers.  The first call must run eagerly, before any
+ * capture: it sets kernel attributes (shared-memory limits) and loads the modules, which a capturing stream cannot do. */
+size_t tome_policy_predict_workspace_bytes(const tome_stack_cfg_t* cfg, const tome_policy_inputs_t* inputs);
+int tome_policy_predict(const tome_stack_cfg_t* cfg, const tome_policy_inputs_t* inputs, const tome_stack_io_t* io,
+                        const tome_ddpm_sample_t* sample, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * 8. Launch accounting and per-op timing (measurement aid; off by default, never on the product path's hot loop)

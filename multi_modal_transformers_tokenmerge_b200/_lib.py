@@ -15,7 +15,7 @@ TOME_OK, TOME_ERR_INVALID, TOME_ERR_CUDA, TOME_ERR_UNSUPPORTED = 0, 1, 2, 3
 TOME_BF16, TOME_F32, TOME_U8 = 0, 1, 2
 TOME_MAJOR_K, TOME_MAJOR_MN = 0, 1
 TOME_MERGE_SUM, TOME_MERGE_WAVG = 0, 1
-ABI_VERSION = 17
+ABI_VERSION = 18
 
 vp, ll, i32, f32, u64, u32 = C.c_void_p, C.c_longlong, C.c_int, C.c_float, C.c_uint64, C.c_uint32
 
@@ -136,6 +136,18 @@ class ImageTokenizerDesc(C.Structure):
                 ("position_interval", i32), ("token_rows", i32), ("out_dtype", i32), ("chunk_rows", i32)]
 
 
+class PolicyRows(C.Structure):
+    """tome_policy_rows_t: one non-image token set copied into the assembled sequence (batch_stride 0 broadcasts it)."""
+    _fields_ = [("rows", vp), ("batch_stride", ll), ("n", i32), ("first_row", i32)]
+
+
+class PolicyInputs(C.Structure):
+    """tome_policy_inputs_t: what tome_policy_predict assembles the sequence from (image_rows is a HOST array)."""
+    _fields_ = [("image", ImageTokenizerDesc), ("image_params_f32", vp), ("image_params_bf16", vp), ("pixels", vp),
+                ("row_tokens", vp), ("col_tokens", vp), ("image_rows", C.POINTER(i32)), ("n_sets", i32),
+                ("sets", PolicyRows * MAX_TOKEN_SETS)]
+
+
 IT_CONV0_KERNEL, IT_CONV0_BIAS, IT_DENSE_KERNEL, IT_DENSE_BIAS, IT_ROW_EMBED, IT_COL_EMBED, IT_BLOCK0 = 0, 1, 2, 3, 4, 5, 16
 
 
@@ -172,7 +184,7 @@ def lib() -> C.CDLL:
         for name in ("tome_gemm_workspace_bytes", "tome_stack_workspace_bytes", "tome_attention_workspace_bytes", "tome_sim_argmax_workspace_bytes",
                      "tome_attention_bwd_workspace_bytes", "tome_action_head_workspace_bytes", "tome_diffusion_head_workspace_bytes",
                      "tome_diffusion_head_sample_workspace_bytes", "tome_stack_predict_workspace_bytes",
-                     "tome_image_tokenizer_workspace_bytes", "tome_adamw_workspace_bytes"):
+                     "tome_image_tokenizer_workspace_bytes", "tome_adamw_workspace_bytes", "tome_policy_predict_workspace_bytes"):
             getattr(L, name).restype = C.c_size_t
         for name in ("tome_stack_param_count", "tome_stack_layer_offset", "tome_stack_head_offset", "tome_launch_count",
                      "tome_diffusion_head_param_count", "tome_diffusion_head_param_offset",
@@ -247,6 +259,8 @@ def lib() -> C.CDLL:
             "tome_stack_predict_workspace_bytes": [P(StackCfg)],
             "tome_stack_predict": [P(StackCfg), P(StackIO), P(DdpmSample), vp],
             "tome_stack_tokens_at": [P(StackCfg), i32],
+            "tome_policy_predict_workspace_bytes": [P(StackCfg), P(PolicyInputs)],
+            "tome_policy_predict": [P(StackCfg), P(PolicyInputs), P(StackIO), P(DdpmSample), vp],
             "tome_stack_final_x": [P(StackCfg), P(StackIO)],
             "tome_stack_final_size": [P(StackCfg), P(StackIO)],
             "tome_stack_layer_edge_idx": [P(StackCfg), P(StackIO), i32],

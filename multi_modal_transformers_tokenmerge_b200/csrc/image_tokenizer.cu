@@ -24,7 +24,9 @@
 //                          adds the pooled tensor (the residual of image_tokenizer.py:170)
 //   it_im2col3_kernel      other widths: the nine shifted copies of the 3x3 SAME im2col row, zero outside the o2 x o2
 //                          window; one 16-byte load and one 16-byte store per thread; residual in the last GEMM's epilogue
-//   it_posadd_kernel       Dense output + row_embedding[row_token] + col_embedding[col_token] -> out dtype
+//   it_posadd_kernel       Dense output + row_embedding[row_token] + col_embedding[col_token] -> out dtype, into
+//                          out [B, N, n_patches, E] or (tome_policy_predict) straight into rows of the assembled sequence
+//   it_seq_rows_kernel     the sequence's text / readout rows (tome_policy_predict), one launch for every set
 // What is left HBM-bound is the input convolution (its im2col rows are k*k*C_in / (s*s*C_in) = 36x the pixels); the batch
 // is processed in chunks of whole batch rows so that buffer stays near 1 GiB whatever the batch.  Measurements and the
 // versions that led here: DESIGN.md 4.5, profiles/r02c_image_tokenizer.md.
@@ -32,6 +34,7 @@
 
 #include "common.cuh"
 #include "host_util.h"
+#include "image_tokenizer.h"
 
 namespace tome {
 
@@ -421,11 +424,13 @@ it_compact_kernel(const __nv_bfloat16* __restrict__ xp, const __nv_bfloat16* __r
   st_na_v4(out + (size_t)v * 8, o);
 }
 
-// tokens + row / column position embeddings (image_tokenizer.py:296-305), 4 features per thread.
+// tokens + row / column position embeddings (image_tokenizer.py:296-305), 4 features per thread.  kPlaced: bf16 token
+// (b, n, p) goes to row place.row0[i] + (n * np + p - place.k0[i]) of the [B, T0, E] sequence `out` instead of out[b, n, p].
+template <bool kPlaced>
 __global__ void __launch_bounds__(IT_THREADS)
 it_posadd_kernel(const float* __restrict__ dense, const float* __restrict__ row_emb, const float* __restrict__ col_emb,
                  const int32_t* __restrict__ row_tok, const int32_t* __restrict__ col_tok, void* __restrict__ out, long long n_vec,
-                 int E, int np, long long img0, int per_image_tokens, int P, int out_bf16) {
+                 int E, int np, long long img0, int per_image_tokens, int P, int out_bf16, const ItPlacement place) {
   const long long v = (long long)blockIdx.x * IT_THREADS + threadIdx.x;
   if (v >= n_vec) return;
   const int e4 = E >> 2;
@@ -440,12 +445,34 @@ it_posadd_kernel(const float* __restrict__ dense, const float* __restrict__ row_
   const float4 r = *reinterpret_cast<const float4*>(row_emb + (long long)rt * E + e);
   const float4 c = *reinterpret_cast<const float4*>(col_emb + (long long)ct * E + e);
   const float4 y = make_float4((d.x + r.x) + c.x, (d.y + r.y) + c.y, (d.z + r.z) + c.z, (d.w + r.w) + c.w);
-  if (out_bf16) {
+  if (kPlaced) {
+    const long long img = img0 + m / np;
+    const int k = (int)(img % place.n_images) * np + p;
+    int i = 0;
+    while (i + 1 < place.n_runs && k >= place.k0[i + 1]) ++i;
+    const long long row = (img / place.n_images) * place.seq_tokens + place.row0[i] + (k - place.k0[i]);
+    uint2 w = make_uint2(pack_bf16(y.x, y.y), pack_bf16(y.z, y.w));
+    *reinterpret_cast<uint2*>(reinterpret_cast<__nv_bfloat16*>(out) + row * E + e) = w;
+  } else if (out_bf16) {
     uint2 w = make_uint2(pack_bf16(y.x, y.y), pack_bf16(y.z, y.w));
     *reinterpret_cast<uint2*>(reinterpret_cast<__nv_bfloat16*>(out) + m * E + e) = w;
   } else {
     *reinterpret_cast<float4*>(reinterpret_cast<float*>(out) + m * E + e) = y;
   }
+}
+
+// The non-image rows of the assembled sequence: CTA column blockIdx.y = token set, thread = 16 bytes of one (batch row,
+// token) row.  A pure copy, so the rows equal TokenSequence.assemble_embeddings's bit for bit.
+__global__ void __launch_bounds__(IT_THREADS)
+it_seq_rows_kernel(const SeqRowSets sets, __nv_bfloat16* __restrict__ seq, int batch, int seq_tokens, int c8) {
+  const int s = blockIdx.y;
+  const long long v = (long long)blockIdx.x * IT_THREADS + threadIdx.x;
+  const long long per_row = (long long)sets.n[s] * c8;
+  if (v >= per_row * batch) return;
+  const long long b = v / per_row, rem = v - b * per_row;
+  const long long t = rem / c8, c = rem - t * c8;
+  const __nv_bfloat16* src = reinterpret_cast<const __nv_bfloat16*>(sets.src[s]) + b * sets.batch_stride[s] + t * c8 * 8 + c * 8;
+  *reinterpret_cast<uint4*>(seq + ((b * seq_tokens + sets.row0[s] + t) * c8 + c) * 8) = ld_nc_v4(src);
 }
 
 static long long it_offset(const tome_image_tokenizer_desc_t* d, const ItGeom& g, int which) {
@@ -512,11 +539,10 @@ static int it_gemm(int m, int n, int k, const void* a, const void* b, void* c, i
   return tome_gemm_bf16(&ga, nullptr, 0, stream);
 }
 
-extern "C" int tome_image_tokenizer_fwd(const tome_image_tokenizer_desc_t* d, const void* image, const float* pf, const void* pb_,
-                                        const int32_t* row_tokens, const int32_t* col_tokens, void* out, void* workspace,
-                                        size_t workspace_bytes, void* stream_) {
-  clear_error();
-  cudaStream_t stream = (cudaStream_t)stream_;
+// The front end; place == nullptr writes out [B, N, n_patches, E], else the bf16 sequence rows of `place`.
+static int it_forward(const tome_image_tokenizer_desc_t* d, const void* image, const float* pf, const void* pb_,
+                      const int32_t* row_tokens, const int32_t* col_tokens, void* out, const ItPlacement* place, void* workspace,
+                      size_t workspace_bytes, cudaStream_t stream) {
   ItGeom g;
   int rc = it_geometry(d, &g, "image_tokenizer_fwd");
   if (rc != TOME_OK) return rc;
@@ -646,12 +672,48 @@ extern "C" int tome_image_tokenizer_fwd(const tome_image_tokenizer_desc_t* d, co
     {
       const long long nv = mt * (E / 4);
       ProfScope prof(PROF_OTHER, (double)nv * 16 * 2, 1, stream);
-      launch_k(it_posadd_kernel, nblk(nv), IT_THREADS, 0, stream, dense, pf + it_offset(d, g, TOME_IT_ROW_EMBED),
-               pf + it_offset(d, g, TOME_IT_COL_EMBED), row_tokens, col_tokens,
-               reinterpret_cast<uint8_t*>(out) + (size_t)img0 * g.np * E * out_bytes, nv, E, g.np, img0, d->token_rows == 1 ? 0 : 1,
-               d->position_interval, d->out_dtype == TOME_BF16 ? 1 : 0);
+      if (place)
+        launch_k(it_posadd_kernel<true>, nblk(nv), IT_THREADS, 0, stream, dense, pf + it_offset(d, g, TOME_IT_ROW_EMBED),
+                 pf + it_offset(d, g, TOME_IT_COL_EMBED), row_tokens, col_tokens, out, nv, E, g.np, img0,
+                 d->token_rows == 1 ? 0 : 1, d->position_interval, 1, *place);
+      else
+        launch_k(it_posadd_kernel<false>, nblk(nv), IT_THREADS, 0, stream, dense, pf + it_offset(d, g, TOME_IT_ROW_EMBED),
+                 pf + it_offset(d, g, TOME_IT_COL_EMBED), row_tokens, col_tokens,
+                 reinterpret_cast<uint8_t*>(out) + (size_t)img0 * g.np * E * out_bytes, nv, E, g.np, img0, d->token_rows == 1 ? 0 : 1,
+                 d->position_interval, d->out_dtype == TOME_BF16 ? 1 : 0, ItPlacement{});
       TOME_CUDA(cudaGetLastError());
     }
   }
   return TOME_OK;
 }
+
+extern "C" int tome_image_tokenizer_fwd(const tome_image_tokenizer_desc_t* d, const void* image, const float* pf, const void* pb,
+                                        const int32_t* row_tokens, const int32_t* col_tokens, void* out, void* workspace,
+                                        size_t workspace_bytes, void* stream) {
+  clear_error();
+  return it_forward(d, image, pf, pb, row_tokens, col_tokens, out, nullptr, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+namespace tome {
+
+int image_tokenizer_fwd_placed(const tome_image_tokenizer_desc_t* d, const void* image, const float* pf, const void* pb,
+                               const int32_t* row_tokens, const int32_t* col_tokens, const ItPlacement& place, void* seq,
+                               void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  TOME_CHECK(d != nullptr && d->out_dtype == TOME_BF16, TOME_ERR_INVALID, "image_tokenizer_fwd: sequence rows are bf16 (out_dtype)");
+  TOME_CHECK(place.n_runs >= 1 && place.n_runs <= IT_MAX_ROW_RUNS && place.n_images == d->n_images, TOME_ERR_INVALID,
+             "image_tokenizer_fwd: bad row placement");
+  return it_forward(d, image, pf, pb, row_tokens, col_tokens, seq, &place, workspace, workspace_bytes, stream);
+}
+
+int fill_sequence_rows(const SeqRowSets& sets, int batch, int seq_tokens, int channels, void* seq, cudaStream_t stream) {
+  if (sets.n_sets == 0) return TOME_OK;
+  long long most = 0;
+  for (int s = 0; s < sets.n_sets; ++s) most = std::max(most, (long long)batch * sets.n[s] * (channels / 8));
+  ProfScope prof(PROF_OTHER, (double)most * sets.n_sets * 32, 1, stream);
+  launch_k(it_seq_rows_kernel, dim3((unsigned)((most + IT_THREADS - 1) / IT_THREADS), sets.n_sets), IT_THREADS, 0, stream, sets,
+           reinterpret_cast<__nv_bfloat16*>(seq), batch, seq_tokens, channels / 8);
+  TOME_CUDA(cudaGetLastError());
+  return TOME_OK;
+}
+
+}  // namespace tome

@@ -15,10 +15,12 @@
 // shapes, so a whole step can be captured in a CUDA graph by the caller.
 #include <string.h>
 
+#include <algorithm>
 #include <vector>
 
 #include "common.cuh"
 #include "host_util.h"
+#include "image_tokenizer.h"
 
 namespace tome {
 
@@ -668,13 +670,8 @@ extern "C" size_t tome_stack_predict_workspace_bytes(const tome_stack_cfg_t* c) 
   return S.total;
 }
 
-extern "C" int tome_stack_predict(const tome_stack_cfg_t* cfg, const tome_stack_io_t* io, const tome_ddpm_sample_t* sample,
-                                  void* stream_) {
-  clear_error();
-  cudaStream_t st = (cudaStream_t)stream_;
-  RC(check_cfg(cfg));
-  const tome_stack_cfg_t p = predict_cfg(cfg);
-  const tome_stack_cfg_t* c = &p;
+// Everything tome_stack_predict checks, before any CUDA call; fills the predict layout over io->workspace.
+static int predict_check(const tome_stack_cfg_t* c, const tome_stack_io_t* io, const tome_ddpm_sample_t* sample, StackLayout* S) {
   TOME_CHECK((c->head == 3) == (sample != nullptr), TOME_ERR_INVALID,
              "stack_predict: the diffusion head (head 3) needs the sampler's draws, every other head takes sample = NULL");
   if (sample) {
@@ -682,10 +679,15 @@ extern "C" int tome_stack_predict(const tome_stack_cfg_t* cfg, const tome_stack_
                "stack_predict: sample->noise_per_step must be 0 or 1");
     TOME_CHECK(sample->clip > 0.f, TOME_ERR_INVALID, "stack_predict: sample->clip must be positive");
   }
-  StackLayout S = make_layout(c, io ? io->workspace : nullptr, true);
-  if (c->head == 3 && S.ws_head_bytes == 0) return TOME_ERR_UNSUPPORTED;   // the sampler's shape check set the message
-  RC(check_io(c, io, S, false));
+  *S = make_layout(c, io ? io->workspace : nullptr, true);
+  if (c->head == 3 && S->ws_head_bytes == 0) return TOME_ERR_UNSUPPORTED;   // the sampler's shape check set the message
+  RC(check_io(c, io, *S, false));
   TOME_CHECK(c->head == 0 || io->head_out, TOME_ERR_INVALID, "stack_predict: head_out missing");
+  return TOME_OK;
+}
+
+static int predict_run(const tome_stack_cfg_t* c, const tome_stack_io_t* io, const tome_ddpm_sample_t* sample, const StackLayout& S,
+                       cudaStream_t st) {
   const int B = c->batch, C = c->channels;
   RC(forward_layers(c, io, S, st));
   const int TL = S.shapes.back().t_out;
@@ -705,6 +707,133 @@ extern "C" int tome_stack_predict(const tome_stack_cfg_t* cfg, const tome_stack_
   }
   if (io->readout) RC(tome_readout_mse(B, TL, C, c->n_readout, xf, S.origin, nullptr, nullptr, nullptr, io->readout, st));
   return TOME_OK;
+}
+
+extern "C" int tome_stack_predict(const tome_stack_cfg_t* cfg, const tome_stack_io_t* io, const tome_ddpm_sample_t* sample,
+                                  void* stream_) {
+  clear_error();
+  RC(check_cfg(cfg));
+  const tome_stack_cfg_t p = predict_cfg(cfg);
+  StackLayout S;
+  RC(predict_check(&p, io, sample, &S));
+  return predict_run(&p, io, sample, S, (cudaStream_t)stream_);
+}
+
+// ---- pixels to actions (tome_policy_predict) ----
+// Workspace: the assembled bf16 sequence [B, T0, C], then ONE region the front end's scratch and the predict layout share
+// (the front end has finished with its scratch when the stack starts).
+struct PolicyPlan {
+  ItPlacement place;
+  SeqRowSets rows;
+  size_t shared_off, it_bytes, stack_bytes, total;   // shared_off: the shared region follows the sequence
+};
+
+static int policy_plan(const tome_stack_cfg_t* c, const tome_policy_inputs_t* in, PolicyPlan* pp) {
+  RC(check_cfg(c));
+  TOME_CHECK(in != nullptr, TOME_ERR_INVALID, "policy: null inputs");
+  const tome_image_tokenizer_desc_t* d = &in->image;
+  TOME_CHECK(d->batch == c->batch, TOME_ERR_INVALID, "policy: batch %d of the image descriptor differs from the stack's %d", d->batch,
+             c->batch);
+  TOME_CHECK(d->embed_dim == c->channels, TOME_ERR_INVALID, "policy: the image tokens have embed_dim %d, the stack %d channels",
+             d->embed_dim, c->channels);
+  TOME_CHECK(d->out_dtype == TOME_BF16, TOME_ERR_INVALID, "policy: the image descriptor's out_dtype must be bf16 (the sequence is bf16)");
+  pp->it_bytes = tome_image_tokenizer_workspace_bytes(d);
+  if (pp->it_bytes == 0) return TOME_ERR_INVALID;   // the front end's own check set the message
+  const int T0 = c->tokens, np = (d->image_size / d->patch_size) * (d->image_size / d->patch_size);
+  const long long n_img = (long long)d->n_images * np;
+  TOME_CHECK(n_img <= T0, TOME_ERR_INVALID, "policy: %lld image tokens do not fit a %d-token sequence", n_img, T0);
+  TOME_CHECK(in->image_rows != nullptr, TOME_ERR_INVALID, "policy: image_rows missing");
+  TOME_CHECK(in->n_sets >= 0 && in->n_sets <= TOME_MAX_TOKEN_SETS, TOME_ERR_INVALID, "policy: n_sets must be in [0, %d]",
+             TOME_MAX_TOKEN_SETS);
+  std::vector<int> owner(T0, -1);   // -1: not covered yet; -2: an image token; s >= 0: non-image set s
+  ItPlacement& pl = pp->place;
+  memset(&pl, 0, sizeof(pl));
+  pl.seq_tokens = T0;
+  pl.n_images = d->n_images;
+  for (int k = 0; k < (int)n_img; ++k) {
+    const int row = in->image_rows[k];
+    TOME_CHECK(row >= 0 && row < T0, TOME_ERR_INVALID, "policy: image_rows[%d] = %d is outside the sequence [0, %d)", k, row, T0);
+    TOME_CHECK(owner[row] == -1, TOME_ERR_INVALID, "policy: sequence row %d is covered twice (image token %d)", row, k);
+    owner[row] = -2;
+    if (k == 0 || row != in->image_rows[k - 1] + 1) {   // a new run of consecutive rows
+      TOME_CHECK(pl.n_runs < IT_MAX_ROW_RUNS, TOME_ERR_UNSUPPORTED, "policy: the image rows form more than %d runs of consecutive rows",
+                 IT_MAX_ROW_RUNS);
+      pl.k0[pl.n_runs] = k;
+      pl.row0[pl.n_runs] = row;
+      ++pl.n_runs;
+    }
+  }
+  pl.k0[pl.n_runs] = (int)n_img;
+  SeqRowSets& rs = pp->rows;
+  memset(&rs, 0, sizeof(rs));
+  rs.n_sets = in->n_sets;
+  for (int s = 0; s < in->n_sets; ++s) {
+    const tome_policy_rows_t& r = in->sets[s];
+    TOME_CHECK(r.n >= 1 && r.first_row >= 0 && (long long)r.first_row + r.n <= T0, TOME_ERR_INVALID,
+               "policy: set %d (rows %d .. %d) is outside the sequence [0, %d)", s, r.first_row, r.first_row + r.n - 1, T0);
+    TOME_CHECK(r.batch_stride == 0 || r.batch_stride >= (long long)r.n * c->channels, TOME_ERR_INVALID,
+               "policy: set %d: batch_stride must be 0 (one set for every batch row) or at least n * channels", s);
+    TOME_CHECK(r.batch_stride % 8 == 0, TOME_ERR_INVALID, "policy: set %d: batch_stride must be a multiple of 8 elements", s);
+    for (int t = r.first_row; t < r.first_row + r.n; ++t) {
+      TOME_CHECK(owner[t] == -1, TOME_ERR_INVALID, "policy: sequence row %d is covered twice (set %d)", t, s);
+      owner[t] = s;
+    }
+    rs.src[s] = r.rows;
+    rs.batch_stride[s] = r.batch_stride;
+    rs.n[s] = r.n;
+    rs.row0[s] = r.first_row;
+  }
+  for (int t = 0; t < T0; ++t)
+    TOME_CHECK(owner[t] != -1, TOME_ERR_INVALID, "policy: sequence row %d is covered by no image token and no set", t);
+  const tome_stack_cfg_t p = predict_cfg(c);
+  pp->stack_bytes = make_layout(&p, nullptr, true).total;
+  if (p.head == 3) {
+    tome_diffusion_desc_t dd = diffusion_desc(&p, 1);
+    if (tome_diffusion_head_sample_workspace_bytes(&dd) == 0) return TOME_ERR_UNSUPPORTED;   // the sampler's check set the message
+  }
+  Bump b{nullptr};
+  b.reserve((size_t)c->batch * T0 * c->channels * 2);
+  pp->shared_off = b.reserve(std::max(pp->it_bytes, pp->stack_bytes));
+  pp->total = b.total();
+  return TOME_OK;
+}
+
+extern "C" size_t tome_policy_predict_workspace_bytes(const tome_stack_cfg_t* cfg, const tome_policy_inputs_t* inputs) {
+  clear_error();
+  PolicyPlan pp;
+  if (policy_plan(cfg, inputs, &pp) != TOME_OK) return 0;
+  return pp.total;
+}
+
+extern "C" int tome_policy_predict(const tome_stack_cfg_t* cfg, const tome_policy_inputs_t* in, const tome_stack_io_t* io,
+                                   const tome_ddpm_sample_t* sample, void* stream_) {
+  clear_error();
+  cudaStream_t st = (cudaStream_t)stream_;
+  PolicyPlan pp;
+  RC(policy_plan(cfg, in, &pp));
+  TOME_CHECK(io != nullptr && io->workspace != nullptr, TOME_ERR_INVALID, "policy: null io / workspace");
+  TOME_CHECK(io->workspace_bytes >= pp.total, TOME_ERR_INVALID, "policy: workspace too small (%zu < %zu)", io->workspace_bytes, pp.total);
+  TOME_CHECK(((uintptr_t)io->workspace & 255) == 0, TOME_ERR_INVALID, "policy: workspace must be 256-byte aligned");
+  TOME_CHECK(in->pixels && in->image_params_f32 && in->image_params_bf16 && in->row_tokens && in->col_tokens, TOME_ERR_INVALID,
+             "policy: null pixels / image parameters / position tokens");
+  TOME_CHECK((((uintptr_t)in->image_params_f32 | (uintptr_t)in->image_params_bf16) & 15) == 0, TOME_ERR_INVALID,
+             "policy: image parameters must be 16-byte aligned");
+  for (int s = 0; s < in->n_sets; ++s)
+    TOME_CHECK(in->sets[s].rows && ((uintptr_t)in->sets[s].rows & 15) == 0, TOME_ERR_INVALID, "policy: set %d: rows null or not 16-byte aligned", s);
+  uint8_t* ws = reinterpret_cast<uint8_t*>(io->workspace);
+  void* seq = ws;
+  tome_stack_io_t sio = *io;
+  sio.x = seq;
+  sio.x_dtype = TOME_BF16;
+  sio.workspace = ws + pp.shared_off;
+  sio.workspace_bytes = io->workspace_bytes - pp.shared_off;
+  const tome_stack_cfg_t p = predict_cfg(cfg);
+  StackLayout S;
+  RC(predict_check(&p, &sio, sample, &S));
+  RC(image_tokenizer_fwd_placed(&in->image, in->pixels, in->image_params_f32, in->image_params_bf16, in->row_tokens, in->col_tokens,
+                                pp.place, seq, ws + pp.shared_off, pp.it_bytes, st));
+  RC(fill_sequence_rows(pp.rows, cfg->batch, cfg->tokens, cfg->channels, seq, st));
+  return predict_run(&p, &sio, sample, S, st);
 }
 
 extern "C" int tome_stack_backward(const tome_stack_cfg_t* c, const tome_stack_io_t* io, void* stream_) {

@@ -379,6 +379,15 @@ class ToMeStackEngine:
         p.layer_gid, p.layer_pos = self.layer_gid, self.layer_pos
         return p
 
+    def policy(self, tokenizer, tokenizer_variables, token_sequence, batch: Optional[int] = None, graph: bool = False):
+        """Camera frames -> actions in one native call (tome_policy_predict): a `policy.PixelPolicy` over THIS engine's
+        params / params_bf16 storage (it sees every optimiser step without a reload), masks and readout indices, at `batch`
+        (default: the engine's).  tokenizer / tokenizer_variables: the ImageTokenizer (bf16 out_dtype) and its Flax variables,
+        packed once; token_sequence: the grammar (TokenSequence or its string) the sequence is assembled by.  graph=True replays
+        every call after the first from a CUDA graph."""
+        from .policy import PixelPolicy
+        return PixelPolicy(self, tokenizer, tokenizer_variables, token_sequence, batch=batch, graph=graph)
+
     def predict(self, x: torch.Tensor, init=None, noise=None, rng=0, x_final: Optional[torch.Tensor] = None):
         """Forward only, dropout off (tome_stack_predict).  Returns (head_out, readout): head_out is the action head's output
         -- tanh actions [B, A] (continuous), logits [B, groups, bins] (categorical), sampled actions [B, A] (diffusion) -- or
