@@ -236,7 +236,11 @@ typedef struct {
   /* block-causal mask as a group table instead of [B,H,T,T] booleans (octo.py:66-68,119):
    * allow[gid[b,q]*num_groups + gid[b,k]] = 0 masked, 1 visible, 2 visible iff pos[b,k] <= pos[b,q].
    * gid == NULL: no mask.  masked logits become -FLT_MAX (finite, like flax's finfo.min), so a fully masked row
-   * yields the uniform distribution, not NaN. */
+   * yields the uniform distribution, not NaN.  Such a row's lse is the mask constant's, below -2^90 * ln 2 (about -8.6e26)
+   * for scale >= 2^-9, and a row that sees any key has an lse of the order of its logits; tome_attention_bwd and
+   * tome_attention_importance recognise the row by that lse.  Its gradient is that of the uniform forward: every key
+   * k < T receives dO / T (times keep[q,k] / (1 - rate) with dropout) in dV, nothing flows into dQ or dK (the masked
+   * logits are constants), and its weights count 1/T per key in both importance modes. */
   const uint8_t* gid;   /* [B,T] */
   const int32_t* pos;   /* [B,T] */
   const uint8_t* allow; /* [G,G], G <= 32 */

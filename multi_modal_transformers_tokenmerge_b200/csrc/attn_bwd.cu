@@ -109,6 +109,14 @@ __device__ __forceinline__ void ab_store_tile(uint8_t* stage, float* part, uint3
   }
 }
 
+// w[i] holds the bf16 pair of columns 2i, 2i + 1; the columns whose bit is set in `cols` (all 0 so far) become bf16(fill)
+__device__ __forceinline__ void or_bf16_lanes(uint32_t (&w)[16], uint32_t cols, float fill) {
+  const uint32_t f = pack_bf16(fill, fill);
+#pragma unroll
+  for (int i = 0; i < 16; ++i)
+    w[i] |= f & ((((cols >> (2 * i)) & 1u) ? 0x0000ffffu : 0u) | (((cols >> (2 * i + 1)) & 1u) ? 0xffff0000u : 0u));
+}
+
 // ------------------------------------------------------------------------------------------------ prep
 __global__ void attn_bwd_prep_kernel(int B, int T, int Tp, int H, const __nv_bfloat16* __restrict__ o, long long o_bs,
                                      long long o_ts, const __nv_bfloat16* __restrict__ dout, long long do_bs, long long do_ts,
@@ -428,6 +436,14 @@ attn_bwd_dkdv_ts_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_c
             g = __fmul2_rn(g, pf);
             dw[c >> 1] = pack_bf16(g.x, g.y);
           }
+        }
+      }
+      if (has_mask) {  // query rows with no visible key (attn_meta.cuh): 1/T of their dO reaches every key's dV; dS stays 0
+        const float lq = reinterpret_cast<const float*>(slot)[hq * 32 + lane];
+        const uint32_t fw = __ballot_sync(0xffffffffu, lq < ATTN_MASKED_ROW_LSE2) & kb;   // warp-uniform, rarely non-zero
+        if (fw) {
+          if constexpr (DROP) or_bf16_lanes(pw, fw, p.inv_keep / (float)T);
+          else or_bf16_lanes(pe, fw, 1.0f / (float)T);
         }
       }
       tmem_st_x16(tm_dpt + lane_sel + hq * 32, dw);

@@ -6,6 +6,7 @@
 // at the literal config (8 x 3 x 74 rows) is microseconds.  Same entry points, same results contract; chosen by head_dim.
 #include <float.h>
 
+#include "attn_meta.cuh"
 #include "common.cuh"
 #include "host_util.h"
 
@@ -206,7 +207,9 @@ attn_generic_dkdv_kernel(const AttnGenericParams p) {
     const bool vis = ag_visible(p, gq, pq, b, kk);
     const float lse2 = p.lse[((long long)b * p.heads + h) * T + q] * 1.4426950408889634f;
     const float pe = vis ? fast_exp2(fmaf(dot, p.scale_log2, bias2) - lse2) : 0.f;
-    const float pd = keep ? pe * p.drop.inv_keep : 0.f;
+    // a query row with no visible key (attn_meta.cuh) weighs every key 1/T in the forward: that reaches dV, not dS
+    const float pv = lse2 < ATTN_MASKED_ROW_LSE2 ? 1.0f / (float)T : pe;
+    const float pd = keep ? pv * p.drop.inv_keep : 0.f;
     const float dpd = keep ? dp * p.drop.inv_keep : 0.f;
     const float ds = pe * (dpd - delta) * p.scale;
 #pragma unroll

@@ -31,6 +31,13 @@ constexpr int ATTN_META_OFF_VIS = 256, ATTN_META_OFF_VISC = 512, ATTN_META_OFF_P
 // (32-byte rows, loaded by TMA with the 32-byte swizzle) and a flag word saying whether the trick applies to this table.
 constexpr int ATTN_AUG_K = 16;
 constexpr float ATTN_AUG_BIG = 1.2676506002282294e30f;   // 2^100, exact in bf16
+// ---- query rows with no visible key ----
+// The forward gives such a row the uniform distribution over its T keys (masked logits are one finite constant, as flax's
+// finfo.min), and leaves its lse at that constant: about -FLT_MAX * ln 2 on the select path, -2^100 * scale on the
+// augmentation path.  A row with a visible key has an lse of the order of its logits.  The backward and the importance
+// kernel therefore recognise the row by lse * log2(e) < ATTN_MASKED_ROW_LSE2, with no pass of their own, and give it the
+// forward's weights: 1/T on every key for dV and importance, and no gradient into the logits.  Holds for scale >= 2^-9.
+constexpr float ATTN_MASKED_ROW_LSE2 = -1.2379400392853803e27f;   // -2^90
 inline size_t attn_tiles(int tokens) { return (size_t)(tokens + ATTN_META_TILE - 1) / ATTN_META_TILE; }
 inline size_t attn_blocks_bytes(int batch, int tokens) { return (size_t)batch * attn_tiles(tokens) * ATTN_META_BYTES; }
 inline size_t attn_aug_array_bytes(int batch, int tokens) { return (size_t)batch * attn_tiles(tokens) * ATTN_META_TILE * ATTN_AUG_K * 2; }

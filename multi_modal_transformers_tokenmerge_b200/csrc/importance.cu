@@ -16,6 +16,7 @@
 // Weights are the UNDROPPED ones (the ranking must not depend on the dropout stream).
 #include <float.h>
 
+#include "attn_meta.cuh"
 #include "common.cuh"
 #include "host_util.h"
 
@@ -115,6 +116,7 @@ attn_importance_kernel(const ImpParams p) {
   };
 
   float acc[2] = {0.f, 0.f};
+  const float inv_t = 1.0f / (float)T;
   uint32_t a[D / 16][4];
   stage(0, 0);
   for (int it = 0; it < n_it; ++it) {
@@ -132,6 +134,10 @@ attn_importance_kernel(const ImpParams p) {
 #pragma unroll
         for (int i = 0; i < 2; ++i)
           r_term[i] = row_ok[i] ? -p.lse[((long long)b * p.heads + h) * T + row[i]] * 1.4426950408889634f : 0.f;
+        // a query with no visible key (attn_meta.cuh) weighs each of the T keys 1/T: its row sums to one
+        if (MASKED && t == 0)
+#pragma unroll
+          for (int i = 0; i < 2; ++i) acc[i] += r_term[i] > -ATTN_MASKED_ROW_LSE2 ? 1.f : 0.f;
       }
     }
     cp_async_wait<0>();
@@ -156,15 +162,18 @@ attn_importance_kernel(const ImpParams p) {
           const float c_term = c_term_s[buf][cl];
           const int gp = MASKED ? c_gp_s[buf][cl] : 0;
           const int cg = gp & 255, cp = gp >> 8;
+          // received: a query with no visible key (attn_meta.cuh) gives 1/T to every key
+          const float c_fill = ROWS_ARE_KEYS && c_term > -ATTN_MASKED_ROW_LSE2 ? inv_t : 0.f;
 #pragma unroll
           for (int i = 0; i < 2; ++i) {
-            float s2 = fmaf(c[2 * i + jj], p.scale_log2, c_term + r_term[i]);
+            const float s2 = fmaf(c[2 * i + jj], p.scale_log2, c_term + r_term[i]);
             if (MASKED) {
               const bool causal_ok = ROWS_ARE_KEYS ? rp[i] <= cp : cp <= rp[i];
               const bool vis = ((vis1[i] >> cg) & 1u) || (((vis2[i] >> cg) & 1u) && causal_ok);
-              s2 = vis ? s2 : -INFINITY;
+              acc[i] += vis ? fast_exp2(s2) : c_fill;
+            } else {
+              acc[i] += fast_exp2(s2);
             }
-            acc[i] += fast_exp2(s2);
           }
         }
       }
